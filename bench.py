@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            our arm (CUDA, sm_100a)
   python bench.py --impl reference [...]                          the reference's CPU path
+  python bench.py [...] --dump-outputs DIR                        also save the last timed step's results
 
 Workload (BASELINE.json configs[1]): 2048x2048 U8 synthetic microscopy-like video, 1000 frames per
 GPU; one STEP = encode the whole batch, then decode it again (device-resident).  Metric: raw-pixel
@@ -24,6 +25,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # no __pycache__ either: the benchmark writes nothing into the source tree
 
 METRIC = "dbde_encode_decode_raw_pixel_throughput"
 UNIT = "GB/s"
@@ -47,7 +49,13 @@ def parse():
     ap.add_argument("--kind", default=KIND, choices=["micro", "mix", "low", "noise"])
     ap.add_argument("--width", type=int, default=W)
     ap.add_argument("--height", type=int, default=H)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed on rank 0 as DIR/*.npy: record "
+                         "sizes, offsets, decode status, and a fixed seeded sample of record bytes and decoded pixels")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
 
 
 def workload_config(a, extra=None):
@@ -118,25 +126,37 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------------ CPU arm
+# what cpu_baseline.kind stands for; only "reference" is the reference's own speed
+CPU_CODECS = {
+    "reference": "dbde_pack_frame/dbde_unpack_frame of the unmodified dbde_util.cpp (g++ -O3 -march=corei7, SSE4.1) "
+                 "via oracle/_ref",
+    "port": "oracle_pack_frame/oracle_unpack_frame of the plain-C port oracle/dbde_oracle.c (oracle/_ref is not built): "
+            "a bit-at-a-time restatement far slower than the reference, not a baseline to quote speed-ups against",
+}
+
+
 def cpu_reference_rates(frames, threads, target_s=1.0):
-    """Time the reference's own CPU implementation (oracle/_ref: dbde_util.cpp compiled unmodified)
-    on `threads` host threads over contiguous frame ranges.  -> dict of rates."""
+    """Time the reference's own CPU implementation (oracle/_ref: dbde_util.cpp compiled unmodified;
+    where that is not built, the plain-C port oracle/dbde_oracle.c, reported as kind "port") on
+    `threads` host threads over contiguous frame ranges.  -> dict of rates."""
     import oracle
-    if oracle.ref is None:
-        raise RuntimeError("oracle/_ref/libdbde_ref.so missing: build it where /root/reference exists")
+    if oracle.ref is not None:
+        encode_mt, decode_mt, kind = oracle.ref_encode_mt, oracle.ref_decode_mt, "reference"
+    else:
+        encode_mt, decode_mt, kind = oracle.port_encode_mt, oracle.port_decode_mt, "port"
     n, Hh, Ww = frames.shape
     # calibrate repetitions so each direction runs for about target_s
-    s, slots, sizes = oracle.ref_encode_mt(frames, threads, 1)
+    s, slots, sizes = encode_mt(frames, threads, 1)
     reps_e = max(1, int(target_s / max(s, 1e-4)))
-    s_e, slots, sizes = oracle.ref_encode_mt(frames, threads, reps_e)
-    s, dec, bad = oracle.ref_decode_mt(slots, Ww, Hh, threads, 1)
+    s_e, slots, sizes = encode_mt(frames, threads, reps_e)
+    s, dec, bad = decode_mt(slots, Ww, Hh, threads, 1)
     reps_d = max(1, int(target_s / max(s, 1e-4)))
-    s_d, dec, bad = oracle.ref_decode_mt(slots, Ww, Hh, threads, reps_d)
-    assert bad == 0 and (dec == frames).all(), "reference round trip failed"
+    s_d, dec, bad = decode_mt(slots, Ww, Hh, threads, reps_d)
+    assert bad == 0 and (dec == frames).all(), "%s round trip failed" % kind
     enc_fps, dec_fps = n * reps_e / s_e, n * reps_d / s_d
     px = Ww * Hh
     t_pair = 1.0 / enc_fps + 1.0 / dec_fps            # seconds to encode AND decode one frame
-    return {"encode_fps": enc_fps, "decode_fps": dec_fps, "value": 2 * px / t_pair / 1e9,
+    return {"encode_fps": enc_fps, "decode_fps": dec_fps, "value": 2 * px / t_pair / 1e9, "kind": kind,
             "cpu_seconds": threads * (s_e + s_d), "reps": [reps_e, reps_d], "sizes": sizes}
 
 
@@ -159,15 +179,15 @@ def run_reference(a):
     val = float(np.mean([p["value"] for p in per]))
     enc = float(np.mean([p["encode_fps"] for p in per]))
     dec = float(np.mean([p["decode_fps"] for p in per]))
-    sample = "%d frames of the same workload, dbde_pack_frame then dbde_unpack_frame, ~%.2f s per direction per step" % (nsample, target)
+    kind = per[0]["kind"]
+    sample = "%d frames of the same workload, ~%.2f s per direction per step" % (nsample, target)
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
             "warmup": a.warmup, "ms_per_step": 1000.0 * wall / max(a.steps, 1), "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "u8", "data": "synthetic",
             "config": workload_config(a), "encode_fps": enc, "decode_fps": dec,
-            "cpu_baseline": {"value": val, "unit": UNIT, "cores": threads, "kind": "reference", "sample": sample},
+            "cpu_baseline": {"value": val, "unit": UNIT, "cores": threads, "kind": kind, "sample": sample},
             "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
-            "note": "unmodified dbde_util.cpp (g++ -O3 -march=corei7, SSE4.1) via oracle/_ref, %d std::threads over "
-                    "contiguous frame ranges; host only, no GPU" % threads}
+            "note": "%s; %d host threads over contiguous frame ranges; host only, no GPU" % (CPU_CODECS[kind], threads)}
     print(json.dumps(line))
     return 0
 
@@ -271,6 +291,34 @@ class DeviceLeg:
                 "enc_ms": float(np.mean([e[0].elapsed_time(e[1]) for e in ev])),
                 "dec_ms": float(np.mean([e[1].elapsed_time(e[2]) for e in ev]))}
 
+    def dump(self, out_dir):
+        """Save what the last encode()/decode() handed back as out_dir/<name>.npy.  Per frame (frames
+        per_frame_index, all of them up to 2^19): record_sizes, record_offsets, decode_status (float64).  For
+        8 frames (sample_frame_index): record_bytes_sample at 2^19 byte positions of the slot
+        (sample_byte_position; -1 past the record's end) and decoded_pixels_sample at 2^19 pixel positions
+        (sample_pixel_position), float32.  The indices are drawn with a fixed seed from the shape alone, so
+        two runs with the same arguments compare entry by entry; at most 56 MB in all."""
+        torch, N, px, stride = self.torch, self.N, self.px, self.stride
+        rng = np.random.default_rng(20261020)
+
+        def pick(n, k):
+            return np.arange(n) if n <= k else np.sort(rng.choice(n, k, replace=False))
+
+        every, frames, bpos, ppos = pick(N, 1 << 19), pick(N, 8), pick(stride, 1 << 19), pick(px, 1 << 19)
+        sizes = self.sizes[:N].cpu().numpy()
+        fi = torch.from_numpy(frames).to(self.dev)
+        slots = self.stream_buf[self.delta:self.delta + N * stride].view(N, stride)
+        rec = slots.index_select(0, fi).index_select(1, torch.from_numpy(bpos).to(self.dev)).cpu().numpy().astype(np.float32)
+        rec[bpos[None, :] >= sizes[frames][:, None]] = -1
+        dec = self.decoded[:N * px].view(N, px).index_select(0, fi).index_select(1, torch.from_numpy(ppos).to(self.dev))
+        os.makedirs(out_dir, exist_ok=True)
+        for name, arr in (("per_frame_index", every), ("record_sizes", sizes[every]),
+                          ("record_offsets", self.offs[:N].cpu().numpy()[every]),
+                          ("decode_status", self.status[:N].cpu().numpy()[every]),
+                          ("sample_frame_index", frames), ("sample_byte_position", bpos), ("sample_pixel_position", ppos),
+                          ("record_bytes_sample", rec), ("decoded_pixels_sample", dec.cpu().numpy().astype(np.float32))):
+            np.save(os.path.join(out_dir, name + ".npy"), arr if arr.dtype == np.float32 else arr.astype(np.float64))
+
     def free(self):
         self.frames = self.stream_buf = self.decoded = None
 
@@ -320,6 +368,8 @@ def run_ours(a):
     sampler = ClockSampler(local) if rank == 0 else None
     tm = leg.timed(a.steps, a.warmup, barrier)
     clocks = sampler.stop(*tm["t_host"]) if sampler else None
+    if a.dump_outputs and rank == 0:
+        leg.dump(a.dump_outputs)        # before the end-to-end leg below reuses the device buffers
     launches, enc_ms, dec_ms = tm["launches"], tm["enc_ms"], tm["dec_ms"]
     t = torch.tensor([tm["elapsed_ms"], enc_ms, dec_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -499,12 +549,12 @@ def run_ours(a):
             ns = min(N, 64)
             sample = frames[:ns * px].cpu().numpy().reshape(ns, Hh, Ww)
             r = cpu_reference_rates(sample, threads, target_s=1.0)
-            cpu = {"value": r["value"], "unit": UNIT, "cores": threads, "kind": "reference",
-                   "sample": "first %d frames of this rank's batch, dbde_pack_frame/dbde_unpack_frame via oracle/_ref, "
-                             "~1 s per direction (%.0f core-seconds)" % (ns, r["cpu_seconds"]),
+            cpu = {"value": r["value"], "unit": UNIT, "cores": threads, "kind": r["kind"],
+                   "sample": "first %d frames of this rank's batch, %s, ~1 s per direction (%.0f core-seconds)"
+                             % (ns, CPU_CODECS[r["kind"]], r["cpu_seconds"]),
                    "encode_fps": r["encode_fps"], "decode_fps": r["decode_fps"]}
         except Exception as ex:            # the baseline must never take the bench line down
-            cpu = {"value": None, "unit": UNIT, "cores": os.cpu_count(), "kind": "reference", "sample": "failed: %s" % ex}
+            cpu = {"value": None, "unit": UNIT, "cores": os.cpu_count(), "kind": None, "sample": "failed: %s" % ex}
 
     line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": a.steps, "warmup": a.warmup,
             "ms_per_step": ms_per_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,

@@ -9,6 +9,7 @@ import this package; the product (dbce-video-cpp_b200/) never does.
 import ctypes as C
 import os
 import subprocess
+import time
 
 import numpy as np
 
@@ -256,3 +257,51 @@ def ref_decode_mt(slots, W, H, threads, reps=1):
     bad = C.c_int(0)
     s = _ref_lib.ref_decode_mt(_ptr(slots), slot, W, H, N, threads, reps, _ptr(frames), C.byref(bad))
     return s, frames, bad.value
+
+
+def _fan_out(n, threads, work):
+    """work(a, b) over `threads` contiguous ranges of range(n) on host threads (ctypes releases the GIL
+    during each call into the library) -> the sum of what the calls return"""
+    from concurrent.futures import ThreadPoolExecutor
+    threads = max(1, min(threads, n))
+    with ThreadPoolExecutor(threads) as ex:
+        return sum(ex.map(lambda t: work(n * t // threads, n * (t + 1) // threads), range(threads)))
+
+
+def port_encode_mt(frames, threads, reps=1):
+    """ref_encode_mt with the port's pack_frame: the CPU baseline where oracle/_ref is not built.
+    -> (seconds, slots (N,slot) u8, sizes)"""
+    frames = np.ascontiguousarray(frames, dtype=np.uint8)
+    N, H, W = frames.shape
+    slot = (frame_record_bound(W, H) + 63) // 64 * 64
+    slots = np.zeros((N, slot), dtype=np.uint8)
+    sizes = np.zeros(N, dtype=np.uint64)
+
+    def work(a, b):
+        for i in range(a, b):
+            sizes[i] = port._pack_frame(i, _ptr(frames[i]), W, H, _ptr(slots[i]))
+        return 0
+
+    t0 = time.perf_counter()
+    for _ in range(reps):
+        _fan_out(N, threads, work)
+    return time.perf_counter() - t0, slots, sizes
+
+
+def port_decode_mt(slots, W, H, threads, reps=1):
+    """ref_decode_mt with the port's unpack_frame -> (seconds, frames, records rejected over all reps)"""
+    slots = np.ascontiguousarray(slots, dtype=np.uint8)
+    N, slot = slots.shape
+    frames = np.zeros((N, H, W), dtype=np.uint8)
+
+    def work(a, b):
+        hdr = np.zeros(3, dtype=np.uint64)
+        bad = 0
+        for i in range(a, b):
+            port._unpack_frame(_ptr(slots[i]), W, H, _ptr(frames[i]), hdr.ctypes.data_as(_u64p))
+            bad += int(hdr[0]) != 2
+        return bad
+
+    t0 = time.perf_counter()
+    bad = sum(_fan_out(N, threads, work) for _ in range(reps))
+    return time.perf_counter() - t0, frames, bad

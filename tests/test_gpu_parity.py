@@ -217,6 +217,37 @@ def test_invert_endian_variant_matches_the_reference_built_with_the_macro(dropin
     assert (dropin.pack_frame(9, fr[0]) == ORA.pack_frame(9, fr[0])).all()
 
 
+def test_stored_differential_and_variant_records(codec, dropin):
+    """tests/golden/golden_differential.json through the CUDA path: the 60 small random frames through the C++
+    drop-in, and the DBDE_INVERT_ENDIAN + DBDE_HZ_AS_INTEGER streams and video header with both variants on"""
+    import importlib.util
+    import json
+    gdir = os.path.join(os.path.dirname(__file__), "golden")
+    spec = importlib.util.spec_from_file_location("make_golden_differential", os.path.join(gdir, "make_golden_differential.py"))
+    mg = importlib.util.module_from_spec(spec); spec.loader.exec_module(mg)
+    gold = json.load(open(os.path.join(gdir, "golden_differential.json")))
+    for (i, W, H, img), c in zip(mg.differential_frames(), gold["differential"], strict=True):
+        rec = dropin.pack_frame(i, img)
+        assert len(rec) == c["record_len"] and sha(rec) == c["record_sha256"], (W, H)
+        used, hdr, dec = dropin.unpack_frame(rec, W, H)
+        assert used == len(rec) and hdr == (2, i, 0) and (dec == img).all()
+    c = pkg.Codec(0)
+    try:
+        c.set_invert_endian(True)
+        for (W, H, style, fr), g in zip(mg.variant_frames(), gold["variants"]["cases"], strict=True):
+            got, offs = c.encode_host(fr, 5)
+            assert np.diff(offs).astype(np.int64).tolist() == g["sizes"] and sha(got) == g["stream_sha256"], (W, H, style)
+            dec, status, _ = c.decode_host(got, offs[:2], W, H)
+            assert (status == 0).all() and (dec == fr).all()
+    finally:
+        c.close()
+    try:
+        pkg.set_format_variants(True, True)
+        assert dropin.pack_video_header(3, 480, 640, 29.97).tobytes().hex() == gold["variants"]["video_header"]["hex"]
+    finally:
+        pkg.set_format_variants(False, False)
+
+
 def test_empty_batch_and_bad_arguments(codec):
     """nframes == 0 is a no-op that succeeds; nonsense dimensions and short output buffers are refused
     with an error code instead of a launch (the reference has no such checks: SURVEY 8b 'no bounds

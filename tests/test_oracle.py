@@ -1,6 +1,7 @@
 """CPU tests: pin the oracle port (oracle/dbde_oracle.c) against the reference's golden vectors
-(tests/golden/golden.json, produced by the unmodified reference) and, when oracle/_ref is built,
-differentially against the reference itself."""
+(tests/golden/golden.json, produced by the unmodified reference), against the stored records of the
+differential and format-variant comparisons (tests/golden/golden_differential.json) and, when
+oracle/_ref is built, differentially against the reference itself."""
 import hashlib
 import os
 
@@ -154,19 +155,33 @@ def test_invalid_streams_rejected(name, cd):
     assert hdr[0] == 0xFFFFFFFF and n == len(rec)             # header parse always advances (:330-337)
 
 
-@pytest.mark.skipif(oracle.ref is None, reason="oracle/_ref not built")
+def differential_golden():
+    """tests/golden/make_golden_differential.py (the inputs) and golden_differential.json (the stored records)"""
+    import importlib.util
+    import json
+    gdir = os.path.join(os.path.dirname(__file__), "golden")
+    spec = importlib.util.spec_from_file_location("make_golden_differential", os.path.join(gdir, "make_golden_differential.py"))
+    mg = importlib.util.module_from_spec(spec); spec.loader.exec_module(mg)
+    return mg, json.load(open(os.path.join(gdir, "golden_differential.json")))
+
+
 def test_port_vs_reference_differential():
-    """Random sizes incl. W<8, H<8, odd; all depth classes; both directions."""
-    rng = np.random.default_rng(3)
-    from conftest import rand_frame
-    for i in range(60):
-        W, H = int(rng.integers(1, 70)), int(rng.integers(1, 50))
-        img = rand_frame(rng, W, H, ["classes", "noise", "flat"][i % 3])
-        a, b = oracle.port.pack_frame(i, img), oracle.ref.pack_frame(i, img)
-        assert len(a) == len(b) and (a == b).all(), (W, H)
-        n1, h1, d1 = oracle.port.unpack_frame(b, W, H)
-        n2, h2, d2 = oracle.ref.unpack_frame(b, W, H)
-        assert n1 == n2 and h1 == h2 and (d1 == d2).all() and (d1 == img).all()
+    """Random sizes incl. W<8, H<8, odd; all depth classes; both directions: every record against the stored
+    vectors, and against the reference itself where oracle/_ref is built."""
+    mg, gold = differential_golden()
+    frames = mg.differential_frames()
+    assert len(frames) == len(gold["differential"]) == 60
+    for (i, W, H, img), c in zip(frames, gold["differential"]):
+        assert (W, H, sha(img)) == (c["W"], c["H"], c["image_sha256"]), "rng drifted; regenerate golden"
+        a = oracle.port.pack_frame(i, img)
+        assert len(a) == c["record_len"] and sha(a) == c["record_sha256"], (W, H)
+        n1, h1, d1 = oracle.port.unpack_frame(a, W, H)
+        assert n1 == len(a) and h1 == (2, i, 0) and (d1 == img).all()
+        if oracle.ref is not None:
+            b = oracle.ref.pack_frame(i, img)
+            assert len(a) == len(b) and (a == b).all(), (W, H)
+            n2, h2, d2 = oracle.ref.unpack_frame(b, W, H)
+            assert n1 == n2 and h1 == h2 and (d1 == d2).all()
 
 
 @pytest.mark.parametrize("name,cd", CODECS, ids=ids)
@@ -180,24 +195,29 @@ def test_depth8_stores_pixel_minus_min(name, cd):
 # ------------------------------------------------------------------ the reference's compile-time variants
 def test_port_variants_match_the_reference_built_with_both_macros():
     """DBDE_INVERT_ENDIAN + DBDE_HZ_AS_INTEGER (dbde_util.cpp:15-19,203-204,352-353): the port's run-time
-    switches against the unmodified reference compiled with the two macros (oracle/_ref)."""
-    if oracle.ref_variants is None:
-        pytest.skip("oracle/_ref/libdbde_ref_variants.so not built")
+    switches against the stored vectors (tests/golden/golden_differential.json) and against the unmodified
+    reference compiled with the two macros where oracle/_ref is built."""
+    mg, gold = differential_golden()
     pv, rv = oracle.port_variants(), oracle.ref_variants
-    rng = np.random.default_rng(77)
+    cases = mg.variant_frames()
+    assert len(cases) == len(gold["variants"]["cases"]) == 15
     differs = False
-    for W, H in [(8, 8), (10, 10), (17, 23), (64, 40), (1001, 24)]:
-        for style in ("classes", "noise", "flat"):
-            fr = np.stack([rand_frame(rng, W, H, style) for _ in range(2)])
-            a, sa = pv.pack_frames(fr, 5)
+    for (W, H, style, fr), c in zip(cases, gold["variants"]["cases"]):
+        assert (W, H, style, sha(fr)) == (c["W"], c["H"], c["style"], c["frames_sha256"]), "rng drifted; regenerate golden"
+        a, sa = pv.pack_frames(fr, 5)
+        assert [int(s) for s in sa] == c["sizes"] and sha(a) == c["stream_sha256"], (W, H, style)
+        if rv is not None:
             b, sb = rv.pack_frames(fr, 5)
             assert list(sa) == list(sb) and (a == b).all(), (W, H, style)
-            differs |= not np.array_equal(a, oracle.port.pack_frames(fr, 5)[0])
-            assert (pv.unpack_frames(a, W, H, 2)[0] == fr).all() and (rv.unpack_frames(a, W, H, 2)[0] == fr).all()
+            assert (rv.unpack_frames(a, W, H, 2)[0] == fr).all()
+        differs |= not np.array_equal(a, oracle.port.pack_frames(fr, 5)[0])
+        assert (pv.unpack_frames(a, W, H, 2)[0] == fr).all()
     assert differs, "the variant must change the payload bytes"
-    hv = rv.pack_video_header(3, 480, 640, 29.97)
-    assert (pv.pack_video_header(3, 480, 640, 29.97) == hv).all() and hv[20:].tolist() == [30, 0, 0, 0, 0, 0, 0, 0]
-    assert pv.unpack_video_header(hv) == rv.unpack_video_header(hv) == (28, (3, 480, 640, 30.0))
+    hv = pv.pack_video_header(3, 480, 640, 29.97)
+    assert hv.tobytes().hex() == gold["variants"]["video_header"]["hex"] and hv[20:].tolist() == [30, 0, 0, 0, 0, 0, 0, 0]
+    assert pv.unpack_video_header(hv) == (28, (3, 480, 640, 30.0))
+    if rv is not None:
+        assert (rv.pack_video_header(3, 480, 640, 29.97) == hv).all() and rv.unpack_video_header(hv) == (28, (3, 480, 640, 30.0))
 
 
 # ------------------------------------------------------------------ DBDE16 (SURVEY 8 f-4; not in the reference)
