@@ -37,6 +37,7 @@ C_SYMBOLS = [
     "dbde_b200_set_format_variants", "dbde_b200_get_format_variants", "dbde_b200_set_invert_endian",
     "dbde_b200_writer_open", "dbde_b200_writer_append", "dbde_b200_writer_close",
     "dbde_b200_reader_open", "dbde_b200_reader_next", "dbde_b200_reader_close", "dbde_b200_file_last_error",
+    "dbde_b200_decode_roi_device", "dbde_b200_decode_roi_host", "dbde_b200_reader_set_roi",
 ]
 # the reference's C++ entry points (include/dbde_util.h), by mangled name (SURVEY.md 8b)
 CXX_SYMBOLS = {
@@ -132,6 +133,11 @@ def load():
     lib.dbde_b200_reader_next.restype = C.c_long
     lib.dbde_b200_reader_next.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     lib.dbde_b200_reader_close.argtypes = [C.c_void_p]
+    lib.dbde_b200_reader_set_roi.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.dbde_b200_decode_roi_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.dbde_b200_decode_roi_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                              C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.dbde_b200_file_last_error.restype = C.c_char_p
     return lib
 
@@ -231,6 +237,13 @@ class Codec:
         self._ck(self.lib.dbde_b200_decode_device(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, n, frames_ptr,
                                                   status_ptr, index_ptr, stream), "decode_device")
 
+    def decode_roi_device(self, stream_ptr, stream_bytes, offs_ptr, W, H, n, roi, out_ptr, status_ptr, index_ptr=None,
+                          stream=0):
+        """region roi = (x0, y0, roi_w, roi_h) of every frame -> out_ptr, n * roi_w * roi_h bytes tightly packed"""
+        x0, y0, rw, rh = (int(v) for v in roi)
+        self._ck(self.lib.dbde_b200_decode_roi_device(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, n, x0, y0, rw, rh,
+                                                      out_ptr, status_ptr, index_ptr, stream), "decode_roi_device")
+
     # ---- host-buffer hot path (numpy or raw host pointers)
     def encode_host(self, frames, first_index=0):
         """frames (N,H,W) u8 -> (stream bytes, offsets[N+1])"""
@@ -258,6 +271,22 @@ class Codec:
         self._ck(self.lib.dbde_b200_decode_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
                                                 frames.ctypes.data, status.ctypes.data, index.ctypes.data),
                  "decode_host")
+        return frames, status, index
+
+    def decode_roi_host(self, stream, offsets, W, H, roi, fill=None):
+        """region roi = (x0, y0, roi_w, roi_h) of every frame -> (frames (N, roi_h, roi_w), status[N], indices[N]);
+        rejected frames keep `fill`"""
+        stream = np.ascontiguousarray(stream, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        x0, y0, rw, rh = (int(v) for v in roi)
+        N = len(offsets)
+        shape = (N, max(rh, 0), max(rw, 0))
+        frames = np.zeros(shape, dtype=np.uint8) if fill is None else np.full(shape, fill, dtype=np.uint8)
+        status = np.zeros(N, dtype=np.uint32)
+        index = np.zeros(N, dtype=np.uint64)
+        self._ck(self.lib.dbde_b200_decode_roi_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
+                                                    x0, y0, rw, rh, frames.ctypes.data, status.ctypes.data, index.ctypes.data),
+                 "decode_roi_host")
         return frames, status, index
 
     def decode_host_raw(self, stream_ptr, stream_bytes, offs_ptr, W, H, N, frames_ptr, status_ptr, index_ptr=None):
@@ -363,16 +392,22 @@ def write_file(codec, path, frames, hz=30.0, first_index=0, batch=16):
     return nf.value, nb.value
 
 
-def read_file(codec, path, batch=16, fill=0xCD):
-    """dbde_b200_reader_*: -> ((W, H, hz), frames (N,H,W), indices[N], status[N])"""
+def read_file(codec, path, batch=16, fill=0xCD, roi=None):
+    """dbde_b200_reader_*: -> ((W, H, hz), frames (N,H,W), indices[N], status[N]).  roi = (x0, y0, roi_w, roi_h):
+    only that region of every frame, frames (N, roi_h, roi_w)"""
     lib = codec.lib
     r, W, H, hz = C.c_void_p(), C.c_int(), C.c_int(), C.c_double()
     if lib.dbde_b200_reader_open(codec.h, path.encode(), batch, C.byref(W), C.byref(H), C.byref(hz), C.byref(r)):
         raise DbdeError("reader_open: " + lib.dbde_b200_file_last_error().decode())
     out, idx, st = [], [], []
+    ow, oh = W.value, H.value
     try:
+        if roi is not None:
+            x0, y0, ow, oh = (int(v) for v in roi)
+            if lib.dbde_b200_reader_set_roi(r, x0, y0, ow, oh):
+                raise DbdeError("reader_set_roi: " + lib.dbde_b200_file_last_error().decode())
         while True:
-            fr = np.full((batch, H.value, W.value), fill, dtype=np.uint8)
+            fr = np.full((batch, oh, ow), fill, dtype=np.uint8)
             ii = np.zeros(batch, dtype=np.uint64)
             ss = np.zeros(batch, dtype=np.uint32)
             n = lib.dbde_b200_reader_next(r, fr.ctypes.data, batch, ii.ctypes.data, ss.ctypes.data)
@@ -384,7 +419,7 @@ def read_file(codec, path, batch=16, fill=0xCD):
     finally:
         lib.dbde_b200_reader_close(r)
     if not out:
-        return (W.value, H.value, hz.value), np.zeros((0, H.value, W.value), np.uint8), np.zeros(0, np.uint64), np.zeros(0, np.uint32)
+        return (W.value, H.value, hz.value), np.zeros((0, oh, ow), np.uint8), np.zeros(0, np.uint64), np.zeros(0, np.uint32)
     return (W.value, H.value, hz.value), np.concatenate(out), np.concatenate(idx), np.concatenate(st)
 
 

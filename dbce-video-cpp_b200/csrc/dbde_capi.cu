@@ -487,6 +487,73 @@ extern "C" int dbde_b200_validate_device(dbde_b200_ctx *c, const uint8_t *stream
                               indices_dev, stream, true);
 }
 
+// ------------------------------------------------------------------ region of interest
+static bool roi_ok(int W, int H, int x0, int y0, int roi_w, int roi_h) {
+    return x0 >= 0 && y0 >= 0 && roi_w >= 1 && roi_h >= 1 && (long long)x0 + roi_w <= W && (long long)y0 + roi_h <= H;
+}
+
+// The validation pre-pass on linear partitions (every check of the full decode, over the whole record),
+// then one warp per 32 tile columns of each tile row of the region (dbde_roi.cu).  A region equal to the
+// frame is the full decode.
+extern "C" int dbde_b200_decode_roi_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
+                                           const uint64_t *frame_offsets_dev, int W, int H, int nframes, int x0, int y0,
+                                           int roi_w, int roi_h, uint8_t *roi_dev, uint32_t *status_dev,
+                                           uint64_t *indices_dev, void *stream) {
+    if (!c || !dims_ok(W, H, nframes) || !roi_ok(W, H, x0, y0, roi_w, roi_h) ||
+        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !roi_dev || !status_dev)))
+        return fail(DBDE_B200_E_INVALID, "decode_roi_device: bad argument");
+    if (nframes == 0) return 0;
+    if (x0 == 0 && y0 == 0 && roi_w == W && roi_h == H)
+        return decode_device_impl(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, roi_dev, status_dev,
+                                  indices_dev, stream, false);
+    CK(cudaSetDevice(c->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    DecParams D;
+    D.g = roi_scan_geom(W, H);
+    const int nitems = D.g.ppf * kConsumerWarps;
+    const size_t sbytes = 4 * (size_t)nframes * ((size_t)nitems + 1);
+    StreamScratch &sc = scratch_for(c, st);
+    int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
+    if (rc) return rc;
+    D.stream = stream_dev;
+    D.stream_bytes = stream_bytes;
+    D.frame_offsets = frame_offsets_dev;
+    D.frames = nullptr;
+    D.status = status_dev;
+    D.indices = indices_dev;
+    D.wprefix = (uint32_t *)sc.dec;
+    D.nframes = nframes;
+    D.nparts = (unsigned)((unsigned long long)nframes * D.g.ppf);
+    D.flags = c->invert_endian ? kFlagInvertRows : 0u;
+    RoiParams R;
+    R.stream = stream_dev;
+    R.frame_offsets = frame_offsets_dev;
+    R.status = status_dev;
+    R.wprefix = D.wprefix;
+    R.out = roi_dev;
+    R.w = D.g.w;
+    R.wh = D.g.wh;
+    R.nitems = nitems;
+    R.x0 = x0; R.y0 = y0; R.roi_w = roi_w; R.roi_h = roi_h;
+    R.tx0 = x0 / 8;
+    R.ty0 = y0 / 8;
+    R.tx_end = (x0 + roi_w + 7) / 8;
+    R.nty = (y0 + roi_h + 7) / 8 - R.ty0;
+    R.nchunks = (R.tx_end - R.tx0 + 31) / 32;
+    // a region narrower than 32 tiles gives each tile row the next power of two >= its width in lanes, and a
+    // warp 32 / that many tile rows: a one-pixel column keeps every lane busy
+    R.seg_shift = 0;
+    while ((1 << R.seg_shift) < R.tx_end - R.tx0 && R.seg_shift < 5) R.seg_shift++;
+    R.nrg = (R.nty + (32 >> R.seg_shift) - 1) / (32 >> R.seg_shift);
+    R.ntasks = (unsigned long long)nframes * (unsigned long long)R.nrg * (unsigned long long)R.nchunks;
+    R.flags = D.flags;
+    CK(launch_decode_scan(D, st));
+    c->launches += 1;
+    CK(launch_decode_roi(R, st));
+    c->launches += 1;
+    return 0;
+}
+
 // ------------------------------------------------------------------ pageable host memory
 // The reference's callers pass malloc'd buffers (dbde_util.h:24-35).  cudaMemcpyAsync on pageable memory
 // goes through the driver's own staging at ~15 GB/s and blocks the caller, and one host thread's memcpy is
@@ -874,7 +941,8 @@ extern "C" int dbde_b200_encode_host(dbde_b200_ctx *c, const uint8_t *frames_hos
 
 static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                             const uint64_t *frame_offsets_host, int W, int H, int nframes, uint8_t *frames_host,
-                            uint32_t *status_host, uint64_t *indices_host, bool scan_only, bool u16 = false) {
+                            uint32_t *status_host, uint64_t *indices_host, bool scan_only, bool u16 = false,
+                            const int *roi = nullptr) {
     if (!c || !dims_ok(W, H, nframes) ||
         (nframes > 0 && (!stream_host || !frame_offsets_host || (!frames_host && !scan_only) || !status_host)))
         return fail(DBDE_B200_E_INVALID, "decode_host: bad argument");
@@ -886,7 +954,7 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
             return fail(DBDE_B200_E_INVALID, "decode_host: frame offsets must ascend within the stream");
     }
     const HostFmt F = host_fmt(W, H, u16);
-    const size_t px = F.px;
+    const size_t px = roi ? (size_t)roi[2] * (size_t)roi[3] : F.px;    // output bytes per frame
     const int chunk = default_chunk(c, W, H, nframes, u16);
     const size_t delta = F.delta;
     const int nchunks = (nframes + chunk - 1) / chunk;
@@ -966,10 +1034,12 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
             CK(cudaMemcpyAsync(s.d_a + delta, stream_host + b0, b1 - b0, cudaMemcpyHostToDevice, s.st));
         }
         prof.mark(1, "h2d");
-        rc_all = u16 ? dbde_b200_decode16_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (uint16_t *)s.d_b, s.d_status,
-                                                 s.d_index, s.st)
-                     : decode_device_impl(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, s.d_b, s.d_status, s.d_index, s.st,
-                                          scan_only);
+        rc_all = u16   ? dbde_b200_decode16_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (uint16_t *)s.d_b, s.d_status,
+                                                   s.d_index, s.st)
+                 : roi ? dbde_b200_decode_roi_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, roi[0], roi[1], roi[2], roi[3],
+                                                     s.d_b, s.d_status, s.d_index, s.st)
+                       : decode_device_impl(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, s.d_b, s.d_status, s.d_index, s.st,
+                                            scan_only);
         if (rc_all) break;
         CK(cudaMemcpyAsync(s.h_status, s.d_status, 4 * (size_t)s.n, cudaMemcpyDeviceToHost, s.st));
         if (indices_host) CK(cudaMemcpyAsync(s.h_index, s.d_index, 8 * (size_t)s.n, cudaMemcpyDeviceToHost, s.st));
@@ -996,6 +1066,20 @@ extern "C" int dbde_b200_decode_host(dbde_b200_ctx *c, const uint8_t *stream_hos
                                      uint8_t *frames_host, uint32_t *status_host, uint64_t *indices_host) {
     return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, frames_host, status_host,
                             indices_host, false);
+}
+
+// The host form of dbde_b200_decode_roi_device: the same chunk pipeline with roi_w * roi_h bytes per frame
+// coming back.  Records still cross PCIe whole.
+extern "C" int dbde_b200_decode_roi_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
+                                         const uint64_t *frame_offsets_host, int W, int H, int nframes, int x0, int y0,
+                                         int roi_w, int roi_h, uint8_t *roi_host, uint32_t *status_host,
+                                         uint64_t *indices_host) {
+    if (!c || !dims_ok(W, H, nframes) || !roi_ok(W, H, x0, y0, roi_w, roi_h) ||
+        (nframes > 0 && (!stream_host || !frame_offsets_host || !roi_host || !status_host)))
+        return fail(DBDE_B200_E_INVALID, "decode_roi_host: bad argument");
+    const int roi[4] = {x0, y0, roi_w, roi_h};
+    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, roi_host, status_host,
+                            indices_host, false, false, roi);
 }
 
 // dbde_b200_validate_device for a stream in host memory: the records cross PCIe once, nothing comes

@@ -185,6 +185,8 @@ struct dbde_b200_reader {
     size_t pos = 0, have = 0;
     size_t ahead = 0;                          // bytes the I/O thread read into buf[1-cur]
     bool ahead_pending = false, eof = false, io_error = false, stopped = false;
+    bool roi = false;                          // hand out the region rx0, ry0, rw x rh of every frame
+    int rx0 = 0, ry0 = 0, rw = 0, rh = 0;
     std::vector<uint64_t> offs;
     Helper io;
 };
@@ -259,8 +261,9 @@ extern "C" int dbde_b200_reader_open(dbde_b200_ctx *ctx, const char *path, int b
     return 0;
 }
 
-// Decodes up to max_frames (<= the reader's batch size) frames into frames_host.  Returns the number of
-// frames handed out (0 at the end of the file) or a negative error.  status[i] != 0 marks a record
+// Decodes up to max_frames (<= the reader's batch size) frames -- or their regions, dbde_b200_reader_set_roi --
+// into frames_host.  Returns the number of frames handed out (0 at the end of the file) or a negative
+// error.  status[i] != 0 marks a record
 // the decoder rejected (its pixels are untouched); reading stops after the first rejected record,
 // like the reference's walker (dbde_util.cpp:416).
 extern "C" long dbde_b200_reader_next(dbde_b200_reader *r, uint8_t *frames_host, int max_frames, uint64_t *indices,
@@ -289,7 +292,9 @@ extern "C" long dbde_b200_reader_next(dbde_b200_reader *r, uint8_t *frames_host,
     uint8_t *p = r->buf[r->cur] + r->pos;
     const long n = dbde_b200_index_stream(p, r->have - r->pos, r->W, r->H, r->offs.data(), max_frames);
     if (n <= 0) return 0;                      // end of file (or a torn last record)
-    int rc = dbde_b200_decode_host(r->ctx, p, (size_t)r->offs[n], r->offs.data(), r->W, r->H, (int)n, frames_host, status, indices);
+    int rc = r->roi ? dbde_b200_decode_roi_host(r->ctx, p, (size_t)r->offs[n], r->offs.data(), r->W, r->H, (int)n, r->rx0, r->ry0,
+                                                r->rw, r->rh, frames_host, status, indices)
+                    : dbde_b200_decode_host(r->ctx, p, (size_t)r->offs[n], r->offs.data(), r->W, r->H, (int)n, frames_host, status, indices);
     if (rc) return ffail(rc, std::string("reader_next: ") + dbde_b200_last_error());
     long ok = n;
     for (long i = 0; i < n; i++)
@@ -297,6 +302,14 @@ extern "C" long dbde_b200_reader_next(dbde_b200_reader *r, uint8_t *frames_host,
     r->pos += (size_t)r->offs[ok];
     if (ok < n || status[ok - 1] != 0) r->stopped = true;                    // stop at the first bad record
     return ok;
+}
+
+extern "C" int dbde_b200_reader_set_roi(dbde_b200_reader *r, int x0, int y0, int roi_w, int roi_h) {
+    if (!r || x0 < 0 || y0 < 0 || roi_w < 1 || roi_h < 1 || (long long)x0 + roi_w > r->W || (long long)y0 + roi_h > r->H)
+        return ffail(DBDE_B200_E_INVALID, "reader_set_roi: the region must lie inside the frame");
+    r->roi = !(x0 == 0 && y0 == 0 && roi_w == r->W && roi_h == r->H);
+    r->rx0 = x0; r->ry0 = y0; r->rw = roi_w; r->rh = roi_h;
+    return 0;
 }
 
 extern "C" int dbde_b200_reader_close(dbde_b200_reader *r) {

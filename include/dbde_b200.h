@@ -168,6 +168,29 @@ DBDE_B200_API int dbde_b200_validate_host(dbde_b200_ctx *ctx, const uint8_t *str
                                           const uint64_t *frame_offsets_host, int W, int H, int nframes,
                                           uint32_t *status_host, uint64_t *indices_host);
 
+/* ---- region of interest: one rectangle of every frame ------------------------------------------------
+ * dbde_unpack_frame (dbde_util.cpp:339-345 -> dbde_unpack_image :291-328) followed by a crop, without
+ * decoding the rest of the frame: roi_out receives nframes * roi_h * roi_w bytes, tightly packed, frame i
+ * at roi_out + i * roi_w * roi_h, byte for byte image_i[y0 .. y0+roi_h-1][x0 .. x0+roi_w-1] of the full
+ * decode.  The region must satisfy 0 <= x0, 0 <= y0, roi_w >= 1, roi_h >= 1, x0 + roi_w <= W and
+ * y0 + roi_h <= H, else DBDE_B200_E_INVALID before any work is queued.  Validation covers the WHOLE record
+ * (dbde_util.cpp:295-303, 335 plus depth <= 8 and bounds): status and indices are exactly what
+ * dbde_b200_decode_device reports for the same records, a record damaged outside the region is rejected
+ * too, and a rejected frame's region of the output is left untouched.  roi_out may have any alignment and
+ * nothing outside [roi_out, roi_out + nframes * roi_w * roi_h) is written.  Follows the context's
+ * DBDE_INVERT_ENDIAN setting.  A region equal to the frame is dbde_b200_decode_device.
+ * _device: asynchronous on `stream`, with decode_device's per-stream scratch.  _host: the chunk pipeline of
+ * dbde_b200_decode_host (staging slots in flight, pageable buffers relayed, only accepted frames copied
+ * out); records still cross PCIe whole, only the region's pixels come back. */
+DBDE_B200_API int dbde_b200_decode_roi_device(dbde_b200_ctx *ctx, const uint8_t *stream_dev, size_t stream_bytes,
+                                              const uint64_t *frame_offsets_dev, int W, int H, int nframes,
+                                              int x0, int y0, int roi_w, int roi_h, uint8_t *roi_dev,
+                                              uint32_t *status_dev, uint64_t *indices_dev, void *stream);
+DBDE_B200_API int dbde_b200_decode_roi_host(dbde_b200_ctx *ctx, const uint8_t *stream_host, size_t stream_bytes,
+                                            const uint64_t *frame_offsets_host, int W, int H, int nframes,
+                                            int x0, int y0, int roi_w, int roi_h, uint8_t *roi_host,
+                                            uint32_t *status_host, uint64_t *indices_host);
+
 /* ---- DBDE16: 16-bit frames (SURVEY.md 8 f-4) -------------------------------------------------------
  * The extension the format note hints at (reference README.md:65, "could expand size to handle higher
  * bit depth images").  NOT in the reference code: the layout is defined here and restated by the test oracle
@@ -222,6 +245,10 @@ DBDE_B200_API int dbde_b200_reader_open(dbde_b200_ctx *ctx, const char *path, in
  * untouched); reading stops after the first one, like the reference's walker (dbde_util.cpp:416). */
 DBDE_B200_API long dbde_b200_reader_next(dbde_b200_reader *r, uint8_t *frames_host, int max_frames,
                                          uint64_t *indices, uint32_t *status);
+/* from the next dbde_b200_reader_next on, hand out the region (x0, y0, roi_w, roi_h) of every frame,
+ * roi_w * roi_h bytes per frame (dbde_b200_decode_roi_host); (0, 0, W, H) restores whole frames.  May be
+ * called between reader_next calls.  A region outside the frame is DBDE_B200_E_INVALID. */
+DBDE_B200_API int dbde_b200_reader_set_roi(dbde_b200_reader *r, int x0, int y0, int roi_w, int roi_h);
 DBDE_B200_API int dbde_b200_reader_close(dbde_b200_reader *r);
 DBDE_B200_API const char *dbde_b200_file_last_error(void);
 
