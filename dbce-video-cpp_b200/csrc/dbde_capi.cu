@@ -168,13 +168,7 @@ static PartGeom make_geom(int W, int H, bool fast) {
     // constant row pitch 2048 -- every lane has a tile (measured: 2304x2304 3.55 -> see DESIGN.md section 6).
     if (fast && g.w >= 32 && g.w % kTilesPerPart != 0) {
         const double used = g.nseg > 1 ? (double)g.w / (g.nseg * kTilesPerPart) : (double)(g.G * g.w) / kTilesPerPart;
-        if (used < 0.9 && getenv("DBDE_B200_NO_LINEAR") == nullptr) {
-            g.linear = 1;
-            g.nseg = 1;
-            g.G = 1;
-            g.ppf = (g.wh + kTilesPerPart - 1) / kTilesPerPart;
-            g.pitch = 8 * kTilesPerPart;
-        }
+        if (used < 0.9 && getenv("DBDE_B200_NO_LINEAR") == nullptr) g = linear_geom(W, H);
     }
     int need = 8 * g.G * g.pitch;
     if (need < 64 * kTilesPerPart) need = 64 * kTilesPerPart;
@@ -432,6 +426,29 @@ extern "C" int dbde_b200_encode_device(dbde_b200_ctx *c, const uint8_t *frames_d
     return 0;
 }
 
+// The validation pre-pass over geometry g.  Its word-prefix table lives in the scratch of stream st.  P->frames
+// is left null.
+static int scan_params(dbde_b200_ctx *c, cudaStream_t st, const PartGeom &g, const uint8_t *stream_dev, size_t stream_bytes,
+                       const uint64_t *frame_offsets_dev, int nframes, uint32_t *status_dev, uint64_t *indices_dev,
+                       DecParams *P) {
+    const size_t sbytes = 4 * (size_t)nframes * ((size_t)g.ppf * kConsumerWarps + 1);
+    StreamScratch &sc = scratch_for(c, st);
+    int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
+    if (rc) return rc;
+    P->g = g;
+    P->stream = stream_dev;
+    P->stream_bytes = stream_bytes;
+    P->frame_offsets = frame_offsets_dev;
+    P->frames = nullptr;
+    P->status = status_dev;
+    P->indices = indices_dev;
+    P->wprefix = (uint32_t *)sc.dec;
+    P->nframes = nframes;
+    P->nparts = (unsigned)((unsigned long long)nframes * g.ppf);
+    P->flags = c->invert_endian ? kFlagInvertRows : 0u;
+    return 0;
+}
+
 // scan_only: run the validation pre-pass alone (status + indices, no pixels): dbde_b200_validate_*
 static int decode_device_impl(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
                               const uint64_t *frame_offsets_dev, int W, int H, int nframes, uint8_t *frames_dev,
@@ -443,24 +460,12 @@ static int decode_device_impl(dbde_b200_ctx *c, const uint8_t *stream_dev, size_
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     const bool fast = (W % 16 == 0) && (H % 8 == 0) && (((uintptr_t)frames_dev & 15) == 0);
+    const PartGeom g = make_geom(W, H, fast);
+    if ((unsigned long long)nframes * g.ppf >= 0xFFFFFFF0ull) return fail(DBDE_B200_E_INVALID, "decode_device: batch too large");
     DecParams P;
-    P.g = make_geom(W, H, fast);
-    const unsigned long long nparts = (unsigned long long)nframes * P.g.ppf;
-    if (nparts >= 0xFFFFFFF0ull) return fail(DBDE_B200_E_INVALID, "decode_device: batch too large");
-    const size_t sbytes = 4 * (size_t)nframes * ((size_t)P.g.ppf * kConsumerWarps + 1);
-    StreamScratch &sc = scratch_for(c, st);
-    int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
+    int rc = scan_params(c, st, g, stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev, indices_dev, &P);
     if (rc) return rc;
-    P.stream = stream_dev;
-    P.stream_bytes = stream_bytes;
-    P.frame_offsets = frame_offsets_dev;
     P.frames = frames_dev;
-    P.status = status_dev;
-    P.indices = indices_dev;
-    P.wprefix = (uint32_t *)sc.dec;
-    P.nframes = nframes;
-    P.nparts = (unsigned)nparts;
-    P.flags = c->invert_endian ? kFlagInvertRows : 0u;
     CK(launch_decode_scan(P, st));
     c->launches += 1;
     if (scan_only) return 0;
@@ -509,47 +514,12 @@ extern "C" int dbde_b200_decode_roi_device(dbde_b200_ctx *c, const uint8_t *stre
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     DecParams D;
-    D.g = roi_scan_geom(W, H);
-    const int nitems = D.g.ppf * kConsumerWarps;
-    const size_t sbytes = 4 * (size_t)nframes * ((size_t)nitems + 1);
-    StreamScratch &sc = scratch_for(c, st);
-    int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
+    int rc = scan_params(c, st, linear_geom(W, H), stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev, indices_dev,
+                         &D);
     if (rc) return rc;
-    D.stream = stream_dev;
-    D.stream_bytes = stream_bytes;
-    D.frame_offsets = frame_offsets_dev;
-    D.frames = nullptr;
-    D.status = status_dev;
-    D.indices = indices_dev;
-    D.wprefix = (uint32_t *)sc.dec;
-    D.nframes = nframes;
-    D.nparts = (unsigned)((unsigned long long)nframes * D.g.ppf);
-    D.flags = c->invert_endian ? kFlagInvertRows : 0u;
-    RoiParams R;
-    R.stream = stream_dev;
-    R.frame_offsets = frame_offsets_dev;
-    R.status = status_dev;
-    R.wprefix = D.wprefix;
-    R.out = roi_dev;
-    R.w = D.g.w;
-    R.wh = D.g.wh;
-    R.nitems = nitems;
-    R.x0 = x0; R.y0 = y0; R.roi_w = roi_w; R.roi_h = roi_h;
-    R.tx0 = x0 / 8;
-    R.ty0 = y0 / 8;
-    R.tx_end = (x0 + roi_w + 7) / 8;
-    R.nty = (y0 + roi_h + 7) / 8 - R.ty0;
-    R.nchunks = (R.tx_end - R.tx0 + 31) / 32;
-    // a region narrower than 32 tiles gives each tile row the next power of two >= its width in lanes, and a
-    // warp 32 / that many tile rows: a one-pixel column keeps every lane busy
-    R.seg_shift = 0;
-    while ((1 << R.seg_shift) < R.tx_end - R.tx0 && R.seg_shift < 5) R.seg_shift++;
-    R.nrg = (R.nty + (32 >> R.seg_shift) - 1) / (32 >> R.seg_shift);
-    R.ntasks = (unsigned long long)nframes * (unsigned long long)R.nrg * (unsigned long long)R.nchunks;
-    R.flags = D.flags;
     CK(launch_decode_scan(D, st));
     c->launches += 1;
-    CK(launch_decode_roi(R, st));
+    CK(launch_decode_roi(D, x0, y0, roi_w, roi_h, roi_dev, st));
     c->launches += 1;
     return 0;
 }

@@ -217,54 +217,7 @@ struct DecSmemT {
 };
 using DecSmem = DecSmemT<kDecStages>;
 
-// ALIGN = 8: payload words are 8-byte aligned in shared memory (LDS.64), 4: 4-byte aligned
-// (LDS.32), 1: any byte offset (funnel-shifted pairs).  Uniform per partition.
-template <int K, int ALIGN>
-__device__ __forceinline__ void load_split(const uint8_t *pay, uint32_t (&q)[16]) {
-    uint32_t x[16];
-#pragma unroll
-    for (int j = 0; j < 16; j++) x[j] = 0;
-    if (ALIGN == 8) {
-#pragma unroll
-        for (int j = 0; j < K; j++) {
-            const uint2 v = reinterpret_cast<const uint2 *>(pay)[j];
-            x[2 * j] = v.x;
-            x[2 * j + 1] = v.y;
-        }
-    } else {
-#pragma unroll
-        for (int j = 0; j < 2 * K; j++)
-            x[j] = ALIGN == 4 ? reinterpret_cast<const uint32_t *>(pay)[j] : lds_u32_unaligned(pay + 4 * j);
-    }
-    split_fields<K>(x, q);
-}
-
-template <int ALIGN>
-__device__ __forceinline__ void load_split_any(int k, const uint8_t *pay, uint32_t (&q)[16]) {
-    switch (k) {
-        case 1: load_split<1, ALIGN>(pay, q); break;
-        case 2: load_split<2, ALIGN>(pay, q); break;
-        case 3: load_split<3, ALIGN>(pay, q); break;
-        case 4: load_split<4, ALIGN>(pay, q); break;
-        case 5: load_split<5, ALIGN>(pay, q); break;
-        case 6: load_split<6, ALIGN>(pay, q); break;
-        case 7: load_split<7, ALIGN>(pay, q); break;
-        default: load_split<8, ALIGN>(pay, q); break;
-    }
-}
-
 // ------------------------------------------------------------------ generic (unaligned / cropped) row stores
-// Bytes [s, e) of the little-endian 64-bit `w` go to q + s .. q + e; q is 8-byte aligned, 0 <= s <= e <= 8.
-// At most six naturally aligned stores (1-2-4 up to alignment, then 4-2-1 down).
-__device__ __forceinline__ void store_partial(uint8_t *q, uint64_t w, uint32_t s, uint32_t e) {
-    if ((s & 1u) && e - s >= 1u) { q[s] = (uint8_t)(w >> (8 * s)); s += 1; }
-    if ((s & 2u) && e - s >= 2u) { *reinterpret_cast<uint16_t *>(q + s) = (uint16_t)(w >> (8 * s)); s += 2; }
-    if ((s & 4u) && e - s >= 4u) { *reinterpret_cast<uint32_t *>(q + s) = (uint32_t)(w >> (8 * s)); s += 4; }
-    if (e - s >= 4u) { *reinterpret_cast<uint32_t *>(q + s) = (uint32_t)(w >> (8 * s)); s += 4; }
-    if (e - s >= 2u) { *reinterpret_cast<uint16_t *>(q + s) = (uint16_t)(w >> (8 * s)); s += 2; }
-    if (e - s >= 1u) q[s] = (uint8_t)(w >> (8 * s));
-}
-
 // One pixel row of a warp's tiles, any alignment, cropped to `ncol` columns (dbde_util.cpp:281-289).
 // Consecutive lanes of a band hold consecutive 8-byte pieces of the row, so every lane assembles the
 // ALIGNED 8-byte word its piece starts in -- the tail of its left neighbour (one shuffle) plus its own
@@ -404,13 +357,9 @@ __device__ __forceinline__ void store_rows_direct_any(uint32_t a0, uint8_t *rp, 
     }
 }
 
-// ------------------------------------------------------------------ one lane == one tile: payload -> pixels
-// Reads the tile's depth and minimum from the staged planes and its k words from the staged payload,
+// ------------------------------------------------------------------ one lane == one tile: stage -> pixels
+// Reads the tile's depth and minimum from the staged planes and finds its k words in the staged payload,
 // returns the 64 pixels (+min applied) in px.  Warp-wide call (scan + vote).
-// Measured (mix-2048, all nine depths per warp): threshold 99 (never) 4.41 TB/s, 3 -> 5.71, 2 -> 5.70; micro-2048
-// is indifferent (5.80-5.92 in all three), low-4096 loses 7 % at 2.  Re-measured with the sliding-window unpacker:
-// threshold 2 costs low-4096 10 % and low-1001x1003 8 %, threshold 1 (always) the same and gains 2 % on noise only.
-constexpr int kDecVarMinDepths = 3;
 __device__ __forceinline__ void dec_unpack_tile(const uint8_t *stage, const uint4 &c1, uint32_t wbase, int tid, int lane,
                                                 bool valid, bool invert, uint32_t (&px)[16]) {
     const uint32_t pres = c1.x;
@@ -422,33 +371,7 @@ __device__ __forceinline__ void dec_unpack_tile(const uint8_t *stage, const uint
     }
     const uint32_t incl = warp_inclusive_scan((uint32_t)k, lane);
     const uint32_t woff = wbase + incl - (uint32_t)k;
-    const uint32_t m4 = mn * 0x01010101u;
-    // how many different non-zero depths does this warp hold?  Each one is a pass through its own
-    // specialisation; from kDecVarMinDepths on, the depth-agnostic row unpacker is shorter.
-    const uint32_t kinds = __reduce_or_sync(0xffffffffu, (1u << k) >> 1);
-    const uint8_t *pay = stage + pres + 8 * (size_t)woff;
-    // (a warp of nothing but depth-8 tiles also goes this way: the K = 8 specialisation reads its 64-byte payloads with
-    // 8-way bank conflicts, the sliding window does not -- noise-2048 5.71 -> 5.83 TB/s)
-    if (__popc(kinds) >= kDecVarMinDepths || kinds == 0x80u) {
-        if (k > 0) {
-            if (DBDE_DEC_VAR64 && (pres & 7u) == 0) unpack_rows_var64(pay, k, px, m4);
-            else unpack_rows_var(pay, k, px, m4);
-        } else {
-#pragma unroll
-            for (int i = 0; i < 16; i++) px[i] = m4;
-        }
-    } else if (k > 0) {
-        uint32_t q[16];
-        if ((pres & 7u) == 0) load_split_any<8>(k, pay, q);     // the usual case: records on 8-byte boundaries
-        else load_split_any<1>(k, pay, q);
-        const SpreadK sk = spread_consts(k);
-#pragma unroll
-        for (int i = 0; i < 16; i++) px[i] = spread4(q[i], sk) + m4;   // +min (dbde_util.cpp:246)
-    } else {
-#pragma unroll
-        for (int i = 0; i < 16; i++) px[i] = m4;                                        // depth 0 (dbde_util.cpp:218-226)
-    }
-    if (invert) reverse_rows(px);                                                       // ENDIAN() at dbde_util.cpp:246-270
+    unpack_tile(stage + pres + 8 * (size_t)woff, k, mn * 0x01010101u, (pres & 7u) == 0, invert, px);
 }
 
 // ------------------------------------------------------------------ producer warp (both unpack kernels)

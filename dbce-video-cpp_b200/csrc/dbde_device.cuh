@@ -37,6 +37,21 @@ struct PartGeom {
                   //    they fall in (aligned frames whose width would leave lanes idle otherwise, see make_geom)
 };
 
+// Linear partitions (make_geom for aligned frames, the region-of-interest scan): word-prefix item i of the scan
+// is exactly tiles [32 i, 32 i + 32).  stage_bytes is left to the caller that stages partitions.
+inline PartGeom linear_geom(int W, int H) {
+    PartGeom g;
+    g.W = W; g.H = H;
+    g.w = (W + 7) / 8; g.h = (H + 7) / 8; g.wh = g.w * g.h;
+    g.linear = 1;
+    g.nseg = 1;
+    g.G = 1;
+    g.ppf = (g.wh + kTilesPerPart - 1) / kTilesPerPart;
+    g.pitch = 8 * kTilesPerPart;
+    g.stage_bytes = 0;
+    return g;
+}
+
 struct PartInfo {
     int f;        // frame within the batch
     int q;        // partition within the frame
@@ -412,6 +427,100 @@ __device__ __forceinline__ void unpack_rows_var64(const uint8_t *pay, int k, uin
     }
 }
 
+// unaligned-safe shared load for payloads that are not 8-byte aligned (records at odd offsets)
+__device__ __forceinline__ uint32_t lds_u32_unaligned(const uint8_t *p) {
+    uint32_t a = smem_u32(p);
+    const uint32_t *q = (const uint32_t *)(p - (a & 3u));
+    uint32_t sh = (a & 3u) * 8u;
+    uint32_t x0 = q[0];
+    if (sh == 0) return x0;
+    return __funnelshift_r(x0, q[1], sh);
+}
+
+// The per-depth specialisations: K payload words -> the sixteen 4K-bit fields.  ALIGN = 8: the words are 8-byte
+// aligned in shared memory (LDS.64); 1: any byte offset (funnel-shifted pairs).  Uniform per warp.
+template <int K, int ALIGN>
+__device__ __forceinline__ void load_split(const uint8_t *pay, uint32_t (&q)[16]) {
+    uint32_t x[16];
+#pragma unroll
+    for (int j = 0; j < 16; j++) x[j] = 0;
+    if (ALIGN == 8) {
+#pragma unroll
+        for (int j = 0; j < K; j++) {
+            const uint2 v = reinterpret_cast<const uint2 *>(pay)[j];
+            x[2 * j] = v.x;
+            x[2 * j + 1] = v.y;
+        }
+    } else {
+#pragma unroll
+        for (int j = 0; j < 2 * K; j++) x[j] = lds_u32_unaligned(pay + 4 * j);
+    }
+    split_fields<K>(x, q);
+}
+
+template <int ALIGN>
+__device__ __forceinline__ void load_split_any(int k, const uint8_t *pay, uint32_t (&q)[16]) {
+    switch (k) {
+        case 1: load_split<1, ALIGN>(pay, q); break;
+        case 2: load_split<2, ALIGN>(pay, q); break;
+        case 3: load_split<3, ALIGN>(pay, q); break;
+        case 4: load_split<4, ALIGN>(pay, q); break;
+        case 5: load_split<5, ALIGN>(pay, q); break;
+        case 6: load_split<6, ALIGN>(pay, q); break;
+        case 7: load_split<7, ALIGN>(pay, q); break;
+        default: load_split<8, ALIGN>(pay, q); break;
+    }
+}
+
+// ------------------------------------------------------------------ one lane == one tile: payload -> pixels
+// The unpacker of both decoders (dbde_decode.cu, dbde_roi.cu).  The warp votes on how many different non-zero
+// depths it holds: each one is a pass through its own specialisation, so from kDecVarMinDepths on the
+// depth-agnostic row unpacker is shorter.
+// Measured (mix-2048, all nine depths per warp): threshold 99 (never) 4.41 TB/s, 3 -> 5.71, 2 -> 5.70; micro-2048
+// is indifferent (5.80-5.92 in all three), low-4096 loses 7 % at 2.  Re-measured with the sliding-window unpacker:
+// threshold 2 costs low-4096 10 % and low-1001x1003 8 %, threshold 1 (always) the same and gains 2 % on noise only.
+constexpr int kDecVarMinDepths = 3;
+// pay: the tile's k payload words in shared memory, 8-byte aligned when al8 (the stage has the unpackers' slack
+// past them); m4: its minimum in every byte.  Returns the 64 pixels (+min applied, rows byte-reversed when
+// invert) in px.  Warp-wide call (the vote); lanes without a tile pass k = 0.
+__device__ __forceinline__ void unpack_tile(const uint8_t *pay, int k, uint32_t m4, bool al8, bool invert, uint32_t (&px)[16]) {
+    const uint32_t kinds = __reduce_or_sync(0xffffffffu, (1u << k) >> 1);
+    // (a warp of nothing but depth-8 tiles also goes this way: the K = 8 specialisation reads its 64-byte payloads with
+    // 8-way bank conflicts, the sliding window does not -- noise-2048 5.71 -> 5.83 TB/s)
+    if (__popc(kinds) >= kDecVarMinDepths || kinds == 0x80u) {
+        if (k > 0) {
+            if (DBDE_DEC_VAR64 && al8) unpack_rows_var64(pay, k, px, m4);
+            else unpack_rows_var(pay, k, px, m4);
+        } else {
+#pragma unroll
+            for (int i = 0; i < 16; i++) px[i] = m4;
+        }
+    } else if (k > 0) {
+        uint32_t q[16];
+        if (al8) load_split_any<8>(k, pay, q);                     // the usual case: records on 8-byte boundaries
+        else load_split_any<1>(k, pay, q);
+        const SpreadK sk = spread_consts(k);
+#pragma unroll
+        for (int i = 0; i < 16; i++) px[i] = spread4(q[i], sk) + m4;   // +min (dbde_util.cpp:246)
+    } else {
+#pragma unroll
+        for (int i = 0; i < 16; i++) px[i] = m4;                                        // depth 0 (dbde_util.cpp:218-226)
+    }
+    if (invert) reverse_rows(px);                                                       // ENDIAN() at dbde_util.cpp:246-270
+}
+
+// ------------------------------------------------------------------ cropped row stores (global memory)
+// Bytes [s, e) of the little-endian 64-bit `w` go to q + s .. q + e; q is 8-byte aligned, 0 <= s <= e <= 8.
+// At most six naturally aligned stores (1-2-4 up to alignment, then 4-2-1 down).
+__device__ __forceinline__ void store_partial(uint8_t *q, uint64_t w, uint32_t s, uint32_t e) {
+    if ((s & 1u) && e - s >= 1u) { q[s] = (uint8_t)(w >> (8 * s)); s += 1; }
+    if ((s & 2u) && e - s >= 2u) { *reinterpret_cast<uint16_t *>(q + s) = (uint16_t)(w >> (8 * s)); s += 2; }
+    if ((s & 4u) && e - s >= 4u) { *reinterpret_cast<uint32_t *>(q + s) = (uint32_t)(w >> (8 * s)); s += 4; }
+    if (e - s >= 4u) { *reinterpret_cast<uint32_t *>(q + s) = (uint32_t)(w >> (8 * s)); s += 4; }
+    if (e - s >= 2u) { *reinterpret_cast<uint16_t *>(q + s) = (uint16_t)(w >> (8 * s)); s += 2; }
+    if (e - s >= 1u) q[s] = (uint8_t)(w >> (8 * s));
+}
+
 // pack: q[16] = the sixteen 4k-bit fields (squeeze4) -> k U64 words at wp (8-byte aligned shared
 // memory).  A 64-bit accumulator takes one k-byte row per step at byte position (k*r) & 7 and is
 // flushed with a predicated store whenever a word completes.
@@ -461,16 +570,6 @@ __device__ __forceinline__ void pack_low_depths(const uint32_t (&px)[16], int k,
     } else if (k == 1) {
         asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(addr), "r"(r[0] + (r[1] << 16)), "r"(r[2] + (r[3] << 16)) : "memory");
     }
-}
-
-// unaligned-safe shared load for payloads that are not 8-byte aligned (records at odd offsets)
-__device__ __forceinline__ uint32_t lds_u32_unaligned(const uint8_t *p) {
-    uint32_t a = smem_u32(p);
-    const uint32_t *q = (const uint32_t *)(p - (a & 3u));
-    uint32_t sh = (a & 3u) * 8u;
-    uint32_t x0 = q[0];
-    if (sh == 0) return x0;
-    return __funnelshift_r(x0, q[1], sh);
 }
 #endif  // __CUDACC__
 

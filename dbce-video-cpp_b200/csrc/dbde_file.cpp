@@ -307,7 +307,7 @@ extern "C" long dbde_b200_reader_next(dbde_b200_reader *r, uint8_t *frames_host,
 extern "C" int dbde_b200_reader_set_roi(dbde_b200_reader *r, int x0, int y0, int roi_w, int roi_h) {
     if (!r || x0 < 0 || y0 < 0 || roi_w < 1 || roi_h < 1 || (long long)x0 + roi_w > r->W || (long long)y0 + roi_h > r->H)
         return ffail(DBDE_B200_E_INVALID, "reader_set_roi: the region must lie inside the frame");
-    r->roi = !(x0 == 0 && y0 == 0 && roi_w == r->W && roi_h == r->H);
+    r->roi = true;                             // dbde_b200_decode_roi_host runs a full-frame region as the full decode
     r->rx0 = x0; r->ry0 = y0; r->rw = roi_w; r->rh = roi_h;
     return 0;
 }

@@ -33,24 +33,6 @@ struct DecParams {
     uint32_t flags;             // kFlagInvertRows
 };
 
-// Region-of-interest decode (dbde_roi.cu): the rectangle [x0, x0 + roi_w) x [y0, y0 + roi_h) of every frame,
-// after dbde_decode_scan_kernel has run on roi_scan_geom(W, H) (word prefixes per 32 consecutive tiles)
-struct RoiParams {
-    const uint8_t *stream;
-    const uint64_t *frame_offsets;
-    const uint32_t *status;     // from the scan: frames with status != 0 are skipped
-    const uint32_t *wprefix;    // nframes * (nitems + 1)
-    uint8_t *out;               // nframes * roi_w * roi_h, tightly packed, any alignment
-    int w, wh, nitems;          // tile columns, tiles, word-prefix items per frame (ppf * 8)
-    int x0, y0, roi_w, roi_h;
-    int tx0, ty0, tx_end;       // the region's first tile column / row, one past its last tile column
-    int nty, nchunks;           // tile rows of the region, 32-tile warps per tile row
-    int seg_shift;              // log2 of the lanes per tile row: 5, or fewer for regions narrower than 32 tiles
-    int nrg;                    // warps (groups of 32 >> seg_shift tile rows) per 32-tile column chunk and frame
-    unsigned long long ntasks;  // nframes * nrg * nchunks warps
-    uint32_t flags;             // kFlagInvertRows
-};
-
 // The reference's DBDE_INVERT_ENDIAN build variant (dbde_util.cpp:15-19,24-27,246-270): every 8-pixel tile
 // row is byte-reversed before packing and after unpacking.  A launch-uniform flag here.
 enum : uint32_t { kFlagInvertRows = 1 };
@@ -104,7 +86,9 @@ cudaError_t launch_compact(const uint8_t *slots, uint64_t slot_stride, const uin
                            cudaStream_t stream);
 cudaError_t launch_decode_scan(const DecParams &P, cudaStream_t stream);
 cudaError_t launch_decode(const DecParams &P, bool fast, int num_sms, cudaStream_t stream);
-PartGeom roi_scan_geom(int W, int H);      // linear partitions: word-prefix item i == tiles [32 i, 32 i + 32)
-cudaError_t launch_decode_roi(const RoiParams &P, cudaStream_t stream);
+// Region-of-interest decode (dbde_roi.cu): the rectangle [x0, x0 + roi_w) x [y0, y0 + roi_h) of every frame into
+// `out` (nframes * roi_w * roi_h bytes, tightly packed, any alignment), after launch_decode_scan(scan) with
+// scan.g = linear_geom(W, H) (word prefixes per 32 consecutive tiles).  Frames the scan rejected stay untouched.
+cudaError_t launch_decode_roi(const DecParams &scan, int x0, int y0, int roi_w, int roi_h, uint8_t *out, cudaStream_t stream);
 
 }  // namespace dbde

@@ -3,14 +3,14 @@
 // (dbde_util.cpp:291-328, 339-345) and with its accept/reject behaviour.
 //
 // Two launches:
-//   dbde_decode_scan_kernel (dbde_decode.cu, unchanged) on a LINEAR geometry (roi_scan_geom): partitions of
+//   dbde_decode_scan_kernel (dbde_decode.cu, unchanged) on a LINEAR geometry (linear_geom): partitions of
 //     256 consecutive tiles, so word-prefix item i is exactly tiles [32 i, 32 i + 32) of the frame's
 //     row-major tile order.  It validates the WHOLE record (a record damaged outside the region is still
 //     rejected, with the same status bits as dbde_b200_decode_device) and reads 1 byte per tile.
 //   dbde_decode_roi_kernel : one warp == 32 consecutive tile columns of one tile row of the region in one
 //     frame, one lane == one tile.  Payloads lie in row-major tile order, so the warp's 32 payloads are ONE
 //     contiguous byte run of the record: the warp stages it into shared memory with coalesced 16-byte loads
-//     and unpacks with the decoder's helpers.  Its first tile's word offset is the item prefix plus at most
+//     and unpacks with the decoder's unpack_tile.  Its first tile's word offset is the item prefix plus at most
 //     31 depth bytes; the rest is a warp scan of the 32 depths.  Rows are cropped on all four sides and
 //     stored at pitch roi_w, any alignment, as runs of aligned 8-byte words assembled across lanes.
 //     A region narrower than 32 tiles gives a tile row a SEGMENT of S lanes (the next power of two >= its
@@ -20,57 +20,30 @@
 #include "dbde_kernels.h"
 
 namespace dbde {
+
+// one launch of dbde_decode_roi_kernel: the scan's outputs and the region's tiling (launch_decode_roi)
+struct RoiParams {
+    const uint8_t *stream;
+    const uint64_t *frame_offsets;
+    const uint32_t *status;     // from the scan: frames with status != 0 are skipped
+    const uint32_t *wprefix;    // nframes * (nitems + 1)
+    uint8_t *out;               // nframes * roi_w * roi_h, tightly packed, any alignment
+    int w, wh, nitems;          // tile columns, tiles, word-prefix items per frame (ppf * 8)
+    int x0, y0, roi_w, roi_h;
+    int tx0, ty0, tx_end;       // the region's first tile column / row, one past its last tile column
+    int nty, nchunks;           // tile rows of the region, 32-tile warps per tile row
+    int seg_shift;              // log2 of the lanes per tile row: 5, or fewer for regions narrower than 32 tiles
+    int nrg;                    // warps (groups of 32 >> seg_shift tile rows) per 32-tile column chunk and frame
+    unsigned long long ntasks;  // nframes * nrg * nchunks warps
+    uint32_t flags;             // kFlagInvertRows
+};
+
 namespace {
 
 constexpr int kRoiWarps = 8;
 // per segment of S lanes: its payload run (<= S tiles x 64 bytes) + its offset inside the first 16-byte granule
 // (< 16) + the unpackers' over-read past a tile's last byte (< 16); 32 / S segments per warp
 constexpr int kRoiBufBytes = 32 * (64 + 32);
-
-// ALIGN = 8: payload words 8-byte aligned in shared memory; 1: any byte offset
-template <int K, int ALIGN>
-__device__ __forceinline__ void roi_load_split(const uint8_t *pay, uint32_t (&q)[16]) {
-    uint32_t x[16];
-#pragma unroll
-    for (int j = 0; j < 16; j++) x[j] = 0;
-    if (ALIGN == 8) {
-#pragma unroll
-        for (int j = 0; j < K; j++) {
-            const uint2 v = reinterpret_cast<const uint2 *>(pay)[j];
-            x[2 * j] = v.x;
-            x[2 * j + 1] = v.y;
-        }
-    } else {
-#pragma unroll
-        for (int j = 0; j < 2 * K; j++) x[j] = lds_u32_unaligned(pay + 4 * j);
-    }
-    split_fields<K>(x, q);
-}
-
-template <int ALIGN>
-__device__ __forceinline__ void roi_load_split_any(int k, const uint8_t *pay, uint32_t (&q)[16]) {
-    switch (k) {
-        case 1: roi_load_split<1, ALIGN>(pay, q); break;
-        case 2: roi_load_split<2, ALIGN>(pay, q); break;
-        case 3: roi_load_split<3, ALIGN>(pay, q); break;
-        case 4: roi_load_split<4, ALIGN>(pay, q); break;
-        case 5: roi_load_split<5, ALIGN>(pay, q); break;
-        case 6: roi_load_split<6, ALIGN>(pay, q); break;
-        case 7: roi_load_split<7, ALIGN>(pay, q); break;
-        default: roi_load_split<8, ALIGN>(pay, q); break;
-    }
-}
-
-// Bytes [s, e) of the little-endian 64-bit `w` go to q + s .. q + e; q is 8-byte aligned, 0 <= s < e <= 8.
-// Naturally aligned pieces: 1-2-4 up to alignment, then 4-2-1 down.
-__device__ __forceinline__ void roi_store_partial(uint8_t *q, uint64_t w, int s, int e) {
-    if ((s & 1) && e - s >= 1) { q[s] = (uint8_t)(w >> (8 * s)); s += 1; }
-    if ((s & 2) && e - s >= 2) { *reinterpret_cast<uint16_t *>(q + s) = (uint16_t)(w >> (8 * s)); s += 2; }
-    if ((s & 4) && e - s >= 4) { *reinterpret_cast<uint32_t *>(q + s) = (uint32_t)(w >> (8 * s)); s += 4; }
-    if (e - s >= 4) { *reinterpret_cast<uint32_t *>(q + s) = (uint32_t)(w >> (8 * s)); s += 4; }
-    if (e - s >= 2) { *reinterpret_cast<uint16_t *>(q + s) = (uint16_t)(w >> (8 * s)); s += 2; }
-    if (e - s >= 1) q[s] = (uint8_t)(w >> (8 * s));
-}
 
 // One pixel row of a segment's tiles into an output row of roi_w bytes at any alignment.  Lane l's 8 pixels
 // belong at row + pos (pos = 8 l + 256 chunk - (x0 & 7), l the lane within its segment: the region's first
@@ -94,11 +67,11 @@ __device__ __forceinline__ void roi_store_row(uint8_t *row, int pos, uint64_t x,
     const int s = max(-qo, first ? (int)a : 0), e = min(roi_w - qo, 8);
     uint8_t *q = row + qo;
     if (s == 0 && e == 8) st_stream_u64(q, w);
-    else if (s < e) roi_store_partial(q, w, s, e);
+    else if (s < e) store_partial(q, w, (uint32_t)s, (uint32_t)e);
     if (last && a) {                                                         // my bytes past that word
         // (a one-tile-wide region can start inside them: the left crop applies here too)
         const int s2 = max(-qo - 8, 0), e2 = min(roi_w - qo - 8, (int)a);
-        if (s2 < e2) roi_store_partial(q + 8, x >> (64 - 8 * a), s2, e2);
+        if (s2 < e2) store_partial(q + 8, x >> (64 - 8 * a), (uint32_t)s2, (uint32_t)e2);
     }
 }
 
@@ -159,33 +132,9 @@ __global__ void __launch_bounds__(kRoiWarps * 32) dbde_decode_roi_kernel(const R
     }
     __syncwarp();
 
-    // unpack, with the full decoder's choice between per-depth specialisations and the depth-agnostic
-    // row unpacker (dec_unpack_tile in dbde_decode.cu)
-    const uint8_t *pay = sbuf + (gs - a0) + 8 * (size_t)(incl - k);
-    const bool al8 = (gs & 7u) == 0;
-    const uint32_t m4 = mn * 0x01010101u;
-    const uint32_t kinds = __reduce_or_sync(0xffffffffu, (1u << k) >> 1);
     uint32_t px[16];
-    if (__popc(kinds) >= 3 || kinds == 0x80u) {
-        if (k > 0) {
-            if (al8) unpack_rows_var64(pay, (int)k, px, m4);
-            else unpack_rows_var(pay, (int)k, px, m4);
-        } else {
-#pragma unroll
-            for (int i = 0; i < 16; i++) px[i] = m4;
-        }
-    } else if (k > 0) {
-        uint32_t q[16];
-        if (al8) roi_load_split_any<8>((int)k, pay, q);
-        else roi_load_split_any<1>((int)k, pay, q);
-        const SpreadK sk = spread_consts((int)k);
-#pragma unroll
-        for (int i = 0; i < 16; i++) px[i] = spread4(q[i], sk) + m4;           // +min (dbde_util.cpp:246)
-    } else {
-#pragma unroll
-        for (int i = 0; i < 16; i++) px[i] = m4;                               // depth 0 (dbde_util.cpp:218-226)
-    }
-    if (P.flags & kFlagInvertRows) reverse_rows(px);                           // ENDIAN() at dbde_util.cpp:246-270
+    unpack_tile(sbuf + (gs - a0) + 8 * (size_t)(incl - k), (int)k, mn * 0x01010101u, (gs & 7u) == 0, (P.flags & kFlagInvertRows) != 0,
+                px);
 
     // crop and store: rows of the tile inside [y0, y0 + roi_h), columns inside [x0, x0 + roi_w)
     uint8_t *fout = P.out + (size_t)f * ((size_t)P.roi_w * (size_t)P.roi_h);
@@ -200,20 +149,28 @@ __global__ void __launch_bounds__(kRoiWarps * 32) dbde_decode_roi_kernel(const R
     }
 }
 
-PartGeom roi_scan_geom(int W, int H) {
-    PartGeom g;
-    g.W = W; g.H = H;
-    g.w = (W + 7) / 8; g.h = (H + 7) / 8; g.wh = g.w * g.h;
-    g.linear = 1;
-    g.nseg = 1;
-    g.G = 1;
-    g.ppf = (g.wh + kTilesPerPart - 1) / kTilesPerPart;
-    g.pitch = 8 * kTilesPerPart;        // unused by the scan
-    g.stage_bytes = 0;
-    return g;
-}
-
-cudaError_t launch_decode_roi(const RoiParams &P, cudaStream_t stream) {
+cudaError_t launch_decode_roi(const DecParams &scan, int x0, int y0, int roi_w, int roi_h, uint8_t *out, cudaStream_t stream) {
+    RoiParams P;
+    P.stream = scan.stream;
+    P.frame_offsets = scan.frame_offsets;
+    P.status = scan.status;
+    P.wprefix = scan.wprefix;
+    P.out = out;
+    P.w = scan.g.w;
+    P.wh = scan.g.wh;
+    P.nitems = scan.g.ppf * kConsumerWarps;
+    P.x0 = x0; P.y0 = y0; P.roi_w = roi_w; P.roi_h = roi_h;
+    P.tx0 = x0 / 8;
+    P.ty0 = y0 / 8;
+    P.tx_end = (x0 + roi_w + 7) / 8;
+    P.nty = (y0 + roi_h + 7) / 8 - P.ty0;
+    P.nchunks = (P.tx_end - P.tx0 + 31) / 32;
+    // segments: the next power of two >= the region's width in tiles, at most 32 lanes
+    P.seg_shift = 0;
+    while ((1 << P.seg_shift) < P.tx_end - P.tx0 && P.seg_shift < 5) P.seg_shift++;
+    P.nrg = (P.nty + (32 >> P.seg_shift) - 1) / (32 >> P.seg_shift);
+    P.ntasks = (unsigned long long)scan.nframes * (unsigned long long)P.nrg * (unsigned long long)P.nchunks;
+    P.flags = scan.flags;
     if (P.ntasks == 0) return cudaSuccess;
     const unsigned long long blocks = (P.ntasks + kRoiWarps - 1) / kRoiWarps;
     if (blocks > 0x7FFFFFFFull) return cudaErrorInvalidConfiguration;
