@@ -38,6 +38,7 @@ C_SYMBOLS = [
     "dbde_b200_writer_open", "dbde_b200_writer_append", "dbde_b200_writer_close",
     "dbde_b200_reader_open", "dbde_b200_reader_next", "dbde_b200_reader_close", "dbde_b200_file_last_error",
     "dbde_b200_decode_roi_device", "dbde_b200_decode_roi_host", "dbde_b200_reader_set_roi",
+    "dbde_b200_decode_crops_device", "dbde_b200_decode_crops_host",
 ]
 # the reference's C++ entry points (include/dbde_util.h), by mangled name (SURVEY.md 8b)
 CXX_SYMBOLS = {
@@ -138,6 +139,12 @@ def load():
                                                 C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.dbde_b200_decode_roi_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                               C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.dbde_b200_decode_crops_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                  C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                                  C.c_void_p, C.c_void_p]
+    lib.dbde_b200_decode_crops_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                                C.c_void_p]
     lib.dbde_b200_file_last_error.restype = C.c_char_p
     return lib
 
@@ -244,6 +251,16 @@ class Codec:
         self._ck(self.lib.dbde_b200_decode_roi_device(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, n, x0, y0, rw, rh,
                                                       out_ptr, status_ptr, index_ptr, stream), "decode_roi_device")
 
+    def decode_crops_device(self, stream_ptr, stream_bytes, offs_ptr, W, H, n, corners_ptr, ncrops, per_frame, size, out_ptr,
+                            status_ptr, index_ptr=None, pad=0, stream=0):
+        """ncrops crops of size = (crop_w, crop_h) per frame at the int32 {x0, y0} corners at corners_ptr (device; per_frame:
+        n * ncrops pairs, else ncrops pairs for every frame) -> out_ptr, n * ncrops * crop_w * crop_h bytes tightly packed;
+        pixels outside the frame are `pad`"""
+        cw, ch = (int(v) for v in size)
+        self._ck(self.lib.dbde_b200_decode_crops_device(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, n, corners_ptr, ncrops,
+                                                        int(per_frame), cw, ch, pad, out_ptr, status_ptr, index_ptr, stream),
+                 "decode_crops_device")
+
     # ---- host-buffer hot path (numpy or raw host pointers)
     def encode_host(self, frames, first_index=0):
         """frames (N,H,W) u8 -> (stream bytes, offsets[N+1])"""
@@ -288,6 +305,31 @@ class Codec:
                                                     x0, y0, rw, rh, frames.ctypes.data, status.ctypes.data, index.ctypes.data),
                  "decode_roi_host")
         return frames, status, index
+
+    def decode_crops_host(self, stream, offsets, W, H, corners, size, pad=0, fill=None):
+        """crops of size = (crop_w, crop_h) at int32 corners (R, 2) (the same for every frame) or (N, R, 2) (per frame) ->
+        (crops (N, R, crop_h, crop_w), status[N], indices[N]); pixels outside the frame are `pad`, rejected frames keep
+        `fill`"""
+        stream = np.ascontiguousarray(stream, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        corners = np.ascontiguousarray(corners, dtype=np.int32)
+        cw, ch = (int(v) for v in size)
+        N = len(offsets)
+        if corners.ndim == 3 and corners.shape[0] == N and corners.shape[2] == 2:
+            per_frame = 1
+        elif corners.ndim == 2 and corners.shape[1] == 2:
+            per_frame = 0
+        else:
+            raise ValueError("corners must have shape (R, 2) or (N, R, 2), got %r" % (corners.shape,))
+        R = corners.shape[-2]
+        shape = (N, R, max(ch, 0), max(cw, 0))
+        crops = np.zeros(shape, dtype=np.uint8) if fill is None else np.full(shape, fill, dtype=np.uint8)
+        status = np.zeros(N, dtype=np.uint32)
+        index = np.zeros(N, dtype=np.uint64)
+        self._ck(self.lib.dbde_b200_decode_crops_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
+                                                      corners.ctypes.data, R, per_frame, cw, ch, pad, crops.ctypes.data,
+                                                      status.ctypes.data, index.ctypes.data), "decode_crops_host")
+        return crops, status, index
 
     def decode_host_raw(self, stream_ptr, stream_bytes, offs_ptr, W, H, N, frames_ptr, status_ptr, index_ptr=None):
         self._ck(self.lib.dbde_b200_decode_host(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, N, frames_ptr,

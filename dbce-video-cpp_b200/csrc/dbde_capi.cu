@@ -89,7 +89,7 @@ struct HostSlot {
     cudaEvent_t ev = nullptr;
     uint8_t *d_a = nullptr;      // encode: frames   | decode: stream bytes
     uint8_t *d_b = nullptr;      // encode: records in their slots | decode: frames
-    uint8_t *d_c = nullptr;      // encode: records back to back (compacted on the device)
+    uint8_t *d_c = nullptr;      // encode: records back to back (compacted on the device) | decode crops: the chunk's corners
     uint64_t *d_off = nullptr;
     uint64_t *d_size = nullptr;
     uint32_t *d_status = nullptr;
@@ -102,6 +102,8 @@ struct HostSlot {
     // bounce buffers the bytes are relayed through in pieces, by parallel memcpy overlapped with the DMA
     uint8_t *h_in = nullptr, *h_out = nullptr;
     size_t cap_hin = 0, cap_hout = 0;
+    int32_t *h_corners = nullptr;   // pinned staging of the chunk's crop corners (decode crops)
+    size_t cap_hcorners = 0;
     // completion flags in pinned memory: a 4-byte D2H copy of the context's device word `1`, queued behind the
     // work it reports, sets one; host threads wait on them by reading memory, not by calling the driver
     volatile uint32_t *h_flag = nullptr;    // kMaxDmaPieces for relayed D2H pieces + 1 for the chunk's kernels
@@ -254,6 +256,7 @@ static void free_slot(HostSlot &s) {
     if (s.h_index) cudaFreeHost(s.h_index);
     if (s.h_in) cudaFreeHost(s.h_in);
     if (s.h_out) cudaFreeHost(s.h_out);
+    if (s.h_corners) cudaFreeHost(s.h_corners);
     if (s.h_flag) cudaFreeHost((void *)s.h_flag);
     if (s.ev) cudaEventDestroy(s.ev);
     if (s.st) cudaStreamDestroy(s.st);
@@ -497,8 +500,19 @@ static bool roi_ok(int W, int H, int x0, int y0, int roi_w, int roi_h) {
     return x0 >= 0 && y0 >= 0 && roi_w >= 1 && roi_h >= 1 && (long long)x0 + roi_w <= W && (long long)y0 + roi_h <= H;
 }
 
-// The validation pre-pass on linear partitions (every check of the full decode, over the whole record),
-// then one warp per 32 tile columns of each tile row of the region (dbde_roi.cu).  A region equal to the
+// The validation pre-pass on linear partitions (every check of the full decode, over the whole record), queued on
+// st: the first launch of the region and crop decodes.  D is what their kernels read.
+static int linear_scan(dbde_b200_ctx *c, cudaStream_t st, int W, int H, const uint8_t *stream_dev, size_t stream_bytes,
+                       const uint64_t *frame_offsets_dev, int nframes, uint32_t *status_dev, uint64_t *indices_dev, DecParams *D) {
+    CK(cudaSetDevice(c->device));
+    int rc = scan_params(c, st, linear_geom(W, H), stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev, indices_dev, D);
+    if (rc) return rc;
+    CK(launch_decode_scan(*D, st));
+    c->launches += 1;
+    return 0;
+}
+
+// The scan, then one warp per 32 tile columns of each tile row of the region (dbde_roi.cu).  A region equal to the
 // frame is the full decode.
 extern "C" int dbde_b200_decode_roi_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
                                            const uint64_t *frame_offsets_dev, int W, int H, int nframes, int x0, int y0,
@@ -511,15 +525,38 @@ extern "C" int dbde_b200_decode_roi_device(dbde_b200_ctx *c, const uint8_t *stre
     if (x0 == 0 && y0 == 0 && roi_w == W && roi_h == H)
         return decode_device_impl(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, roi_dev, status_dev,
                                   indices_dev, stream, false);
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
     DecParams D;
-    int rc = scan_params(c, st, linear_geom(W, H), stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev, indices_dev,
-                         &D);
+    int rc = linear_scan(c, (cudaStream_t)stream, W, H, stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev,
+                         indices_dev, &D);
     if (rc) return rc;
-    CK(launch_decode_scan(D, st));
+    CK(launch_decode_roi(D, x0, y0, roi_w, roi_h, roi_dev, (cudaStream_t)stream));
     c->launches += 1;
-    CK(launch_decode_roi(D, x0, y0, roi_w, roi_h, roi_dev, st));
+    return 0;
+}
+
+// ------------------------------------------------------------------ crops
+static bool crops_ok(int ncrops, int corners_per_frame, int crop_w, int crop_h, int pad) {
+    return ncrops >= 1 && crop_w >= 1 && crop_h >= 1 && dims_ok(crop_w, crop_h, 0) &&
+           (long long)ncrops * crop_w * crop_h <= 0x7FFFFFFFLL && (corners_per_frame == 0 || corners_per_frame == 1) && pad >= 0 &&
+           pad <= 255;
+}
+
+// The region decode's scan and kernel body with one rectangle per task taken from `corners` (dbde_roi.cu).  A crop
+// equal to the frame still runs the crop kernel: its output layout is the crop layout whatever the corners.
+extern "C" int dbde_b200_decode_crops_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
+                                             const uint64_t *frame_offsets_dev, int W, int H, int nframes,
+                                             const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
+                                             int crop_h, int pad, uint8_t *crops_dev, uint32_t *status_dev,
+                                             uint64_t *indices_dev, void *stream) {
+    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
+        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !corners_dev || !crops_dev || !status_dev)))
+        return fail(DBDE_B200_E_INVALID, "decode_crops_device: bad argument");
+    if (nframes == 0) return 0;
+    DecParams D;
+    int rc = linear_scan(c, (cudaStream_t)stream, W, H, stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev,
+                         indices_dev, &D);
+    if (rc) return rc;
+    CK(launch_decode_crops(D, corners_dev, ncrops, corners_per_frame != 0, crop_w, crop_h, pad, crops_dev, (cudaStream_t)stream));
     c->launches += 1;
     return 0;
 }
@@ -909,10 +946,20 @@ extern "C" int dbde_b200_encode_host(dbde_b200_ctx *c, const uint8_t *frames_hos
     return 0;
 }
 
+// What the host pipeline hands back per frame instead of the whole image: the region (x0, y0, w, h), or ncrops crops
+// of w x h with host corners (per_frame: nframes * ncrops {x0, y0} pairs, else ncrops pairs for every frame)
+struct SubFrame {
+    int x0, y0, w, h;
+    const int32_t *corners;     // null: the region
+    int ncrops, per_frame, pad;
+    size_t bytes() const { return (size_t)w * (size_t)h * (size_t)(corners ? ncrops : 1); }
+    size_t corner_bytes(int n) const { return corners ? 8 * (size_t)ncrops * (size_t)(per_frame ? n : 1) : 0; }
+};
+
 static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                             const uint64_t *frame_offsets_host, int W, int H, int nframes, uint8_t *frames_host,
                             uint32_t *status_host, uint64_t *indices_host, bool scan_only, bool u16 = false,
-                            const int *roi = nullptr) {
+                            const SubFrame *sub = nullptr) {
     if (!c || !dims_ok(W, H, nframes) ||
         (nframes > 0 && (!stream_host || !frame_offsets_host || (!frames_host && !scan_only) || !status_host)))
         return fail(DBDE_B200_E_INVALID, "decode_host: bad argument");
@@ -924,8 +971,12 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
             return fail(DBDE_B200_E_INVALID, "decode_host: frame offsets must ascend within the stream");
     }
     const HostFmt F = host_fmt(W, H, u16);
-    const size_t px = roi ? (size_t)roi[2] * (size_t)roi[3] : F.px;    // output bytes per frame
-    const int chunk = default_chunk(c, W, H, nframes, u16);
+    const size_t px = sub ? sub->bytes() : F.px;    // output bytes per frame
+    int chunk = default_chunk(c, W, H, nframes, u16);
+    if (px > F.px) {                                 // crops larger than the frame: a chunk's output stays within 64 MiB
+        const size_t most = (64u << 20) / px;
+        if ((size_t)chunk > most) chunk = most > 0 ? (int)most : 1;
+    }
     const size_t delta = F.delta;
     const int nchunks = (nframes + chunk - 1) / chunk;
     size_t need_a = 0;
@@ -945,10 +996,18 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
     const int ns = nchunks < c->nslots ? nchunks : c->nslots;
     // pageable caller memory is relayed through pinned bounce buffers (see CopyPool)
     const bool in_pageable = is_pageable(stream_host), out_pageable = !scan_only && is_pageable(frames_host);
+    const size_t need_corners = sub ? sub->corner_bytes(chunk) : 0;
     for (int i = 0; i < ns; i++) {
-        int rc = ensure_slot(c, c->slots[i], need_a, need_b, 0, chunk);
-        if (!rc) rc = ensure_bounce(c, c->slots[i], in_pageable ? need_a : 0, out_pageable ? px * chunk : 0);
+        HostSlot &s = c->slots[i];
+        int rc = ensure_slot(c, s, need_a, need_b, need_corners, chunk);
+        if (!rc) rc = ensure_bounce(c, s, in_pageable ? need_a : 0, out_pageable ? px * chunk : 0);
         if (rc) return rc;
+        if (s.cap_hcorners < need_corners) {
+            if (s.h_corners) CK(cudaFreeHost(s.h_corners));
+            s.h_corners = nullptr;
+            CK(cudaHostAlloc(&s.h_corners, need_corners, cudaHostAllocDefault));
+            s.cap_hcorners = need_corners;
+        }
     }
     // finish(): wait for a chunk's status words, then queue the D2H of its accepted frames.  A
     // rejected frame must leave the caller's image untouched (dbde_util.cpp:296-303), so pixels
@@ -1003,10 +1062,20 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
         } else {
             CK(cudaMemcpyAsync(s.d_a + delta, stream_host + b0, b1 - b0, cudaMemcpyHostToDevice, s.st));
         }
+        if (sub && sub->corners) {
+            // this chunk's corners (the staging is free: the slot's stream has drained)
+            const size_t nb = sub->corner_bytes(s.n);
+            memcpy(s.h_corners, sub->corners + (sub->per_frame ? 2 * (size_t)sub->ncrops * (size_t)s.first : 0), nb);
+            CK(cudaMemcpyAsync(s.d_c, s.h_corners, nb, cudaMemcpyHostToDevice, s.st));
+        }
         prof.mark(1, "h2d");
         rc_all = u16   ? dbde_b200_decode16_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (uint16_t *)s.d_b, s.d_status,
                                                    s.d_index, s.st)
-                 : roi ? dbde_b200_decode_roi_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, roi[0], roi[1], roi[2], roi[3],
+                 : sub && sub->corners
+                       ? dbde_b200_decode_crops_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (const int32_t *)s.d_c,
+                                                       sub->ncrops, sub->per_frame, sub->w, sub->h, sub->pad, s.d_b, s.d_status,
+                                                       s.d_index, s.st)
+                 : sub ? dbde_b200_decode_roi_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, sub->x0, sub->y0, sub->w, sub->h,
                                                      s.d_b, s.d_status, s.d_index, s.st)
                        : decode_device_impl(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, s.d_b, s.d_status, s.d_index, s.st,
                                             scan_only);
@@ -1047,9 +1116,24 @@ extern "C" int dbde_b200_decode_roi_host(dbde_b200_ctx *c, const uint8_t *stream
     if (!c || !dims_ok(W, H, nframes) || !roi_ok(W, H, x0, y0, roi_w, roi_h) ||
         (nframes > 0 && (!stream_host || !frame_offsets_host || !roi_host || !status_host)))
         return fail(DBDE_B200_E_INVALID, "decode_roi_host: bad argument");
-    const int roi[4] = {x0, y0, roi_w, roi_h};
+    const SubFrame roi = {x0, y0, roi_w, roi_h, nullptr, 1, 0, 0};
     return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, roi_host, status_host,
-                            indices_host, false, false, roi);
+                            indices_host, false, false, &roi);
+}
+
+// The host form of dbde_b200_decode_crops_device: the same chunk pipeline with ncrops * crop_w * crop_h bytes per
+// frame coming back; each chunk's corners go up on its slot's stream.
+extern "C" int dbde_b200_decode_crops_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
+                                           const uint64_t *frame_offsets_host, int W, int H, int nframes,
+                                           const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
+                                           int crop_h, int pad, uint8_t *crops_host, uint32_t *status_host,
+                                           uint64_t *indices_host) {
+    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
+        (nframes > 0 && (!stream_host || !frame_offsets_host || !corners_host || !crops_host || !status_host)))
+        return fail(DBDE_B200_E_INVALID, "decode_crops_host: bad argument");
+    const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad};
+    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, crops_host, status_host,
+                            indices_host, false, false, &crops);
 }
 
 // dbde_b200_validate_device for a stream in host memory: the records cross PCIe once, nothing comes

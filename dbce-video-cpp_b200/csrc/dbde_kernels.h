@@ -90,5 +90,11 @@ cudaError_t launch_decode(const DecParams &P, bool fast, int num_sms, cudaStream
 // `out` (nframes * roi_w * roi_h bytes, tightly packed, any alignment), after launch_decode_scan(scan) with
 // scan.g = linear_geom(W, H) (word prefixes per 32 consecutive tiles).  Frames the scan rejected stay untouched.
 cudaError_t launch_decode_roi(const DecParams &scan, int x0, int y0, int roi_w, int roi_h, uint8_t *out, cudaStream_t stream);
+// Crop decode (dbde_roi.cu, the same kernel body): ncrops rectangles of crop_w x crop_h per frame with top-left
+// corners {x0, y0} at corners (device; per_frame: nframes * ncrops pairs, else ncrops pairs for every frame), any
+// int32 values; pixels outside the frame are `pad`.  Crop r of frame f goes to out + (f * ncrops + r) * crop_w * crop_h.
+// Same scan as launch_decode_roi; frames the scan rejected stay untouched.
+cudaError_t launch_decode_crops(const DecParams &scan, const int32_t *corners, int ncrops, bool per_frame, int crop_w, int crop_h,
+                                int pad, uint8_t *out, cudaStream_t stream);
 
 }  // namespace dbde

@@ -191,6 +191,36 @@ DBDE_B200_API int dbde_b200_decode_roi_host(dbde_b200_ctx *ctx, const uint8_t *s
                                             int x0, int y0, int roi_w, int roi_h, uint8_t *roi_host,
                                             uint32_t *status_host, uint64_t *indices_host);
 
+/* ---- crops: N fixed-size windows of every frame, anywhere, padded outside the frame ---------------------------
+ * Many rectangles of crop_w x crop_h per frame in one call -- the wells of a plate, a window that follows an animal
+ * from frame to frame, animal-centred windows that run past the frame's edge -- without decoding the rest of the
+ * frame.  corners: {x0, y0} int32 pairs, the top-left corner of each crop; any values, including negative ones and
+ * ones past the frame.  corners_per_frame = 0: ncrops pairs used for every frame; 1: nframes * ncrops pairs, frame
+ * f's crops at corners + 2 * f * ncrops.  Crop r of frame f goes to crops + ((size_t)f * ncrops + r) * crop_w *
+ * crop_h: crop_h rows of crop_w bytes, tightly packed, any alignment.  Pixel (x, y) of a crop is
+ * image[y0 + y][x0 + x] of the full decode where that lies inside the frame, and `pad` elsewhere; a crop entirely
+ * outside the frame is all `pad` and reads nothing of the record.  Validation covers the WHOLE record: status and
+ * indices are exactly what dbde_b200_decode_device reports for the same records, a record damaged outside every
+ * crop is rejected too, and all crops of a rejected frame are left untouched.  Nothing outside
+ * [crops, crops + nframes * ncrops * crop_w * crop_h) is written.  Follows the context's DBDE_INVERT_ENDIAN setting
+ * (a tile row is byte-reversed before the columns past W are set to `pad`; pad bytes are never reversed).
+ * DBDE_B200_E_INVALID before any work is queued for: NULL pointers (when nframes > 0), ncrops < 1, crop_w or
+ * crop_h < 1, a crop size the frame limits reject, ncrops * crop_w * crop_h > 2^31 - 1, corners_per_frame not 0 or
+ * 1, pad outside 0..255.  nframes == 0 returns 0.
+ * _device: corners in device memory (a tracker on the GPU can feed its positions straight in), asynchronous on
+ * `stream`.  _host: host memory, the chunk pipeline of dbde_b200_decode_host (records still cross PCIe whole, only
+ * the accepted frames' crops come back; a chunk's corners go up with it). */
+DBDE_B200_API int dbde_b200_decode_crops_device(dbde_b200_ctx *ctx, const uint8_t *stream_dev, size_t stream_bytes,
+                                                const uint64_t *frame_offsets_dev, int W, int H, int nframes,
+                                                const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
+                                                int crop_h, int pad, uint8_t *crops_dev, uint32_t *status_dev,
+                                                uint64_t *indices_dev, void *stream);
+DBDE_B200_API int dbde_b200_decode_crops_host(dbde_b200_ctx *ctx, const uint8_t *stream_host, size_t stream_bytes,
+                                              const uint64_t *frame_offsets_host, int W, int H, int nframes,
+                                              const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
+                                              int crop_h, int pad, uint8_t *crops_host, uint32_t *status_host,
+                                              uint64_t *indices_host);
+
 /* ---- DBDE16: 16-bit frames (SURVEY.md 8 f-4) -------------------------------------------------------
  * The extension the format note hints at (reference README.md:65, "could expand size to handle higher
  * bit depth images").  NOT in the reference code: the layout is defined here and restated by the test oracle
