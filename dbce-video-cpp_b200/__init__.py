@@ -39,6 +39,7 @@ C_SYMBOLS = [
     "dbde_b200_reader_open", "dbde_b200_reader_next", "dbde_b200_reader_close", "dbde_b200_file_last_error",
     "dbde_b200_decode_roi_device", "dbde_b200_decode_roi_host", "dbde_b200_reader_set_roi",
     "dbde_b200_decode_crops_device", "dbde_b200_decode_crops_host",
+    "dbde_b200_decode_binned_device", "dbde_b200_decode_binned_host",
 ]
 # the reference's C++ entry points (include/dbde_util.h), by mangled name (SURVEY.md 8b)
 CXX_SYMBOLS = {
@@ -145,6 +146,10 @@ def load():
     lib.dbde_b200_decode_crops_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                                 C.c_void_p]
+    lib.dbde_b200_decode_binned_device.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                   C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.dbde_b200_decode_binned_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                 C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.dbde_b200_file_last_error.restype = C.c_char_p
     return lib
 
@@ -261,6 +266,13 @@ class Codec:
                                                         int(per_frame), cw, ch, pad, out_ptr, status_ptr, index_ptr, stream),
                  "decode_crops_device")
 
+    def decode_binned_device(self, stream_ptr, stream_bytes, offs_ptr, W, H, n, factor, out_ptr, status_ptr, index_ptr=None,
+                             stream=0):
+        """every frame binned by factor (1, 2, 4 or 8): the rounded means of its in-frame factor x factor blocks -> out_ptr,
+        n * ceil(H / factor) * ceil(W / factor) bytes tightly packed"""
+        self._ck(self.lib.dbde_b200_decode_binned_device(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, n, int(factor), out_ptr,
+                                                         status_ptr, index_ptr, stream), "decode_binned_device")
+
     # ---- host-buffer hot path (numpy or raw host pointers)
     def encode_host(self, frames, first_index=0):
         """frames (N,H,W) u8 -> (stream bytes, offsets[N+1])"""
@@ -330,6 +342,22 @@ class Codec:
                                                       corners.ctypes.data, R, per_frame, cw, ch, pad, crops.ctypes.data,
                                                       status.ctypes.data, index.ctypes.data), "decode_crops_host")
         return crops, status, index
+
+    def decode_binned_host(self, stream, offsets, W, H, factor, fill=None):
+        """every frame binned by factor (1, 2, 4 or 8) -> (frames (N, ceil(H / factor), ceil(W / factor)), status[N],
+        indices[N]); rejected frames keep `fill`"""
+        stream = np.ascontiguousarray(stream, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        factor = int(factor)
+        N = len(offsets)
+        shape = (N, -(-H // factor), -(-W // factor)) if factor > 0 else (N, 0, 0)
+        frames = np.zeros(shape, dtype=np.uint8) if fill is None else np.full(shape, fill, dtype=np.uint8)
+        status = np.zeros(N, dtype=np.uint32)
+        index = np.zeros(N, dtype=np.uint64)
+        self._ck(self.lib.dbde_b200_decode_binned_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
+                                                       factor, frames.ctypes.data, status.ctypes.data, index.ctypes.data),
+                 "decode_binned_host")
+        return frames, status, index
 
     def decode_host_raw(self, stream_ptr, stream_bytes, offs_ptr, W, H, N, frames_ptr, status_ptr, index_ptr=None):
         self._ck(self.lib.dbde_b200_decode_host(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, N, frames_ptr,

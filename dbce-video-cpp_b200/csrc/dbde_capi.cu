@@ -561,6 +561,32 @@ extern "C" int dbde_b200_decode_crops_device(dbde_b200_ctx *c, const uint8_t *st
     return 0;
 }
 
+// ------------------------------------------------------------------ binned
+static bool factor_ok(int factor) { return factor == 1 || factor == 2 || factor == 4 || factor == 8; }
+
+// The scan on linear partitions, then the full decoder's pipeline with each tile reduced to its block means in
+// registers (dbde_decode.cu).  Factor 1 is the full decode.
+extern "C" int dbde_b200_decode_binned_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
+                                              const uint64_t *frame_offsets_dev, int W, int H, int nframes, int factor,
+                                              uint8_t *out_dev, uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
+    if (!c || !dims_ok(W, H, nframes) || !factor_ok(factor) ||
+        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !out_dev || !status_dev)))
+        return fail(DBDE_B200_E_INVALID, "decode_binned_device: bad argument");
+    if (nframes == 0) return 0;
+    if (factor == 1)
+        return decode_device_impl(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, out_dev, status_dev,
+                                  indices_dev, stream, false);
+    if ((unsigned long long)nframes * linear_geom(W, H).ppf >= 0xFFFFFFF0ull)
+        return fail(DBDE_B200_E_INVALID, "decode_binned_device: batch too large");
+    DecParams D;
+    int rc = linear_scan(c, (cudaStream_t)stream, W, H, stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev,
+                         indices_dev, &D);
+    if (rc) return rc;
+    CK(launch_decode_binned(D, factor, out_dev, c->num_sms, (cudaStream_t)stream));
+    c->launches += 1;
+    return 0;
+}
+
 // ------------------------------------------------------------------ pageable host memory
 // The reference's callers pass malloc'd buffers (dbde_util.h:24-35).  cudaMemcpyAsync on pageable memory
 // goes through the driver's own staging at ~15 GB/s and blocks the caller, and one host thread's memcpy is
@@ -946,12 +972,14 @@ extern "C" int dbde_b200_encode_host(dbde_b200_ctx *c, const uint8_t *frames_hos
     return 0;
 }
 
-// What the host pipeline hands back per frame instead of the whole image: the region (x0, y0, w, h), or ncrops crops
-// of w x h with host corners (per_frame: nframes * ncrops {x0, y0} pairs, else ncrops pairs for every frame)
+// What the host pipeline hands back per frame instead of the whole image: the region (x0, y0, w, h), ncrops crops
+// of w x h with host corners (per_frame: nframes * ncrops {x0, y0} pairs, else ncrops pairs for every frame), or the
+// frame binned by `factor` (w x h = ceil(W / factor) x ceil(H / factor))
 struct SubFrame {
     int x0, y0, w, h;
-    const int32_t *corners;     // null: the region
+    const int32_t *corners;     // null: the region or the binned frame
     int ncrops, per_frame, pad;
+    int factor;                 // > 0: the binned frame
     size_t bytes() const { return (size_t)w * (size_t)h * (size_t)(corners ? ncrops : 1); }
     size_t corner_bytes(int n) const { return corners ? 8 * (size_t)ncrops * (size_t)(per_frame ? n : 1) : 0; }
 };
@@ -1075,6 +1103,9 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
                        ? dbde_b200_decode_crops_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (const int32_t *)s.d_c,
                                                        sub->ncrops, sub->per_frame, sub->w, sub->h, sub->pad, s.d_b, s.d_status,
                                                        s.d_index, s.st)
+                 : sub && sub->factor
+                       ? dbde_b200_decode_binned_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, sub->factor, s.d_b, s.d_status,
+                                                        s.d_index, s.st)
                  : sub ? dbde_b200_decode_roi_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, sub->x0, sub->y0, sub->w, sub->h,
                                                      s.d_b, s.d_status, s.d_index, s.st)
                        : decode_device_impl(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, s.d_b, s.d_status, s.d_index, s.st,
@@ -1116,7 +1147,7 @@ extern "C" int dbde_b200_decode_roi_host(dbde_b200_ctx *c, const uint8_t *stream
     if (!c || !dims_ok(W, H, nframes) || !roi_ok(W, H, x0, y0, roi_w, roi_h) ||
         (nframes > 0 && (!stream_host || !frame_offsets_host || !roi_host || !status_host)))
         return fail(DBDE_B200_E_INVALID, "decode_roi_host: bad argument");
-    const SubFrame roi = {x0, y0, roi_w, roi_h, nullptr, 1, 0, 0};
+    const SubFrame roi = {x0, y0, roi_w, roi_h, nullptr, 1, 0, 0, 0};
     return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, roi_host, status_host,
                             indices_host, false, false, &roi);
 }
@@ -1131,9 +1162,22 @@ extern "C" int dbde_b200_decode_crops_host(dbde_b200_ctx *c, const uint8_t *stre
     if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
         (nframes > 0 && (!stream_host || !frame_offsets_host || !corners_host || !crops_host || !status_host)))
         return fail(DBDE_B200_E_INVALID, "decode_crops_host: bad argument");
-    const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad};
+    const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad, 0};
     return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, crops_host, status_host,
                             indices_host, false, false, &crops);
+}
+
+// The host form of dbde_b200_decode_binned_device: the same chunk pipeline with ceil(W / factor) * ceil(H / factor)
+// bytes per frame coming back.  Records still cross PCIe whole.
+extern "C" int dbde_b200_decode_binned_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
+                                            const uint64_t *frame_offsets_host, int W, int H, int nframes, int factor,
+                                            uint8_t *out_host, uint32_t *status_host, uint64_t *indices_host) {
+    if (!c || !dims_ok(W, H, nframes) || !factor_ok(factor) ||
+        (nframes > 0 && (!stream_host || !frame_offsets_host || !out_host || !status_host)))
+        return fail(DBDE_B200_E_INVALID, "decode_binned_host: bad argument");
+    const SubFrame binned = {0, 0, (W - 1) / factor + 1, (H - 1) / factor + 1, nullptr, 1, 0, 0, factor};
+    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, out_host, status_host,
+                            indices_host, false, false, &binned);
 }
 
 // dbde_b200_validate_device for a stream in host memory: the records cross PCIe once, nothing comes

@@ -20,6 +20,8 @@
 //   dbde_decode_staged_kernel<WM> : odd frames whose partitions span the full width (W <= 2048): the
 //                               partition's pixels are built in shared memory as they lie in the frame
 //                               (compile-time row shapes) and leave with one bulk-TMA store.
+//   dbde_decode_binned_kernel<B> : any frame on linear partitions, each tile reduced in registers to the
+//                               rounded means of its B x B blocks (B = 2, 4, 8) before it is stored.
 #include "dbde_device.cuh"
 #include "dbde_kernels.h"
 #include <stdlib.h>
@@ -582,6 +584,160 @@ __global__ void __launch_bounds__(kDecThreads, MODE == -1 ? 3 : 4) dbde_decode_k
     }
 }
 
+// ------------------------------------------------------------------ binned decode (B x B block means)
+// Bin sums of a tile whose px[i] hold the 16-bit sums of their two byte pairs (px[2r] = [c0+c1, c2+c3] of row r,
+// px[2r+1] = [c4+c5, c6+c7]).  Bin row j of the tile's 8 / B; the sums come back as 16-bit halves:
+//   B = 2: s0 = [bin 0, bin 1], s1 = [bin 2, bin 3];  B = 4: s0 = [bin 0, bin 1];  B = 8: s0 = bin 0.
+// The largest, an 8x8 sum, is 64 * 255 = 16320: no half ever carries into the next.
+template <int B>
+__device__ __forceinline__ void bin_row_sums(const uint32_t (&px)[16], int j, uint32_t &s0, uint32_t &s1) {
+    s1 = 0;
+    if constexpr (B == 2) {
+        s0 = px[4 * j] + px[4 * j + 2];
+        s1 = px[4 * j + 1] + px[4 * j + 3];
+    } else if constexpr (B == 4) {
+        const uint32_t a0 = px[8 * j] + px[8 * j + 2] + px[8 * j + 4] + px[8 * j + 6];
+        const uint32_t a1 = px[8 * j + 1] + px[8 * j + 3] + px[8 * j + 5] + px[8 * j + 7];
+        s0 = __byte_perm(a0, a1, 0x5410) + __byte_perm(a0, a1, 0x7632);
+    } else {
+        uint32_t a = 0;
+#pragma unroll
+        for (int i = 0; i < 16; i++) a += px[i];
+        s0 = (a & 0xffffu) + (a >> 16);
+    }
+}
+
+// n <= 4 bytes of v to p, any alignment, as naturally aligned pieces
+__device__ __forceinline__ void store_bytes(uint8_t *p, uint32_t v, uint32_t n) {
+    const uint32_t a = (uint32_t)(uintptr_t)p & 7u;
+    uint8_t *q = p - a;
+    if (a + n <= 8u) {
+        store_partial(q, (uint64_t)v << (8 * a), a, a + n);
+    } else {
+        store_partial(q, (uint64_t)v << (8 * a), a, 8u);
+        store_partial(q + 8, v >> (8 * (8 - a)), 0u, a + n - 8u);
+    }
+}
+
+// The full decoder's pipeline (dec_producer, dec_unpack_tile) on linear partitions, with each lane's 64 pixels
+// reduced in registers to the (8 / B)^2 rounded means of its B x B bins before anything is stored: a lane writes
+// 8 / B pieces of 8 / B bytes, one per bin row, and the 4 MiB full-size frame never exists.  Interior tiles divide by
+// shifting; the frame's last tile column / row (W % 8 or H % 8 != 0) first zeroes the encoder's clamp padding past
+// W and H -- it must not enter the mean -- and divides each bin by its count of in-frame pixels.
+template <int B>
+__global__ void __launch_bounds__(kDecThreads, 4) dbde_decode_binned_kernel(const DecParams P) {
+    constexpr int NB = 8 / B;                 // bins per tile side
+    extern __shared__ __align__(128) uint8_t smem_raw[];
+    DecSmem &S = *reinterpret_cast<DecSmem *>(smem_raw);
+    uint8_t *stages = smem_raw + ((sizeof(DecSmem) + 127) & ~127);
+    const PartGeom &g = P.g;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int Wb = (g.W + B - 1) / B, Hb = (g.H + B - 1) / B;
+    const size_t fbytes = (size_t)Wb * (size_t)Hb;
+
+    if (tid == 0) {
+        for (int s = 0; s < kDecStages; s++) {
+            mbar_init(&S.full[s], 1);
+            mbar_init(&S.empty[s], kConsumerWarps);
+        }
+        mbar_fence_init();
+    }
+    __syncthreads();
+
+    if (warp == kConsumerWarps) {
+        dec_producer<kDecStages, kDecInflightBytes>(P, S, stages, lane);
+        return;
+    }
+    // my tile is tile tid after the partition's first one: lin_dy bands down, lin_dx columns right, wrapping once
+    // more if that passes the last column
+    const int lin_dy = tid / g.w, lin_dx = tid - lin_dy * g.w;
+    for (unsigned it = 0;; it++) {
+        const int s = it % kDecStages;
+        const uint32_t ph = (it / kDecStages) & 1;
+        mbar_wait(&S.full[s], ph);
+        const int4 c0 = *reinterpret_cast<const int4 *>(&S.ctl[s].part);      // part, flags, f, nt
+        if (c0.x < 0) break;
+        if (c0.y & kCtlSkip) {
+            __syncwarp();
+            if (lane == 0) mbar_arrive(&S.empty[s]);
+            continue;
+        }
+        const uint4 c1 = *reinterpret_cast<const uint4 *>(&S.ctl[s].pres);    // pres, kres, mres, pixoff
+        const int2 c2 = *reinterpret_cast<const int2 *>(&S.ctl[s].y0);        // first tile's band and column
+        const uint8_t *stage = stages + (size_t)s * kDecStageBytes;
+        const bool valid = tid < c0.w;
+        uint32_t px[16];
+        dec_unpack_tile(stage, c1, S.ctl[s].wbase[warp], tid, lane, valid, (P.flags & kFlagInvertRows) != 0, px);
+        fence_proxy_async();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&S.empty[s]);       // payload is in registers: free the stage early
+        if (!valid) continue;
+
+        int ty = c2.x + lin_dy, tx = c2.y + lin_dx;
+        if (tx >= g.w) {
+            tx -= g.w;
+            ty++;
+        }
+        const int wc = g.W - 8 * tx, hr = g.H - 8 * ty;                    // in-frame columns / rows of the tile, if < 8
+        const bool edge = wc < 8 || hr < 8;
+        if (edge) {
+            // the clamp padding past W and H (after the invert-endian row reversal) leaves the sums
+            const uint32_t mlo = wc >= 4 ? ~0u : (1u << (8 * wc)) - 1u;
+            const uint32_t mhi = wc >= 8 ? ~0u : wc > 4 ? (1u << (8 * (wc - 4))) - 1u : 0u;
+#pragma unroll
+            for (int r = 0; r < 8; r++) {
+                px[2 * r] = r < hr ? px[2 * r] & mlo : 0u;
+                px[2 * r + 1] = r < hr ? px[2 * r + 1] & mhi : 0u;
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < 16; i++) px[i] = (px[i] & 0x00ff00ffu) + ((px[i] >> 8) & 0x00ff00ffu);
+
+        uint8_t *op = P.frames + (size_t)c0.z * fbytes + (size_t)(NB * ty) * (size_t)Wb + (size_t)(NB * tx);
+        if (!edge) {
+#pragma unroll
+            for (int j = 0; j < NB; j++) {
+                uint32_t s0, s1;
+                bin_row_sums<B>(px, j, s0, s1);
+                if constexpr (B == 2) {
+                    const uint32_t m0 = ((s0 + 0x00020002u) >> 2) & 0x00ff00ffu, m1 = ((s1 + 0x00020002u) >> 2) & 0x00ff00ffu;
+                    const uint32_t v = __byte_perm(m0, m1, 0x6420);
+                    if (((uintptr_t)op & 3u) == 0) st_stream_u32(op, v);
+                    else store_bytes(op, v, 4u);
+                } else if constexpr (B == 4) {
+                    const uint32_t m = ((s0 + 0x00080008u) >> 4) & 0x00ff00ffu;
+                    const uint32_t v = __byte_perm(m, 0u, 0x4420);
+                    if (((uintptr_t)op & 1u) == 0) *reinterpret_cast<uint16_t *>(op) = (uint16_t)v;
+                    else store_bytes(op, v, 2u);
+                } else {
+                    *op = (uint8_t)((s0 + 32u) >> 6);
+                }
+                op += Wb;
+            }
+        } else {
+            // the frame's last tile column / row: bins past W / H are not in the output, the others divide their sum
+            // by their in-frame pixel count, rounded half up
+            const int ncb = min(NB, Wb - NB * tx), nrb = min(NB, Hb - NB * ty);
+#pragma unroll
+            for (int j = 0; j < NB; j++) {                 // unrolled: px is indexed with constants only
+                if (j < nrb) {
+                    uint32_t s0, s1;
+                    bin_row_sums<B>(px, j, s0, s1);
+                    const uint32_t rows = (uint32_t)min(B, hr - B * j);
+                    uint32_t v = 0;
+                    for (int i = 0; i < ncb; i++) {
+                        const uint32_t sum = B == 8 ? s0 : ((i < 2 ? s0 : s1) >> (16 * (i & 1))) & 0xffffu;
+                        const uint32_t n = rows * (uint32_t)min(B, wc - B * i);
+                        v |= ((sum + n / 2) / n) << (8 * i);
+                    }
+                    store_bytes(op, v, (uint32_t)ncb);
+                }
+                op += Wb;
+            }
+        }
+    }
+}
+
 // ------------------------------------------------------------------ staged-store kernel (odd sizes, W <= 2048)
 // Frames whose rows are not 8-byte aligned (W % 8 != 0), or that end in partial tiles, cannot use the
 // direct row stores: a warp's row would be cut into unaligned pieces.  But a full-width partition's
@@ -858,6 +1014,18 @@ cudaError_t launch_decode(const DecParams &P, bool fast, int num_sms, cudaStream
         case 5: return launch_persistent(dbde_decode_kernel<5>, P, kDecThreads, smem, num_sms, stream);
         case 6: return launch_persistent(dbde_decode_kernel<6>, P, kDecThreads, smem, num_sms, stream);
         default: return launch_persistent(dbde_decode_kernel<7>, P, kDecThreads, smem, num_sms, stream);
+    }
+}
+
+cudaError_t launch_decode_binned(const DecParams &scan, int factor, uint8_t *out, int num_sms, cudaStream_t stream) {
+    DecParams P = scan;
+    P.frames = out;
+    const size_t smem = dec_smem_bytes(P.g);
+    switch (factor) {
+        case 2: return launch_persistent(dbde_decode_binned_kernel<2>, P, kDecThreads, smem, num_sms, stream);
+        case 4: return launch_persistent(dbde_decode_binned_kernel<4>, P, kDecThreads, smem, num_sms, stream);
+        case 8: return launch_persistent(dbde_decode_binned_kernel<8>, P, kDecThreads, smem, num_sms, stream);
+        default: return cudaErrorInvalidValue;
     }
 }
 

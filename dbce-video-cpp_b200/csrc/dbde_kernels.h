@@ -96,5 +96,9 @@ cudaError_t launch_decode_roi(const DecParams &scan, int x0, int y0, int roi_w, 
 // Same scan as launch_decode_roi; frames the scan rejected stay untouched.
 cudaError_t launch_decode_crops(const DecParams &scan, const int32_t *corners, int ncrops, bool per_frame, int crop_w, int crop_h,
                                 int pad, uint8_t *out, cudaStream_t stream);
+// Binned decode (dbde_decode.cu): every frame reduced to the rounded means of its factor x factor blocks (factor 2, 4
+// or 8), ceil(H / factor) rows of ceil(W / factor) bytes per frame, tightly packed from `out`, any alignment.  Same
+// scan as launch_decode_roi; frames the scan rejected stay untouched.
+cudaError_t launch_decode_binned(const DecParams &scan, int factor, uint8_t *out, int num_sms, cudaStream_t stream);
 
 }  // namespace dbde

@@ -221,6 +221,27 @@ DBDE_B200_API int dbde_b200_decode_crops_host(dbde_b200_ctx *ctx, const uint8_t 
                                               int crop_h, int pad, uint8_t *crops_host, uint32_t *status_host,
                                               uint64_t *indices_host);
 
+/* ---- binned: every frame at 1/2, 1/4 or 1/8 of its size, as block means ---------------------------------------
+ * The whole field of view at lower resolution -- a tracker on a quarter-size image, previews, motion energy over a
+ * plate, a network that takes downsampled frames -- without writing the full-size frame anywhere.  factor must be
+ * 1, 2, 4 or 8; factor 1 is dbde_b200_decode_device.  Frame i's output is Hb = ceil(H / factor) rows of
+ * Wb = ceil(W / factor) bytes, tightly packed, at out + i * Wb * Hb; any alignment, and nothing outside
+ * [out, out + nframes * Wb * Hb) is written.  Output pixel (X, Y) is the mean of the IN-FRAME pixels of the full
+ * decode in [factor X, factor X + factor) x [factor Y, factor Y + factor), rounded half up: (sum + n / 2) / n in
+ * integers, n the number of in-frame pixels (factor^2 except in the last column when W % factor != 0 and the last row
+ * when H % factor != 0).  "The full decode" follows the context's DBDE_INVERT_ENDIAN setting.  Validation covers the
+ * WHOLE record: status and indices are exactly what dbde_b200_decode_device reports for the same records, and a
+ * rejected frame's output is left untouched.  DBDE_B200_E_INVALID before any work is queued for: NULL pointers (when
+ * nframes > 0), a factor other than 1, 2, 4 or 8, frame dimensions the frame limits reject.  nframes == 0 returns 0.
+ * _device: asynchronous on `stream`.  _host: the chunk pipeline of dbde_b200_decode_host (records still cross PCIe
+ * whole, only the accepted frames' binned pixels come back). */
+DBDE_B200_API int dbde_b200_decode_binned_device(dbde_b200_ctx *ctx, const uint8_t *stream_dev, size_t stream_bytes,
+                                                 const uint64_t *frame_offsets_dev, int W, int H, int nframes, int factor,
+                                                 uint8_t *out_dev, uint32_t *status_dev, uint64_t *indices_dev, void *stream);
+DBDE_B200_API int dbde_b200_decode_binned_host(dbde_b200_ctx *ctx, const uint8_t *stream_host, size_t stream_bytes,
+                                               const uint64_t *frame_offsets_host, int W, int H, int nframes, int factor,
+                                               uint8_t *out_host, uint32_t *status_host, uint64_t *indices_host);
+
 /* ---- DBDE16: 16-bit frames (SURVEY.md 8 f-4) -------------------------------------------------------
  * The extension the format note hints at (reference README.md:65, "could expand size to handle higher
  * bit depth images").  NOT in the reference code: the layout is defined here and restated by the test oracle
