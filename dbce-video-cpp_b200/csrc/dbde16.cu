@@ -233,13 +233,14 @@ __global__ void __launch_bounds__(256) dbde16_scan_kernel(const Dec16Params P) {
     const uint64_t fixed = 32 + 3 * (uint64_t)P.wh;
     const int ng = (P.wh + 31) / 32;
     uint32_t *wp = P.wprefix + (size_t)f * (ng + 1);
-    if (off + fixed > P.stream_bytes) {
+    if (off > P.stream_bytes || P.stream_bytes - off < fixed) {   // no wrap for any off
         if (tid == 0) {
             P.status[f] = kStTruncated;
             if (P.indices) P.indices[f] = 0;
         }
         return;
     }
+    const uint64_t room = P.stream_bytes - off - fixed;      // payload bytes the stream has after the fixed fields
     const uint8_t *rec = P.stream + off;
     auto le32 = [](const uint8_t *p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); };
     uint32_t status = 0;
@@ -299,7 +300,7 @@ __global__ void __launch_bounds__(256) dbde16_scan_kernel(const Dec16Params P) {
         wp[ng] = carry;
         if (carry != n64) status |= kStBadWordCount;
         if (s_flag) status |= kStDepthTooBig;
-        if (off + fixed + 8ull * carry > P.stream_bytes) status |= kStTruncated;
+        if (room < 8ull * carry) status |= kStTruncated;
         P.status[f] = status;
         if (P.indices) P.indices[f] = (uint64_t)le32(rec + 4) | ((uint64_t)le32(rec + 8) << 32);
     }

@@ -57,13 +57,14 @@ __global__ void __launch_bounds__(256) dbde_decode_scan_kernel(const DecParams P
     const uint64_t fixed = 32 + 2 * (uint64_t)g.wh;
     const int nitems = g.ppf * kConsumerWarps;
     uint32_t *wp = P.wprefix + (size_t)f * (nitems + 1);
-    if (off + fixed > P.stream_bytes) {          // cannot even read the fixed fields
+    if (off > P.stream_bytes || P.stream_bytes - off < fixed) {   // cannot even read the fixed fields (no wrap for any off)
         if (tid == 0) {
             P.status[f] = kStTruncated;
             if (P.indices) P.indices[f] = 0;
         }
         return;
     }
+    const uint64_t room = P.stream_bytes - off - fixed;      // payload bytes the stream has after the fixed fields
     const uint8_t *rec = P.stream + off;
     uint32_t status = 0;
     if (ldg_u32_bytes(rec) != 2u) status |= kStBadFrameHeader;
@@ -189,7 +190,7 @@ __global__ void __launch_bounds__(256) dbde_decode_scan_kernel(const DecParams P
         wp[nitems] = carry;
         if (carry != n64) status |= kStBadWordCount;
         if (s_flag) status |= kStDepthTooBig;
-        if (off + fixed + 8ull * carry > P.stream_bytes) status |= kStTruncated;
+        if (room < 8ull * carry) status |= kStTruncated;
         P.status[f] = status;
         if (P.indices) {
             uint64_t idx = (uint64_t)ldg_u32_bytes(rec + 4) | ((uint64_t)ldg_u32_bytes(rec + 8) << 32);
