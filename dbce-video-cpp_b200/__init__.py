@@ -40,6 +40,8 @@ C_SYMBOLS = [
     "dbde_b200_decode_roi_device", "dbde_b200_decode_roi_host", "dbde_b200_reader_set_roi",
     "dbde_b200_decode_crops_device", "dbde_b200_decode_crops_host",
     "dbde_b200_decode_binned_device", "dbde_b200_decode_binned_host",
+    "dbde_b200_decode16_crops_device", "dbde_b200_decode16_crops_host",
+    "dbde_b200_decode16_binned_device", "dbde_b200_decode16_binned_host",
 ]
 # the reference's C++ entry points (include/dbde_util.h), by mangled name (SURVEY.md 8b)
 CXX_SYMBOLS = {
@@ -150,6 +152,10 @@ def load():
                                                    C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.dbde_b200_decode_binned_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                  C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.dbde_b200_decode16_crops_device.argtypes = lib.dbde_b200_decode_crops_device.argtypes
+    lib.dbde_b200_decode16_crops_host.argtypes = lib.dbde_b200_decode_crops_host.argtypes
+    lib.dbde_b200_decode16_binned_device.argtypes = lib.dbde_b200_decode_binned_device.argtypes
+    lib.dbde_b200_decode16_binned_host.argtypes = lib.dbde_b200_decode_binned_host.argtypes
     lib.dbde_b200_file_last_error.restype = C.c_char_p
     return lib
 
@@ -385,6 +391,64 @@ class Codec:
         index = np.zeros(N, dtype=np.uint64)
         self._ck(self.lib.dbde_b200_decode16_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
                                                   frames.ctypes.data, status.ctypes.data, index.ctypes.data), "decode16_host")
+        return frames, status, index
+
+    def decode16_crops_device(self, stream_ptr, stream_bytes, offs_ptr, W, H, n, corners_ptr, ncrops, per_frame, size, out_ptr,
+                              status_ptr, index_ptr=None, pad=0, stream=0):
+        """DBDE16 records: ncrops crops of size = (crop_w, crop_h) per frame at the int32 {x0, y0} corners at corners_ptr
+        (device; per_frame: n * ncrops pairs, else ncrops pairs for every frame) -> out_ptr (2-byte aligned), n * ncrops *
+        crop_w * crop_h U16 tightly packed; pixels outside the frame are `pad` (0..65535)"""
+        cw, ch = (int(v) for v in size)
+        self._ck(self.lib.dbde_b200_decode16_crops_device(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, n, corners_ptr, ncrops,
+                                                          int(per_frame), cw, ch, pad, out_ptr, status_ptr, index_ptr, stream),
+                 "decode16_crops_device")
+
+    def decode16_binned_device(self, stream_ptr, stream_bytes, offs_ptr, W, H, n, factor, out_ptr, status_ptr, index_ptr=None,
+                               stream=0):
+        """DBDE16 records, every frame binned by factor (1, 2, 4 or 8): the rounded means of its in-frame factor x factor
+        blocks -> out_ptr (2-byte aligned), n * ceil(H / factor) * ceil(W / factor) U16 tightly packed"""
+        self._ck(self.lib.dbde_b200_decode16_binned_device(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, n, int(factor),
+                                                           out_ptr, status_ptr, index_ptr, stream), "decode16_binned_device")
+
+    def decode16_crops_host(self, stream, offsets, W, H, corners, size, pad=0, fill=None):
+        """DBDE16 records: crops of size = (crop_w, crop_h) at int32 corners (R, 2) (the same for every frame) or (N, R, 2)
+        (per frame) -> (crops (N, R, crop_h, crop_w) u16, status[N], indices[N]); pixels outside the frame are `pad`,
+        rejected frames keep `fill`"""
+        stream = np.ascontiguousarray(stream, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        corners = np.ascontiguousarray(corners, dtype=np.int32)
+        cw, ch = (int(v) for v in size)
+        N = len(offsets)
+        if corners.ndim == 3 and corners.shape[0] == N and corners.shape[2] == 2:
+            per_frame = 1
+        elif corners.ndim == 2 and corners.shape[1] == 2:
+            per_frame = 0
+        else:
+            raise ValueError("corners must have shape (R, 2) or (N, R, 2), got %r" % (corners.shape,))
+        R = corners.shape[-2]
+        shape = (N, R, max(ch, 0), max(cw, 0))
+        crops = np.zeros(shape, dtype=np.uint16) if fill is None else np.full(shape, fill, dtype=np.uint16)
+        status = np.zeros(N, dtype=np.uint32)
+        index = np.zeros(N, dtype=np.uint64)
+        self._ck(self.lib.dbde_b200_decode16_crops_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
+                                                        corners.ctypes.data, R, per_frame, cw, ch, pad, crops.ctypes.data,
+                                                        status.ctypes.data, index.ctypes.data), "decode16_crops_host")
+        return crops, status, index
+
+    def decode16_binned_host(self, stream, offsets, W, H, factor, fill=None):
+        """DBDE16 records, every frame binned by factor (1, 2, 4 or 8) -> (frames (N, ceil(H / factor), ceil(W / factor))
+        u16, status[N], indices[N]); rejected frames keep `fill`"""
+        stream = np.ascontiguousarray(stream, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        factor = int(factor)
+        N = len(offsets)
+        shape = (N, -(-H // factor), -(-W // factor)) if factor > 0 else (N, 0, 0)
+        frames = np.zeros(shape, dtype=np.uint16) if fill is None else np.full(shape, fill, dtype=np.uint16)
+        status = np.zeros(N, dtype=np.uint32)
+        index = np.zeros(N, dtype=np.uint64)
+        self._ck(self.lib.dbde_b200_decode16_binned_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
+                                                         factor, frames.ctypes.data, status.ctypes.data, index.ctypes.data),
+                 "decode16_binned_host")
         return frames, status, index
 
     def validate_host(self, stream, offsets, W, H):

@@ -10,6 +10,9 @@
 // consecutive tiles per CTA iteration, frame-interleaved tickets + the single-word decoupled look-back for
 // the word offsets, words staged in shared memory and copied out coalesced.  Pixels are read and written
 // with 16-byte accesses when rows allow it (W % 8 == 0, aligned base), element-wise with clamp/crop otherwise.
+// Sub-frame decodes run after the same scan and share the decoder's pair extraction (unpack_tile16):
+// dbde16_decode_crops_kernel unpacks only the tiles under each crop, dbde16_decode_binned_kernel<B> stores each tile's
+// B x B block means instead of its pixels.
 #include "dbde_device.cuh"
 #include "dbde_kernels.h"
 
@@ -307,6 +310,127 @@ __global__ void __launch_bounds__(256) dbde16_scan_kernel(const Dec16Params P) {
 }
 
 // ------------------------------------------------------------------ decoder: unpack
+// The pair extraction every DBDE16 decoder shares.  `su` is staged payload in the padded layout (pad16): after every
+// 32 units comes one padding unit holding a COPY of the unit that follows it, so "this unit and the next" is always
+// two adjacent loads.  The tile's k words start at word `woff` of the staging; px[4r + j] = pixels (2j, 2j+1) of tile
+// row r.  Depth 0 is the minimum everywhere.
+__device__ __forceinline__ void unpack_tile16(const uint32_t *su, uint32_t woff, int k, uint32_t mn, uint32_t (&px)[32]) {
+    const uint32_t m2 = mn * 0x00010001u;
+    if (k > 0) {
+        const uint32_t kk = 2u * (uint32_t)k, mk = (1u << k) - 1u;
+#pragma unroll
+        for (int i = 0; i < 32; i++) {
+            const uint32_t bit = kk * (uint32_t)i;                               // pair i: bits [2k i, 2k i + 2k)
+            const uint32_t at = pad16(2u * woff + (bit >> 5));
+            const uint32_t a = su[at], b = su[at + 1u];                          // the next unit, or its copy in the padding slot
+            const uint32_t v = __funnelshift_r(a, b, bit);                       // low 2k bits = the pair
+            px[i] = ((v & mk) | (((v >> k) & mk) << 16)) + m2;                    // + min, wrapping per pixel is impossible: <= 65535
+        }
+    } else {
+#pragma unroll
+        for (int i = 0; i < 32; i++) px[i] = m2;
+    }
+}
+
+// bytes [s, e) of the 64-bit word w at the 8-byte-aligned q: store_partial, which leaves the whole word to its
+// callers, or one 8-byte store
+__device__ __forceinline__ void store_word_part(uint8_t *q, uint64_t w, uint32_t s, uint32_t e) {
+    if (s == 0u && e == 8u) *reinterpret_cast<uint64_t *>(q) = w;
+    else store_partial(q, w, s, e);
+}
+
+// n <= 4 U16 values (v, lowest first) to p, any even address, as naturally aligned pieces
+__device__ __forceinline__ void store_u16s(uint16_t *p, uint64_t v, uint32_t n) {
+    const uint32_t a = (uint32_t)(uintptr_t)p & 7u, e = a + 2u * n;
+    uint8_t *q = reinterpret_cast<uint8_t *>(p) - a;
+    if (e <= 8u) {
+        store_word_part(q, v << (8 * a), a, e);
+    } else {                                                  // a > 0 here
+        store_partial(q, v << (8 * a), a, 8u);
+        store_partial(q + 8, v >> (64 - 8 * a), 0u, e - 8u);
+    }
+}
+
+// Binned epilogue: one tile's pixels -> the rounded means of its (8 / B)^2 bins of B x B, one piece of 8 / B values
+// per bin row at `op` (frame row pitch Wb).  wc / hr: the tile's in-frame columns / rows.  A tile in the frame's last
+// tile column / row (W % 8 or H % 8 != 0) first zeroes the encoder's clamp padding past W and H -- it must not enter
+// the mean -- divides each bin by its count of in-frame pixels and skips the bins past ceil(W / B) and ceil(H / B).
+// Sums are 32-bit: an 8 x 8 bin sums to at most 64 * 65535.
+template <int B>
+__device__ __forceinline__ void store_bins16(uint16_t *op, int Wb, int ncb, int nrb, int wc, int hr, uint32_t (&px)[32]) {
+    constexpr int NB = 8 / B;                                 // bins per tile side
+    const bool edge = wc < 8 || hr < 8;
+    if (edge) {
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const uint32_t m = 2 * j + 2 <= wc ? ~0u : 2 * j + 1 == wc ? 0xffffu : 0u;
+#pragma unroll
+            for (int r = 0; r < 8; r++) px[4 * r + j] = r < hr ? px[4 * r + j] & m : 0u;
+        }
+    }
+#pragma unroll
+    for (int by = 0; by < NB; by++) {
+        uint64_t v = 0;
+#pragma unroll
+        for (int bx = 0; bx < NB; bx++) {
+            uint32_t s = 0;
+#pragma unroll
+            for (int r = B * by; r < B * by + B; r++)
+#pragma unroll
+                for (int j = B * bx / 2; j < (B * bx + B) / 2; j++) s += (px[4 * r + j] & 0xffffu) + (px[4 * r + j] >> 16);
+            uint32_t m;
+            if (!edge) {
+                m = (s + B * B / 2) >> (B == 2 ? 2 : B == 4 ? 4 : 6);
+            } else {
+                const uint32_t n = (uint32_t)max(1, min(B, hr - B * by)) * (uint32_t)max(1, min(B, wc - B * bx));
+                m = (s + n / 2) / n;
+            }
+            v |= (uint64_t)m << (16 * bx);
+        }
+        if (!edge) {
+            if constexpr (B == 2) {
+                if (((uintptr_t)op & 7u) == 0) st_stream_u64(op, v);
+                else store_u16s(op, v, 4u);
+            } else if constexpr (B == 4) {
+                if (((uintptr_t)op & 3u) == 0) st_stream_u32(op, (uint32_t)v);
+                else store_u16s(op, v, 2u);
+            } else {
+                *op = (uint16_t)v;
+            }
+        } else if (by < nrb) {
+            store_u16s(op, v, (uint32_t)ncb);
+        }
+        op += Wb;
+    }
+}
+
+// A partition's agg words at src (any alignment), coalesced over the CTA's threads, into the padded layout of
+// unpack_tile16 at s_words.  Padded layout (pad16): after every 32 units comes one padding unit, and that padding
+// unit holds a COPY of the unit that follows it, so the reader's "this unit and the next" is always two adjacent loads.
+__device__ __forceinline__ void stage_words16(uint8_t *s_words, const uint8_t *src, uint32_t agg, int tid) {
+    uint32_t *su = reinterpret_cast<uint32_t *>(s_words);
+    if (((uintptr_t)src & 7) == 0) {
+        for (uint32_t i = (uint32_t)tid; i < agg; i += kT16) {
+            const uint64_t v = __ldcs(reinterpret_cast<const uint64_t *>(src) + i);
+            const uint32_t at = pad16(2u * i);                                  // units 2i and 2i+1 share a block of 32
+            su[at] = (uint32_t)v;
+            su[at + 1u] = (uint32_t)(v >> 32);
+            if (((2u * i) & 31u) == 0u && i > 0u) su[at - 1u] = (uint32_t)v;    // the copy in the padding slot before it
+        }
+    } else {
+        for (uint32_t i = (uint32_t)tid; i < 8u * agg; i += kT16) {
+            const uint32_t u = i >> 2;
+            s_words[4u * pad16(u) + (i & 3u)] = src[i];
+            if ((u & 31u) == 0u && u > 0u) s_words[4u * (pad16(u) - 1u) + (i & 3u)] = src[i];
+        }
+    }
+    if (tid < 2) {                                                            // the reader looks one unit past the end
+        const uint32_t u = 2u * agg + (uint32_t)tid;
+        su[pad16(u)] = 0u;
+        if ((u & 31u) == 0u && u > 0u) su[pad16(u) - 1u] = 0u;
+    }
+}
+
 __global__ void __launch_bounds__(kT16) dbde16_decode_kernel(const Dec16Params P) {
     extern __shared__ __align__(16) uint8_t s_words[];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -321,29 +445,7 @@ __global__ void __launch_bounds__(kT16) dbde16_decode_kernel(const Dec16Params P
         const uint32_t w0 = wp[g0], agg = wp[g1] - w0;
         // the partition's words, coalesced, into shared memory
         const uint8_t *src = rec + 32 + 3 * (size_t)P.wh + 8ull * w0;
-        // Padded layout (pad16): after every 32 units comes one padding unit, and that padding unit holds a
-        // COPY of the unit that follows it, so the reader's "this unit and the next" is always two adjacent loads.
-        uint32_t *su = reinterpret_cast<uint32_t *>(s_words);
-        if (((uintptr_t)src & 7) == 0) {
-            for (uint32_t i = (uint32_t)tid; i < agg; i += kT16) {
-                const uint64_t v = __ldcs(reinterpret_cast<const uint64_t *>(src) + i);
-                const uint32_t at = pad16(2u * i);                                  // units 2i and 2i+1 share a block of 32
-                su[at] = (uint32_t)v;
-                su[at + 1u] = (uint32_t)(v >> 32);
-                if (((2u * i) & 31u) == 0u && i > 0u) su[at - 1u] = (uint32_t)v;    // the copy in the padding slot before it
-            }
-        } else {
-            for (uint32_t i = (uint32_t)tid; i < 8u * agg; i += kT16) {
-                const uint32_t u = i >> 2;
-                s_words[4u * pad16(u) + (i & 3u)] = src[i];
-                if ((u & 31u) == 0u && u > 0u) s_words[4u * (pad16(u) - 1u) + (i & 3u)] = src[i];
-            }
-        }
-        if (tid < 2) {                                                            // the reader looks one unit past the end
-            const uint32_t u = 2u * agg + (uint32_t)tid;
-            su[pad16(u)] = 0u;
-            if ((u & 31u) == 0u && u > 0u) su[pad16(u) - 1u] = 0u;
-        }
+        stage_words16(s_words, src, agg, tid);
         const int tile = (int)q * kT16 + tid;
         const bool valid = tile < P.wh;
         int k = 0;
@@ -357,27 +459,242 @@ __global__ void __launch_bounds__(kT16) dbde16_decode_kernel(const Dec16Params P
         const uint32_t woff = (g0 + warp < ng ? wp[g0 + warp] - w0 : 0u) + incl - (uint32_t)k;
         __syncthreads();
         uint32_t px[32];
-        const uint32_t m2 = mn * 0x00010001u;
-        if (k > 0) {
-            const uint32_t kk = 2u * (uint32_t)k, mk = (1u << k) - 1u;
-            const uint32_t *su = reinterpret_cast<const uint32_t *>(s_words);
-#pragma unroll
-            for (int i = 0; i < 32; i++) {
-                const uint32_t bit = kk * (uint32_t)i;                               // pair i: bits [2k i, 2k i + 2k)
-                const uint32_t at = pad16(2u * woff + (bit >> 5));
-                const uint32_t a = su[at], b = su[at + 1u];                          // the next unit, or its copy in the padding slot
-                const uint32_t v = __funnelshift_r(a, b, bit);                       // low 2k bits = the pair
-                px[i] = ((v & mk) | (((v >> k) & mk) << 16)) + m2;                    // + min, wrapping per pixel is impossible: <= 65535
-            }
-        } else {
-#pragma unroll
-            for (int i = 0; i < 32; i++) px[i] = m2;
-        }
+        unpack_tile16(reinterpret_cast<const uint32_t *>(s_words), woff, k, mn, px);
         if (valid) {
             const int ty = tile / P.w, tx = tile - ty * P.w;
             store_tile16(P.frames + (size_t)f * fpix, P.W, P.H, ty, tx, P.aligned != 0, px);
         }
         __syncthreads();                                      // s_words is reused by the next partition
+    }
+}
+
+// Binned decode: dbde16_decode_kernel's partition loop with the bin epilogue (store_bins16) in place of the tile
+// store; P.frames is the binned output, frames of ceil(W / B) x ceil(H / B) U16.  B divides 8, so no bin crosses a
+// tile.  A kernel of its own, not a template of the full decoder: folding the two into one loop changes the full
+// decoder's code.
+template <int B>
+__global__ void __launch_bounds__(kT16) dbde16_decode_binned_kernel(const Dec16Params P) {
+    extern __shared__ __align__(16) uint8_t s_words[];
+    constexpr int NB = 8 / B;                                 // bins per tile side
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int ng = (P.wh + 31) / 32;
+    const int Wb = (P.W + B - 1) / B, Hb = (P.H + B - 1) / B;
+    const size_t fbins = (size_t)Wb * (size_t)Hb;
+    for (unsigned p = blockIdx.x; p < P.nparts; p += gridDim.x) {
+        const unsigned f = p / (unsigned)P.ppf, q = p - f * (unsigned)P.ppf;
+        if (P.status[f] != 0) continue;                       // rejected by the scan: the output stays untouched
+        const uint8_t *rec = P.stream + P.frame_offsets[f];
+        const uint32_t *wp = P.wprefix + (size_t)f * (ng + 1);
+        const int g0 = (int)q * (kT16 / 32), g1 = min(g0 + kT16 / 32, ng);
+        const uint32_t w0 = wp[g0], agg = wp[g1] - w0;
+        stage_words16(s_words, rec + 32 + 3 * (size_t)P.wh + 8ull * w0, agg, tid);
+        const int tile = (int)q * kT16 + tid;
+        const bool valid = tile < P.wh;
+        int k = 0;
+        uint32_t mn = 0;
+        if (valid) {
+            k = rec[24 + tile];
+            const uint8_t *mp = rec + 28 + (size_t)P.wh + 2 * (size_t)tile;
+            mn = (uint32_t)mp[0] | ((uint32_t)mp[1] << 8);
+        }
+        const uint32_t incl = warp_inclusive_scan((uint32_t)k, lane);
+        const uint32_t woff = (g0 + warp < ng ? wp[g0 + warp] - w0 : 0u) + incl - (uint32_t)k;
+        __syncthreads();
+        uint32_t px[32];
+        unpack_tile16(reinterpret_cast<const uint32_t *>(s_words), woff, k, mn, px);
+        if (valid) {
+            const int ty = tile / P.w, tx = tile - ty * P.w;
+            uint16_t *op = P.frames + (size_t)f * fbins + (size_t)(NB * ty) * (size_t)Wb + (size_t)(NB * tx);
+            store_bins16<B>(op, Wb, min(NB, Wb - NB * tx), min(NB, Hb - NB * ty), P.W - 8 * tx, P.H - 8 * ty, px);
+        }
+        __syncthreads();                                      // s_words is reused by the next partition
+    }
+}
+
+// ------------------------------------------------------------------ decoder: crops
+// ncrops rectangles of crop_w x crop_h per frame at int32 corners, after dbde16_scan_kernel.  The scan's word prefix
+// item g covers tiles [32 g, 32 g + 32) in raster order, so a run of consecutive tiles of one tile row has ONE
+// contiguous payload run, starting at the item's prefix plus the depths of the item's tiles before the run.
+// One warp == up to 32 consecutive tile columns of one tile row of a crop of one frame, one lane == one tile; a crop
+// narrower than 32 tiles gives each tile row a SEGMENT of S lanes (the next power of two >= its width in tiles) and a
+// warp 32 / S tile rows.  A segment stages its run in the padded layout and unpacks with unpack_tile16.  Lanes whose
+// tile lies outside the frame load nothing and unpack depth 0 with the pad value as minimum; a crop entirely outside
+// the frame reads nothing of the record.  Rows are cropped on all four sides and leave as aligned 16-byte words
+// assembled across lanes.
+struct Crop16Params {
+    const uint8_t *stream;
+    const uint64_t *frame_offsets;
+    const uint32_t *status;     // from the scan: frames with status != 0 are skipped
+    const uint32_t *wprefix;    // nframes * (ng + 1)
+    const int32_t *corners;     // {x0, y0} of crop r of frame f at corners + 2 * (f * corner_stride + r)
+    uint16_t *out;              // nframes * ncrops * crop_w * crop_h, tightly packed, 2-byte aligned
+    int W, H, w, h, wh, ng;     // the frame in pixels and tiles, word-prefix items per frame
+    int crop_w, crop_h, ncrops, corner_stride;   // corner_stride: ncrops (per-frame corners) or 0 (shared)
+    int nchunks, seg_shift, nrg;                 // 32-tile chunks per tile row, log2 lanes per segment, warps per chunk
+    unsigned long long ntasks;                   // nframes * ncrops * nrg * nchunks warps
+    uint32_t pad2;              // the pad value in both halves
+};
+
+constexpr int kCrop16Warps = 8;
+// per segment of S lanes: 32 S units of payload (S tiles of <= 16 words), the unit past the end, the padding: 33 S + 2
+// units; 32 / S segments per warp
+constexpr int kCrop16BufUnits = 1120;
+
+// The 8 pixels of the combined row [prev (pixels 0-7), x (pixels 8-15)] starting at pixel 8 - s, s = 0..7: a shifter
+// of selects that is branch-free for any s, so segments of one warp may differ in s
+__device__ __forceinline__ uint4 shift_in16(uint4 prev, uint4 x, uint32_t s) {
+    const uint32_t v[8] = {prev.x, prev.y, prev.z, prev.w, x.x, x.y, x.z, x.w};
+    const uint32_t q = s >> 1;
+    uint32_t a[6], u[5];
+#pragma unroll
+    for (int i = 0; i < 6; i++) a[i] = (q & 2u) ? v[i] : v[i + 2];            // a[i] = v[2 + i - 2 (q >> 1)]
+#pragma unroll
+    for (int i = 0; i < 5; i++) u[i] = (q & 1u) ? a[i] : a[i + 1];            // u[i] = v[3 + i - q]
+    uint32_t r[4];
+#pragma unroll
+    for (int j = 0; j < 4; j++) r[j] = (s & 1u) ? __funnelshift_r(u[j], u[j + 1], 16) : u[j + 1];
+    return make_uint4(r[0], r[1], r[2], r[3]);
+}
+
+// pixels [st, en) of the 16-byte-aligned 8-pixel word w at q, as naturally aligned pieces
+__device__ __forceinline__ void store_pixels16(uint16_t *q, uint4 w, int st, int en) {
+    uint8_t *q8 = reinterpret_cast<uint8_t *>(q);
+    if (st < 4) store_word_part(q8, ((uint64_t)w.y << 32) | w.x, 2u * st, 2u * min(en, 4));
+    if (en > 4) store_word_part(q8 + 8, ((uint64_t)w.w << 32) | w.z, 2u * max(st - 4, 0), 2u * (en - 4));
+}
+
+// One pixel row of a segment's tiles into a crop row of cw pixels.  Lane l's 8 pixels belong at row + pos.
+// Consecutive lanes hold consecutive 16-byte pieces, so every lane assembles the ALIGNED 16-byte word its piece
+// starts in -- its left neighbour's tail and its own head -- and stores the part inside [row, row + cw).  A segment's
+// first lane leaves the pixels before its piece to the last lane of the previous chunk, which stores its tail past its
+// word.  Warp-wide call; `live`: this lane has a tile of the crop in a row of the crop.
+__device__ __forceinline__ void crop16_store_row(uint16_t *row, int pos, uint4 x, int cw, bool live, bool first, bool last) {
+    uint4 prev;
+    prev.x = __shfl_up_sync(0xffffffffu, x.x, 1);
+    prev.y = __shfl_up_sync(0xffffffffu, x.y, 1);
+    prev.z = __shfl_up_sync(0xffffffffu, x.z, 1);
+    prev.w = __shfl_up_sync(0xffffffffu, x.w, 1);
+    if (!live) return;
+    const uint32_t s = (((uint32_t)(uintptr_t)row + 2u * (uint32_t)pos) & 15u) >> 1;   // the same in every lane of a segment
+    const int qo = pos - (int)s;                                                         // my aligned word: row + qo
+    const uint4 w = shift_in16(prev, x, s);
+    const int st = max(-qo, first ? (int)s : 0), en = min(cw - qo, 8);
+    uint16_t *q = row + qo;
+    if (st == 0 && en == 8) st_stream_v4u32(q, w);
+    else if (st < en) store_pixels16(q, w, st, en);
+    if (last && s) {                                                                      // my pixels past that word
+        const int st2 = max(-qo - 8, 0), en2 = min(cw - qo - 8, (int)s);
+        if (st2 < en2) store_pixels16(q + 8, shift_in16(x, make_uint4(0u, 0u, 0u, 0u), s), st2, en2);
+    }
+}
+
+__global__ void __launch_bounds__(kCrop16Warps * 32) dbde16_decode_crops_kernel(const Crop16Params P) {
+    __shared__ __align__(16) uint32_t s_buf[kCrop16Warps][kCrop16BufUnits];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const unsigned long long task = (unsigned long long)blockIdx.x * kCrop16Warps + warp;
+    if (task >= P.ntasks) return;
+    // task = ((f * ncrops + r) * nrg + row group) * nchunks + chunk: neighbouring warps read neighbouring payloads
+    const int chunk = (int)(task % (unsigned)P.nchunks);
+    const unsigned long long fr = task / (unsigned)P.nchunks;
+    const unsigned long long fc = fr / (unsigned)P.nrg;
+    const int rg = (int)(fr - fc * (unsigned)P.nrg);
+    const int f = (int)(fc / (unsigned)P.ncrops);
+    const int r = (int)(fc - (unsigned long long)f * (unsigned)P.ncrops);
+    if (P.status[f] != 0) return;                            // rejected by the scan: its crops stay untouched
+    const int32_t *cp = P.corners + 2 * ((size_t)f * (size_t)P.corner_stride + (size_t)r);
+    const int x0 = __ldg(cp), y0 = __ldg(cp + 1);
+    // floor division (negative corners), the far edge in 64 bits (corners up to INT32_MAX)
+    const int tx0 = x0 >> 3, ty0 = y0 >> 3;
+    const int tx_end = (int)(((long long)x0 + P.crop_w + 7) >> 3);
+    const int nty = (int)(((long long)y0 + P.crop_h + 7) >> 3) - ty0;
+    uint16_t *rout = P.out + (size_t)fc * ((size_t)P.crop_w * (size_t)P.crop_h);
+    const int S = 1 << P.seg_shift;
+    const int seg = lane >> P.seg_shift, sl = lane & (S - 1);
+    const int rowi = (rg << (5 - P.seg_shift)) + seg;        // tile row of the crop
+    const bool rowok = rowi < nty;
+    const int ty = ty0 + rowi;
+    const int txc = tx0 + 32 * chunk;                        // my segment's first tile column
+    const int tx = txc + sl;
+    const bool live = rowok && tx < tx_end;
+    // the segment's tiles inside the frame: columns [txa, txb) of tile row ty, one contiguous payload run
+    const int txa = max(txc, 0), txb = min(min(txc + S, tx_end), P.w);
+    const bool segin = rowok && ty >= 0 && ty < P.h && txa < txb;
+    const bool inframe = live && segin && tx >= 0 && tx < P.w;
+    const uint8_t *rec = P.stream + P.frame_offsets[f];
+    const int t0 = segin ? ty * P.w + txa : 0;               // the run's first raster tile
+    const int item = t0 >> 5, rem = t0 & 31;
+    const int tl = inframe ? ty * P.w + tx : 0;              // my tile
+
+    // word offset of tile t0: the item's exclusive prefix plus the depths of the item's tiles before t0
+    uint32_t before = 0;
+    if (segin)
+        for (int j = sl; j < rem; j += S) before += rec[24 + 32 * item + j];
+    for (int o = 1; o < S; o <<= 1) before += __shfl_xor_sync(0xffffffffu, before, o);
+    int k = 0;
+    uint32_t mn = P.pad2 & 0xffffu;                          // outside the frame: depth 0 with the pad value as minimum
+    if (inframe) {
+        k = rec[24 + tl];
+        const uint8_t *mp = rec + 28 + (size_t)P.wh + 2 * (size_t)tl;
+        mn = (uint32_t)mp[0] | ((uint32_t)mp[1] << 8);
+    }
+    const uint32_t wbase = segin ? P.wprefix[(size_t)f * (P.ng + 1) + item] + before : 0u;
+    uint32_t incl = (uint32_t)k;                             // inclusive scan of the depths inside the segment
+    for (int d = 1; d < S; d <<= 1) {
+        const uint32_t t = __shfl_up_sync(0xffffffffu, incl, d, S);
+        if (sl >= d) incl += t;
+    }
+    const uint32_t nwords = __shfl_sync(0xffffffffu, incl, S - 1, S);
+
+    // stage the segment's run (nothing outside it is read): 8-byte loads when it is 8-byte aligned, else 4 byte loads
+    // per unit
+    uint32_t *su = s_buf[warp] + seg * (33 * S + 2);
+    const uint8_t *src = rec + 32 + 3 * (size_t)P.wh + 8 * (size_t)wbase;
+    if (((uintptr_t)src & 7) == 0) {
+        for (uint32_t i = (uint32_t)sl; i < nwords; i += (uint32_t)S) {
+            const uint64_t v = __ldg(reinterpret_cast<const unsigned long long *>(src) + i);
+            const uint32_t at = pad16(2u * i);
+            su[at] = (uint32_t)v;
+            su[at + 1u] = (uint32_t)(v >> 32);
+            if (((2u * i) & 31u) == 0u && i > 0u) su[at - 1u] = (uint32_t)v;
+        }
+    } else {
+        for (uint32_t u = (uint32_t)sl; u < 2u * nwords; u += (uint32_t)S) {
+            const uint8_t *b = src + 4u * u;
+            const uint32_t v = (uint32_t)b[0] | ((uint32_t)b[1] << 8) | ((uint32_t)b[2] << 16) | ((uint32_t)b[3] << 24);
+            const uint32_t at = pad16(u);
+            su[at] = v;
+            if ((u & 31u) == 0u && u > 0u) su[at - 1u] = v;
+        }
+    }
+    if (sl == 0) {                                           // the reader looks one unit past the end
+        const uint32_t u = 2u * nwords;
+        su[pad16(u)] = 0u;
+        if ((u & 31u) == 0u && u > 0u) su[pad16(u) - 1u] = 0u;
+    }
+    __syncwarp();
+
+    uint32_t px[32];
+    unpack_tile16(su, incl - (uint32_t)k, k, mn, px);
+
+    // the frame's partial last tile column / row: pixels past column W and rows past H are pad
+    const int wc = inframe && tx == P.w - 1 ? (P.W & 7) : 0;              // kept pixels of each row, 0 = all
+    const int hr = inframe && ty == P.h - 1 ? P.H - 8 * ty : 8;           // kept rows
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        const uint32_t m = wc == 0 || 2 * j + 2 <= wc ? ~0u : 2 * j + 1 == wc ? 0xffffu : 0u;
+#pragma unroll
+        for (int rr = 0; rr < 8; rr++) px[4 * rr + j] = rr < hr ? (px[4 * rr + j] & m) | (P.pad2 & ~m) : P.pad2;
+    }
+    // crop and store: rows of the tile inside [y0, y0 + crop_h), columns inside [x0, x0 + crop_w).  Offsets are taken
+    // from the crop's first tile, so corners near INT32_MAX do not overflow
+    const int pos = 8 * (tx - tx0) - (x0 & 7);
+    const bool last = sl == S - 1 || tx + 1 >= tx_end;
+#pragma unroll
+    for (int rr = 0; rr < 8; rr++) {
+        const int yr = 8 * rowi + rr - (y0 & 7);                               // the same in every lane of a segment
+        const bool in = live && yr >= 0 && yr < P.crop_h;
+        crop16_store_row(rout + (in ? (size_t)yr * (size_t)P.crop_w : 0), pos,
+                         make_uint4(px[4 * rr], px[4 * rr + 1], px[4 * rr + 2], px[4 * rr + 3]), P.crop_w, in, sl == 0, last);
     }
 }
 
@@ -406,6 +723,46 @@ cudaError_t launch_decode16_scan(const Dec16Params &P, cudaStream_t stream) {
 }
 cudaError_t launch_decode16(const Dec16Params &P, int num_sms, cudaStream_t stream) {
     return launch16(dbde16_decode_kernel, P, P.nparts, num_sms, stream);
+}
+
+cudaError_t launch_decode16_binned(const Dec16Params &scan, int factor, uint16_t *out, int num_sms, cudaStream_t stream) {
+    Dec16Params P = scan;
+    P.frames = out;
+    switch (factor) {
+        case 2: return launch16(dbde16_decode_binned_kernel<2>, P, P.nparts, num_sms, stream);
+        case 4: return launch16(dbde16_decode_binned_kernel<4>, P, P.nparts, num_sms, stream);
+        case 8: return launch16(dbde16_decode_binned_kernel<8>, P, P.nparts, num_sms, stream);
+        default: return cudaErrorInvalidValue;
+    }
+}
+
+cudaError_t launch_decode16_crops(const Dec16Params &scan, const int32_t *corners, int ncrops, bool per_frame, int crop_w,
+                                  int crop_h, int pad, uint16_t *out, cudaStream_t stream) {
+    Crop16Params P = Crop16Params();
+    P.stream = scan.stream;
+    P.frame_offsets = scan.frame_offsets;
+    P.status = scan.status;
+    P.wprefix = scan.wprefix;
+    P.corners = corners;
+    P.out = out;
+    P.W = scan.W; P.H = scan.H; P.w = scan.w; P.h = scan.h; P.wh = scan.wh;
+    P.ng = (scan.wh + 31) / 32;
+    P.crop_w = crop_w; P.crop_h = crop_h; P.ncrops = ncrops;
+    P.corner_stride = per_frame ? ncrops : 0;
+    // a crop starting 7 columns / rows into a tile spans one tile more than one starting on a tile boundary
+    const int span = (int)(((long long)crop_w + 14) / 8), nty = (int)(((long long)crop_h + 14) / 8);
+    P.nchunks = (span + 31) / 32;
+    P.seg_shift = 0;                                          // segments: the next power of two >= the span, <= 32 lanes
+    while ((1 << P.seg_shift) < span && P.seg_shift < 5) P.seg_shift++;
+    P.nrg = (nty + (32 >> P.seg_shift) - 1) / (32 >> P.seg_shift);
+    P.ntasks = (unsigned long long)scan.nframes * (unsigned long long)ncrops * (unsigned long long)P.nrg *
+               (unsigned long long)P.nchunks;
+    P.pad2 = (uint32_t)(pad & 0xFFFF) * 0x00010001u;
+    if (P.ntasks == 0) return cudaSuccess;
+    const unsigned long long blocks = (P.ntasks + kCrop16Warps - 1) / kCrop16Warps;
+    if (blocks > 0x7FFFFFFFull) return cudaErrorInvalidConfiguration;
+    dbde16_decode_crops_kernel<<<(unsigned)blocks, kCrop16Warps * 32, 0, stream>>>(P);
+    return cudaGetLastError();
 }
 
 }  // namespace dbde

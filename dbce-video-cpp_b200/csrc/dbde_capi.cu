@@ -535,10 +535,11 @@ extern "C" int dbde_b200_decode_roi_device(dbde_b200_ctx *c, const uint8_t *stre
 }
 
 // ------------------------------------------------------------------ crops
-static bool crops_ok(int ncrops, int corners_per_frame, int crop_w, int crop_h, int pad) {
+// pad_max: 255 for 8-bit frames, 65535 for DBDE16; the size limit counts pixels whatever their width
+static bool crops_ok(int ncrops, int corners_per_frame, int crop_w, int crop_h, int pad, int pad_max = 255) {
     return ncrops >= 1 && crop_w >= 1 && crop_h >= 1 && dims_ok(crop_w, crop_h, 0) &&
            (long long)ncrops * crop_w * crop_h <= 0x7FFFFFFFLL && (corners_per_frame == 0 || corners_per_frame == 1) && pad >= 0 &&
-           pad <= 255;
+           pad <= pad_max;
 }
 
 // The region decode's scan and kernel body with one rectangle per task taken from `corners` (dbde_roi.cu).  A crop
@@ -974,7 +975,8 @@ extern "C" int dbde_b200_encode_host(dbde_b200_ctx *c, const uint8_t *frames_hos
 
 // What the host pipeline hands back per frame instead of the whole image: the region (x0, y0, w, h), ncrops crops
 // of w x h with host corners (per_frame: nframes * ncrops {x0, y0} pairs, else ncrops pairs for every frame), or the
-// frame binned by `factor` (w x h = ceil(W / factor) x ceil(H / factor))
+// frame binned by `factor` (w x h = ceil(W / factor) x ceil(H / factor)).  Sizes count pixels: DBDE16 frames (u16)
+// have two bytes each, and no region form.
 struct SubFrame {
     int x0, y0, w, h;
     const int32_t *corners;     // null: the region or the binned frame
@@ -999,7 +1001,7 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
             return fail(DBDE_B200_E_INVALID, "decode_host: frame offsets must ascend within the stream");
     }
     const HostFmt F = host_fmt(W, H, u16);
-    const size_t px = sub ? sub->bytes() : F.px;    // output bytes per frame
+    const size_t px = sub ? sub->bytes() * (u16 ? 2 : 1) : F.px;    // output bytes per frame
     int chunk = default_chunk(c, W, H, nframes, u16);
     if (px > F.px) {                                 // crops larger than the frame: a chunk's output stays within 64 MiB
         const size_t most = (64u << 20) / px;
@@ -1097,7 +1099,13 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
             CK(cudaMemcpyAsync(s.d_c, s.h_corners, nb, cudaMemcpyHostToDevice, s.st));
         }
         prof.mark(1, "h2d");
-        rc_all = u16   ? dbde_b200_decode16_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (uint16_t *)s.d_b, s.d_status,
+        rc_all = u16 && sub && sub->corners
+                       ? dbde_b200_decode16_crops_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (const int32_t *)s.d_c,
+                                                         sub->ncrops, sub->per_frame, sub->w, sub->h, sub->pad, (uint16_t *)s.d_b,
+                                                         s.d_status, s.d_index, s.st)
+                 : u16 && sub ? dbde_b200_decode16_binned_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, sub->factor,
+                                                                 (uint16_t *)s.d_b, s.d_status, s.d_index, s.st)
+                 : u16 ? dbde_b200_decode16_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (uint16_t *)s.d_b, s.d_status,
                                                    s.d_index, s.st)
                  : sub && sub->corners
                        ? dbde_b200_decode_crops_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (const int32_t *)s.d_c,
@@ -1231,6 +1239,31 @@ extern "C" int dbde_b200_encode16_device(dbde_b200_ctx *c, const uint16_t *frame
     return 0;
 }
 
+// The DBDE16 validation pass (dbde16_scan_kernel: every check, over the whole record, and the word prefix of every
+// 32 raster-order tiles), queued on st: the first launch of every DBDE16 decode.  P is what the second kernel reads;
+// its output fields are left to the caller.
+static int decode16_scan(dbde_b200_ctx *c, cudaStream_t st, const uint8_t *stream_dev, size_t stream_bytes,
+                         const uint64_t *frame_offsets_dev, int W, int H, int nframes, uint32_t *status_dev, uint64_t *indices_dev,
+                         Dec16Params *P, const char *what) {
+    CK(cudaSetDevice(c->device));
+    *P = Dec16Params();
+    P->W = W; P->H = H; P->w = (W + 7) / 8; P->h = (H + 7) / 8; P->wh = P->w * P->h;
+    P->ppf = (P->wh + 255) / 256;
+    const unsigned long long nparts = (unsigned long long)nframes * P->ppf;
+    if (nparts >= 0xFFFFFFF0ull) return fail(DBDE_B200_E_INVALID, what);
+    const size_t sbytes = 4 * (size_t)nframes * ((size_t)(P->wh + 31) / 32 + 1);
+    StreamScratch &sc = scratch_for(c, st);
+    int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
+    if (rc) return rc;
+    P->stream = stream_dev; P->stream_bytes = stream_bytes; P->frame_offsets = frame_offsets_dev;
+    P->status = status_dev; P->indices = indices_dev;
+    P->wprefix = (uint32_t *)sc.dec;
+    P->nframes = nframes; P->nparts = (unsigned)nparts;
+    CK(launch_decode16_scan(*P, st));
+    c->launches += 1;
+    return 0;
+}
+
 extern "C" int dbde_b200_decode16_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
                                          const uint64_t *frame_offsets_dev, int W, int H, int nframes, uint16_t *frames_dev,
                                          uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
@@ -1238,25 +1271,59 @@ extern "C" int dbde_b200_decode16_device(dbde_b200_ctx *c, const uint8_t *stream
         ((uintptr_t)frames_dev & 1))
         return fail(DBDE_B200_E_INVALID, "decode16_device: bad argument");
     if (nframes == 0) return 0;
-    CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     Dec16Params P;
-    P.W = W; P.H = H; P.w = (W + 7) / 8; P.h = (H + 7) / 8; P.wh = P.w * P.h;
-    P.ppf = (P.wh + 255) / 256;
-    const unsigned long long nparts = (unsigned long long)nframes * P.ppf;
-    if (nparts >= 0xFFFFFFF0ull) return fail(DBDE_B200_E_INVALID, "decode16_device: batch too large");
-    const size_t sbytes = 4 * (size_t)nframes * ((size_t)(P.wh + 31) / 32 + 1);
-    StreamScratch &sc = scratch_for(c, st);
-    int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
+    int rc = decode16_scan(c, st, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, status_dev, indices_dev, &P,
+                           "decode16_device: batch too large");
     if (rc) return rc;
-    P.stream = stream_dev; P.stream_bytes = stream_bytes; P.frame_offsets = frame_offsets_dev;
-    P.frames = frames_dev; P.status = status_dev; P.indices = indices_dev;
-    P.wprefix = (uint32_t *)sc.dec;
-    P.nframes = nframes; P.nparts = (unsigned)nparts;
+    P.frames = frames_dev;
     P.aligned = (W % 8 == 0) && (((uintptr_t)frames_dev & 15) == 0);
-    CK(launch_decode16_scan(P, st));
     CK(launch_decode16(P, c->num_sms, st));
-    c->launches += 2;
+    c->launches += 1;
+    return 0;
+}
+
+// The scan, then one warp per 32 tile columns of each tile row of each crop (dbde16.cu).  A crop equal to the frame
+// still runs the crop kernel: its output layout is the crop layout whatever the corners.
+extern "C" int dbde_b200_decode16_crops_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
+                                               const uint64_t *frame_offsets_dev, int W, int H, int nframes,
+                                               const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
+                                               int crop_h, int pad, uint16_t *crops_dev, uint32_t *status_dev,
+                                               uint64_t *indices_dev, void *stream) {
+    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad, 65535) ||
+        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !corners_dev || !crops_dev || !status_dev)) ||
+        ((uintptr_t)crops_dev & 1))
+        return fail(DBDE_B200_E_INVALID, "decode16_crops_device: bad argument");
+    if (nframes == 0) return 0;
+    cudaStream_t st = (cudaStream_t)stream;
+    Dec16Params P;
+    int rc = decode16_scan(c, st, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, status_dev, indices_dev, &P,
+                           "decode16_crops_device: batch too large");
+    if (rc) return rc;
+    CK(launch_decode16_crops(P, corners_dev, ncrops, corners_per_frame != 0, crop_w, crop_h, pad, crops_dev, st));
+    c->launches += 1;
+    return 0;
+}
+
+// The scan, then the full decoder's partitions with each tile reduced to its bin means in registers (dbde16.cu).
+// Factor 1 is the full decode.
+extern "C" int dbde_b200_decode16_binned_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
+                                                const uint64_t *frame_offsets_dev, int W, int H, int nframes, int factor,
+                                                uint16_t *out_dev, uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
+    if (!c || !dims_ok(W, H, nframes) || !factor_ok(factor) ||
+        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !out_dev || !status_dev)) || ((uintptr_t)out_dev & 1))
+        return fail(DBDE_B200_E_INVALID, "decode16_binned_device: bad argument");
+    if (nframes == 0) return 0;
+    if (factor == 1)
+        return dbde_b200_decode16_device(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, out_dev, status_dev,
+                                         indices_dev, stream);
+    cudaStream_t st = (cudaStream_t)stream;
+    Dec16Params P;
+    int rc = decode16_scan(c, st, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, status_dev, indices_dev, &P,
+                           "decode16_binned_device: batch too large");
+    if (rc) return rc;
+    CK(launch_decode16_binned(P, factor, out_dev, c->num_sms, st));
+    c->launches += 1;
     return 0;
 }
 
@@ -1285,6 +1352,36 @@ extern "C" int dbde_b200_decode16_host(dbde_b200_ctx *c, const uint8_t *stream_h
         return fail(DBDE_B200_E_INVALID, "decode16_host: bad argument");
     return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, (uint8_t *)frames_host, status_host,
                             indices_host, false, true);
+}
+
+// The host forms of the DBDE16 crop and binned decodes: the same chunk pipeline with the crops' or the bins' pixels
+// coming back.  Records still cross PCIe whole.
+extern "C" int dbde_b200_decode16_crops_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
+                                             const uint64_t *frame_offsets_host, int W, int H, int nframes,
+                                             const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
+                                             int crop_h, int pad, uint16_t *crops_host, uint32_t *status_host,
+                                             uint64_t *indices_host) {
+    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad, 65535) ||
+        (nframes > 0 && (!stream_host || !frame_offsets_host || !corners_host || !crops_host || !status_host)) ||
+        ((uintptr_t)crops_host & 1))
+        return fail(DBDE_B200_E_INVALID, "decode16_crops_host: bad argument");
+    const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad, 0};
+    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, (uint8_t *)crops_host, status_host,
+                            indices_host, false, true, &crops);
+}
+
+extern "C" int dbde_b200_decode16_binned_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
+                                              const uint64_t *frame_offsets_host, int W, int H, int nframes, int factor,
+                                              uint16_t *out_host, uint32_t *status_host, uint64_t *indices_host) {
+    if (!c || !dims_ok(W, H, nframes) || !factor_ok(factor) ||
+        (nframes > 0 && (!stream_host || !frame_offsets_host || !out_host || !status_host)) || ((uintptr_t)out_host & 1))
+        return fail(DBDE_B200_E_INVALID, "decode16_binned_host: bad argument");
+    if (factor == 1)
+        return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, (uint8_t *)out_host, status_host,
+                                indices_host, false, true);
+    const SubFrame binned = {0, 0, (W - 1) / factor + 1, (H - 1) / factor + 1, nullptr, 1, 0, 0, factor};
+    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, (uint8_t *)out_host, status_host,
+                            indices_host, false, true, &binned);
 }
 
 // ------------------------------------------------------------------ multi-GPU sharding

@@ -73,6 +73,16 @@ struct Dec16Params {
 cudaError_t launch_encode16(const Enc16Params &P, int num_sms, cudaStream_t stream);
 cudaError_t launch_decode16_scan(const Dec16Params &P, cudaStream_t stream);
 cudaError_t launch_decode16(const Dec16Params &P, int num_sms, cudaStream_t stream);
+// DBDE16 crop decode (dbde16.cu), after launch_decode16_scan(scan): ncrops rectangles of crop_w x crop_h per frame with
+// top-left corners {x0, y0} at corners (device; per_frame: nframes * ncrops pairs, else ncrops pairs for every frame),
+// any int32 values; pixels outside the frame are `pad`.  Crop r of frame f goes to out + (f * ncrops + r) * crop_w *
+// crop_h U16.  Frames the scan rejected stay untouched.
+cudaError_t launch_decode16_crops(const Dec16Params &scan, const int32_t *corners, int ncrops, bool per_frame, int crop_w,
+                                  int crop_h, int pad, uint16_t *out, cudaStream_t stream);
+// DBDE16 binned decode (dbde16.cu), after launch_decode16_scan(scan): every frame reduced to the rounded means of its
+// factor x factor blocks (factor 2, 4 or 8), ceil(H / factor) rows of ceil(W / factor) U16 per frame, tightly packed
+// from `out`.  Frames the scan rejected stay untouched.
+cudaError_t launch_decode16_binned(const Dec16Params &scan, int factor, uint16_t *out, int num_sms, cudaStream_t stream);
 
 // The persistent kernels' launch configuration (dynamic shared memory opt-in + resident CTAs per SM) is a
 // property of (device, kernel, shared-memory size): looked up once and remembered, because the two runtime

@@ -271,6 +271,53 @@ DBDE_B200_API int dbde_b200_decode16_host(dbde_b200_ctx *ctx, const uint8_t *str
                                           const uint64_t *frame_offsets_host, int W, int H, int nframes,
                                           uint16_t *frames_host, uint32_t *status_host, uint64_t *indices_host);
 
+/* ---- DBDE16 crops: N fixed-size windows of every 16-bit frame, anywhere, padded outside the frame ---------------
+ * dbde_b200_decode_crops_* for DBDE16 records: the wells of a plate, a tracked window or animal-centred windows from
+ * a scientific camera's frames without decoding the rest of each frame.  corners, corners_per_frame and the output
+ * layout are those of dbde_b200_decode_crops_*, counted in U16 pixels: crop r of frame f goes to crops +
+ * ((size_t)f * ncrops + r) * crop_w * crop_h, crop_h rows of crop_w U16, tightly packed.  Pixel (x, y) of a crop is
+ * image[y0 + y][x0 + x] of dbde_b200_decode16_device's image where that lies inside the frame, and `pad` elsewhere; a
+ * crop entirely outside the frame is all `pad` and reads nothing of the record.  A region of interest is one crop
+ * with a shared corner inside the frame.  Validation covers the WHOLE record: status and indices are exactly what
+ * dbde_b200_decode16_device reports for the same records, a record damaged outside every crop is rejected too, and
+ * all crops of a rejected frame are left untouched.  Nothing outside [crops, crops + nframes * ncrops * crop_w *
+ * crop_h * 2 bytes) is written.  Like dbde_b200_decode16_device, these ignore the context's DBDE_INVERT_ENDIAN
+ * setting: DBDE16 has no such variant.  DBDE_B200_E_INVALID before any work is queued for: NULL pointers (when
+ * nframes > 0), an output pointer that is not 2-byte aligned (any even address works), ncrops < 1, crop_w or crop_h
+ * < 1, a crop size the frame limits reject, ncrops * crop_w * crop_h > 2^31 - 1 pixels, corners_per_frame not 0 or 1,
+ * pad outside 0..65535.  nframes == 0 returns 0.
+ * _device: corners in device memory, asynchronous on `stream`.  _host: host memory, the chunk pipeline of
+ * dbde_b200_decode16_host (records still cross PCIe whole, only the accepted frames' crops come back). */
+DBDE_B200_API int dbde_b200_decode16_crops_device(dbde_b200_ctx *ctx, const uint8_t *stream_dev, size_t stream_bytes,
+                                                  const uint64_t *frame_offsets_dev, int W, int H, int nframes,
+                                                  const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
+                                                  int crop_h, int pad, uint16_t *crops_dev, uint32_t *status_dev,
+                                                  uint64_t *indices_dev, void *stream);
+DBDE_B200_API int dbde_b200_decode16_crops_host(dbde_b200_ctx *ctx, const uint8_t *stream_host, size_t stream_bytes,
+                                                const uint64_t *frame_offsets_host, int W, int H, int nframes,
+                                                const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
+                                                int crop_h, int pad, uint16_t *crops_host, uint32_t *status_host,
+                                                uint64_t *indices_host);
+
+/* ---- DBDE16 binned: every 16-bit frame at 1/2, 1/4 or 1/8 of its size, as block means -----------------------------
+ * dbde_b200_decode_binned_* for DBDE16 records.  factor must be 1, 2, 4 or 8; factor 1 is dbde_b200_decode16_device.
+ * Frame i's output is Hb = ceil(H / factor) rows of Wb = ceil(W / factor) U16, tightly packed, at out + i * Wb * Hb
+ * U16; nothing outside [out, out + nframes * Wb * Hb * 2 bytes) is written.  Output pixel (X, Y) is the mean of the
+ * IN-FRAME pixels of dbde_b200_decode16_device's image in [factor X, factor X + factor) x [factor Y, factor Y +
+ * factor), rounded half up: (sum + n / 2) / n in integers with 32-bit sums, n the number of in-frame pixels (factor^2
+ * except in the last column when W % factor != 0 and the last row when H % factor != 0).  Validation, status, indices
+ * and rejected frames as for the DBDE16 crops above; DBDE_INVERT_ENDIAN is ignored.  DBDE_B200_E_INVALID before any
+ * work is queued for: NULL pointers (when nframes > 0), an output pointer that is not 2-byte aligned, a factor other
+ * than 1, 2, 4 or 8, frame dimensions the frame limits reject.  nframes == 0 returns 0.
+ * _device: asynchronous on `stream`.  _host: the chunk pipeline of dbde_b200_decode16_host (records still cross PCIe
+ * whole, only the accepted frames' binned pixels come back). */
+DBDE_B200_API int dbde_b200_decode16_binned_device(dbde_b200_ctx *ctx, const uint8_t *stream_dev, size_t stream_bytes,
+                                                   const uint64_t *frame_offsets_dev, int W, int H, int nframes, int factor,
+                                                   uint16_t *out_dev, uint32_t *status_dev, uint64_t *indices_dev, void *stream);
+DBDE_B200_API int dbde_b200_decode16_binned_host(dbde_b200_ctx *ctx, const uint8_t *stream_host, size_t stream_bytes,
+                                                 const uint64_t *frame_offsets_host, int W, int H, int nframes, int factor,
+                                                 uint16_t *out_host, uint32_t *status_host, uint64_t *indices_host);
+
 /* ---- .dbde files (SURVEY.md 8 f-1): 28-byte video header + frame records back to back ------------- */
 /* The container the reference's walker reads (dbde_util.cpp:362-426; dbde_start_file_walk /
  * dbde_walk_a_file / dbde_end_file_walk in include/dbde_util.h remain available as the drop-in).
