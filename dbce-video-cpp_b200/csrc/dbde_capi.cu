@@ -562,6 +562,48 @@ extern "C" int dbde_b200_decode_crops_device(dbde_b200_ctx *c, const uint8_t *st
     return 0;
 }
 
+// One CTA per record of a persistent grid, one lane per crop tile (dbde_encode.cu).  A crop equal to the frame still
+// runs the crop kernel: its records are the frame encoder's records, byte for byte.
+extern "C" int dbde_b200_encode_crops_device(dbde_b200_ctx *c, const uint8_t *frames_dev, int W, int H, uint64_t first_index,
+                                             int nframes, const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
+                                             int crop_h, int pad, uint8_t *out_dev, size_t out_capacity, size_t slot_stride,
+                                             uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev, void *stream) {
+    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
+        (nframes > 0 && (!frames_dev || !corners_dev || !out_dev || !frame_offsets_dev || !frame_sizes_dev)))
+        return fail(DBDE_B200_E_INVALID, "encode_crops_device: bad argument");
+    if (nframes == 0) return 0;
+    if (slot_stride == 0) slot_stride = dbde_b200_slot_stride(crop_w, crop_h);
+    if (slot_stride < dbde_b200_frame_record_bound(crop_w, crop_h))
+        return fail(DBDE_B200_E_INVALID, "encode_crops_device: slot_stride < dbde_b200_frame_record_bound(crop_w, crop_h)");
+    const long long nrec = (long long)nframes * ncrops;
+    if (nrec > 0x7FFFFFFFLL) return fail(DBDE_B200_E_INVALID, "encode_crops_device: nframes * ncrops > 2^31 - 1");
+    if (slot_stride > out_capacity / (size_t)nrec)
+        return fail(DBDE_B200_E_CAPACITY, "encode_crops_device: out_capacity < nframes * ncrops * slot_stride");
+    CK(cudaSetDevice(c->device));
+    EncCropParams P;
+    P.frames = frames_dev;
+    P.W = W;
+    P.H = H;
+    P.corners = corners_dev;
+    P.ncrops = ncrops;
+    P.corner_stride = corners_per_frame ? ncrops : 0;
+    P.crop_w = crop_w;
+    P.crop_h = crop_h;
+    P.w = (crop_w + 7) / 8;
+    P.wh = P.w * ((crop_h + 7) / 8);
+    P.pad8 = (uint64_t)pad * 0x0101010101010101ull;
+    P.out = out_dev;
+    P.slot_stride = slot_stride;
+    P.frame_offsets = frame_offsets_dev;
+    P.frame_sizes = frame_sizes_dev;
+    P.first_index = first_index;
+    P.nrec = (int)nrec;
+    P.flags = c->invert_endian ? kFlagInvertRows : 0u;
+    CK(launch_encode_crops(P, c->num_sms, (cudaStream_t)stream));
+    c->launches += 1;
+    return 0;
+}
+
 // ------------------------------------------------------------------ binned
 static bool factor_ok(int factor) { return factor == 1 || factor == 2 || factor == 4 || factor == 8; }
 
@@ -828,6 +870,30 @@ static int ensure_slot(dbde_b200_ctx *c, HostSlot &s, size_t need_a, size_t need
     return 0;
 }
 
+// What the host pipeline hands back per frame instead of the whole image: the region (x0, y0, w, h), ncrops crops
+// of w x h with host corners (per_frame: nframes * ncrops {x0, y0} pairs, else ncrops pairs for every frame), or the
+// frame binned by `factor` (w x h = ceil(W / factor) x ceil(H / factor)).  Sizes count pixels: DBDE16 frames (u16)
+// have two bytes each, and no region form.  The encoder takes the crops form: ncrops records of w x h per frame.
+struct SubFrame {
+    int x0, y0, w, h;
+    const int32_t *corners;     // null: the region or the binned frame
+    int ncrops, per_frame, pad;
+    int factor;                 // > 0: the binned frame
+    size_t bytes() const { return (size_t)w * (size_t)h * (size_t)(corners ? ncrops : 1); }
+    size_t corner_bytes(int n) const { return corners ? 8 * (size_t)ncrops * (size_t)(per_frame ? n : 1) : 0; }
+};
+
+// pinned staging of a chunk's crop corners
+static int ensure_corner_staging(HostSlot &s, size_t need) {
+    if (s.cap_hcorners >= need) return 0;
+    if (s.h_corners) CK(cudaFreeHost(s.h_corners));
+    s.h_corners = nullptr;
+    s.cap_hcorners = 0;
+    CK(cudaHostAlloc(&s.h_corners, need, cudaHostAllocDefault));
+    s.cap_hcorners = need;
+    return 0;
+}
+
 // Where the next chunk's records go in the output stream.  Chunks are claimed strictly in chunk
 // order -- by one worker (plain encode_host) or by several (encode_host_sharded: chunk ci belongs to
 // worker ci mod G) -- so the records land back to back without any pass over the bytes afterwards.
@@ -837,29 +903,35 @@ struct EncSequencer {
     size_t out_pos = 0;            // guarded by `next`
 };
 
-// Worker `my` of `nworkers`: encodes chunks my, my + nworkers, ... of the batch on context c.
+// Worker `my` of `nworkers`: encodes chunks my, my + nworkers, ... of the batch on context c.  crops: every frame
+// gives crops->ncrops records of crops->w x crops->h (dbde_b200_encode_crops_device) instead of its own record; the
+// chunk's corners travel behind its frames in the slot's frame buffer.
 static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index,
                               int nframes, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host,
-                              int chunk, int my, int nworkers, EncSequencer *seq, bool u16 = false) {
+                              int chunk, int my, int nworkers, EncSequencer *seq, bool u16 = false, const SubFrame *crops = nullptr) {
     CK(cudaSetDevice(c->device));
-    const HostFmt F = host_fmt(W, H, u16);
-    const size_t px = F.px;
+    const HostFmt F = crops ? host_fmt(crops->w, crops->h, false) : host_fmt(W, H, u16);   // the records' format
+    const size_t px = crops ? (size_t)W * (size_t)H : F.px;                                  // input bytes per frame
+    const int per = crops ? crops->ncrops : 1;                                                // records per frame
+    const int nrec = chunk * per;                                                             // records per chunk
     const size_t delta = F.delta;
-    const size_t need_a = px * chunk + 32, need_b = F.stream_bound(chunk) + 32;
+    const size_t corner_at = (px * chunk + 15) & ~(size_t)15, need_corners = crops ? crops->corner_bytes(chunk) : 0;
+    const size_t need_a = crops ? corner_at + need_corners : px * chunk + 32, need_b = F.stream_bound(nrec) + 32;
     const int nchunks = (nframes + chunk - 1) / chunk;
     const int mine = nchunks > my ? (nchunks - my + nworkers - 1) / nworkers : 0;
     const int ns = mine < c->nslots ? mine : c->nslots;            // a one-frame call sets up one slot
     // pageable caller memory is relayed through pinned bounce buffers (see CopyPool)
     const bool in_pageable = is_pageable(frames_host), out_pageable = is_pageable(out_host);
     for (int i = 0; i < ns; i++) {
-        int rc = ensure_slot(c, c->slots[i], need_a, need_b, chunk > 1 ? need_b : 0, chunk);
+        int rc = ensure_slot(c, c->slots[i], need_a, need_b, nrec > 1 ? need_b : 0, nrec);
         if (!rc) rc = ensure_bounce(c, c->slots[i], in_pageable ? px * chunk : 0, out_pageable ? need_b : 0);
+        if (!rc) rc = ensure_corner_staging(c->slots[i], need_corners);
         if (rc) return rc;
     }
     const size_t stride = F.stride;
     // One frame per call into pageable memory (the drop-in functions): the record's size is not known until the
     // kernel has run, but its first DMA piece can follow the kernel at once -- most records are longer than a piece.
-    const size_t spec_piece = (chunk == 1 && out_pageable) ? d2h_piece_bytes(stride) : 0;
+    const size_t spec_piece = (nrec == 1 && out_pageable) ? d2h_piece_bytes(stride) : 0;
     // finish(): wait for a chunk's kernels, learn the record sizes, claim the chunk's place in the
     // stream, and queue ONE D2H copy of its records -- already laid back to back on the device
     // (a one-frame chunk's record is contiguous in its slot as it is: no compaction pass).
@@ -870,8 +942,9 @@ static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int 
         else CK(cudaEventSynchronize(s.ev));
         g_enc_prof.mark(3, "gpu");
         g_enc_prof.gpu_collect();
+        const int nr = s.n * per;
         uint64_t total = 0;
-        for (int i = 0; i < s.n; i++) total += s.h_size[i];
+        for (int i = 0; i < nr; i++) total += s.h_size[i];
         while (seq->next.load(std::memory_order_acquire) != ci) {
             if (seq->err.load(std::memory_order_relaxed)) return DBDE_B200_E_INVALID;   // another worker failed
             std::this_thread::yield();
@@ -881,11 +954,11 @@ static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int 
         seq->out_pos = pos + total;
         seq->next.store(ci + 1, std::memory_order_release);
         uint64_t run = pos;
-        for (int i = 0; i < s.n; i++) {
-            frame_offsets_host[s.first + i] = run;
+        for (int i = 0; i < nr; i++) {
+            frame_offsets_host[(size_t)s.first * per + i] = run;
             run += s.h_size[i];
         }
-        const uint8_t *d_rec = chunk > 1 ? s.d_c : s.d_b + delta;
+        const uint8_t *d_rec = nrec > 1 ? s.d_c : s.d_b + delta;
         if (out_pageable && spec_piece) {
             // the record's first piece has been on its way since the kernel was queued; now that the size is known
             // the remaining pieces follow, and everything up to `total` leaves the bounce buffer
@@ -923,16 +996,29 @@ static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int 
         } else {
             CK(cudaMemcpyAsync(s.d_a, frames_host + px * s.first, px * s.n, cudaMemcpyHostToDevice, s.st));
         }
+        if (crops) {
+            // this chunk's corners (the staging is free: the slot's stream has drained)
+            const size_t nb = crops->corner_bytes(s.n);
+            memcpy(s.h_corners, crops->corners + (crops->per_frame ? 2 * (size_t)crops->ncrops * (size_t)s.first : 0), nb);
+            CK(cudaMemcpyAsync(s.d_a + corner_at, s.h_corners, nb, cudaMemcpyHostToDevice, s.st));
+        }
         prof.mark(1, "h2d");
         prof.gpu_mark(1, s.st);
-        rc_all = u16 ? dbde_b200_encode16_device(c, (const uint16_t *)s.d_a, W, H, first_index + s.first, s.n, s.d_b + delta,
-                                                 need_b - 32, stride, s.d_off, s.d_size, s.st)
-                     : dbde_b200_encode_device(c, s.d_a, W, H, first_index + s.first, s.n, s.d_b + delta, need_b - 32, stride,
-                                               s.d_off, s.d_size, s.st);
+        rc_all = crops ? dbde_b200_encode_crops_device(c, s.d_a, W, H, first_index + s.first, s.n, (const int32_t *)(s.d_a + corner_at),
+                                                       crops->ncrops, crops->per_frame, crops->w, crops->h, crops->pad, s.d_b + delta,
+                                                       need_b - 32, stride, s.d_off, s.d_size, s.st)
+                 : u16 ? dbde_b200_encode16_device(c, (const uint16_t *)s.d_a, W, H, first_index + s.first, s.n, s.d_b + delta,
+                                                   need_b - 32, stride, s.d_off, s.d_size, s.st)
+                       : dbde_b200_encode_device(c, s.d_a, W, H, first_index + s.first, s.n, s.d_b + delta, need_b - 32, stride,
+                                                 s.d_off, s.d_size, s.st);
         if (rc_all) break;
         prof.gpu_mark(2, s.st);
-        CK(cudaMemcpyAsync(s.h_size, s.d_size, 8 * (size_t)s.n, cudaMemcpyDeviceToHost, s.st));
-        if (chunk > 1) {
+        CK(cudaMemcpyAsync(s.h_size, s.d_size, 8 * (size_t)s.n * per, cudaMemcpyDeviceToHost, s.st));
+        if (crops && nrec > 1) {
+            // thousands of records per chunk: the prefix once (into d_off, which the host does not read back)
+            CK(launch_compact_prefixed(s.d_b + delta, stride, s.d_size, s.d_off, s.n * per, s.d_c, s.st));
+            c->launches += 2;
+        } else if (chunk > 1) {
             CK(launch_compact(s.d_b + delta, stride, s.d_size, s.n, s.d_c, s.st));
             c->launches += 1;
         }
@@ -973,18 +1059,33 @@ extern "C" int dbde_b200_encode_host(dbde_b200_ctx *c, const uint8_t *frames_hos
     return 0;
 }
 
-// What the host pipeline hands back per frame instead of the whole image: the region (x0, y0, w, h), ncrops crops
-// of w x h with host corners (per_frame: nframes * ncrops {x0, y0} pairs, else ncrops pairs for every frame), or the
-// frame binned by `factor` (w x h = ceil(W / factor) x ceil(H / factor)).  Sizes count pixels: DBDE16 frames (u16)
-// have two bytes each, and no region form.
-struct SubFrame {
-    int x0, y0, w, h;
-    const int32_t *corners;     // null: the region or the binned frame
-    int ncrops, per_frame, pad;
-    int factor;                 // > 0: the binned frame
-    size_t bytes() const { return (size_t)w * (size_t)h * (size_t)(corners ? ncrops : 1); }
-    size_t corner_bytes(int n) const { return corners ? 8 * (size_t)ncrops * (size_t)(per_frame ? n : 1) : 0; }
-};
+// The host form of dbde_b200_encode_crops_device: the encode_host chunk pipeline with ncrops records per frame; each
+// chunk's corners go up behind its frames.
+extern "C" int dbde_b200_encode_crops_host(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index,
+                                           int nframes, const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
+                                           int crop_h, int pad, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host) {
+    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
+        (nframes > 0 && (!frames_host || !corners_host || !out_host || !frame_offsets_host)))
+        return fail(DBDE_B200_E_INVALID, "encode_crops_host: bad argument");
+    if (nframes == 0) {
+        if (frame_offsets_host) frame_offsets_host[0] = 0;
+        return 0;
+    }
+    if ((long long)nframes * ncrops > 0x7FFFFFFFLL) return fail(DBDE_B200_E_INVALID, "encode_crops_host: nframes * ncrops > 2^31 - 1");
+    int chunk = default_chunk(c, W, H, nframes);
+    const size_t rec = (size_t)ncrops * dbde_b200_slot_stride(crop_w, crop_h);    // one frame's record slots
+    if (rec > dbde_b200_slot_stride(W, H)) {       // crops larger than the frame: a chunk's records stay within 64 MiB
+        const size_t most = (64u << 20) / rec;
+        if ((size_t)chunk > most) chunk = most > 0 ? (int)most : 1;
+    }
+    const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad, 0};
+    EncSequencer seq;
+    int rc = encode_host_worker(c, frames_host, W, H, first_index, nframes, out_host, out_capacity, frame_offsets_host, chunk, 0, 1,
+                                &seq, false, &crops);
+    if (rc) return rc;
+    frame_offsets_host[(size_t)nframes * ncrops] = seq.out_pos;
+    return 0;
+}
 
 static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                             const uint64_t *frame_offsets_host, int W, int H, int nframes, uint8_t *frames_host,
@@ -1031,13 +1132,8 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
         HostSlot &s = c->slots[i];
         int rc = ensure_slot(c, s, need_a, need_b, need_corners, chunk);
         if (!rc) rc = ensure_bounce(c, s, in_pageable ? need_a : 0, out_pageable ? px * chunk : 0);
+        if (!rc) rc = ensure_corner_staging(s, need_corners);
         if (rc) return rc;
-        if (s.cap_hcorners < need_corners) {
-            if (s.h_corners) CK(cudaFreeHost(s.h_corners));
-            s.h_corners = nullptr;
-            CK(cudaHostAlloc(&s.h_corners, need_corners, cudaHostAllocDefault));
-            s.cap_hcorners = need_corners;
-        }
     }
     // finish(): wait for a chunk's status words, then queue the D2H of its accepted frames.  A
     // rejected frame must leave the caller's image untouched (dbde_util.cpp:296-303), so pixels

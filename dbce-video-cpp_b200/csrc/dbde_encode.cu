@@ -566,6 +566,167 @@ __global__ void __launch_bounds__(kEncThreads, 3) dbde_encode_kernel(const EncPa
     }
 }
 
+// ------------------------------------------------------------------ crop encoder
+// One CTA per record (frame f, crop r) of a persistent grid, one lane per tile of the crop.  The CTA walks the crop's
+// tiles in raster order, 256 at a time; a record's word offsets depend on its own tiles only, so a CTA-wide scan per
+// chunk plus a running carry replaces the frame encoder's look-back and tickets, and no scratch is zeroed.
+
+// The 8 rows of crop tile (tx, ty): pixel (x, y) of the crop image is frame[y0 + y][x0 + x] inside the frame and the
+// pad byte outside it; the reference's clamp padding at the crop's own partial last column / row repeats the crop
+// image's last valid pixel (dbde_util.cpp:105-135), which may be pad.  A tile inside the frame and the crop loads each
+// row as the one or two aligned 8-byte words it touches (32 lanes of a tile row read 256 consecutive bytes); a tile
+// at an edge reads each in-frame pixel it needs as a byte and nothing else.
+__device__ __forceinline__ void load_crop_tile(const EncCropParams &P, const uint8_t *fr, long long x0, long long y0, int tx, int ty,
+                                               uint32_t (&px)[16]) {
+    const long long xs = x0 + 8 * tx, ys = y0 + 8 * ty;
+    const bool inner = 8 * tx + 8 <= P.crop_w && 8 * ty + 8 <= P.crop_h && xs >= 0 && xs + 8 <= P.W && ys >= 0 && ys + 8 <= P.H;
+    if (inner) {
+        const uint8_t *p = fr + (size_t)ys * (size_t)P.W + (size_t)xs;
+#pragma unroll
+        for (int r = 0; r < 8; r++) {
+            const uint64_t *a = reinterpret_cast<const uint64_t *>((uintptr_t)p & ~(uintptr_t)7);
+            const uint32_t sh = ((uint32_t)(uintptr_t)p & 7u) * 8u;
+            uint64_t v = __ldg(a);
+            if (sh) v = (v >> sh) | (__ldg(a + 1) << (64u - sh));
+            px[2 * r] = (uint32_t)v;
+            px[2 * r + 1] = (uint32_t)(v >> 32);
+            p += P.W;
+        }
+        return;
+    }
+#pragma unroll
+    for (int r = 0; r < 8; r++) {
+        const long long y = y0 + min(8 * ty + r, P.crop_h - 1);
+        uint64_t v = P.pad8;
+        if (y >= 0 && y < P.H) {
+            const uint8_t *row = fr + (size_t)y * (size_t)P.W;
+            v = 0;
+#pragma unroll
+            for (int i = 0; i < 8; i++) {
+                const long long x = x0 + min(8 * tx + i, P.crop_w - 1);
+                const uint64_t b = x >= 0 && x < P.W ? (uint64_t)__ldg(row + x) : (P.pad8 & 0xffu);
+                v |= b << (8 * i);
+            }
+        }
+        px[2 * r] = (uint32_t)v;
+        px[2 * r + 1] = (uint32_t)(v >> 32);
+    }
+}
+
+__global__ void __launch_bounds__(kTilesPerPart) dbde_encode_crops_kernel(const EncCropParams P) {
+    __shared__ __align__(16) uint8_t s_words[kConsumerWarps][kEncWarpBytes];   // each warp's packed words of one chunk
+    __shared__ uint32_t s_wtot[2][kConsumerWarps];                            // each warp's word count, by chunk parity
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    uint8_t *stage_out = s_words[warp];
+    const size_t fbytes = (size_t)P.W * (size_t)P.H;
+    const size_t fixed = 32 + 2 * (size_t)P.wh;
+    unsigned cc = 0;                                   // chunks done by this CTA: selects the s_wtot half
+    for (int j = blockIdx.x; j < P.nrec; j += gridDim.x) {
+        const int f = j / P.ncrops, r = j - f * P.ncrops;
+        const int32_t *cp = P.corners + 2 * ((size_t)f * (size_t)P.corner_stride + (size_t)r);
+        const long long x0 = __ldg(cp), y0 = __ldg(cp + 1);
+        const uint8_t *fr = P.frames + (size_t)f * fbytes;
+        uint8_t *rec = P.out + (size_t)j * P.slot_stride;
+        uint32_t carry = 0;                            // U64 words of the record's earlier chunks
+        for (int t0 = 0; t0 < P.wh; t0 += kTilesPerPart, cc++) {
+            const int t = t0 + tid;
+            const bool valid = t < P.wh;
+            uint32_t px[16];
+            if (valid) {
+                const int ty = t / P.w;
+                load_crop_tile(P, fr, x0, y0, t - ty * P.w, ty, px);
+            } else {
+#pragma unroll
+                for (int i = 0; i < 16; i++) px[i] = 0;
+            }
+            if (P.flags & kFlagInvertRows) reverse_rows(px);      // after the clamp padding, as ENDIAN() at dbde_util.cpp:24-27
+            uint32_t mn = tile_min(px);
+            int k = tile_subtract_depth(px, mn);
+            if (!valid) { k = 0; mn = 0; }
+            const uint32_t incl = warp_inclusive_scan((uint32_t)k, lane);
+            if (lane == 31) s_wtot[cc & 1][warp] = incl;
+            const uint32_t off = incl - (uint32_t)k;
+            // the frame encoder's depth vote and packers (dbde_encode_kernel, stage (4))
+            const uint32_t kinds = __reduce_or_sync(0xffffffffu, (1u << k) >> 1);
+            const bool many_depths = __popc(kinds) >= kEncVarMinDepths;
+            if ((kinds & ~3u) == 0u) {
+                if (kinds) pack_low_depths(px, k, stage_out + 8 * off);
+            } else if (k > 0) {
+                const uint32_t c1 = (1u << k) - 256u, c2 = (1u << (2 * k)) - 65536u;
+                uint32_t q[16];
+#pragma unroll
+                for (int i = 0; i < 16; i++) q[i] = squeeze4(px[i], c1, c2);
+                uint2 *wp = reinterpret_cast<uint2 *>(stage_out + 8 * off);
+                auto store = [&](int n, uint32_t lo, uint32_t hi) { wp[n] = make_uint2(lo, hi); };
+                if (many_depths) pack_rows_var(q, k, stage_out + 8 * off);
+                else switch (k) {
+                    case 1: concat_fields<1>(q, store); break;
+                    case 2: concat_fields<2>(q, store); break;
+                    case 3: concat_fields<3>(q, store); break;
+                    case 4: concat_fields<4>(q, store); break;
+                    case 5: concat_fields<5>(q, store); break;
+                    case 6: concat_fields<6>(q, store); break;
+                    case 7: concat_fields<7>(q, store); break;
+                    default: enc_store_depth8(q, stage_out + 8 * off, off); break;
+                }
+            }
+            __syncthreads();                           // every warp's count and words are in shared memory
+            uint32_t wbase = 0, tot = 0;
+#pragma unroll
+            for (int w = 0; w < kConsumerWarps; w++) {
+                const uint32_t v = s_wtot[cc & 1][w];
+                wbase += w < warp ? v : 0u;
+                tot += v;
+            }
+            // depth and minimum planes (dbde_util.cpp:156-157)
+            if (valid) {
+                rec[24 + (size_t)t] = (uint8_t)k;
+                rec[28 + (size_t)P.wh + (size_t)t] = (uint8_t)mn;
+            }
+            // this warp's words: one coalesced run
+            const uint32_t n = s_wtot[cc & 1][warp];
+            uint8_t *dst = rec + fixed + 8 * ((size_t)carry + wbase);
+            if (((uintptr_t)dst & 7) == 0) {
+                for (uint32_t i = lane; i < n; i += 32)
+                    st_stream_u64(dst + 8 * i, *reinterpret_cast<const uint64_t *>(stage_out + 8 * i));
+            } else {
+                for (uint32_t i = lane; i < 8 * n; i += 32) dst[i] = stage_out[i];
+            }
+            carry += tot;
+            __syncwarp();                              // the copy has read the staging before the next chunk packs into it
+        }
+        if (warp == 0) {
+            // the fixed fields (dbde_util.cpp:141-146,182-188,191), as the frame encoder's scan warp writes them
+            const uint64_t index = P.first_index + (uint64_t)f;
+            const uint32_t wh = (uint32_t)P.wh;
+            uint32_t b;
+            uint8_t *dst;
+            if (lane < 4) { b = (2u >> (8 * lane)) & 0xff; dst = rec + lane; }
+            else if (lane < 12) { b = (uint32_t)(index >> (8 * (lane - 4))) & 0xff; dst = rec + lane; }
+            else if (lane < 20) { b = 0; dst = rec + lane; }
+            else if (lane < 24) { b = (wh >> (8 * (lane - 20))) & 0xff; dst = rec + lane; }
+            else if (lane < 28) { b = (wh >> (8 * (lane - 24))) & 0xff; dst = rec + 24 + (size_t)wh + (lane - 24); }
+            else { b = (carry >> (8 * (lane - 28))) & 0xff; dst = rec + 28 + 2 * (size_t)wh + (lane - 28); }
+            *dst = (uint8_t)b;
+            if (lane == 0) {
+                P.frame_offsets[j] = (uint64_t)j * P.slot_stride;
+                P.frame_sizes[j] = fixed + 8ull * carry;
+            }
+        }
+    }
+}
+
+cudaError_t launch_encode_crops(const EncCropParams &P, int num_sms, cudaStream_t stream) {
+    if (P.nrec <= 0) return cudaSuccess;
+    int occ = 0;
+    cudaError_t e = cached_occupancy((const void *)dbde_encode_crops_kernel, kTilesPerPart, 0, &occ);
+    if (e != cudaSuccess) return e;
+    unsigned grid = (unsigned)(num_sms * occ);
+    if (grid > (unsigned)P.nrec) grid = (unsigned)P.nrec;
+    dbde_encode_crops_kernel<<<grid, kTilesPerPart, 0, stream>>>(P);
+    return cudaGetLastError();
+}
+
 // ------------------------------------------------------------------ record compaction
 // Lays the records of a batch back to back on the device (slot f -> dst + sum of the sizes before f),
 // so the host path brings a chunk home with ONE large D2H copy instead of one per record: small
@@ -597,6 +758,65 @@ cudaError_t launch_compact(const uint8_t *slots, uint64_t slot_stride, const uin
     if (bx < 1) bx = 1;
     if (bx > 64) bx = 64;
     dbde_compact_kernel<<<dim3(bx, (unsigned)n), 256, 0, stream>>>(slots, slot_stride, sizes, n, dst);
+    return cudaGetLastError();
+}
+
+// The exclusive prefix of n record sizes, once, by one CTA: prefix[0..n], prefix[n] = the total.
+__global__ void __launch_bounds__(1024) dbde_prefix_kernel(const uint64_t *sizes, int n, uint64_t *prefix) {
+    __shared__ uint64_t s_warp[32];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    uint64_t carry = 0;
+    for (int b = 0; b < n; b += 1024) {
+        const int i = b + tid;
+        const uint64_t v = i < n ? sizes[i] : 0ull;
+        uint64_t incl = v;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const uint64_t u = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += u;
+        }
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        uint64_t before = carry, tot = 0;
+        for (int w = 0; w < 32; w++) {
+            before += w < warp ? s_warp[w] : 0ull;
+            tot += s_warp[w];
+        }
+        if (i < n) prefix[i] = before + incl - v;
+        carry += tot;
+        __syncthreads();
+    }
+    if (tid == 0) prefix[n] = carry;
+}
+
+// dbde_compact_kernel with the prefix given, one record row per gridDim.y rows
+__global__ void __launch_bounds__(256) dbde_compact_prefixed_kernel(const uint8_t *slots, uint64_t slot_stride, const uint64_t *sizes,
+                                                                    const uint64_t *prefix, int n, uint8_t *dst) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x, nt = (uint64_t)gridDim.x * blockDim.x;
+    for (int f = blockIdx.y; f < n; f += gridDim.y) {
+        const uint64_t bytes = sizes[f];
+        const uint8_t *src = slots + (uint64_t)f * slot_stride;
+        uint8_t *d = dst + prefix[f];
+        if ((((uintptr_t)src | (uintptr_t)d) & 7) == 0) {
+            const uint64_t *s8 = reinterpret_cast<const uint64_t *>(src);
+            const uint64_t n8 = bytes >> 3;
+            for (uint64_t i = t; i < n8; i += nt) st_stream_u64(d + 8 * i, __ldcs(s8 + i));
+            for (uint64_t i = (n8 << 3) + t; i < bytes; i += nt) d[i] = src[i];
+        } else {
+            for (uint64_t i = t; i < bytes; i += nt) d[i] = src[i];
+        }
+    }
+}
+
+cudaError_t launch_compact_prefixed(const uint8_t *slots, uint64_t slot_stride, const uint64_t *sizes, uint64_t *prefix, int n,
+                                    uint8_t *dst, cudaStream_t stream) {
+    if (n <= 0) return cudaSuccess;
+    dbde_prefix_kernel<<<1, 1024, 0, stream>>>(sizes, n, prefix);
+    unsigned bx = (unsigned)((slot_stride / 8 + 256 * 8 - 1) / (256 * 8));
+    if (bx < 1) bx = 1;
+    if (bx > 64) bx = 64;
+    const unsigned by = n < 65535 ? (unsigned)n : 65535u;
+    dbde_compact_prefixed_kernel<<<dim3(bx, by), 256, 0, stream>>>(slots, slot_stride, sizes, prefix, n, dst);
     return cudaGetLastError();
 }
 

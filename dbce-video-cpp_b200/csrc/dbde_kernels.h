@@ -19,6 +19,24 @@ struct EncParams {
     uint32_t flags;             // kFlagInvertRows
 };
 
+// Crop encode (dbde_encode.cu): record j = f * ncrops + r is the reference's record of the crop_w x crop_h image at
+// corner r of frame f (pixels outside the frame are the pad byte), at out + j * slot_stride.
+struct EncCropParams {
+    const uint8_t *frames;      // nframes * W * H, tightly packed, device, any alignment
+    int W, H;
+    const int32_t *corners;     // {x0, y0} of crop r of frame f at corners + 2 * (f * corner_stride + r), any int32 values
+    int ncrops, corner_stride;  // corner_stride: ncrops (per-frame corners) or 0 (shared)
+    int crop_w, crop_h, w, wh;  // the crop in pixels, its tile columns and tiles
+    uint64_t pad8;              // the pad byte in every byte
+    uint8_t *out;
+    uint64_t slot_stride;       // >= 32 + 66 * wh
+    uint64_t *frame_offsets;    // nrec entries (= j * slot_stride), device
+    uint64_t *frame_sizes;      // nrec entries (record bytes), device
+    uint64_t first_index;
+    int nrec;                   // nframes * ncrops
+    uint32_t flags;             // kFlagInvertRows
+};
+
 struct DecParams {
     PartGeom g;
     const uint8_t *stream;      // frame records, device
@@ -94,6 +112,12 @@ size_t dec_smem_bytes(const PartGeom &g);
 cudaError_t launch_encode(const EncParams &P, bool fast, int num_sms, cudaStream_t stream);
 cudaError_t launch_compact(const uint8_t *slots, uint64_t slot_stride, const uint64_t *sizes, int n, uint8_t *dst,
                            cudaStream_t stream);
+cudaError_t launch_encode_crops(const EncCropParams &P, int num_sms, cudaStream_t stream);
+// launch_compact for batches of thousands of records (crop encodes): the exclusive prefix of the sizes is computed
+// once into prefix (n + 1 entries, device; prefix[n] = the total), then the records are copied by a grid of at most
+// 65535 record rows.
+cudaError_t launch_compact_prefixed(const uint8_t *slots, uint64_t slot_stride, const uint64_t *sizes, uint64_t *prefix, int n,
+                                    uint8_t *dst, cudaStream_t stream);
 cudaError_t launch_decode_scan(const DecParams &P, cudaStream_t stream);
 cudaError_t launch_decode(const DecParams &P, bool fast, int num_sms, cudaStream_t stream);
 // Region-of-interest decode (dbde_roi.cu): the rectangle [x0, x0 + roi_w) x [y0, y0 + roi_h) of every frame into

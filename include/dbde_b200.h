@@ -221,6 +221,41 @@ DBDE_B200_API int dbde_b200_decode_crops_host(dbde_b200_ctx *ctx, const uint8_t 
                                               int crop_h, int pad, uint8_t *crops_host, uint32_t *status_host,
                                               uint64_t *indices_host);
 
+/* ---- crop encoding: N fixed-size windows of every frame, each recorded as a frame of its own ---------------------
+ * Records only the wells of a plate or a window that follows an animal instead of the whole sensor, without first
+ * gathering the windows into frames of their own.  The crop image is exactly what dbde_b200_decode_crops_* returns
+ * for the same arguments: corners are {x0, y0} int32 pairs, any values; corners_per_frame = 0: ncrops pairs for
+ * every frame, 1: nframes * ncrops pairs, frame f's at corners + 2 * f * ncrops; pixel (x, y) is frame[y0 + y][x0 + x]
+ * inside the frame and `pad` (0..255) outside it.  Record j = f * ncrops + r is byte for byte dbde_pack_frame(
+ * first_index + f, crop image (f, r), crop_w, crop_h): the reference's record of a crop_w x crop_h frame, so the
+ * records of one crop, in frame order behind a video header of crop_h x crop_w, are a .dbde video the reference's
+ * walker reads, and every crop keeps the source frame's index.  The clamp padding of the crop's partial last tile
+ * column and row repeats the crop image's last valid pixel, which may be `pad`.  Follows the context's
+ * DBDE_INVERT_ENDIAN setting (tile rows are reversed after the crop image is assembled).  frames: nframes * W * H
+ * bytes, tightly packed, any alignment; the only frame bytes read are in aligned 8-byte words that hold in-frame
+ * pixels of some crop, and a crop entirely outside the frame reads none.
+ * DBDE_B200_E_INVALID before any work is queued for: NULL pointers (when nframes > 0), the crop arguments
+ * dbde_b200_decode_crops_* rejects, frame dimensions the frame limits reject, a slot_stride below
+ * dbde_b200_frame_record_bound(crop_w, crop_h) (device form), and nframes * ncrops > 2^31 - 1.
+ * DBDE_B200_E_CAPACITY for out_capacity < nframes * ncrops * slot_stride (device form) or less than the records'
+ * total (host form).  nframes == 0 returns 0 (the host form writes frame_offsets_host[0] = 0).
+ * _device: record j at out_dev + j * slot_stride (slot_stride 0 = dbde_b200_slot_stride(crop_w, crop_h));
+ * frame_offsets_dev[j] = j * slot_stride and frame_sizes_dev[j] = the record's size, nframes * ncrops entries each;
+ * nothing outside [out_dev, out_dev + nframes * ncrops * slot_stride) is written.  Corners in device memory (a
+ * tracker on the GPU can feed its positions straight in); asynchronous on `stream`.  One CTA encodes one record, so
+ * a batch of fewer records than the GPU holds CTAs (a few large crops) does not fill the GPU.
+ * _host: the chunk pipeline of dbde_b200_encode_host, pinned or pageable buffers, synchronous; the records back to
+ * back in the same order, frame_offsets_host[0 .. nframes * ncrops] (the last entry is the total size). */
+DBDE_B200_API int dbde_b200_encode_crops_device(dbde_b200_ctx *ctx, const uint8_t *frames_dev, int W, int H,
+                                                uint64_t first_index, int nframes, const int32_t *corners_dev, int ncrops,
+                                                int corners_per_frame, int crop_w, int crop_h, int pad, uint8_t *out_dev,
+                                                size_t out_capacity, size_t slot_stride, uint64_t *frame_offsets_dev,
+                                                uint64_t *frame_sizes_dev, void *stream);
+DBDE_B200_API int dbde_b200_encode_crops_host(dbde_b200_ctx *ctx, const uint8_t *frames_host, int W, int H,
+                                              uint64_t first_index, int nframes, const int32_t *corners_host, int ncrops,
+                                              int corners_per_frame, int crop_w, int crop_h, int pad, uint8_t *out_host,
+                                              size_t out_capacity, uint64_t *frame_offsets_host);
+
 /* ---- binned: every frame at 1/2, 1/4 or 1/8 of its size, as block means ---------------------------------------
  * The whole field of view at lower resolution -- a tracker on a quarter-size image, previews, motion energy over a
  * plate, a network that takes downsampled frames -- without writing the full-size frame anywhere.  factor must be
