@@ -43,6 +43,7 @@ C_SYMBOLS = [
     "dbde_b200_decode16_crops_device", "dbde_b200_decode16_crops_host",
     "dbde_b200_decode16_binned_device", "dbde_b200_decode16_binned_host",
     "dbde_b200_encode_crops_device", "dbde_b200_encode_crops_host",
+    "dbde_b200_encode16_crops_device", "dbde_b200_encode16_crops_host",
 ]
 # the reference's C++ entry points (include/dbde_util.h), by mangled name (SURVEY.md 8b)
 CXX_SYMBOLS = {
@@ -162,6 +163,8 @@ def load():
                                                   C.c_void_p, C.c_void_p]
     lib.dbde_b200_encode_crops_host.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_uint64, C.c_int, C.c_void_p, C.c_int,
                                                 C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]
+    lib.dbde_b200_encode16_crops_device.argtypes = lib.dbde_b200_encode_crops_device.argtypes
+    lib.dbde_b200_encode16_crops_host.argtypes = lib.dbde_b200_encode_crops_host.argtypes
     lib.dbde_b200_file_last_error.restype = C.c_char_p
     return lib
 
@@ -420,6 +423,41 @@ class Codec:
         self._ck(self.lib.dbde_b200_encode16_host(self.h, frames.ctypes.data, W, H, first_index, N, out.ctypes.data, cap,
                                                   offs.ctypes.data), "encode16_host")
         return out[:int(offs[N])].copy(), offs
+
+    def encode16_crops_device(self, frames_ptr, W, H, first_index, n, corners_ptr, ncrops, per_frame, size, out_ptr, out_cap,
+                              offs_ptr, sizes_ptr, pad=0, stream=0, slot_stride=0):
+        """U16 frames (2-byte aligned): ncrops crops of size = (crop_w, crop_h) per frame at the int32 {x0, y0} corners at
+        corners_ptr (device; per_frame: n * ncrops pairs, else ncrops pairs for every frame), pixels outside the frame
+        `pad` (0..65535): record f * ncrops + r is the DBDE16 record of crop r of frame f as a crop_w x crop_h frame with
+        index first_index + f, at out_ptr + (f * ncrops + r) * slot_stride; offs[j] = j * slot_stride, sizes[j] = record
+        bytes"""
+        cw, ch = (int(v) for v in size)
+        self._ck(self.lib.dbde_b200_encode16_crops_device(self.h, frames_ptr, W, H, first_index, n, corners_ptr, ncrops,
+                                                          int(per_frame), cw, ch, pad, out_ptr, out_cap, slot_stride, offs_ptr,
+                                                          sizes_ptr, stream), "encode16_crops_device")
+
+    def encode16_crops_host(self, frames, corners, size, pad=0, first_index=0):
+        """frames (N,H,W) u16, crops of size = (crop_w, crop_h) at int32 corners (R, 2) (the same for every frame) or
+        (N, R, 2) (per frame), pixels outside the frame `pad` -> (stream bytes, offsets[N*R+1]); record f * R + r is the
+        DBDE16 record of crop r of frame f, with frame index first_index + f"""
+        frames = np.ascontiguousarray(frames, dtype=np.uint16)
+        corners = np.ascontiguousarray(corners, dtype=np.int32)
+        N, H, W = frames.shape
+        cw, ch = (int(v) for v in size)
+        if corners.ndim == 3 and corners.shape[0] == N and corners.shape[2] == 2:
+            per_frame = 1
+        elif corners.ndim == 2 and corners.shape[1] == 2:
+            per_frame = 0
+        else:
+            raise ValueError("corners must have shape (R, 2) or (N, R, 2), got %r" % (corners.shape,))
+        R = corners.shape[-2]
+        cap = int(self.lib.dbde_b200_slot_stride16(cw, ch)) * max(N * R, 1) + 16 if cw > 0 and ch > 0 else 16
+        out = np.empty(cap, dtype=np.uint8)
+        offs = np.zeros(N * R + 1, dtype=np.uint64)
+        self._ck(self.lib.dbde_b200_encode16_crops_host(self.h, frames.ctypes.data, W, H, first_index, N, corners.ctypes.data, R,
+                                                        per_frame, cw, ch, pad, out.ctypes.data, cap, offs.ctypes.data),
+                 "encode16_crops_host")
+        return out[:int(offs[N * R])].copy(), offs
 
     def decode16_host(self, stream, offsets, W, H, fill=None):
         """-> (frames (N,H,W) u16, status[N], indices[N]); rejected frames keep `fill`"""

@@ -108,7 +108,47 @@ __device__ __forceinline__ void store_tile16(uint16_t *frame, int W, int H, int 
     }
 }
 
+// The 8 pixels of the combined row [prev (pixels 0-7), x (pixels 8-15)] starting at pixel 8 - s, s = 0..7: a shifter
+// of selects that is branch-free for any s, so segments of one warp may differ in s
+__device__ __forceinline__ uint4 shift_in16(uint4 prev, uint4 x, uint32_t s) {
+    const uint32_t v[8] = {prev.x, prev.y, prev.z, prev.w, x.x, x.y, x.z, x.w};
+    const uint32_t q = s >> 1;
+    uint32_t a[6], u[5];
+#pragma unroll
+    for (int i = 0; i < 6; i++) a[i] = (q & 2u) ? v[i] : v[i + 2];            // a[i] = v[2 + i - 2 (q >> 1)]
+#pragma unroll
+    for (int i = 0; i < 5; i++) u[i] = (q & 1u) ? a[i] : a[i + 1];            // u[i] = v[3 + i - q]
+    uint32_t r[4];
+#pragma unroll
+    for (int j = 0; j < 4; j++) r[j] = (s & 1u) ? __funnelshift_r(u[j], u[j + 1], 16) : u[j + 1];
+    return make_uint4(r[0], r[1], r[2], r[3]);
+}
+
 // ------------------------------------------------------------------ encoder
+// The pair packer every DBDE16 encoder shares: (p - min), k bits each, LSB first, two pixels (2k bits) per step into a
+// 64-bit accumulator, flushed 32 bits at a time to the staging at shared address sbase in the padded layout (pad16);
+// the tile's k U64 words start at 32-bit unit `unit` of the staging.  k = 1..16: a tile of depth 0 has no words.
+__device__ __forceinline__ void pack_tile16(uint32_t sbase, uint32_t unit, int k, uint32_t mn, const uint32_t (&px)[32]) {
+    const uint32_t m2 = mn * 0x00010001u, kk = 2u * (uint32_t)k;
+    uint32_t acc = 0, fill = 0;                                          // `fill` (< 32) valid low bits in acc
+    const uint32_t kmul = 1u << k;
+#pragma unroll
+    for (int i = 0; i < 32; i++) {
+        const uint32_t d = px[i] - m2;                                   // no borrow: every pixel >= min
+        const uint32_t pair = (d >> 16) * kmul + (d & 0xffffu);          // 2k bits
+        const uint32_t lo = acc | (pair << fill);
+        const uint32_t hi = __funnelshift_l(pair, 0u, fill);             // what does not fit in 32 bits (0 when fill == 0)
+        fill += kk;
+        // a unit is complete: predicated store (no branch), carry the overflow
+        asm volatile("{\n\t.reg .pred p;\n\tsetp.ge.u32 p, %2, 32;\n\t@p st.shared.u32 [%0], %1;\n\t}"
+                     ::"r"(sbase + 4u * pad16(unit)), "r"(lo), "r"(fill) : "memory");
+        const bool full = fill >= 32u;
+        acc = full ? hi : lo;
+        unit += full ? 1u : 0u;
+        fill &= 31u;
+    }
+}
+
 __global__ void __launch_bounds__(kT16, 4) dbde16_encode_kernel(const Enc16Params P) {
     extern __shared__ __align__(16) uint8_t s_words[];
     __shared__ uint32_t s_ticket, s_wtot[kT16 / 32];
@@ -163,30 +203,8 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_kernel(const Enc16Param
                 s_excl = excl;
             }
         }
-        // pack (p - min), k bits each, LSB first: two pixels (2k bits) per step into a 64-bit accumulator,
-        // flushed to shared memory 32 bits at a time; the tile's k U64 words start at word `off` of the partition
-        if (k > 0) {
-            const uint32_t m2 = mn * 0x00010001u, kk = 2u * (uint32_t)k;
-            const uint32_t sbase = smem_u32(s_words);
-            uint32_t unit = 2u * (wbase + incl - (uint32_t)k);                   // 32-bit unit inside the partition's words
-            uint32_t acc = 0, fill = 0;                                          // `fill` (< 32) valid low bits in acc
-            const uint32_t kmul = 1u << k;
-#pragma unroll
-            for (int i = 0; i < 32; i++) {
-                const uint32_t d = px[i] - m2;                                   // no borrow: every pixel >= min
-                const uint32_t pair = (d >> 16) * kmul + (d & 0xffffu);          // 2k bits
-                const uint32_t lo = acc | (pair << fill);
-                const uint32_t hi = __funnelshift_l(pair, 0u, fill);             // what does not fit in 32 bits (0 when fill == 0)
-                fill += kk;
-                // a unit is complete: predicated store (no branch), carry the overflow
-                asm volatile("{\n\t.reg .pred p;\n\tsetp.ge.u32 p, %2, 32;\n\t@p st.shared.u32 [%0], %1;\n\t}"
-                             ::"r"(sbase + 4u * pad16(unit)), "r"(lo), "r"(fill) : "memory");
-                const bool full = fill >= 32u;
-                acc = full ? hi : lo;
-                unit += full ? 1u : 0u;
-                fill &= 31u;
-            }
-        }
+        // the tile's words start at word wbase + incl - k of the partition
+        if (k > 0) pack_tile16(smem_u32(s_words), 2u * (wbase + incl - (uint32_t)k), k, mn, px);
         __syncthreads();                                      // words staged, s_excl published
         const uint64_t excl = s_excl;
         uint8_t *rec = P.out + (size_t)f * P.slot_stride;
@@ -222,6 +240,142 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_kernel(const Enc16Param
             }
         }
         __syncthreads();                                      // s_words / s_ticket are reused by the next partition
+    }
+}
+
+// ------------------------------------------------------------------ crop encoder
+// dbde_encode_crops_kernel's scheme with DBDE16 tiles: one CTA per record (frame f, crop r) of a persistent grid, one
+// lane per tile of the crop.  The CTA walks the crop's tiles in raster order, 256 at a time; a record's word offsets
+// depend on its own tiles only, so a CTA-wide scan per chunk plus a running carry replaces the frame encoder's look-back
+// and tickets, and no scratch is zeroed.  Each warp packs its 32 tiles into a region of its own of the staging (1024
+// units, at most 32 tiles of 16 words), so the scan's one barrier per chunk is the only CTA-wide wait.
+
+// The 8 rows of crop tile (tx, ty): pixel (x, y) of the crop image is frame[y0 + y][x0 + x] inside the frame and pad
+// outside it; the clamp padding at the crop's own partial last column / row repeats the crop image's last valid pixel
+// (dbde_util.cpp:105-135), which may be pad.  A tile inside the frame and the crop loads each row as the one or two
+// aligned 16-byte words it touches and shifts the 8 pixels out of them (any x0, any W, any 2-byte aligned frame base);
+// a tile at an edge reads each in-frame pixel it needs as a U16 and nothing else.
+__device__ __forceinline__ void load_crop_tile16(const Enc16CropParams &P, const uint16_t *fr, long long x0, long long y0, int tx, int ty,
+                                                 uint32_t (&px)[32]) {
+    const long long xs = x0 + 8 * tx, ys = y0 + 8 * ty;
+    const bool inner = 8 * tx + 8 <= P.crop_w && 8 * ty + 8 <= P.crop_h && xs >= 0 && xs + 8 <= P.W && ys >= 0 && ys + 8 <= P.H;
+    if (inner) {
+        const uint16_t *p = fr + (size_t)ys * (size_t)P.W + (size_t)xs;
+#pragma unroll
+        for (int r = 0; r < 8; r++) {
+            const uint4 *a = reinterpret_cast<const uint4 *>((uintptr_t)p & ~(uintptr_t)15);
+            const uint32_t s = ((uint32_t)(uintptr_t)p & 15u) >> 1;              // the row starts at pixel s of word a
+            uint4 v = __ldg(a);
+            if (s) v = shift_in16(v, __ldg(a + 1), 8u - s);
+            px[4 * r] = v.x; px[4 * r + 1] = v.y; px[4 * r + 2] = v.z; px[4 * r + 3] = v.w;
+            p += P.W;
+        }
+        return;
+    }
+#pragma unroll
+    for (int r = 0; r < 8; r++) {
+        const long long y = y0 + min(8 * ty + r, P.crop_h - 1);
+        if (y >= 0 && y < P.H) {
+            const uint16_t *row = fr + (size_t)y * (size_t)P.W;
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                const long long xa = x0 + min(8 * tx + 2 * j, P.crop_w - 1), xb = x0 + min(8 * tx + 2 * j + 1, P.crop_w - 1);
+                const uint32_t a = xa >= 0 && xa < P.W ? (uint32_t)__ldg(row + xa) : P.pad;
+                const uint32_t b = xb >= 0 && xb < P.W ? (uint32_t)__ldg(row + xb) : P.pad;
+                px[4 * r + j] = a | (b << 16);
+            }
+        } else {
+#pragma unroll
+            for (int j = 0; j < 4; j++) px[4 * r + j] = P.pad * 0x00010001u;
+        }
+    }
+}
+
+constexpr uint32_t kCropWarpUnits16 = 32 * 16 * 2;   // one warp's staging region: 32 tiles of at most 16 U64 words
+
+__global__ void __launch_bounds__(kT16, 4) dbde16_encode_crops_kernel(const Enc16CropParams P) {
+    extern __shared__ __align__(16) uint8_t s_words[];
+    __shared__ uint32_t s_wtot[2][kT16 / 32];                // each warp's word count, by chunk parity
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const size_t fpix = (size_t)P.W * (size_t)P.H;
+    const size_t fixed = 32 + 3 * (size_t)P.wh;
+    const uint32_t wunit = (uint32_t)warp * kCropWarpUnits16;   // a multiple of 32: pad16(wunit + u) = pad16(wunit) + pad16(u)
+    const uint32_t *su = reinterpret_cast<const uint32_t *>(s_words);
+    unsigned cc = 0;                                         // chunks done by this CTA: selects the s_wtot half
+    for (int j = blockIdx.x; j < P.nrec; j += gridDim.x) {
+        const int f = j / P.ncrops, r = j - f * P.ncrops;
+        const int32_t *cp = P.corners + 2 * ((size_t)f * (size_t)P.corner_stride + (size_t)r);
+        const long long x0 = __ldg(cp), y0 = __ldg(cp + 1);
+        const uint16_t *fr = P.frames + (size_t)f * fpix;
+        uint8_t *rec = P.out + (size_t)j * P.slot_stride;
+        uint32_t carry = 0;                                  // U64 words of the record's earlier chunks
+        for (int t0 = 0; t0 < P.wh; t0 += kT16, cc++) {
+            const int t = t0 + tid;
+            const bool valid = t < P.wh;
+            uint32_t px[32];
+            if (valid) {
+                const int ty = t / P.w;
+                load_crop_tile16(P, fr, x0, y0, t - ty * P.w, ty, px);
+            } else {
+#pragma unroll
+                for (int i = 0; i < 32; i++) px[i] = 0;
+            }
+            // dbde16_encode_kernel's tile: min / max (VIMNMX.U16x2), depth, the pair packer
+            uint32_t lo2 = px[0], hi2 = px[0];
+#pragma unroll
+            for (int i = 1; i < 32; i++) {
+                lo2 = __vminu2(lo2, px[i]);
+                hi2 = __vmaxu2(hi2, px[i]);
+            }
+            const uint32_t mn = min(lo2 & 0xffffu, lo2 >> 16), mx = max(hi2 & 0xffffu, hi2 >> 16);
+            const int k = 32 - __clz((int)(mx - mn));        // 0 for the zeros past the crop's last tile
+            const uint32_t incl = warp_inclusive_scan((uint32_t)k, lane);
+            if (lane == 31) s_wtot[cc & 1][warp] = incl;
+            if (k > 0) pack_tile16(smem_u32(s_words), wunit + 2u * (incl - (uint32_t)k), k, mn, px);
+            // depth and minimum planes (dbde_util.cpp:156-157), the minimum little-endian U16
+            if (valid) {
+                rec[24 + (size_t)t] = (uint8_t)k;
+                rec[28 + (size_t)P.wh + 2 * (size_t)t] = (uint8_t)mn;
+                rec[29 + (size_t)P.wh + 2 * (size_t)t] = (uint8_t)(mn >> 8);
+            }
+            __syncthreads();                                 // every warp's count is in shared memory
+            uint32_t wbase = 0, tot = 0;
+#pragma unroll
+            for (int w = 0; w < kT16 / 32; w++) {
+                const uint32_t v = s_wtot[cc & 1][w];
+                wbase += w < warp ? v : 0u;
+                tot += v;
+            }
+            // this warp's words: one coalesced run
+            const uint32_t n = s_wtot[cc & 1][warp];
+            uint8_t *dst = rec + fixed + 8 * ((size_t)carry + wbase);
+            if (((uintptr_t)dst & 7) == 0) {
+                for (uint32_t i = lane; i < n; i += 32)
+                    st_stream_u64(dst + 8 * (size_t)i, (uint64_t)su[pad16(wunit + 2u * i)] | ((uint64_t)su[pad16(wunit + 2u * i + 1u)] << 32));
+            } else {
+                for (uint32_t i = lane; i < 8u * n; i += 32) dst[i] = s_words[4u * pad16(wunit + (i >> 2)) + (i & 3u)];
+            }
+            carry += tot;
+            __syncwarp();                                    // the copy has read the staging before the next chunk packs into it
+        }
+        if (warp == 0) {
+            // the fixed fields (dbde_util.cpp:141-146,182-188,191), as dbde16_encode_kernel writes them
+            const uint64_t index = P.first_index + (uint64_t)f;
+            const uint32_t wh = (uint32_t)P.wh;
+            uint32_t b;
+            uint8_t *d8;
+            if (lane < 4) { b = (2u >> (8 * lane)) & 0xff; d8 = rec + lane; }
+            else if (lane < 12) { b = (uint32_t)(index >> (8 * (lane - 4))) & 0xff; d8 = rec + lane; }
+            else if (lane < 20) { b = 0; d8 = rec + lane; }
+            else if (lane < 24) { b = (wh >> (8 * (lane - 20))) & 0xff; d8 = rec + lane; }
+            else if (lane < 28) { b = ((2u * wh) >> (8 * (lane - 24))) & 0xff; d8 = rec + 24 + (size_t)wh + (lane - 24); }
+            else { b = (carry >> (8 * (lane - 28))) & 0xff; d8 = rec + 28 + 3 * (size_t)wh + (lane - 28); }
+            *d8 = (uint8_t)b;
+            if (lane == 0) {
+                P.frame_offsets[j] = (uint64_t)j * P.slot_stride;
+                P.frame_sizes[j] = fixed + 8ull * carry;
+            }
+        }
     }
 }
 
@@ -540,22 +694,6 @@ constexpr int kCrop16Warps = 8;
 // units; 32 / S segments per warp
 constexpr int kCrop16BufUnits = 1120;
 
-// The 8 pixels of the combined row [prev (pixels 0-7), x (pixels 8-15)] starting at pixel 8 - s, s = 0..7: a shifter
-// of selects that is branch-free for any s, so segments of one warp may differ in s
-__device__ __forceinline__ uint4 shift_in16(uint4 prev, uint4 x, uint32_t s) {
-    const uint32_t v[8] = {prev.x, prev.y, prev.z, prev.w, x.x, x.y, x.z, x.w};
-    const uint32_t q = s >> 1;
-    uint32_t a[6], u[5];
-#pragma unroll
-    for (int i = 0; i < 6; i++) a[i] = (q & 2u) ? v[i] : v[i + 2];            // a[i] = v[2 + i - 2 (q >> 1)]
-#pragma unroll
-    for (int i = 0; i < 5; i++) u[i] = (q & 1u) ? a[i] : a[i + 1];            // u[i] = v[3 + i - q]
-    uint32_t r[4];
-#pragma unroll
-    for (int j = 0; j < 4; j++) r[j] = (s & 1u) ? __funnelshift_r(u[j], u[j + 1], 16) : u[j + 1];
-    return make_uint4(r[0], r[1], r[2], r[3]);
-}
-
 // pixels [st, en) of the 16-byte-aligned 8-pixel word w at q, as naturally aligned pieces
 __device__ __forceinline__ void store_pixels16(uint16_t *q, uint4 w, int st, int en) {
     uint8_t *q8 = reinterpret_cast<uint8_t *>(q);
@@ -715,6 +853,10 @@ static cudaError_t launch16(Kern kern, const Params &P, unsigned nparts, int num
 
 cudaError_t launch_encode16(const Enc16Params &P, int num_sms, cudaStream_t stream) {
     return launch16(dbde16_encode_kernel, P, P.nparts, num_sms, stream);
+}
+cudaError_t launch_encode16_crops(const Enc16CropParams &P, int num_sms, cudaStream_t stream) {
+    if (P.nrec <= 0) return cudaSuccess;
+    return launch16(dbde16_encode_crops_kernel, P, (unsigned)P.nrec, num_sms, stream);
 }
 cudaError_t launch_decode16_scan(const Dec16Params &P, cudaStream_t stream) {
     if (P.nframes <= 0) return cudaSuccess;

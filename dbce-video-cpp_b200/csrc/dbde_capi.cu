@@ -904,14 +904,14 @@ struct EncSequencer {
 };
 
 // Worker `my` of `nworkers`: encodes chunks my, my + nworkers, ... of the batch on context c.  crops: every frame
-// gives crops->ncrops records of crops->w x crops->h (dbde_b200_encode_crops_device) instead of its own record; the
-// chunk's corners travel behind its frames in the slot's frame buffer.
+// gives crops->ncrops records of crops->w x crops->h (dbde_b200_encode_crops_device, or dbde_b200_encode16_crops_device
+// when u16) instead of its own record; the chunk's corners travel behind its frames in the slot's frame buffer.
 static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index,
                               int nframes, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host,
                               int chunk, int my, int nworkers, EncSequencer *seq, bool u16 = false, const SubFrame *crops = nullptr) {
     CK(cudaSetDevice(c->device));
-    const HostFmt F = crops ? host_fmt(crops->w, crops->h, false) : host_fmt(W, H, u16);   // the records' format
-    const size_t px = crops ? (size_t)W * (size_t)H : F.px;                                  // input bytes per frame
+    const HostFmt F = crops ? host_fmt(crops->w, crops->h, u16) : host_fmt(W, H, u16);     // the records' format
+    const size_t px = crops ? (size_t)W * (size_t)H * (u16 ? 2 : 1) : F.px;                 // input bytes per frame
     const int per = crops ? crops->ncrops : 1;                                                // records per frame
     const int nrec = chunk * per;                                                             // records per chunk
     const size_t delta = F.delta;
@@ -1004,9 +1004,13 @@ static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int 
         }
         prof.mark(1, "h2d");
         prof.gpu_mark(1, s.st);
-        rc_all = crops ? dbde_b200_encode_crops_device(c, s.d_a, W, H, first_index + s.first, s.n, (const int32_t *)(s.d_a + corner_at),
-                                                       crops->ncrops, crops->per_frame, crops->w, crops->h, crops->pad, s.d_b + delta,
-                                                       need_b - 32, stride, s.d_off, s.d_size, s.st)
+        rc_all = crops && u16 ? dbde_b200_encode16_crops_device(c, (const uint16_t *)s.d_a, W, H, first_index + s.first, s.n,
+                                                                (const int32_t *)(s.d_a + corner_at), crops->ncrops, crops->per_frame,
+                                                                crops->w, crops->h, crops->pad, s.d_b + delta, need_b - 32, stride,
+                                                                s.d_off, s.d_size, s.st)
+                 : crops ? dbde_b200_encode_crops_device(c, s.d_a, W, H, first_index + s.first, s.n, (const int32_t *)(s.d_a + corner_at),
+                                                         crops->ncrops, crops->per_frame, crops->w, crops->h, crops->pad, s.d_b + delta,
+                                                         need_b - 32, stride, s.d_off, s.d_size, s.st)
                  : u16 ? dbde_b200_encode16_device(c, (const uint16_t *)s.d_a, W, H, first_index + s.first, s.n, s.d_b + delta,
                                                    need_b - 32, stride, s.d_off, s.d_size, s.st)
                        : dbde_b200_encode_device(c, s.d_a, W, H, first_index + s.first, s.n, s.d_b + delta, need_b - 32, stride,
@@ -1059,32 +1063,48 @@ extern "C" int dbde_b200_encode_host(dbde_b200_ctx *c, const uint8_t *frames_hos
     return 0;
 }
 
-// The host form of dbde_b200_encode_crops_device: the encode_host chunk pipeline with ncrops records per frame; each
-// chunk's corners go up behind its frames.
-extern "C" int dbde_b200_encode_crops_host(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index,
-                                           int nframes, const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
-                                           int crop_h, int pad, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host) {
-    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
+// The host forms of dbde_b200_encode_crops_device and dbde_b200_encode16_crops_device (u16): the encode_host chunk
+// pipeline with ncrops records per frame; each chunk's corners go up behind its frames.
+static int encode_crops_host_impl(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index, int nframes,
+                                  const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w, int crop_h, int pad,
+                                  uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host, bool u16) {
+    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad, u16 ? 65535 : 255) ||
         (nframes > 0 && (!frames_host || !corners_host || !out_host || !frame_offsets_host)))
-        return fail(DBDE_B200_E_INVALID, "encode_crops_host: bad argument");
+        return fail(DBDE_B200_E_INVALID, u16 ? "encode16_crops_host: bad argument" : "encode_crops_host: bad argument");
     if (nframes == 0) {
         if (frame_offsets_host) frame_offsets_host[0] = 0;
         return 0;
     }
-    if ((long long)nframes * ncrops > 0x7FFFFFFFLL) return fail(DBDE_B200_E_INVALID, "encode_crops_host: nframes * ncrops > 2^31 - 1");
-    int chunk = default_chunk(c, W, H, nframes);
-    const size_t rec = (size_t)ncrops * dbde_b200_slot_stride(crop_w, crop_h);    // one frame's record slots
-    if (rec > dbde_b200_slot_stride(W, H)) {       // crops larger than the frame: a chunk's records stay within 64 MiB
+    if ((long long)nframes * ncrops > 0x7FFFFFFFLL)
+        return fail(DBDE_B200_E_INVALID, u16 ? "encode16_crops_host: nframes * ncrops > 2^31 - 1" : "encode_crops_host: nframes * ncrops > 2^31 - 1");
+    int chunk = default_chunk(c, W, H, nframes, u16);
+    const HostFmt crop = host_fmt(crop_w, crop_h, u16), frame = host_fmt(W, H, u16);
+    const size_t rec = (size_t)ncrops * crop.stride;                   // one frame's record slots
+    if (rec > frame.stride) {                      // crops larger than the frame: a chunk's records stay within 64 MiB
         const size_t most = (64u << 20) / rec;
         if ((size_t)chunk > most) chunk = most > 0 ? (int)most : 1;
     }
     const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad, 0};
     EncSequencer seq;
     int rc = encode_host_worker(c, frames_host, W, H, first_index, nframes, out_host, out_capacity, frame_offsets_host, chunk, 0, 1,
-                                &seq, false, &crops);
+                                &seq, u16, &crops);
     if (rc) return rc;
     frame_offsets_host[(size_t)nframes * ncrops] = seq.out_pos;
     return 0;
+}
+
+extern "C" int dbde_b200_encode_crops_host(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index,
+                                           int nframes, const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
+                                           int crop_h, int pad, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host) {
+    return encode_crops_host_impl(c, frames_host, W, H, first_index, nframes, corners_host, ncrops, corners_per_frame, crop_w, crop_h,
+                                  pad, out_host, out_capacity, frame_offsets_host, false);
+}
+
+extern "C" int dbde_b200_encode16_crops_host(dbde_b200_ctx *c, const uint16_t *frames_host, int W, int H, uint64_t first_index,
+                                             int nframes, const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
+                                             int crop_h, int pad, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host) {
+    return encode_crops_host_impl(c, (const uint8_t *)frames_host, W, H, first_index, nframes, corners_host, ncrops, corners_per_frame,
+                                  crop_w, crop_h, pad, out_host, out_capacity, frame_offsets_host, true);
 }
 
 static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
@@ -1331,6 +1351,48 @@ extern "C" int dbde_b200_encode16_device(dbde_b200_ctx *c, const uint16_t *frame
     P.first_index = first_index; P.nframes = nframes; P.nparts = (unsigned)nparts;
     P.aligned = (W % 8 == 0) && (((uintptr_t)frames_dev & 15) == 0);
     CK(launch_encode16(P, c->num_sms, st));
+    c->launches += 1;
+    return 0;
+}
+
+// One CTA per record of a persistent grid, one lane per crop tile (dbde16.cu): dbde_b200_encode_crops_device with U16
+// pixels.  A crop equal to the frame still runs the crop kernel: its records are the frame encoder's records.
+extern "C" int dbde_b200_encode16_crops_device(dbde_b200_ctx *c, const uint16_t *frames_dev, int W, int H, uint64_t first_index,
+                                               int nframes, const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
+                                               int crop_h, int pad, uint8_t *out_dev, size_t out_capacity, size_t slot_stride,
+                                               uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev, void *stream) {
+    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad, 65535) ||
+        (nframes > 0 && (!frames_dev || !corners_dev || !out_dev || !frame_offsets_dev || !frame_sizes_dev)) ||
+        ((uintptr_t)frames_dev & 1))
+        return fail(DBDE_B200_E_INVALID, "encode16_crops_device: bad argument");
+    if (nframes == 0) return 0;
+    if (slot_stride == 0) slot_stride = dbde_b200_slot_stride16(crop_w, crop_h);
+    if (slot_stride < dbde_b200_frame_record_bound16(crop_w, crop_h))
+        return fail(DBDE_B200_E_INVALID, "encode16_crops_device: slot_stride < dbde_b200_frame_record_bound16(crop_w, crop_h)");
+    const long long nrec = (long long)nframes * ncrops;
+    if (nrec > 0x7FFFFFFFLL) return fail(DBDE_B200_E_INVALID, "encode16_crops_device: nframes * ncrops > 2^31 - 1");
+    if (slot_stride > out_capacity / (size_t)nrec)
+        return fail(DBDE_B200_E_CAPACITY, "encode16_crops_device: out_capacity < nframes * ncrops * slot_stride");
+    CK(cudaSetDevice(c->device));
+    Enc16CropParams P;
+    P.frames = frames_dev;
+    P.W = W;
+    P.H = H;
+    P.corners = corners_dev;
+    P.ncrops = ncrops;
+    P.corner_stride = corners_per_frame ? ncrops : 0;
+    P.crop_w = crop_w;
+    P.crop_h = crop_h;
+    P.w = (crop_w + 7) / 8;
+    P.wh = P.w * ((crop_h + 7) / 8);
+    P.pad = (uint32_t)pad;
+    P.out = out_dev;
+    P.slot_stride = slot_stride;
+    P.frame_offsets = frame_offsets_dev;
+    P.frame_sizes = frame_sizes_dev;
+    P.first_index = first_index;
+    P.nrec = (int)nrec;
+    CK(launch_encode16_crops(P, c->num_sms, (cudaStream_t)stream));
     c->launches += 1;
     return 0;
 }

@@ -88,7 +88,24 @@ struct Dec16Params {
     int W, H, w, h, wh, ppf, nframes, aligned;
     unsigned nparts;
 };
+// DBDE16 crop encode (dbde16.cu): record j = f * ncrops + r is the DBDE16 record of the crop_w x crop_h image at corner
+// r of frame f (pixels outside the frame are pad), at out + j * slot_stride.
+struct Enc16CropParams {
+    const uint16_t *frames;     // nframes * W * H u16, tightly packed, device, 2-byte aligned
+    int W, H;
+    const int32_t *corners;     // {x0, y0} of crop r of frame f at corners + 2 * (f * corner_stride + r), any int32 values
+    int ncrops, corner_stride;  // corner_stride: ncrops (per-frame corners) or 0 (shared)
+    int crop_w, crop_h, w, wh;  // the crop in pixels, its tile columns and tiles
+    uint32_t pad;               // 0..65535
+    uint8_t *out;
+    uint64_t slot_stride;       // >= 32 + 131 * wh
+    uint64_t *frame_offsets;    // nrec entries (= j * slot_stride), device
+    uint64_t *frame_sizes;      // nrec entries (record bytes), device
+    uint64_t first_index;
+    int nrec;                   // nframes * ncrops
+};
 cudaError_t launch_encode16(const Enc16Params &P, int num_sms, cudaStream_t stream);
+cudaError_t launch_encode16_crops(const Enc16CropParams &P, int num_sms, cudaStream_t stream);
 cudaError_t launch_decode16_scan(const Dec16Params &P, cudaStream_t stream);
 cudaError_t launch_decode16(const Dec16Params &P, int num_sms, cudaStream_t stream);
 // DBDE16 crop decode (dbde16.cu), after launch_decode16_scan(scan): ncrops rectangles of crop_w x crop_h per frame with

@@ -334,6 +334,42 @@ DBDE_B200_API int dbde_b200_decode16_crops_host(dbde_b200_ctx *ctx, const uint8_
                                                 int crop_h, int pad, uint16_t *crops_host, uint32_t *status_host,
                                                 uint64_t *indices_host);
 
+/* ---- DBDE16 crop encoding: N fixed-size windows of every 16-bit frame, each recorded as a frame of its own ----------
+ * dbde_b200_encode_crops_* for 16-bit frames: records only the wells of a plate or a window that follows an animal
+ * instead of the whole sensor, without first gathering the windows into frames of their own.  Arguments and semantics
+ * are those of dbde_b200_encode_crops_*, with pixels counted as U16.  The crop image is exactly what
+ * dbde_b200_decode16_crops_* returns for the same arguments: corners are {x0, y0} int32 pairs, any values;
+ * corners_per_frame = 0: ncrops pairs for every frame, 1: nframes * ncrops pairs, frame f's at corners + 2 * f * ncrops;
+ * pixel (x, y) is frame[y0 + y][x0 + x] inside the frame and `pad` (0..65535) outside it.  Record j = f * ncrops + r is
+ * byte for byte the DBDE16 record of the crop_w x crop_h crop image (f, r) with frame index first_index + f:
+ *   I32 2 | U64 index | F64 0.0 | I32 wh | U8 depth[wh] | I32 2*wh | U16 min[wh] | I32 n64 | U64 words[n64]
+ * The clamp padding of the crop's partial last tile column and row repeats the crop image's last valid pixel, which may
+ * be `pad`.  Like every DBDE16 call, these ignore the context's DBDE_INVERT_ENDIAN setting: DBDE16 has no such
+ * variant.  frames: nframes * W * H U16, tightly packed, 2-byte aligned; the only frame bytes read are in aligned
+ * 16-byte words that hold in-frame pixels of some crop, and a crop entirely outside the frame reads none.
+ * DBDE_B200_E_INVALID before any work is queued for: NULL pointers (when nframes > 0), a frame pointer that is not
+ * 2-byte aligned (device form), the crop arguments dbde_b200_decode16_crops_* rejects, frame dimensions the frame limits
+ * reject, a slot_stride below dbde_b200_frame_record_bound16(crop_w, crop_h) (device form), and nframes * ncrops >
+ * 2^31 - 1.  DBDE_B200_E_CAPACITY for out_capacity < nframes * ncrops * slot_stride (device form) or less than the
+ * records' total (host form).  nframes == 0 returns 0 (the host form writes frame_offsets_host[0] = 0).
+ * _device: record j at out_dev + j * slot_stride (slot_stride 0 = dbde_b200_slot_stride16(crop_w, crop_h));
+ * frame_offsets_dev[j] = j * slot_stride and frame_sizes_dev[j] = the record's size, nframes * ncrops entries each;
+ * nothing outside [out_dev, out_dev + nframes * ncrops * slot_stride) is written, nor anything between a record's end
+ * and its slot's end.  Corners in device memory; asynchronous on `stream`; one kernel launch and nothing else (no
+ * scratch, no memset).  One CTA encodes one record, so a batch of fewer records than the GPU holds CTAs does not
+ * fill the GPU.
+ * _host: the chunk pipeline of dbde_b200_encode16_host, pinned or pageable buffers, synchronous; the records back to
+ * back in the same order, frame_offsets_host[0 .. nframes * ncrops] (the last entry is the total size). */
+DBDE_B200_API int dbde_b200_encode16_crops_device(dbde_b200_ctx *ctx, const uint16_t *frames_dev, int W, int H,
+                                                  uint64_t first_index, int nframes, const int32_t *corners_dev, int ncrops,
+                                                  int corners_per_frame, int crop_w, int crop_h, int pad, uint8_t *out_dev,
+                                                  size_t out_capacity, size_t slot_stride, uint64_t *frame_offsets_dev,
+                                                  uint64_t *frame_sizes_dev, void *stream);
+DBDE_B200_API int dbde_b200_encode16_crops_host(dbde_b200_ctx *ctx, const uint16_t *frames_host, int W, int H,
+                                                uint64_t first_index, int nframes, const int32_t *corners_host, int ncrops,
+                                                int corners_per_frame, int crop_w, int crop_h, int pad, uint8_t *out_host,
+                                                size_t out_capacity, uint64_t *frame_offsets_host);
+
 /* ---- DBDE16 binned: every 16-bit frame at 1/2, 1/4 or 1/8 of its size, as block means -----------------------------
  * dbde_b200_decode_binned_* for DBDE16 records.  factor must be 1, 2, 4 or 8; factor 1 is dbde_b200_decode16_device.
  * Frame i's output is Hb = ceil(H / factor) rows of Wb = ceil(W / factor) U16, tightly packed, at out + i * Wb * Hb
