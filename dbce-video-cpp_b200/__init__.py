@@ -165,8 +165,26 @@ def load():
                                                 C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p]
     lib.dbde_b200_encode16_crops_device.argtypes = lib.dbde_b200_encode_crops_device.argtypes
     lib.dbde_b200_encode16_crops_host.argtypes = lib.dbde_b200_encode_crops_host.argtypes
+    lib.dbde_b200_validate_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                            C.c_void_p]
     lib.dbde_b200_file_last_error.restype = C.c_char_p
     return lib
+
+
+def _corners(corners, N):
+    """int32 crop corners (R, 2), the same for every frame, or (N, R, 2), per frame -> (contiguous corners, per_frame, R)"""
+    corners = np.ascontiguousarray(corners, dtype=np.int32)
+    if corners.ndim == 3 and corners.shape[0] == N and corners.shape[2] == 2:
+        per_frame = 1
+    elif corners.ndim == 2 and corners.shape[1] == 2:
+        per_frame = 0
+    else:
+        raise ValueError("corners must have shape (R, 2) or (N, R, 2), got %r" % (corners.shape,))
+    return corners, per_frame, corners.shape[-2]
+
+
+def _binned_shape(W, H, factor):
+    return (-(-H // factor), -(-W // factor)) if factor > 0 else (0, 0)
 
 
 class DbdeError(RuntimeError):
@@ -302,36 +320,30 @@ class Codec:
     # ---- host-buffer hot path (numpy or raw host pointers)
     def encode_host(self, frames, first_index=0):
         """frames (N,H,W) u8 -> (stream bytes, offsets[N+1])"""
-        frames = np.ascontiguousarray(frames, dtype=np.uint8)
-        N, H, W = frames.shape
-        cap = self.stream_bound(W, H, N)
-        out = np.empty(cap, dtype=np.uint8)
-        offs = np.zeros(N + 1, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_encode_host(self.h, frames.ctypes.data, W, H, first_index, N, out.ctypes.data,
-                                                cap, offs.ctypes.data), "encode_host")
-        return out[:int(offs[N])].copy(), offs
+        return self._encode_host(self.lib.dbde_b200_encode_host, "encode_host", frames, np.uint8, first_index)
 
     def encode_crops_host(self, frames, corners, size, pad=0, first_index=0):
         """frames (N,H,W) u8, crops of size = (crop_w, crop_h) at int32 corners (R, 2) (the same for every frame) or
         (N, R, 2) (per frame), pixels outside the frame `pad` -> (stream bytes, offsets[N*R+1]); record f * R + r is crop r
         of frame f, with frame index first_index + f"""
-        frames = np.ascontiguousarray(frames, dtype=np.uint8)
-        corners = np.ascontiguousarray(corners, dtype=np.int32)
+        return self._encode_host(self.lib.dbde_b200_encode_crops_host, "encode_crops_host", frames, np.uint8, first_index, corners,
+                                 size, pad)
+
+    def _encode_host(self, fn, name, frames, dtype, first_index, corners=None, size=None, pad=0):
+        """the numpy host encodes: frames (N,H,W) of dtype -> (stream bytes, offsets[N*R+1]), R = 1 or, with corners, the
+        crops per frame"""
+        frames = np.ascontiguousarray(frames, dtype=dtype)
         N, H, W = frames.shape
-        cw, ch = (int(v) for v in size)
-        if corners.ndim == 3 and corners.shape[0] == N and corners.shape[2] == 2:
-            per_frame = 1
-        elif corners.ndim == 2 and corners.shape[1] == 2:
-            per_frame = 0
-        else:
-            raise ValueError("corners must have shape (R, 2) or (N, R, 2), got %r" % (corners.shape,))
-        R = corners.shape[-2]
-        cap = self.stream_bound(cw, ch, N * R) if cw > 0 and ch > 0 else 16
+        rw, rh, R, crops = W, H, 1, ()
+        if corners is not None:
+            rw, rh = (int(v) for v in size)
+            corners, per_frame, R = _corners(corners, N)
+            crops = (corners.ctypes.data, R, per_frame, rw, rh, pad)
+        stride = self.lib.dbde_b200_slot_stride16 if dtype == np.uint16 else self.lib.dbde_b200_slot_stride
+        cap = int(stride(rw, rh)) * max(N * R, 1) + 16 if rw > 0 and rh > 0 else 16
         out = np.empty(cap, dtype=np.uint8)
         offs = np.zeros(N * R + 1, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_encode_crops_host(self.h, frames.ctypes.data, W, H, first_index, N, corners.ctypes.data, R,
-                                                      per_frame, cw, ch, pad, out.ctypes.data, cap, offs.ctypes.data),
-                 "encode_crops_host")
+        self._ck(fn(self.h, frames.ctypes.data, W, H, first_index, N, *crops, out.ctypes.data, cap, offs.ctypes.data), name)
         return out[:int(offs[N * R])].copy(), offs
 
     def encode_host_raw(self, frames_ptr, W, H, first_index, N, out_ptr, out_cap, offs_ptr):
@@ -340,73 +352,44 @@ class Codec:
 
     def decode_host(self, stream, offsets, W, H, fill=None):
         """-> (frames (N,H,W), status[N], indices[N]); rejected frames keep `fill`"""
-        stream = np.ascontiguousarray(stream, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
-        N = len(offsets)
-        frames = np.zeros((N, H, W), dtype=np.uint8) if fill is None else np.full((N, H, W), fill, dtype=np.uint8)
-        status = np.zeros(N, dtype=np.uint32)
-        index = np.zeros(N, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_decode_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
-                                                frames.ctypes.data, status.ctypes.data, index.ctypes.data),
-                 "decode_host")
-        return frames, status, index
+        return self._decode_host(self.lib.dbde_b200_decode_host, "decode_host", stream, offsets, W, H, (H, W), np.uint8, fill)
 
     def decode_roi_host(self, stream, offsets, W, H, roi, fill=None):
         """region roi = (x0, y0, roi_w, roi_h) of every frame -> (frames (N, roi_h, roi_w), status[N], indices[N]);
         rejected frames keep `fill`"""
-        stream = np.ascontiguousarray(stream, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
         x0, y0, rw, rh = (int(v) for v in roi)
-        N = len(offsets)
-        shape = (N, max(rh, 0), max(rw, 0))
-        frames = np.zeros(shape, dtype=np.uint8) if fill is None else np.full(shape, fill, dtype=np.uint8)
-        status = np.zeros(N, dtype=np.uint32)
-        index = np.zeros(N, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_decode_roi_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
-                                                    x0, y0, rw, rh, frames.ctypes.data, status.ctypes.data, index.ctypes.data),
-                 "decode_roi_host")
-        return frames, status, index
+        return self._decode_host(self.lib.dbde_b200_decode_roi_host, "decode_roi_host", stream, offsets, W, H, (max(rh, 0), max(rw, 0)),
+                                 np.uint8, fill, x0, y0, rw, rh)
 
     def decode_crops_host(self, stream, offsets, W, H, corners, size, pad=0, fill=None):
         """crops of size = (crop_w, crop_h) at int32 corners (R, 2) (the same for every frame) or (N, R, 2) (per frame) ->
         (crops (N, R, crop_h, crop_w), status[N], indices[N]); pixels outside the frame are `pad`, rejected frames keep
         `fill`"""
-        stream = np.ascontiguousarray(stream, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
-        corners = np.ascontiguousarray(corners, dtype=np.int32)
         cw, ch = (int(v) for v in size)
-        N = len(offsets)
-        if corners.ndim == 3 and corners.shape[0] == N and corners.shape[2] == 2:
-            per_frame = 1
-        elif corners.ndim == 2 and corners.shape[1] == 2:
-            per_frame = 0
-        else:
-            raise ValueError("corners must have shape (R, 2) or (N, R, 2), got %r" % (corners.shape,))
-        R = corners.shape[-2]
-        shape = (N, R, max(ch, 0), max(cw, 0))
-        crops = np.zeros(shape, dtype=np.uint8) if fill is None else np.full(shape, fill, dtype=np.uint8)
-        status = np.zeros(N, dtype=np.uint32)
-        index = np.zeros(N, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_decode_crops_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
-                                                      corners.ctypes.data, R, per_frame, cw, ch, pad, crops.ctypes.data,
-                                                      status.ctypes.data, index.ctypes.data), "decode_crops_host")
-        return crops, status, index
+        corners, per_frame, R = _corners(corners, len(offsets))
+        return self._decode_host(self.lib.dbde_b200_decode_crops_host, "decode_crops_host", stream, offsets, W, H, (R, max(ch, 0), max(cw, 0)),
+                                 np.uint8, fill, corners.ctypes.data, R, per_frame, cw, ch, pad)
 
     def decode_binned_host(self, stream, offsets, W, H, factor, fill=None):
         """every frame binned by factor (1, 2, 4 or 8) -> (frames (N, ceil(H / factor), ceil(W / factor)), status[N],
         indices[N]); rejected frames keep `fill`"""
+        factor = int(factor)
+        return self._decode_host(self.lib.dbde_b200_decode_binned_host, "decode_binned_host", stream, offsets, W, H,
+                                 _binned_shape(W, H, factor), np.uint8, fill, factor)
+
+    def _decode_host(self, fn, name, stream, offsets, W, H, shape, dtype, fill, *args):
+        """the numpy host decodes: N = len(offsets) records -> (output (N,) + shape of dtype, status[N], indices[N]) with
+        rejected frames keeping `fill`; shape None (validation): -> (status[N], indices[N])"""
         stream = np.ascontiguousarray(stream, dtype=np.uint8)
         offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
-        factor = int(factor)
         N = len(offsets)
-        shape = (N, -(-H // factor), -(-W // factor)) if factor > 0 else (N, 0, 0)
-        frames = np.zeros(shape, dtype=np.uint8) if fill is None else np.full(shape, fill, dtype=np.uint8)
+        out = None if shape is None else np.zeros((N,) + shape, dtype=dtype) if fill is None else np.full((N,) + shape, fill, dtype=dtype)
         status = np.zeros(N, dtype=np.uint32)
         index = np.zeros(N, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_decode_binned_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
-                                                       factor, frames.ctypes.data, status.ctypes.data, index.ctypes.data),
-                 "decode_binned_host")
-        return frames, status, index
+        out_ptr = () if out is None else (out.ctypes.data,)
+        self._ck(fn(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N, *args, *out_ptr, status.ctypes.data,
+                    index.ctypes.data), name)
+        return (status, index) if out is None else (out, status, index)
 
     def decode_host_raw(self, stream_ptr, stream_bytes, offs_ptr, W, H, N, frames_ptr, status_ptr, index_ptr=None):
         self._ck(self.lib.dbde_b200_decode_host(self.h, stream_ptr, stream_bytes, offs_ptr, W, H, N, frames_ptr,
@@ -415,14 +398,7 @@ class Codec:
     # ---- DBDE16, the 16-bit extension (SURVEY 8 f-4)
     def encode16_host(self, frames, first_index=0):
         """frames (N,H,W) u16 -> (stream bytes, offsets[N+1])"""
-        frames = np.ascontiguousarray(frames, dtype=np.uint16)
-        N, H, W = frames.shape
-        cap = int(self.lib.dbde_b200_slot_stride16(W, H)) * max(N, 1) + 16
-        out = np.empty(cap, dtype=np.uint8)
-        offs = np.zeros(N + 1, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_encode16_host(self.h, frames.ctypes.data, W, H, first_index, N, out.ctypes.data, cap,
-                                                  offs.ctypes.data), "encode16_host")
-        return out[:int(offs[N])].copy(), offs
+        return self._encode_host(self.lib.dbde_b200_encode16_host, "encode16_host", frames, np.uint16, first_index)
 
     def encode16_crops_device(self, frames_ptr, W, H, first_index, n, corners_ptr, ncrops, per_frame, size, out_ptr, out_cap,
                               offs_ptr, sizes_ptr, pad=0, stream=0, slot_stride=0):
@@ -440,36 +416,12 @@ class Codec:
         """frames (N,H,W) u16, crops of size = (crop_w, crop_h) at int32 corners (R, 2) (the same for every frame) or
         (N, R, 2) (per frame), pixels outside the frame `pad` -> (stream bytes, offsets[N*R+1]); record f * R + r is the
         DBDE16 record of crop r of frame f, with frame index first_index + f"""
-        frames = np.ascontiguousarray(frames, dtype=np.uint16)
-        corners = np.ascontiguousarray(corners, dtype=np.int32)
-        N, H, W = frames.shape
-        cw, ch = (int(v) for v in size)
-        if corners.ndim == 3 and corners.shape[0] == N and corners.shape[2] == 2:
-            per_frame = 1
-        elif corners.ndim == 2 and corners.shape[1] == 2:
-            per_frame = 0
-        else:
-            raise ValueError("corners must have shape (R, 2) or (N, R, 2), got %r" % (corners.shape,))
-        R = corners.shape[-2]
-        cap = int(self.lib.dbde_b200_slot_stride16(cw, ch)) * max(N * R, 1) + 16 if cw > 0 and ch > 0 else 16
-        out = np.empty(cap, dtype=np.uint8)
-        offs = np.zeros(N * R + 1, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_encode16_crops_host(self.h, frames.ctypes.data, W, H, first_index, N, corners.ctypes.data, R,
-                                                        per_frame, cw, ch, pad, out.ctypes.data, cap, offs.ctypes.data),
-                 "encode16_crops_host")
-        return out[:int(offs[N * R])].copy(), offs
+        return self._encode_host(self.lib.dbde_b200_encode16_crops_host, "encode16_crops_host", frames, np.uint16, first_index, corners,
+                                 size, pad)
 
     def decode16_host(self, stream, offsets, W, H, fill=None):
         """-> (frames (N,H,W) u16, status[N], indices[N]); rejected frames keep `fill`"""
-        stream = np.ascontiguousarray(stream, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
-        N = len(offsets)
-        frames = np.zeros((N, H, W), dtype=np.uint16) if fill is None else np.full((N, H, W), fill, dtype=np.uint16)
-        status = np.zeros(N, dtype=np.uint32)
-        index = np.zeros(N, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_decode16_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
-                                                  frames.ctypes.data, status.ctypes.data, index.ctypes.data), "decode16_host")
-        return frames, status, index
+        return self._decode_host(self.lib.dbde_b200_decode16_host, "decode16_host", stream, offsets, W, H, (H, W), np.uint16, fill)
 
     def decode16_crops_device(self, stream_ptr, stream_bytes, offs_ptr, W, H, n, corners_ptr, ncrops, per_frame, size, out_ptr,
                               status_ptr, index_ptr=None, pad=0, stream=0):
@@ -492,55 +444,21 @@ class Codec:
         """DBDE16 records: crops of size = (crop_w, crop_h) at int32 corners (R, 2) (the same for every frame) or (N, R, 2)
         (per frame) -> (crops (N, R, crop_h, crop_w) u16, status[N], indices[N]); pixels outside the frame are `pad`,
         rejected frames keep `fill`"""
-        stream = np.ascontiguousarray(stream, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
-        corners = np.ascontiguousarray(corners, dtype=np.int32)
         cw, ch = (int(v) for v in size)
-        N = len(offsets)
-        if corners.ndim == 3 and corners.shape[0] == N and corners.shape[2] == 2:
-            per_frame = 1
-        elif corners.ndim == 2 and corners.shape[1] == 2:
-            per_frame = 0
-        else:
-            raise ValueError("corners must have shape (R, 2) or (N, R, 2), got %r" % (corners.shape,))
-        R = corners.shape[-2]
-        shape = (N, R, max(ch, 0), max(cw, 0))
-        crops = np.zeros(shape, dtype=np.uint16) if fill is None else np.full(shape, fill, dtype=np.uint16)
-        status = np.zeros(N, dtype=np.uint32)
-        index = np.zeros(N, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_decode16_crops_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
-                                                        corners.ctypes.data, R, per_frame, cw, ch, pad, crops.ctypes.data,
-                                                        status.ctypes.data, index.ctypes.data), "decode16_crops_host")
-        return crops, status, index
+        corners, per_frame, R = _corners(corners, len(offsets))
+        return self._decode_host(self.lib.dbde_b200_decode16_crops_host, "decode16_crops_host", stream, offsets, W, H, (R, max(ch, 0), max(cw, 0)),
+                                 np.uint16, fill, corners.ctypes.data, R, per_frame, cw, ch, pad)
 
     def decode16_binned_host(self, stream, offsets, W, H, factor, fill=None):
         """DBDE16 records, every frame binned by factor (1, 2, 4 or 8) -> (frames (N, ceil(H / factor), ceil(W / factor))
         u16, status[N], indices[N]); rejected frames keep `fill`"""
-        stream = np.ascontiguousarray(stream, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
         factor = int(factor)
-        N = len(offsets)
-        shape = (N, -(-H // factor), -(-W // factor)) if factor > 0 else (N, 0, 0)
-        frames = np.zeros(shape, dtype=np.uint16) if fill is None else np.full(shape, fill, dtype=np.uint16)
-        status = np.zeros(N, dtype=np.uint32)
-        index = np.zeros(N, dtype=np.uint64)
-        self._ck(self.lib.dbde_b200_decode16_binned_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
-                                                         factor, frames.ctypes.data, status.ctypes.data, index.ctypes.data),
-                 "decode16_binned_host")
-        return frames, status, index
+        return self._decode_host(self.lib.dbde_b200_decode16_binned_host, "decode16_binned_host", stream, offsets, W, H,
+                                 _binned_shape(W, H, factor), np.uint16, fill, factor)
 
     def validate_host(self, stream, offsets, W, H):
         """GPU validation without decoding (SURVEY 8 f-2) -> (status[N], indices[N])"""
-        stream = np.ascontiguousarray(stream, dtype=np.uint8)
-        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
-        N = len(offsets)
-        status = np.zeros(N, dtype=np.uint32)
-        index = np.zeros(N, dtype=np.uint64)
-        self.lib.dbde_b200_validate_host.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_int, C.c_int, C.c_int,
-                                                     C.c_void_p, C.c_void_p]
-        self._ck(self.lib.dbde_b200_validate_host(self.h, stream.ctypes.data, stream.nbytes, offsets.ctypes.data, W, H, N,
-                                                  status.ctypes.data, index.ctypes.data), "validate_host")
-        return status, index
+        return self._decode_host(self.lib.dbde_b200_validate_host, "validate_host", stream, offsets, W, H, None, None, None)
 
     def index_stream(self, stream, W, H, max_frames=1 << 20):
         stream = np.ascontiguousarray(stream, dtype=np.uint8)

@@ -386,54 +386,214 @@ static StreamScratch &scratch_for(dbde_b200_ctx *c, cudaStream_t st) {
     return *lru;
 }
 
-// ------------------------------------------------------------------ device-resident hot path
-extern "C" int dbde_b200_encode_device(dbde_b200_ctx *c, const uint8_t *frames_dev, int W, int H,
-                                       uint64_t first_index, int nframes, uint8_t *out_dev, size_t out_capacity,
-                                       size_t slot_stride, uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev,
-                                       void *stream) {
-    if (!c || !dims_ok(W, H, nframes) ||
-        (nframes > 0 && (!frames_dev || !out_dev || !frame_offsets_dev || !frame_sizes_dev)))
-        return fail(DBDE_B200_E_INVALID, "encode_device: bad argument");
-    if (nframes == 0) return 0;
-    if (slot_stride == 0) slot_stride = dbde_b200_slot_stride(W, H);
-    if (slot_stride < dbde_b200_frame_record_bound(W, H))
-        return fail(DBDE_B200_E_INVALID, "encode_device: slot_stride < dbde_b200_frame_record_bound()");
-    if (out_capacity < slot_stride * (size_t)nframes)
-        return fail(DBDE_B200_E_CAPACITY, "encode_device: out_capacity < nframes * slot_stride");
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const bool fast = (W % 16 == 0) && (H % 8 == 0) && (((uintptr_t)frames_dev & 15) == 0);
-    EncParams P;
-    P.g = make_geom(W, H, fast);
-    const unsigned long long nparts = (unsigned long long)nframes * P.g.ppf;
-    if (nparts >= 0xFFFFFFF0ull) return fail(DBDE_B200_E_INVALID, "encode_device: batch too large");
-    // scratch: [ticket | pad to 128][desc: nparts u64], zeroed per launch
+// ------------------------------------------------------------------ requests
+// Every codec entry point describes its call as one Request: the pixel format, the output form and its fields, and
+// its public name.  check_decode / check_encode hold every argument rule; enqueue_decode / enqueue_encode pick and
+// queue the kernels and check nothing.  A device entry point is request, check, enqueue; a host entry point is
+// request, check, then the chunk pipeline, which enqueues once per chunk.
+enum class Form { Full, Validate, Region, Crops, Binned };
+
+// What the pixel format fixes for frames of w x h pixels
+struct Fmt {
+    size_t px, bound, stride;   // bytes per frame, the record bound, the slot stride
+    size_t delta;               // where a slot's record starts so that its U64 words are 16-byte aligned
+    size_t stream_bound(int n) const { return stride * (size_t)(n < 0 ? 0 : n) + 16; }
+};
+
+struct Request {
+    const char *name;           // the entry point, for dbde_b200_last_error()
+    bool u16;                   // DBDE16 records of U16 frames, else the reference's 8-bit records
+    Form form;                  // encoders: Full or Crops
+    int W, H, nframes;
+    int factor = 0;             // Binned: 1, 2, 4 or 8
+    int x0 = 0, y0 = 0;         // Region: the rectangle's corner
+    int w = 0, h = 0;           // Region: its size; Crops: the crop size
+    const int32_t *corners = nullptr;    // Crops, in the caller's memory: nframes * ncrops {x0, y0} pairs if per_frame, else ncrops
+    int ncrops = 1, per_frame = 0, pad = 0;
+
+    int pad_max() const { return u16 ? 65535 : 255; }
+    Fmt fmt(int fw, int fh) const {
+        const size_t wh = (size_t)((fw + 7) / 8) * ((fh + 7) / 8);
+        Fmt f;
+        f.px = (size_t)fw * fh * (u16 ? 2 : 1);
+        f.bound = u16 ? dbde_b200_frame_record_bound16(fw, fh) : dbde_b200_frame_record_bound(fw, fh);
+        f.stride = (f.bound + 15) & ~(size_t)15;
+        f.delta = (16 - (32 + (u16 ? 3 : 2) * wh) % 16) % 16;
+        return f;
+    }
+    int records() const { return form == Form::Crops ? ncrops : 1; }      // per frame
+    Fmt record_fmt() const { return form == Form::Crops ? fmt(w, h) : fmt(W, H); }
+    // bytes per frame a decode writes: the frame, the region, the crops or the bins
+    size_t out_bytes() const {
+        switch (form) {
+        case Form::Region: return fmt(w, h).px;
+        case Form::Crops: return fmt(w, h).px * (size_t)ncrops;
+        case Form::Binned: return fmt((W - 1) / factor + 1, (H - 1) / factor + 1).px;
+        default: return fmt(W, H).px;
+        }
+    }
+    size_t corner_bytes(int n) const { return form == Form::Crops ? 8 * (size_t)ncrops * (size_t)(per_frame ? n : 1) : 0; }
+};
+
+static int reject(const Request &r, int code, const char *why) {
+    g_err = std::string(r.name) + ": " + why;
+    return code;
+}
+
+static bool roi_ok(int W, int H, int x0, int y0, int roi_w, int roi_h) {
+    return x0 >= 0 && y0 >= 0 && roi_w >= 1 && roi_h >= 1 && (long long)x0 + roi_w <= W && (long long)y0 + roi_h <= H;
+}
+// the size limit counts pixels whatever their width
+static bool crops_ok(int ncrops, int corners_per_frame, int crop_w, int crop_h, int pad, int pad_max) {
+    return ncrops >= 1 && crop_w >= 1 && crop_h >= 1 && dims_ok(crop_w, crop_h, 0) &&
+           (long long)ncrops * crop_w * crop_h <= 0x7FFFFFFFLL && (corners_per_frame == 0 || corners_per_frame == 1) && pad >= 0 &&
+           pad <= pad_max;
+}
+static bool factor_ok(int factor) { return factor == 1 || factor == 2 || factor == 4 || factor == 8; }
+
+// the rules every form shares: the frame, and the output form's own fields
+static bool request_ok(const dbde_b200_ctx *c, const Request &r) {
+    if (!c || !dims_ok(r.W, r.H, r.nframes)) return false;
+    switch (r.form) {
+    case Form::Region: return roi_ok(r.W, r.H, r.x0, r.y0, r.w, r.h);
+    case Form::Crops: return crops_ok(r.ncrops, r.per_frame, r.w, r.h, r.pad, r.pad_max());
+    case Form::Binned: return factor_ok(r.factor);
+    default: return true;
+    }
+}
+
+// Every argument rule of the decoders.  `out` is the frames, region, crops or bins (unused by Validate).  host: the
+// buffers are in host memory; the offsets must then ascend within the stream.  0: run the request (nothing to run for
+// an empty batch).
+static int check_decode(const dbde_b200_ctx *c, const Request &r, const uint8_t *stream, size_t stream_bytes, const uint64_t *offs,
+                        const void *out, const uint32_t *status, bool host) {
+    // DBDE16 output is 2-byte aligned, but for decode16_host, which has always copied out of staging to any address
+    const bool odd_ok = !r.u16 || (host && r.form == Form::Full);
+    if (!request_ok(c, r) || (!odd_ok && ((uintptr_t)out & 1)) ||
+        (r.nframes > 0 && (!stream || !offs || (!out && r.form != Form::Validate) || !status || (r.form == Form::Crops && !r.corners))))
+        return reject(r, DBDE_B200_E_INVALID, "bad argument");
+    if (host)
+        for (int i = 0; i < r.nframes; i++) {
+            const uint64_t end = i + 1 < r.nframes ? offs[i + 1] : stream_bytes;
+            if (offs[i] > end || end > stream_bytes) return reject(r, DBDE_B200_E_INVALID, "frame offsets must ascend within the stream");
+        }
+    return 0;
+}
+
+// Every argument rule of the encoders.  slot_stride: the device forms' (0 picks the default and is replaced by it);
+// null for the host forms, whose capacity can only be checked against the records' sizes once they are known.
+static int check_encode(const dbde_b200_ctx *c, const Request &r, const void *frames, const uint8_t *out, size_t out_capacity,
+                        size_t *slot_stride, const uint64_t *offs, const uint64_t *sizes) {
+    const bool device = slot_stride != nullptr;
+    // the device forms read DBDE16 frames in place, 2-byte aligned; the host forms copy them into staging first
+    if (!request_ok(c, r) || (r.u16 && device && ((uintptr_t)frames & 1)) ||
+        (r.nframes > 0 && (!frames || !out || !offs || (device && !sizes) || (r.form == Form::Crops && !r.corners))))
+        return reject(r, DBDE_B200_E_INVALID, "bad argument");
+    if (r.nframes == 0) return 0;
+    const Fmt f = r.record_fmt();
+    if (device) {
+        if (*slot_stride == 0) *slot_stride = f.stride;
+        if (*slot_stride < f.bound) return reject(r, DBDE_B200_E_INVALID, "slot_stride < the record bound");
+    }
+    const long long nrec = (long long)r.nframes * r.records();
+    if (nrec > 0x7FFFFFFFLL) return reject(r, DBDE_B200_E_INVALID, "nframes * ncrops > 2^31 - 1");
+    if (device && *slot_stride > out_capacity / (size_t)nrec)
+        return reject(r, DBDE_B200_E_CAPACITY, "out_capacity < records * slot_stride");
+    return 0;
+}
+
+// ------------------------------------------------------------------ the kernels of a request
+// The frame encoders' look-back scratch on stream st, zeroed: [ticket | pad to 128][desc: nparts u64]
+static int encode_scratch(dbde_b200_ctx *c, cudaStream_t st, const Request &r, unsigned long long nparts, unsigned int **ticket,
+                          uint64_t **desc) {
+    if (nparts >= 0xFFFFFFF0ull) return reject(r, DBDE_B200_E_INVALID, "batch too large");
     const size_t sbytes = 128 + 8 * (size_t)nparts;
     StreamScratch &sc = scratch_for(c, st);
     int rc = grow(&sc.enc, &sc.enc_bytes, sbytes);
     if (rc) return rc;
     CK(cudaMemsetAsync(sc.enc, 0, sbytes, st));
-    P.frames = frames_dev;
-    P.out = out_dev;
-    P.slot_stride = slot_stride;
-    P.frame_offsets = frame_offsets_dev;
-    P.frame_sizes = frame_sizes_dev;
-    P.ticket = (unsigned int *)sc.enc;
-    P.desc = (uint64_t *)((uint8_t *)sc.enc + 128);
-    P.first_index = first_index;
-    P.nframes = nframes;
-    P.nparts = (unsigned)nparts;
-    P.flags = c->invert_endian ? kFlagInvertRows : 0u;
-    CK(launch_encode(P, fast, c->num_sms, st));
+    *ticket = (unsigned int *)sc.enc;
+    *desc = (uint64_t *)((uint8_t *)sc.enc + 128);
+    return 0;
+}
+
+// the fields the 8-bit and DBDE16 crop encoders share
+template <class P>
+static P crop_params(const Request &r, const uint8_t *frames, uint64_t first_index, int n, const int32_t *corners, uint8_t *out,
+                     size_t slot_stride, uint64_t *offs, uint64_t *sizes) {
+    P p;
+    p.frames = (decltype(p.frames))frames;
+    p.W = r.W;
+    p.H = r.H;
+    p.corners = corners;
+    p.ncrops = r.ncrops;
+    p.corner_stride = r.per_frame ? r.ncrops : 0;
+    p.crop_w = r.w;
+    p.crop_h = r.h;
+    p.w = (r.w + 7) / 8;
+    p.wh = p.w * ((r.h + 7) / 8);
+    p.out = out;
+    p.slot_stride = slot_stride;
+    p.frame_offsets = offs;
+    p.frame_sizes = sizes;
+    p.first_index = first_index;
+    p.nrec = n * r.ncrops;
+    return p;
+}
+
+// The encoder of a checked request for n frames at `frames` (device; Crops: the corners at `corners`, device), queued on st.
+// A crop equal to the frame still runs the crop kernel: its records are the frame encoder's records, byte for byte.
+static int enqueue_encode(dbde_b200_ctx *c, const Request &r, const uint8_t *frames, uint64_t first_index, int n, const int32_t *corners,
+                          uint8_t *out, size_t slot_stride, uint64_t *offs, uint64_t *sizes, cudaStream_t st) {
+    CK(cudaSetDevice(c->device));
+    int rc = 0;
+    if (r.form == Form::Crops && r.u16) {
+        Enc16CropParams P = crop_params<Enc16CropParams>(r, frames, first_index, n, corners, out, slot_stride, offs, sizes);
+        P.pad = (uint32_t)r.pad;
+        CK(launch_encode16_crops(P, c->num_sms, st));
+    } else if (r.form == Form::Crops) {
+        EncCropParams P = crop_params<EncCropParams>(r, frames, first_index, n, corners, out, slot_stride, offs, sizes);
+        P.pad8 = (uint64_t)r.pad * 0x0101010101010101ull;
+        P.flags = c->invert_endian ? kFlagInvertRows : 0u;
+        CK(launch_encode_crops(P, c->num_sms, st));
+    } else if (r.u16) {
+        Enc16Params P;
+        P.W = r.W; P.H = r.H; P.w = (r.W + 7) / 8; P.h = (r.H + 7) / 8; P.wh = P.w * P.h;
+        P.ppf = (P.wh + 255) / 256;
+        const unsigned long long nparts = (unsigned long long)n * P.ppf;
+        if ((rc = encode_scratch(c, st, r, nparts, &P.ticket, &P.desc))) return rc;
+        P.frames = (const uint16_t *)frames; P.out = out; P.slot_stride = slot_stride;
+        P.frame_offsets = offs; P.frame_sizes = sizes;
+        P.first_index = first_index; P.nframes = n; P.nparts = (unsigned)nparts;
+        P.aligned = (r.W % 8 == 0) && (((uintptr_t)frames & 15) == 0);
+        CK(launch_encode16(P, c->num_sms, st));
+    } else {
+        const bool fast = (r.W % 16 == 0) && (r.H % 8 == 0) && (((uintptr_t)frames & 15) == 0);
+        EncParams P;
+        P.g = make_geom(r.W, r.H, fast);
+        const unsigned long long nparts = (unsigned long long)n * P.g.ppf;
+        if ((rc = encode_scratch(c, st, r, nparts, &P.ticket, &P.desc))) return rc;
+        P.frames = frames;
+        P.out = out;
+        P.slot_stride = slot_stride;
+        P.frame_offsets = offs;
+        P.frame_sizes = sizes;
+        P.first_index = first_index;
+        P.nframes = n;
+        P.nparts = (unsigned)nparts;
+        P.flags = c->invert_endian ? kFlagInvertRows : 0u;
+        CK(launch_encode(P, fast, c->num_sms, st));
+    }
     c->launches += 1;
     return 0;
 }
 
-// The validation pre-pass over geometry g.  Its word-prefix table lives in the scratch of stream st.  P->frames
-// is left null.
-static int scan_params(dbde_b200_ctx *c, cudaStream_t st, const PartGeom &g, const uint8_t *stream_dev, size_t stream_bytes,
-                       const uint64_t *frame_offsets_dev, int nframes, uint32_t *status_dev, uint64_t *indices_dev,
-                       DecParams *P) {
+// The 8-bit validation pre-pass over geometry g, queued on st.  Its word-prefix table lives in the scratch of st.
+// P->frames is what a full decode writes (null for the other forms).
+static int decode_scan(dbde_b200_ctx *c, cudaStream_t st, const Request &r, const PartGeom &g, const uint8_t *stream_dev,
+                       size_t stream_bytes, const uint64_t *frame_offsets_dev, int nframes, uint8_t *frames_dev, uint32_t *status_dev,
+                       uint64_t *indices_dev, DecParams *P) {
+    if ((unsigned long long)nframes * g.ppf >= 0xFFFFFFF0ull) return reject(r, DBDE_B200_E_INVALID, "batch too large");
     const size_t sbytes = 4 * (size_t)nframes * ((size_t)g.ppf * kConsumerWarps + 1);
     StreamScratch &sc = scratch_for(c, st);
     int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
@@ -442,47 +602,120 @@ static int scan_params(dbde_b200_ctx *c, cudaStream_t st, const PartGeom &g, con
     P->stream = stream_dev;
     P->stream_bytes = stream_bytes;
     P->frame_offsets = frame_offsets_dev;
-    P->frames = nullptr;
+    P->frames = frames_dev;
     P->status = status_dev;
     P->indices = indices_dev;
     P->wprefix = (uint32_t *)sc.dec;
     P->nframes = nframes;
     P->nparts = (unsigned)((unsigned long long)nframes * g.ppf);
     P->flags = c->invert_endian ? kFlagInvertRows : 0u;
+    CK(launch_decode_scan(*P, st));
+    c->launches += 1;
     return 0;
 }
 
-// scan_only: run the validation pre-pass alone (status + indices, no pixels): dbde_b200_validate_*
-static int decode_device_impl(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
-                              const uint64_t *frame_offsets_dev, int W, int H, int nframes, uint8_t *frames_dev,
-                              uint32_t *status_dev, uint64_t *indices_dev, void *stream, bool scan_only) {
-    if (!c || !dims_ok(W, H, nframes) ||
-        (nframes > 0 && (!stream_dev || !frame_offsets_dev || (!frames_dev && !scan_only) || !status_dev)))
-        return fail(DBDE_B200_E_INVALID, "decode_device: bad argument");
-    if (nframes == 0) return 0;
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const bool fast = (W % 16 == 0) && (H % 8 == 0) && (((uintptr_t)frames_dev & 15) == 0);
-    const PartGeom g = make_geom(W, H, fast);
-    if ((unsigned long long)nframes * g.ppf >= 0xFFFFFFF0ull) return fail(DBDE_B200_E_INVALID, "decode_device: batch too large");
-    DecParams P;
-    int rc = scan_params(c, st, g, stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev, indices_dev, &P);
+// The DBDE16 validation pass (dbde16_scan_kernel: every check, over the whole record, and the word prefix of every
+// 32 raster-order tiles), queued on st: the first launch of every DBDE16 decode.  P is what the second kernel reads;
+// its output fields are left to the caller.
+static int decode16_scan(dbde_b200_ctx *c, cudaStream_t st, const Request &r, const uint8_t *stream_dev, size_t stream_bytes,
+                         const uint64_t *frame_offsets_dev, int nframes, uint32_t *status_dev, uint64_t *indices_dev, Dec16Params *P) {
+    *P = Dec16Params();
+    P->W = r.W; P->H = r.H; P->w = (r.W + 7) / 8; P->h = (r.H + 7) / 8; P->wh = P->w * P->h;
+    P->ppf = (P->wh + 255) / 256;
+    const unsigned long long nparts = (unsigned long long)nframes * P->ppf;
+    if (nparts >= 0xFFFFFFF0ull) return reject(r, DBDE_B200_E_INVALID, "batch too large");
+    const size_t sbytes = 4 * (size_t)nframes * ((size_t)(P->wh + 31) / 32 + 1);
+    StreamScratch &sc = scratch_for(c, st);
+    int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
     if (rc) return rc;
-    P.frames = frames_dev;
-    CK(launch_decode_scan(P, st));
-    c->launches += 1;
-    if (scan_only) return 0;
-    CK(launch_decode(P, fast, c->num_sms, st));
+    P->stream = stream_dev; P->stream_bytes = stream_bytes; P->frame_offsets = frame_offsets_dev;
+    P->status = status_dev; P->indices = indices_dev;
+    P->wprefix = (uint32_t *)sc.dec;
+    P->nframes = nframes; P->nparts = (unsigned)nparts;
+    CK(launch_decode16_scan(*P, st));
     c->launches += 1;
     return 0;
+}
+
+// The kernels of a checked decode request for n records (Crops: the corners at `corners`, device), queued on st: the
+// validation scan, then the pixels of the output form into `out`.  Validate stops after the scan.  The full decode's
+// 8-bit scan runs on the geometry the full decoder picks from the output's alignment; the region, crop and binned
+// decoders read a scan on linear partitions (dbde_roi.cu).  A region equal to the frame and factor 1 are the full
+// decode; a crop equal to the frame still runs the crop kernel, whose output layout is the crop layout.
+static int enqueue_decode(dbde_b200_ctx *c, const Request &r, const uint8_t *stream, size_t stream_bytes, const uint64_t *offs, int n,
+                          const int32_t *corners, void *out, uint32_t *status, uint64_t *indices, cudaStream_t st) {
+    CK(cudaSetDevice(c->device));
+    Form form = r.form;
+    if ((form == Form::Region && r.x0 == 0 && r.y0 == 0 && r.w == r.W && r.h == r.H) || (form == Form::Binned && r.factor == 1))
+        form = Form::Full;
+    const bool whole = form == Form::Full || form == Form::Validate;
+    const bool fast = whole && (r.W % 16 == 0) && (r.H % 8 == 0) && (((uintptr_t)out & 15) == 0);
+    uint8_t *out8 = (uint8_t *)out;
+    uint16_t *out16 = (uint16_t *)out;
+    DecParams D;
+    Dec16Params P;
+    int rc = r.u16 ? decode16_scan(c, st, r, stream, stream_bytes, offs, n, status, indices, &P)
+                   : decode_scan(c, st, r, whole ? make_geom(r.W, r.H, fast) : linear_geom(r.W, r.H), stream, stream_bytes, offs, n,
+                                 whole ? out8 : nullptr, status, indices, &D);
+    if (rc) return rc;
+    switch (form) {
+    case Form::Validate:
+        return 0;
+    case Form::Full:
+        if (r.u16) {
+            P.frames = out16;
+            P.aligned = (r.W % 8 == 0) && (((uintptr_t)out & 15) == 0);
+            CK(launch_decode16(P, c->num_sms, st));
+        } else {
+            CK(launch_decode(D, fast, c->num_sms, st));
+        }
+        break;
+    case Form::Region:          // 8-bit only
+        CK(launch_decode_roi(D, r.x0, r.y0, r.w, r.h, out8, st));
+        break;
+    case Form::Crops:
+        CK(r.u16 ? launch_decode16_crops(P, corners, r.ncrops, r.per_frame != 0, r.w, r.h, r.pad, out16, st)
+                 : launch_decode_crops(D, corners, r.ncrops, r.per_frame != 0, r.w, r.h, r.pad, out8, st));
+        break;
+    case Form::Binned:
+        CK(r.u16 ? launch_decode16_binned(P, r.factor, out16, c->num_sms, st) : launch_decode_binned(D, r.factor, out8, c->num_sms, st));
+        break;
+    }
+    c->launches += 1;
+    return 0;
+}
+
+// ------------------------------------------------------------------ device-resident hot path
+static int encode_device(dbde_b200_ctx *c, const Request &r, const void *frames_dev, uint64_t first_index, uint8_t *out_dev,
+                         size_t out_capacity, size_t slot_stride, uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev, void *stream) {
+    int rc = check_encode(c, r, frames_dev, out_dev, out_capacity, &slot_stride, frame_offsets_dev, frame_sizes_dev);
+    if (rc || r.nframes == 0) return rc;
+    return enqueue_encode(c, r, (const uint8_t *)frames_dev, first_index, r.nframes, r.corners, out_dev, slot_stride, frame_offsets_dev,
+                          frame_sizes_dev, (cudaStream_t)stream);
+}
+
+static int decode_device(dbde_b200_ctx *c, const Request &r, const uint8_t *stream_dev, size_t stream_bytes,
+                         const uint64_t *frame_offsets_dev, void *out_dev, uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
+    int rc = check_decode(c, r, stream_dev, stream_bytes, frame_offsets_dev, out_dev, status_dev, false);
+    if (rc || r.nframes == 0) return rc;
+    return enqueue_decode(c, r, stream_dev, stream_bytes, frame_offsets_dev, r.nframes, r.corners, out_dev, status_dev, indices_dev,
+                          (cudaStream_t)stream);
+}
+
+extern "C" int dbde_b200_encode_device(dbde_b200_ctx *c, const uint8_t *frames_dev, int W, int H,
+                                       uint64_t first_index, int nframes, uint8_t *out_dev, size_t out_capacity,
+                                       size_t slot_stride, uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev,
+                                       void *stream) {
+    return encode_device(c, {"encode_device", false, Form::Full, W, H, nframes}, frames_dev, first_index, out_dev, out_capacity,
+                         slot_stride, frame_offsets_dev, frame_sizes_dev, stream);
 }
 
 extern "C" int dbde_b200_decode_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
                                        const uint64_t *frame_offsets_dev, int W, int H, int nframes,
                                        uint8_t *frames_dev, uint32_t *status_dev, uint64_t *indices_dev,
                                        void *stream) {
-    return decode_device_impl(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, frames_dev, status_dev,
-                              indices_dev, stream, false);
+    return decode_device(c, {"decode_device", false, Form::Full, W, H, nframes}, stream_dev, stream_bytes, frame_offsets_dev,
+                         frames_dev, status_dev, indices_dev, stream);
 }
 
 // The indexer's optional GPU validation (SURVEY 8 f-2): the checks dbde_unpack_image makes before it
@@ -491,143 +724,98 @@ extern "C" int dbde_b200_decode_device(dbde_b200_ctx *c, const uint8_t *stream_d
 extern "C" int dbde_b200_validate_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
                                          const uint64_t *frame_offsets_dev, int W, int H, int nframes,
                                          uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
-    return decode_device_impl(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, nullptr, status_dev,
-                              indices_dev, stream, true);
+    return decode_device(c, {"validate_device", false, Form::Validate, W, H, nframes}, stream_dev, stream_bytes, frame_offsets_dev,
+                         nullptr, status_dev, indices_dev, stream);
 }
 
-// ------------------------------------------------------------------ region of interest
-static bool roi_ok(int W, int H, int x0, int y0, int roi_w, int roi_h) {
-    return x0 >= 0 && y0 >= 0 && roi_w >= 1 && roi_h >= 1 && (long long)x0 + roi_w <= W && (long long)y0 + roi_h <= H;
-}
-
-// The validation pre-pass on linear partitions (every check of the full decode, over the whole record), queued on
-// st: the first launch of the region and crop decodes.  D is what their kernels read.
-static int linear_scan(dbde_b200_ctx *c, cudaStream_t st, int W, int H, const uint8_t *stream_dev, size_t stream_bytes,
-                       const uint64_t *frame_offsets_dev, int nframes, uint32_t *status_dev, uint64_t *indices_dev, DecParams *D) {
-    CK(cudaSetDevice(c->device));
-    int rc = scan_params(c, st, linear_geom(W, H), stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev, indices_dev, D);
-    if (rc) return rc;
-    CK(launch_decode_scan(*D, st));
-    c->launches += 1;
-    return 0;
-}
-
-// The scan, then one warp per 32 tile columns of each tile row of the region (dbde_roi.cu).  A region equal to the
-// frame is the full decode.
+// The scan, then one warp per 32 tile columns of each tile row of the region (dbde_roi.cu).
 extern "C" int dbde_b200_decode_roi_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
                                            const uint64_t *frame_offsets_dev, int W, int H, int nframes, int x0, int y0,
                                            int roi_w, int roi_h, uint8_t *roi_dev, uint32_t *status_dev,
                                            uint64_t *indices_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || !roi_ok(W, H, x0, y0, roi_w, roi_h) ||
-        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !roi_dev || !status_dev)))
-        return fail(DBDE_B200_E_INVALID, "decode_roi_device: bad argument");
-    if (nframes == 0) return 0;
-    if (x0 == 0 && y0 == 0 && roi_w == W && roi_h == H)
-        return decode_device_impl(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, roi_dev, status_dev,
-                                  indices_dev, stream, false);
-    DecParams D;
-    int rc = linear_scan(c, (cudaStream_t)stream, W, H, stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev,
-                         indices_dev, &D);
-    if (rc) return rc;
-    CK(launch_decode_roi(D, x0, y0, roi_w, roi_h, roi_dev, (cudaStream_t)stream));
-    c->launches += 1;
-    return 0;
+    return decode_device(c, {"decode_roi_device", false, Form::Region, W, H, nframes, 0, x0, y0, roi_w, roi_h}, stream_dev,
+                         stream_bytes, frame_offsets_dev, roi_dev, status_dev, indices_dev, stream);
 }
 
-// ------------------------------------------------------------------ crops
-// pad_max: 255 for 8-bit frames, 65535 for DBDE16; the size limit counts pixels whatever their width
-static bool crops_ok(int ncrops, int corners_per_frame, int crop_w, int crop_h, int pad, int pad_max = 255) {
-    return ncrops >= 1 && crop_w >= 1 && crop_h >= 1 && dims_ok(crop_w, crop_h, 0) &&
-           (long long)ncrops * crop_w * crop_h <= 0x7FFFFFFFLL && (corners_per_frame == 0 || corners_per_frame == 1) && pad >= 0 &&
-           pad <= pad_max;
-}
-
-// The region decode's scan and kernel body with one rectangle per task taken from `corners` (dbde_roi.cu).  A crop
-// equal to the frame still runs the crop kernel: its output layout is the crop layout whatever the corners.
+// The region decode's scan and kernel body with one rectangle per task taken from `corners` (dbde_roi.cu).
 extern "C" int dbde_b200_decode_crops_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
                                              const uint64_t *frame_offsets_dev, int W, int H, int nframes,
                                              const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
                                              int crop_h, int pad, uint8_t *crops_dev, uint32_t *status_dev,
                                              uint64_t *indices_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
-        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !corners_dev || !crops_dev || !status_dev)))
-        return fail(DBDE_B200_E_INVALID, "decode_crops_device: bad argument");
-    if (nframes == 0) return 0;
-    DecParams D;
-    int rc = linear_scan(c, (cudaStream_t)stream, W, H, stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev,
-                         indices_dev, &D);
-    if (rc) return rc;
-    CK(launch_decode_crops(D, corners_dev, ncrops, corners_per_frame != 0, crop_w, crop_h, pad, crops_dev, (cudaStream_t)stream));
-    c->launches += 1;
-    return 0;
+    return decode_device(c, {"decode_crops_device", false, Form::Crops, W, H, nframes, 0, 0, 0, crop_w, crop_h, corners_dev, ncrops,
+                             corners_per_frame, pad},
+                         stream_dev, stream_bytes, frame_offsets_dev, crops_dev, status_dev, indices_dev, stream);
 }
 
-// One CTA per record of a persistent grid, one lane per crop tile (dbde_encode.cu).  A crop equal to the frame still
-// runs the crop kernel: its records are the frame encoder's records, byte for byte.
+// One CTA per record of a persistent grid, one lane per crop tile (dbde_encode.cu).
 extern "C" int dbde_b200_encode_crops_device(dbde_b200_ctx *c, const uint8_t *frames_dev, int W, int H, uint64_t first_index,
                                              int nframes, const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
                                              int crop_h, int pad, uint8_t *out_dev, size_t out_capacity, size_t slot_stride,
                                              uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
-        (nframes > 0 && (!frames_dev || !corners_dev || !out_dev || !frame_offsets_dev || !frame_sizes_dev)))
-        return fail(DBDE_B200_E_INVALID, "encode_crops_device: bad argument");
-    if (nframes == 0) return 0;
-    if (slot_stride == 0) slot_stride = dbde_b200_slot_stride(crop_w, crop_h);
-    if (slot_stride < dbde_b200_frame_record_bound(crop_w, crop_h))
-        return fail(DBDE_B200_E_INVALID, "encode_crops_device: slot_stride < dbde_b200_frame_record_bound(crop_w, crop_h)");
-    const long long nrec = (long long)nframes * ncrops;
-    if (nrec > 0x7FFFFFFFLL) return fail(DBDE_B200_E_INVALID, "encode_crops_device: nframes * ncrops > 2^31 - 1");
-    if (slot_stride > out_capacity / (size_t)nrec)
-        return fail(DBDE_B200_E_CAPACITY, "encode_crops_device: out_capacity < nframes * ncrops * slot_stride");
-    CK(cudaSetDevice(c->device));
-    EncCropParams P;
-    P.frames = frames_dev;
-    P.W = W;
-    P.H = H;
-    P.corners = corners_dev;
-    P.ncrops = ncrops;
-    P.corner_stride = corners_per_frame ? ncrops : 0;
-    P.crop_w = crop_w;
-    P.crop_h = crop_h;
-    P.w = (crop_w + 7) / 8;
-    P.wh = P.w * ((crop_h + 7) / 8);
-    P.pad8 = (uint64_t)pad * 0x0101010101010101ull;
-    P.out = out_dev;
-    P.slot_stride = slot_stride;
-    P.frame_offsets = frame_offsets_dev;
-    P.frame_sizes = frame_sizes_dev;
-    P.first_index = first_index;
-    P.nrec = (int)nrec;
-    P.flags = c->invert_endian ? kFlagInvertRows : 0u;
-    CK(launch_encode_crops(P, c->num_sms, (cudaStream_t)stream));
-    c->launches += 1;
-    return 0;
+    return encode_device(c, {"encode_crops_device", false, Form::Crops, W, H, nframes, 0, 0, 0, crop_w, crop_h, corners_dev, ncrops,
+                             corners_per_frame, pad},
+                         frames_dev, first_index, out_dev, out_capacity, slot_stride, frame_offsets_dev, frame_sizes_dev, stream);
 }
 
-// ------------------------------------------------------------------ binned
-static bool factor_ok(int factor) { return factor == 1 || factor == 2 || factor == 4 || factor == 8; }
-
 // The scan on linear partitions, then the full decoder's pipeline with each tile reduced to its block means in
-// registers (dbde_decode.cu).  Factor 1 is the full decode.
+// registers (dbde_decode.cu).
 extern "C" int dbde_b200_decode_binned_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
                                               const uint64_t *frame_offsets_dev, int W, int H, int nframes, int factor,
                                               uint8_t *out_dev, uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || !factor_ok(factor) ||
-        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !out_dev || !status_dev)))
-        return fail(DBDE_B200_E_INVALID, "decode_binned_device: bad argument");
-    if (nframes == 0) return 0;
-    if (factor == 1)
-        return decode_device_impl(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, out_dev, status_dev,
-                                  indices_dev, stream, false);
-    if ((unsigned long long)nframes * linear_geom(W, H).ppf >= 0xFFFFFFF0ull)
-        return fail(DBDE_B200_E_INVALID, "decode_binned_device: batch too large");
-    DecParams D;
-    int rc = linear_scan(c, (cudaStream_t)stream, W, H, stream_dev, stream_bytes, frame_offsets_dev, nframes, status_dev,
-                         indices_dev, &D);
-    if (rc) return rc;
-    CK(launch_decode_binned(D, factor, out_dev, c->num_sms, (cudaStream_t)stream));
-    c->launches += 1;
-    return 0;
+    return decode_device(c, {"decode_binned_device", false, Form::Binned, W, H, nframes, factor}, stream_dev, stream_bytes,
+                         frame_offsets_dev, out_dev, status_dev, indices_dev, stream);
+}
+
+// ------------------------------------------------------------------ DBDE16 (SURVEY 8 f-4)
+extern "C" size_t dbde_b200_frame_record_bound16(int W, int H) {
+    const size_t wh = (size_t)((W + 7) / 8) * ((H + 7) / 8);
+    return 32 + 3 * wh + 128 * wh;
+}
+extern "C" size_t dbde_b200_slot_stride16(int W, int H) { return (dbde_b200_frame_record_bound16(W, H) + 15) & ~(size_t)15; }
+
+extern "C" int dbde_b200_encode16_device(dbde_b200_ctx *c, const uint16_t *frames_dev, int W, int H, uint64_t first_index,
+                                         int nframes, uint8_t *out_dev, size_t out_capacity, size_t slot_stride,
+                                         uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev, void *stream) {
+    return encode_device(c, {"encode16_device", true, Form::Full, W, H, nframes}, frames_dev, first_index, out_dev, out_capacity,
+                         slot_stride, frame_offsets_dev, frame_sizes_dev, stream);
+}
+
+// One CTA per record of a persistent grid, one lane per crop tile (dbde16.cu): dbde_b200_encode_crops_device with U16
+// pixels.
+extern "C" int dbde_b200_encode16_crops_device(dbde_b200_ctx *c, const uint16_t *frames_dev, int W, int H, uint64_t first_index,
+                                               int nframes, const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
+                                               int crop_h, int pad, uint8_t *out_dev, size_t out_capacity, size_t slot_stride,
+                                               uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev, void *stream) {
+    return encode_device(c, {"encode16_crops_device", true, Form::Crops, W, H, nframes, 0, 0, 0, crop_w, crop_h, corners_dev, ncrops,
+                             corners_per_frame, pad},
+                         frames_dev, first_index, out_dev, out_capacity, slot_stride, frame_offsets_dev, frame_sizes_dev, stream);
+}
+
+extern "C" int dbde_b200_decode16_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
+                                         const uint64_t *frame_offsets_dev, int W, int H, int nframes, uint16_t *frames_dev,
+                                         uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
+    return decode_device(c, {"decode16_device", true, Form::Full, W, H, nframes}, stream_dev, stream_bytes, frame_offsets_dev,
+                         frames_dev, status_dev, indices_dev, stream);
+}
+
+// The scan, then one warp per 32 tile columns of each tile row of each crop (dbde16.cu).
+extern "C" int dbde_b200_decode16_crops_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
+                                               const uint64_t *frame_offsets_dev, int W, int H, int nframes,
+                                               const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
+                                               int crop_h, int pad, uint16_t *crops_dev, uint32_t *status_dev,
+                                               uint64_t *indices_dev, void *stream) {
+    return decode_device(c, {"decode16_crops_device", true, Form::Crops, W, H, nframes, 0, 0, 0, crop_w, crop_h, corners_dev, ncrops,
+                             corners_per_frame, pad},
+                         stream_dev, stream_bytes, frame_offsets_dev, crops_dev, status_dev, indices_dev, stream);
+}
+
+// The scan, then the full decoder's partitions with each tile reduced to its bin means in registers (dbde16.cu).
+extern "C" int dbde_b200_decode16_binned_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
+                                                const uint64_t *frame_offsets_dev, int W, int H, int nframes, int factor,
+                                                uint16_t *out_dev, uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
+    return decode_device(c, {"decode16_binned_device", true, Form::Binned, W, H, nframes, factor}, stream_dev, stream_bytes,
+                         frame_offsets_dev, out_dev, status_dev, indices_dev, stream);
 }
 
 // ------------------------------------------------------------------ pageable host memory
@@ -797,31 +985,16 @@ static int relay_d2h(dbde_b200_ctx *c, HostSlot &s, uint8_t *dst, const uint8_t 
 }
 
 // ------------------------------------------------------------------ host-buffer hot path
-// What differs on the host path between the reference's 8-bit records and the DBDE16 extension: bytes per
-// frame, slot stride, where a slot's record starts so that its U64 words are 16-byte aligned.
-struct HostFmt {
-    bool u16;
-    size_t px, stride, delta;
-    size_t stream_bound(int n) const { return stride * (size_t)(n < 0 ? 0 : n) + 16; }
-};
-static HostFmt host_fmt(int W, int H, bool u16) {
-    HostFmt f;
-    const size_t wh = (size_t)((W + 7) / 8) * ((H + 7) / 8);
-    f.u16 = u16;
-    f.px = (size_t)W * H * (u16 ? 2 : 1);
-    f.stride = u16 ? dbde_b200_slot_stride16(W, H) : dbde_b200_slot_stride(W, H);
-    f.delta = (16 - (32 + (u16 ? 3 : 2) * wh) % 16) % 16;
-    return f;
-}
-
-static int default_chunk(const dbde_b200_ctx *c, int W, int H, int nframes, bool u16 = false) {
+// The 8-bit and DBDE16 host forms share one encode and one decode chunk pipeline (staging slots in flight, records
+// compacted on the device, pageable buffers relayed through the copy pool); the request picks the kernels.
+static int default_chunk(const dbde_b200_ctx *c, const Request &r) {
     int n = c->chunk_frames;
     if (n <= 0) {
-        const size_t px = (size_t)W * H * (u16 ? 2 : 1);
+        const size_t px = r.fmt(r.W, r.H).px;
         n = (int)((64u << 20) / (px ? px : 1));
         if (n < 1) n = 1;
     }
-    if (n > nframes) n = nframes;
+    if (n > r.nframes) n = r.nframes;
     return n;
 }
 
@@ -869,20 +1042,6 @@ static int ensure_slot(dbde_b200_ctx *c, HostSlot &s, size_t need_a, size_t need
     }
     return 0;
 }
-
-// What the host pipeline hands back per frame instead of the whole image: the region (x0, y0, w, h), ncrops crops
-// of w x h with host corners (per_frame: nframes * ncrops {x0, y0} pairs, else ncrops pairs for every frame), or the
-// frame binned by `factor` (w x h = ceil(W / factor) x ceil(H / factor)).  Sizes count pixels: DBDE16 frames (u16)
-// have two bytes each, and no region form.  The encoder takes the crops form: ncrops records of w x h per frame.
-struct SubFrame {
-    int x0, y0, w, h;
-    const int32_t *corners;     // null: the region or the binned frame
-    int ncrops, per_frame, pad;
-    int factor;                 // > 0: the binned frame
-    size_t bytes() const { return (size_t)w * (size_t)h * (size_t)(corners ? ncrops : 1); }
-    size_t corner_bytes(int n) const { return corners ? 8 * (size_t)ncrops * (size_t)(per_frame ? n : 1) : 0; }
-};
-
 // pinned staging of a chunk's crop corners
 static int ensure_corner_staging(HostSlot &s, size_t need) {
     if (s.cap_hcorners >= need) return 0;
@@ -903,19 +1062,22 @@ struct EncSequencer {
     size_t out_pos = 0;            // guarded by `next`
 };
 
-// Worker `my` of `nworkers`: encodes chunks my, my + nworkers, ... of the batch on context c.  crops: every frame
-// gives crops->ncrops records of crops->w x crops->h (dbde_b200_encode_crops_device, or dbde_b200_encode16_crops_device
-// when u16) instead of its own record; the chunk's corners travel behind its frames in the slot's frame buffer.
-static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index,
-                              int nframes, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host,
-                              int chunk, int my, int nworkers, EncSequencer *seq, bool u16 = false, const SubFrame *crops = nullptr) {
+
+// Worker `my` of `nworkers`: encodes chunks my, my + nworkers, ... of the checked request r on context c.  Crops: every
+// frame gives r.ncrops records of r.w x r.h instead of its own record; the chunk's corners travel behind its frames in
+// the slot's frame buffer.
+static int encode_host_worker(dbde_b200_ctx *c, const Request &r, const uint8_t *frames_host, uint64_t first_index,
+                              uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host, int chunk, int my, int nworkers,
+                              EncSequencer *seq) {
     CK(cudaSetDevice(c->device));
-    const HostFmt F = crops ? host_fmt(crops->w, crops->h, u16) : host_fmt(W, H, u16);     // the records' format
-    const size_t px = crops ? (size_t)W * (size_t)H * (u16 ? 2 : 1) : F.px;                 // input bytes per frame
-    const int per = crops ? crops->ncrops : 1;                                                // records per frame
-    const int nrec = chunk * per;                                                             // records per chunk
+    const bool crops = r.form == Form::Crops;
+    const int nframes = r.nframes;
+    const Fmt F = r.record_fmt();                                      // the records' format
+    const size_t px = r.fmt(r.W, r.H).px;                              // input bytes per frame
+    const int per = r.records();                                       // records per frame
+    const int nrec = chunk * per;                                      // records per chunk
     const size_t delta = F.delta;
-    const size_t corner_at = (px * chunk + 15) & ~(size_t)15, need_corners = crops ? crops->corner_bytes(chunk) : 0;
+    const size_t corner_at = (px * chunk + 15) & ~(size_t)15, need_corners = r.corner_bytes(chunk);
     const size_t need_a = crops ? corner_at + need_corners : px * chunk + 32, need_b = F.stream_bound(nrec) + 32;
     const int nchunks = (nframes + chunk - 1) / chunk;
     const int mine = nchunks > my ? (nchunks - my + nworkers - 1) / nworkers : 0;
@@ -998,23 +1160,14 @@ static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int 
         }
         if (crops) {
             // this chunk's corners (the staging is free: the slot's stream has drained)
-            const size_t nb = crops->corner_bytes(s.n);
-            memcpy(s.h_corners, crops->corners + (crops->per_frame ? 2 * (size_t)crops->ncrops * (size_t)s.first : 0), nb);
+            const size_t nb = r.corner_bytes(s.n);
+            memcpy(s.h_corners, r.corners + (r.per_frame ? 2 * (size_t)r.ncrops * (size_t)s.first : 0), nb);
             CK(cudaMemcpyAsync(s.d_a + corner_at, s.h_corners, nb, cudaMemcpyHostToDevice, s.st));
         }
         prof.mark(1, "h2d");
         prof.gpu_mark(1, s.st);
-        rc_all = crops && u16 ? dbde_b200_encode16_crops_device(c, (const uint16_t *)s.d_a, W, H, first_index + s.first, s.n,
-                                                                (const int32_t *)(s.d_a + corner_at), crops->ncrops, crops->per_frame,
-                                                                crops->w, crops->h, crops->pad, s.d_b + delta, need_b - 32, stride,
-                                                                s.d_off, s.d_size, s.st)
-                 : crops ? dbde_b200_encode_crops_device(c, s.d_a, W, H, first_index + s.first, s.n, (const int32_t *)(s.d_a + corner_at),
-                                                         crops->ncrops, crops->per_frame, crops->w, crops->h, crops->pad, s.d_b + delta,
-                                                         need_b - 32, stride, s.d_off, s.d_size, s.st)
-                 : u16 ? dbde_b200_encode16_device(c, (const uint16_t *)s.d_a, W, H, first_index + s.first, s.n, s.d_b + delta,
-                                                   need_b - 32, stride, s.d_off, s.d_size, s.st)
-                       : dbde_b200_encode_device(c, s.d_a, W, H, first_index + s.first, s.n, s.d_b + delta, need_b - 32, stride,
-                                                 s.d_off, s.d_size, s.st);
+        rc_all = enqueue_encode(c, r, s.d_a, first_index + s.first, s.n, (const int32_t *)(s.d_a + corner_at), s.d_b + delta, stride,
+                                s.d_off, s.d_size, s.st);
         if (rc_all) break;
         prof.gpu_mark(2, s.st);
         CK(cudaMemcpyAsync(s.h_size, s.d_size, 8 * (size_t)s.n * per, cudaMemcpyDeviceToHost, s.st));
@@ -1046,84 +1199,73 @@ static int encode_host_worker(dbde_b200_ctx *c, const uint8_t *frames_host, int 
     return rc_all;
 }
 
-extern "C" int dbde_b200_encode_host(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H,
-                                     uint64_t first_index, int nframes, uint8_t *out_host, size_t out_capacity,
-                                     uint64_t *frame_offsets_host) {
-    if (!c || !dims_ok(W, H, nframes) || (nframes > 0 && (!frames_host || !out_host || !frame_offsets_host)))
-        return fail(DBDE_B200_E_INVALID, "encode_host: bad argument");
-    if (nframes == 0) {
-        if (frame_offsets_host) frame_offsets_host[0] = 0;
-        return 0;
-    }
-    EncSequencer seq;
-    int rc = encode_host_worker(c, frames_host, W, H, first_index, nframes, out_host, out_capacity, frame_offsets_host,
-                                default_chunk(c, W, H, nframes), 0, 1, &seq);
+// The host form of an encode request: the chunk pipeline, for crops with ncrops records per frame.
+static int encode_host(dbde_b200_ctx *c, const Request &r, const uint8_t *frames_host, uint64_t first_index, uint8_t *out_host,
+                       size_t out_capacity, uint64_t *frame_offsets_host) {
+    int rc = check_encode(c, r, frames_host, out_host, out_capacity, nullptr, frame_offsets_host, nullptr);
     if (rc) return rc;
-    frame_offsets_host[nframes] = seq.out_pos;
-    return 0;
-}
-
-// The host forms of dbde_b200_encode_crops_device and dbde_b200_encode16_crops_device (u16): the encode_host chunk
-// pipeline with ncrops records per frame; each chunk's corners go up behind its frames.
-static int encode_crops_host_impl(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index, int nframes,
-                                  const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w, int crop_h, int pad,
-                                  uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host, bool u16) {
-    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad, u16 ? 65535 : 255) ||
-        (nframes > 0 && (!frames_host || !corners_host || !out_host || !frame_offsets_host)))
-        return fail(DBDE_B200_E_INVALID, u16 ? "encode16_crops_host: bad argument" : "encode_crops_host: bad argument");
-    if (nframes == 0) {
+    if (r.nframes == 0) {
         if (frame_offsets_host) frame_offsets_host[0] = 0;
         return 0;
     }
-    if ((long long)nframes * ncrops > 0x7FFFFFFFLL)
-        return fail(DBDE_B200_E_INVALID, u16 ? "encode16_crops_host: nframes * ncrops > 2^31 - 1" : "encode_crops_host: nframes * ncrops > 2^31 - 1");
-    int chunk = default_chunk(c, W, H, nframes, u16);
-    const HostFmt crop = host_fmt(crop_w, crop_h, u16), frame = host_fmt(W, H, u16);
-    const size_t rec = (size_t)ncrops * crop.stride;                   // one frame's record slots
-    if (rec > frame.stride) {                      // crops larger than the frame: a chunk's records stay within 64 MiB
+    int chunk = default_chunk(c, r);
+    const size_t rec = (size_t)r.records() * r.record_fmt().stride;      // one frame's record slots
+    if (rec > r.fmt(r.W, r.H).stride) {            // crops larger than the frame: a chunk's records stay within 64 MiB
         const size_t most = (64u << 20) / rec;
         if ((size_t)chunk > most) chunk = most > 0 ? (int)most : 1;
     }
-    const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad, 0};
     EncSequencer seq;
-    int rc = encode_host_worker(c, frames_host, W, H, first_index, nframes, out_host, out_capacity, frame_offsets_host, chunk, 0, 1,
-                                &seq, u16, &crops);
+    rc = encode_host_worker(c, r, frames_host, first_index, out_host, out_capacity, frame_offsets_host, chunk, 0, 1, &seq);
     if (rc) return rc;
-    frame_offsets_host[(size_t)nframes * ncrops] = seq.out_pos;
+    frame_offsets_host[(size_t)r.nframes * r.records()] = seq.out_pos;
     return 0;
 }
 
+extern "C" int dbde_b200_encode_host(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H,
+                                     uint64_t first_index, int nframes, uint8_t *out_host, size_t out_capacity,
+                                     uint64_t *frame_offsets_host) {
+    return encode_host(c, {"encode_host", false, Form::Full, W, H, nframes}, frames_host, first_index, out_host, out_capacity,
+                       frame_offsets_host);
+}
+
+// The host forms of dbde_b200_encode_crops_device and dbde_b200_encode16_crops_device: each chunk's corners go up behind
+// its frames.
 extern "C" int dbde_b200_encode_crops_host(dbde_b200_ctx *c, const uint8_t *frames_host, int W, int H, uint64_t first_index,
                                            int nframes, const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
                                            int crop_h, int pad, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host) {
-    return encode_crops_host_impl(c, frames_host, W, H, first_index, nframes, corners_host, ncrops, corners_per_frame, crop_w, crop_h,
-                                  pad, out_host, out_capacity, frame_offsets_host, false);
+    return encode_host(c, {"encode_crops_host", false, Form::Crops, W, H, nframes, 0, 0, 0, crop_w, crop_h, corners_host, ncrops,
+                           corners_per_frame, pad},
+                       frames_host, first_index, out_host, out_capacity, frame_offsets_host);
+}
+
+extern "C" int dbde_b200_encode16_host(dbde_b200_ctx *c, const uint16_t *frames_host, int W, int H, uint64_t first_index,
+                                       int nframes, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host) {
+    return encode_host(c, {"encode16_host", true, Form::Full, W, H, nframes}, (const uint8_t *)frames_host, first_index, out_host,
+                       out_capacity, frame_offsets_host);
 }
 
 extern "C" int dbde_b200_encode16_crops_host(dbde_b200_ctx *c, const uint16_t *frames_host, int W, int H, uint64_t first_index,
                                              int nframes, const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
                                              int crop_h, int pad, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host) {
-    return encode_crops_host_impl(c, (const uint8_t *)frames_host, W, H, first_index, nframes, corners_host, ncrops, corners_per_frame,
-                                  crop_w, crop_h, pad, out_host, out_capacity, frame_offsets_host, true);
+    return encode_host(c, {"encode16_crops_host", true, Form::Crops, W, H, nframes, 0, 0, 0, crop_w, crop_h, corners_host, ncrops,
+                           corners_per_frame, pad},
+                       (const uint8_t *)frames_host, first_index, out_host, out_capacity, frame_offsets_host);
 }
 
-static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
-                            const uint64_t *frame_offsets_host, int W, int H, int nframes, uint8_t *frames_host,
-                            uint32_t *status_host, uint64_t *indices_host, bool scan_only, bool u16 = false,
-                            const SubFrame *sub = nullptr) {
-    if (!c || !dims_ok(W, H, nframes) ||
-        (nframes > 0 && (!stream_host || !frame_offsets_host || (!frames_host && !scan_only) || !status_host)))
-        return fail(DBDE_B200_E_INVALID, "decode_host: bad argument");
-    if (nframes == 0) return 0;
+// The host form of a decode request: the records cross PCIe whole, and what the request asks for comes back -- the
+// frames, the region, the crops (each chunk's corners go up on its slot's stream) or the bins; nothing for Validate
+// but 4 (+8) bytes per frame.
+static int decode_host(dbde_b200_ctx *c, const Request &r, const uint8_t *stream_host, size_t stream_bytes,
+                       const uint64_t *frame_offsets_host, void *out_host, uint32_t *status_host, uint64_t *indices_host) {
+    int rc = check_decode(c, r, stream_host, stream_bytes, frame_offsets_host, out_host, status_host, true);
+    if (rc || r.nframes == 0) return rc;
     CK(cudaSetDevice(c->device));
-    for (int i = 0; i < nframes; i++) {
-        const uint64_t end = i + 1 < nframes ? frame_offsets_host[i + 1] : stream_bytes;
-        if (frame_offsets_host[i] > end || end > stream_bytes)
-            return fail(DBDE_B200_E_INVALID, "decode_host: frame offsets must ascend within the stream");
-    }
-    const HostFmt F = host_fmt(W, H, u16);
-    const size_t px = sub ? sub->bytes() * (u16 ? 2 : 1) : F.px;    // output bytes per frame
-    int chunk = default_chunk(c, W, H, nframes, u16);
+    const int nframes = r.nframes;
+    const bool scan_only = r.form == Form::Validate;
+    uint8_t *frames_host = (uint8_t *)out_host;
+    const Fmt F = r.fmt(r.W, r.H);
+    const size_t px = r.out_bytes();                 // output bytes per frame
+    int chunk = default_chunk(c, r);
     if (px > F.px) {                                 // crops larger than the frame: a chunk's output stays within 64 MiB
         const size_t most = (64u << 20) / px;
         if ((size_t)chunk > most) chunk = most > 0 ? (int)most : 1;
@@ -1147,7 +1289,7 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
     const int ns = nchunks < c->nslots ? nchunks : c->nslots;
     // pageable caller memory is relayed through pinned bounce buffers (see CopyPool)
     const bool in_pageable = is_pageable(stream_host), out_pageable = !scan_only && is_pageable(frames_host);
-    const size_t need_corners = sub ? sub->corner_bytes(chunk) : 0;
+    const size_t need_corners = r.corner_bytes(chunk);
     for (int i = 0; i < ns; i++) {
         HostSlot &s = c->slots[i];
         int rc = ensure_slot(c, s, need_a, need_b, need_corners, chunk);
@@ -1208,32 +1350,14 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
         } else {
             CK(cudaMemcpyAsync(s.d_a + delta, stream_host + b0, b1 - b0, cudaMemcpyHostToDevice, s.st));
         }
-        if (sub && sub->corners) {
+        if (r.form == Form::Crops) {
             // this chunk's corners (the staging is free: the slot's stream has drained)
-            const size_t nb = sub->corner_bytes(s.n);
-            memcpy(s.h_corners, sub->corners + (sub->per_frame ? 2 * (size_t)sub->ncrops * (size_t)s.first : 0), nb);
+            const size_t nb = r.corner_bytes(s.n);
+            memcpy(s.h_corners, r.corners + (r.per_frame ? 2 * (size_t)r.ncrops * (size_t)s.first : 0), nb);
             CK(cudaMemcpyAsync(s.d_c, s.h_corners, nb, cudaMemcpyHostToDevice, s.st));
         }
         prof.mark(1, "h2d");
-        rc_all = u16 && sub && sub->corners
-                       ? dbde_b200_decode16_crops_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (const int32_t *)s.d_c,
-                                                         sub->ncrops, sub->per_frame, sub->w, sub->h, sub->pad, (uint16_t *)s.d_b,
-                                                         s.d_status, s.d_index, s.st)
-                 : u16 && sub ? dbde_b200_decode16_binned_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, sub->factor,
-                                                                 (uint16_t *)s.d_b, s.d_status, s.d_index, s.st)
-                 : u16 ? dbde_b200_decode16_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (uint16_t *)s.d_b, s.d_status,
-                                                   s.d_index, s.st)
-                 : sub && sub->corners
-                       ? dbde_b200_decode_crops_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, (const int32_t *)s.d_c,
-                                                       sub->ncrops, sub->per_frame, sub->w, sub->h, sub->pad, s.d_b, s.d_status,
-                                                       s.d_index, s.st)
-                 : sub && sub->factor
-                       ? dbde_b200_decode_binned_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, sub->factor, s.d_b, s.d_status,
-                                                        s.d_index, s.st)
-                 : sub ? dbde_b200_decode_roi_device(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, sub->x0, sub->y0, sub->w, sub->h,
-                                                     s.d_b, s.d_status, s.d_index, s.st)
-                       : decode_device_impl(c, s.d_a + delta, b1 - b0, s.d_off, W, H, s.n, s.d_b, s.d_status, s.d_index, s.st,
-                                            scan_only);
+        rc_all = enqueue_decode(c, r, s.d_a + delta, b1 - b0, s.d_off, s.n, (const int32_t *)s.d_c, s.d_b, s.d_status, s.d_index, s.st);
         if (rc_all) break;
         CK(cudaMemcpyAsync(s.h_status, s.d_status, 4 * (size_t)s.n, cudaMemcpyDeviceToHost, s.st));
         if (indices_host) CK(cudaMemcpyAsync(s.h_index, s.d_index, 8 * (size_t)s.n, cudaMemcpyDeviceToHost, s.st));
@@ -1258,288 +1382,64 @@ static int decode_host_impl(dbde_b200_ctx *c, const uint8_t *stream_host, size_t
 extern "C" int dbde_b200_decode_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                                      const uint64_t *frame_offsets_host, int W, int H, int nframes,
                                      uint8_t *frames_host, uint32_t *status_host, uint64_t *indices_host) {
-    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, frames_host, status_host,
-                            indices_host, false);
+    return decode_host(c, {"decode_host", false, Form::Full, W, H, nframes}, stream_host, stream_bytes, frame_offsets_host, frames_host,
+                       status_host, indices_host);
 }
 
-// The host form of dbde_b200_decode_roi_device: the same chunk pipeline with roi_w * roi_h bytes per frame
-// coming back.  Records still cross PCIe whole.
 extern "C" int dbde_b200_decode_roi_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                                          const uint64_t *frame_offsets_host, int W, int H, int nframes, int x0, int y0,
                                          int roi_w, int roi_h, uint8_t *roi_host, uint32_t *status_host,
                                          uint64_t *indices_host) {
-    if (!c || !dims_ok(W, H, nframes) || !roi_ok(W, H, x0, y0, roi_w, roi_h) ||
-        (nframes > 0 && (!stream_host || !frame_offsets_host || !roi_host || !status_host)))
-        return fail(DBDE_B200_E_INVALID, "decode_roi_host: bad argument");
-    const SubFrame roi = {x0, y0, roi_w, roi_h, nullptr, 1, 0, 0, 0};
-    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, roi_host, status_host,
-                            indices_host, false, false, &roi);
+    return decode_host(c, {"decode_roi_host", false, Form::Region, W, H, nframes, 0, x0, y0, roi_w, roi_h}, stream_host, stream_bytes,
+                       frame_offsets_host, roi_host, status_host, indices_host);
 }
 
-// The host form of dbde_b200_decode_crops_device: the same chunk pipeline with ncrops * crop_w * crop_h bytes per
-// frame coming back; each chunk's corners go up on its slot's stream.
 extern "C" int dbde_b200_decode_crops_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                                            const uint64_t *frame_offsets_host, int W, int H, int nframes,
                                            const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
                                            int crop_h, int pad, uint8_t *crops_host, uint32_t *status_host,
                                            uint64_t *indices_host) {
-    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad) ||
-        (nframes > 0 && (!stream_host || !frame_offsets_host || !corners_host || !crops_host || !status_host)))
-        return fail(DBDE_B200_E_INVALID, "decode_crops_host: bad argument");
-    const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad, 0};
-    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, crops_host, status_host,
-                            indices_host, false, false, &crops);
+    return decode_host(c, {"decode_crops_host", false, Form::Crops, W, H, nframes, 0, 0, 0, crop_w, crop_h, corners_host, ncrops,
+                           corners_per_frame, pad},
+                       stream_host, stream_bytes, frame_offsets_host, crops_host, status_host, indices_host);
 }
 
-// The host form of dbde_b200_decode_binned_device: the same chunk pipeline with ceil(W / factor) * ceil(H / factor)
-// bytes per frame coming back.  Records still cross PCIe whole.
 extern "C" int dbde_b200_decode_binned_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                                             const uint64_t *frame_offsets_host, int W, int H, int nframes, int factor,
                                             uint8_t *out_host, uint32_t *status_host, uint64_t *indices_host) {
-    if (!c || !dims_ok(W, H, nframes) || !factor_ok(factor) ||
-        (nframes > 0 && (!stream_host || !frame_offsets_host || !out_host || !status_host)))
-        return fail(DBDE_B200_E_INVALID, "decode_binned_host: bad argument");
-    const SubFrame binned = {0, 0, (W - 1) / factor + 1, (H - 1) / factor + 1, nullptr, 1, 0, 0, factor};
-    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, out_host, status_host,
-                            indices_host, false, false, &binned);
+    return decode_host(c, {"decode_binned_host", false, Form::Binned, W, H, nframes, factor}, stream_host, stream_bytes,
+                       frame_offsets_host, out_host, status_host, indices_host);
 }
 
-// dbde_b200_validate_device for a stream in host memory: the records cross PCIe once, nothing comes
-// back but 4 (+8) bytes per frame.
 extern "C" int dbde_b200_validate_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                                        const uint64_t *frame_offsets_host, int W, int H, int nframes,
                                        uint32_t *status_host, uint64_t *indices_host) {
-    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, nullptr, status_host,
-                            indices_host, true);
-}
-
-// ------------------------------------------------------------------ DBDE16 (SURVEY 8 f-4)
-extern "C" size_t dbde_b200_frame_record_bound16(int W, int H) {
-    const size_t wh = (size_t)((W + 7) / 8) * ((H + 7) / 8);
-    return 32 + 3 * wh + 128 * wh;
-}
-extern "C" size_t dbde_b200_slot_stride16(int W, int H) { return (dbde_b200_frame_record_bound16(W, H) + 15) & ~(size_t)15; }
-
-extern "C" int dbde_b200_encode16_device(dbde_b200_ctx *c, const uint16_t *frames_dev, int W, int H, uint64_t first_index,
-                                         int nframes, uint8_t *out_dev, size_t out_capacity, size_t slot_stride,
-                                         uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || (nframes > 0 && (!frames_dev || !out_dev || !frame_offsets_dev || !frame_sizes_dev)) ||
-        ((uintptr_t)frames_dev & 1))
-        return fail(DBDE_B200_E_INVALID, "encode16_device: bad argument");
-    if (nframes == 0) return 0;
-    if (slot_stride == 0) slot_stride = dbde_b200_slot_stride16(W, H);
-    if (slot_stride < dbde_b200_frame_record_bound16(W, H))
-        return fail(DBDE_B200_E_INVALID, "encode16_device: slot_stride < dbde_b200_frame_record_bound16()");
-    if (out_capacity < slot_stride * (size_t)nframes)
-        return fail(DBDE_B200_E_CAPACITY, "encode16_device: out_capacity < nframes * slot_stride");
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    Enc16Params P;
-    P.W = W; P.H = H; P.w = (W + 7) / 8; P.h = (H + 7) / 8; P.wh = P.w * P.h;
-    P.ppf = (P.wh + 255) / 256;
-    const unsigned long long nparts = (unsigned long long)nframes * P.ppf;
-    if (nparts >= 0xFFFFFFF0ull) return fail(DBDE_B200_E_INVALID, "encode16_device: batch too large");
-    const size_t sbytes = 128 + 8 * (size_t)nparts;
-    StreamScratch &sc = scratch_for(c, st);
-    int rc = grow(&sc.enc, &sc.enc_bytes, sbytes);
-    if (rc) return rc;
-    CK(cudaMemsetAsync(sc.enc, 0, sbytes, st));
-    P.frames = frames_dev; P.out = out_dev; P.slot_stride = slot_stride;
-    P.frame_offsets = frame_offsets_dev; P.frame_sizes = frame_sizes_dev;
-    P.ticket = (unsigned int *)sc.enc;
-    P.desc = (uint64_t *)((uint8_t *)sc.enc + 128);
-    P.first_index = first_index; P.nframes = nframes; P.nparts = (unsigned)nparts;
-    P.aligned = (W % 8 == 0) && (((uintptr_t)frames_dev & 15) == 0);
-    CK(launch_encode16(P, c->num_sms, st));
-    c->launches += 1;
-    return 0;
-}
-
-// One CTA per record of a persistent grid, one lane per crop tile (dbde16.cu): dbde_b200_encode_crops_device with U16
-// pixels.  A crop equal to the frame still runs the crop kernel: its records are the frame encoder's records.
-extern "C" int dbde_b200_encode16_crops_device(dbde_b200_ctx *c, const uint16_t *frames_dev, int W, int H, uint64_t first_index,
-                                               int nframes, const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
-                                               int crop_h, int pad, uint8_t *out_dev, size_t out_capacity, size_t slot_stride,
-                                               uint64_t *frame_offsets_dev, uint64_t *frame_sizes_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad, 65535) ||
-        (nframes > 0 && (!frames_dev || !corners_dev || !out_dev || !frame_offsets_dev || !frame_sizes_dev)) ||
-        ((uintptr_t)frames_dev & 1))
-        return fail(DBDE_B200_E_INVALID, "encode16_crops_device: bad argument");
-    if (nframes == 0) return 0;
-    if (slot_stride == 0) slot_stride = dbde_b200_slot_stride16(crop_w, crop_h);
-    if (slot_stride < dbde_b200_frame_record_bound16(crop_w, crop_h))
-        return fail(DBDE_B200_E_INVALID, "encode16_crops_device: slot_stride < dbde_b200_frame_record_bound16(crop_w, crop_h)");
-    const long long nrec = (long long)nframes * ncrops;
-    if (nrec > 0x7FFFFFFFLL) return fail(DBDE_B200_E_INVALID, "encode16_crops_device: nframes * ncrops > 2^31 - 1");
-    if (slot_stride > out_capacity / (size_t)nrec)
-        return fail(DBDE_B200_E_CAPACITY, "encode16_crops_device: out_capacity < nframes * ncrops * slot_stride");
-    CK(cudaSetDevice(c->device));
-    Enc16CropParams P;
-    P.frames = frames_dev;
-    P.W = W;
-    P.H = H;
-    P.corners = corners_dev;
-    P.ncrops = ncrops;
-    P.corner_stride = corners_per_frame ? ncrops : 0;
-    P.crop_w = crop_w;
-    P.crop_h = crop_h;
-    P.w = (crop_w + 7) / 8;
-    P.wh = P.w * ((crop_h + 7) / 8);
-    P.pad = (uint32_t)pad;
-    P.out = out_dev;
-    P.slot_stride = slot_stride;
-    P.frame_offsets = frame_offsets_dev;
-    P.frame_sizes = frame_sizes_dev;
-    P.first_index = first_index;
-    P.nrec = (int)nrec;
-    CK(launch_encode16_crops(P, c->num_sms, (cudaStream_t)stream));
-    c->launches += 1;
-    return 0;
-}
-
-// The DBDE16 validation pass (dbde16_scan_kernel: every check, over the whole record, and the word prefix of every
-// 32 raster-order tiles), queued on st: the first launch of every DBDE16 decode.  P is what the second kernel reads;
-// its output fields are left to the caller.
-static int decode16_scan(dbde_b200_ctx *c, cudaStream_t st, const uint8_t *stream_dev, size_t stream_bytes,
-                         const uint64_t *frame_offsets_dev, int W, int H, int nframes, uint32_t *status_dev, uint64_t *indices_dev,
-                         Dec16Params *P, const char *what) {
-    CK(cudaSetDevice(c->device));
-    *P = Dec16Params();
-    P->W = W; P->H = H; P->w = (W + 7) / 8; P->h = (H + 7) / 8; P->wh = P->w * P->h;
-    P->ppf = (P->wh + 255) / 256;
-    const unsigned long long nparts = (unsigned long long)nframes * P->ppf;
-    if (nparts >= 0xFFFFFFF0ull) return fail(DBDE_B200_E_INVALID, what);
-    const size_t sbytes = 4 * (size_t)nframes * ((size_t)(P->wh + 31) / 32 + 1);
-    StreamScratch &sc = scratch_for(c, st);
-    int rc = grow(&sc.dec, &sc.dec_bytes, sbytes);
-    if (rc) return rc;
-    P->stream = stream_dev; P->stream_bytes = stream_bytes; P->frame_offsets = frame_offsets_dev;
-    P->status = status_dev; P->indices = indices_dev;
-    P->wprefix = (uint32_t *)sc.dec;
-    P->nframes = nframes; P->nparts = (unsigned)nparts;
-    CK(launch_decode16_scan(*P, st));
-    c->launches += 1;
-    return 0;
-}
-
-extern "C" int dbde_b200_decode16_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
-                                         const uint64_t *frame_offsets_dev, int W, int H, int nframes, uint16_t *frames_dev,
-                                         uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || (nframes > 0 && (!stream_dev || !frame_offsets_dev || !frames_dev || !status_dev)) ||
-        ((uintptr_t)frames_dev & 1))
-        return fail(DBDE_B200_E_INVALID, "decode16_device: bad argument");
-    if (nframes == 0) return 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    Dec16Params P;
-    int rc = decode16_scan(c, st, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, status_dev, indices_dev, &P,
-                           "decode16_device: batch too large");
-    if (rc) return rc;
-    P.frames = frames_dev;
-    P.aligned = (W % 8 == 0) && (((uintptr_t)frames_dev & 15) == 0);
-    CK(launch_decode16(P, c->num_sms, st));
-    c->launches += 1;
-    return 0;
-}
-
-// The scan, then one warp per 32 tile columns of each tile row of each crop (dbde16.cu).  A crop equal to the frame
-// still runs the crop kernel: its output layout is the crop layout whatever the corners.
-extern "C" int dbde_b200_decode16_crops_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
-                                               const uint64_t *frame_offsets_dev, int W, int H, int nframes,
-                                               const int32_t *corners_dev, int ncrops, int corners_per_frame, int crop_w,
-                                               int crop_h, int pad, uint16_t *crops_dev, uint32_t *status_dev,
-                                               uint64_t *indices_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad, 65535) ||
-        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !corners_dev || !crops_dev || !status_dev)) ||
-        ((uintptr_t)crops_dev & 1))
-        return fail(DBDE_B200_E_INVALID, "decode16_crops_device: bad argument");
-    if (nframes == 0) return 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    Dec16Params P;
-    int rc = decode16_scan(c, st, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, status_dev, indices_dev, &P,
-                           "decode16_crops_device: batch too large");
-    if (rc) return rc;
-    CK(launch_decode16_crops(P, corners_dev, ncrops, corners_per_frame != 0, crop_w, crop_h, pad, crops_dev, st));
-    c->launches += 1;
-    return 0;
-}
-
-// The scan, then the full decoder's partitions with each tile reduced to its bin means in registers (dbde16.cu).
-// Factor 1 is the full decode.
-extern "C" int dbde_b200_decode16_binned_device(dbde_b200_ctx *c, const uint8_t *stream_dev, size_t stream_bytes,
-                                                const uint64_t *frame_offsets_dev, int W, int H, int nframes, int factor,
-                                                uint16_t *out_dev, uint32_t *status_dev, uint64_t *indices_dev, void *stream) {
-    if (!c || !dims_ok(W, H, nframes) || !factor_ok(factor) ||
-        (nframes > 0 && (!stream_dev || !frame_offsets_dev || !out_dev || !status_dev)) || ((uintptr_t)out_dev & 1))
-        return fail(DBDE_B200_E_INVALID, "decode16_binned_device: bad argument");
-    if (nframes == 0) return 0;
-    if (factor == 1)
-        return dbde_b200_decode16_device(c, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, out_dev, status_dev,
-                                         indices_dev, stream);
-    cudaStream_t st = (cudaStream_t)stream;
-    Dec16Params P;
-    int rc = decode16_scan(c, st, stream_dev, stream_bytes, frame_offsets_dev, W, H, nframes, status_dev, indices_dev, &P,
-                           "decode16_binned_device: batch too large");
-    if (rc) return rc;
-    CK(launch_decode16_binned(P, factor, out_dev, c->num_sms, st));
-    c->launches += 1;
-    return 0;
-}
-
-// Host-buffer forms: the 8-bit path's chunk pipeline (staging slots in flight, records compacted on the
-// device, pageable buffers relayed through the copy pool), with the DBDE16 kernels underneath.
-extern "C" int dbde_b200_encode16_host(dbde_b200_ctx *c, const uint16_t *frames_host, int W, int H, uint64_t first_index,
-                                       int nframes, uint8_t *out_host, size_t out_capacity, uint64_t *frame_offsets_host) {
-    if (!c || !dims_ok(W, H, nframes) || (nframes > 0 && (!frames_host || !out_host || !frame_offsets_host)))
-        return fail(DBDE_B200_E_INVALID, "encode16_host: bad argument");
-    if (nframes == 0) {
-        if (frame_offsets_host) frame_offsets_host[0] = 0;
-        return 0;
-    }
-    EncSequencer seq;
-    int rc = encode_host_worker(c, (const uint8_t *)frames_host, W, H, first_index, nframes, out_host, out_capacity,
-                                frame_offsets_host, default_chunk(c, W, H, nframes, true), 0, 1, &seq, true);
-    if (rc) return rc;
-    frame_offsets_host[nframes] = seq.out_pos;
-    return 0;
+    return decode_host(c, {"validate_host", false, Form::Validate, W, H, nframes}, stream_host, stream_bytes, frame_offsets_host,
+                       nullptr, status_host, indices_host);
 }
 
 extern "C" int dbde_b200_decode16_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                                        const uint64_t *frame_offsets_host, int W, int H, int nframes, uint16_t *frames_host,
                                        uint32_t *status_host, uint64_t *indices_host) {
-    if (!c || !dims_ok(W, H, nframes) || (nframes > 0 && (!stream_host || !frame_offsets_host || !frames_host || !status_host)))
-        return fail(DBDE_B200_E_INVALID, "decode16_host: bad argument");
-    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, (uint8_t *)frames_host, status_host,
-                            indices_host, false, true);
+    return decode_host(c, {"decode16_host", true, Form::Full, W, H, nframes}, stream_host, stream_bytes, frame_offsets_host,
+                       frames_host, status_host, indices_host);
 }
 
-// The host forms of the DBDE16 crop and binned decodes: the same chunk pipeline with the crops' or the bins' pixels
-// coming back.  Records still cross PCIe whole.
 extern "C" int dbde_b200_decode16_crops_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                                              const uint64_t *frame_offsets_host, int W, int H, int nframes,
                                              const int32_t *corners_host, int ncrops, int corners_per_frame, int crop_w,
                                              int crop_h, int pad, uint16_t *crops_host, uint32_t *status_host,
                                              uint64_t *indices_host) {
-    if (!c || !dims_ok(W, H, nframes) || !crops_ok(ncrops, corners_per_frame, crop_w, crop_h, pad, 65535) ||
-        (nframes > 0 && (!stream_host || !frame_offsets_host || !corners_host || !crops_host || !status_host)) ||
-        ((uintptr_t)crops_host & 1))
-        return fail(DBDE_B200_E_INVALID, "decode16_crops_host: bad argument");
-    const SubFrame crops = {0, 0, crop_w, crop_h, corners_host, ncrops, corners_per_frame, pad, 0};
-    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, (uint8_t *)crops_host, status_host,
-                            indices_host, false, true, &crops);
+    return decode_host(c, {"decode16_crops_host", true, Form::Crops, W, H, nframes, 0, 0, 0, crop_w, crop_h, corners_host, ncrops,
+                           corners_per_frame, pad},
+                       stream_host, stream_bytes, frame_offsets_host, crops_host, status_host, indices_host);
 }
 
 extern "C" int dbde_b200_decode16_binned_host(dbde_b200_ctx *c, const uint8_t *stream_host, size_t stream_bytes,
                                               const uint64_t *frame_offsets_host, int W, int H, int nframes, int factor,
                                               uint16_t *out_host, uint32_t *status_host, uint64_t *indices_host) {
-    if (!c || !dims_ok(W, H, nframes) || !factor_ok(factor) ||
-        (nframes > 0 && (!stream_host || !frame_offsets_host || !out_host || !status_host)) || ((uintptr_t)out_host & 1))
-        return fail(DBDE_B200_E_INVALID, "decode16_binned_host: bad argument");
-    if (factor == 1)
-        return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, (uint8_t *)out_host, status_host,
-                                indices_host, false, true);
-    const SubFrame binned = {0, 0, (W - 1) / factor + 1, (H - 1) / factor + 1, nullptr, 1, 0, 0, factor};
-    return decode_host_impl(c, stream_host, stream_bytes, frame_offsets_host, W, H, nframes, (uint8_t *)out_host, status_host,
-                            indices_host, false, true, &binned);
+    return decode_host(c, {"decode16_binned_host", true, Form::Binned, W, H, nframes, factor}, stream_host, stream_bytes,
+                       frame_offsets_host, out_host, status_host, indices_host);
 }
 
 // ------------------------------------------------------------------ multi-GPU sharding
@@ -1548,27 +1448,28 @@ extern "C" int dbde_b200_decode16_binned_host(dbde_b200_ctx *c, const uint8_t *s
 extern "C" int dbde_b200_encode_host_sharded(dbde_b200_ctx **ctxs, int nctx, const uint8_t *frames_host, int W,
                                              int H, uint64_t first_index, int nframes, uint8_t *out_host,
                                              size_t out_capacity, uint64_t *frame_offsets_host) {
-    if (!ctxs || nctx < 1 || !dims_ok(W, H, nframes) || (nframes > 0 && (!frames_host || !out_host || !frame_offsets_host)))
-        return fail(DBDE_B200_E_INVALID, "encode_host_sharded: bad argument");
+    const Request r = {"encode_host_sharded", false, Form::Full, W, H, nframes};
+    if (!ctxs || nctx < 1) return reject(r, DBDE_B200_E_INVALID, "bad argument");
     for (int g = 0; g < nctx; g++)
-        if (!ctxs[g]) return fail(DBDE_B200_E_INVALID, "encode_host_sharded: null context");
+        if (!ctxs[g]) return reject(r, DBDE_B200_E_INVALID, "null context");
+    if (int bad = check_encode(ctxs[0], r, frames_host, out_host, out_capacity, nullptr, frame_offsets_host, nullptr)) return bad;
     if (nframes == 0) {
-        frame_offsets_host[0] = 0;
+        if (frame_offsets_host) frame_offsets_host[0] = 0;
         return 0;
     }
     // The batch is cut into contiguous frame ranges of one chunk each; range ci goes to context
     // ci mod G.  Every context streams its ranges over its own PCIe link, and the ranges' records are
     // placed in stream order as their sizes become known (EncSequencer): the stream is complete when
     // the last copy lands -- no shard is moved afterwards.
-    const int chunk = default_chunk(ctxs[0], W, H, nframes);
+    const int chunk = default_chunk(ctxs[0], r);
     EncSequencer seq;
     std::vector<int> rc(nctx, 0);
     std::vector<std::string> err(nctx);
     std::vector<std::thread> th;
     for (int g = 0; g < nctx; g++) {
         th.emplace_back([&, g]() {
-            rc[g] = encode_host_worker(ctxs[g], frames_host, W, H, first_index, nframes, out_host, out_capacity,
-                                       frame_offsets_host, chunk, g, nctx, &seq);
+            rc[g] = encode_host_worker(ctxs[g], r, frames_host, first_index, out_host, out_capacity, frame_offsets_host, chunk, g,
+                                       nctx, &seq);
             if (rc[g]) {
                 err[g] = dbde_b200_last_error();
                 seq.err.store(rc[g], std::memory_order_relaxed);
