@@ -149,13 +149,26 @@ __device__ __forceinline__ void pack_tile16(uint32_t sbase, uint32_t unit, int k
     }
 }
 
+// min of the 64 pixels (two per word, VIMNMX.U16x2) into mn; returns the depth bits(max - min), 0..16
+__device__ __forceinline__ int tile_stats16(const uint32_t (&px)[32], uint32_t &mn) {
+    uint32_t lo2 = px[0], hi2 = px[0];
+#pragma unroll
+    for (int i = 1; i < 32; i++) {
+        lo2 = __vminu2(lo2, px[i]);
+        hi2 = __vmaxu2(hi2, px[i]);
+    }
+    mn = min(lo2 & 0xffffu, lo2 >> 16);
+    const uint32_t mx = max(hi2 & 0xffffu, hi2 >> 16);
+    return 32 - __clz((int)(mx - mn));
+}
+
 __global__ void __launch_bounds__(kT16, 4) dbde16_encode_kernel(const Enc16Params P) {
     extern __shared__ __align__(16) uint8_t s_words[];
     __shared__ uint32_t s_ticket, s_wtot[kT16 / 32];
     __shared__ uint64_t s_excl;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const size_t fpix = (size_t)P.W * P.H;
-    const size_t fixed = 32 + 3 * (size_t)P.wh;
+    const size_t fixed = rec_fixed(P.wh, 2);
     for (;;) {
         if (tid == 0) s_ticket = atomicAdd(P.ticket, 1u);
         __syncthreads();
@@ -170,15 +183,8 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_kernel(const Enc16Param
         const int ty = valid ? tile / P.w : 0, tx = valid ? tile - ty * P.w : 0;
         uint32_t px[32];
         load_tile16(P.frames + (size_t)f * fpix, P.W, P.H, ty, tx, P.aligned != 0, px);
-        // min / max of the 64 pixels, two per word (VIMNMX.U16x2)
-        uint32_t lo2 = px[0], hi2 = px[0];
-#pragma unroll
-        for (int i = 1; i < 32; i++) {
-            lo2 = __vminu2(lo2, px[i]);
-            hi2 = __vmaxu2(hi2, px[i]);
-        }
-        uint32_t mn = min(lo2 & 0xffffu, lo2 >> 16), mx = max(hi2 & 0xffffu, hi2 >> 16);
-        int k = 32 - __clz((int)(mx - mn));                      // bits(max - min): 0..16
+        uint32_t mn;
+        int k = tile_stats16(px, mn);
         if (!valid) { k = 0; mn = 0; }
         const uint32_t incl = warp_inclusive_scan((uint32_t)k, lane);
         if (lane == 31) s_wtot[warp] = incl;
@@ -209,9 +215,9 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_kernel(const Enc16Param
         const uint64_t excl = s_excl;
         uint8_t *rec = P.out + (size_t)f * P.slot_stride;
         if (valid) {
-            rec[24 + tile] = (uint8_t)k;                                                  // depth plane
-            rec[28 + (size_t)P.wh + 2 * (size_t)tile] = (uint8_t)mn;                      // minimum plane, little-endian U16
-            rec[29 + (size_t)P.wh + 2 * (size_t)tile] = (uint8_t)(mn >> 8);
+            rec[kRecDepth + tile] = (uint8_t)k;                                           // depth plane
+            rec[rec_min(P.wh) + 2 * (size_t)tile] = (uint8_t)mn;                          // minimum plane, little-endian U16
+            rec[rec_min(P.wh) + 2 * (size_t)tile + 1] = (uint8_t)(mn >> 8);
         }
         uint8_t *dst = rec + fixed + 8 * excl;
         const uint32_t *su = reinterpret_cast<const uint32_t *>(s_words);
@@ -221,24 +227,9 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_kernel(const Enc16Param
         } else {
             for (uint32_t i = (uint32_t)tid; i < 8u * agg; i += kT16) dst[i] = s_words[4u * pad16(i >> 2) + (i & 3u)];
         }
-        if (q == (unsigned)P.ppf - 1 && warp == 0) {
-            // fixed fields: {I32 2 | U64 index | F64 0.0 | I32 wh} {I32 2*wh} {I32 n64}  (dbde_util.cpp:141-146,182-191)
-            const uint32_t n64 = (uint32_t)(excl + agg);
-            const uint64_t index = P.first_index + f;
-            uint32_t b;
-            uint8_t *d8;
-            if (lane < 4) { b = (2u >> (8 * lane)) & 0xff; d8 = rec + lane; }
-            else if (lane < 12) { b = (uint32_t)(index >> (8 * (lane - 4))) & 0xff; d8 = rec + lane; }
-            else if (lane < 20) { b = 0; d8 = rec + lane; }
-            else if (lane < 24) { b = ((uint32_t)P.wh >> (8 * (lane - 20))) & 0xff; d8 = rec + lane; }
-            else if (lane < 28) { b = ((uint32_t)(2 * P.wh) >> (8 * (lane - 24))) & 0xff; d8 = rec + 24 + P.wh + (lane - 24); }
-            else { b = (n64 >> (8 * (lane - 28))) & 0xff; d8 = rec + 28 + 3 * (size_t)P.wh + (lane - 28); }
-            *d8 = (uint8_t)b;
-            if (lane == 0) {
-                P.frame_offsets[f] = (uint64_t)f * P.slot_stride;
-                P.frame_sizes[f] = fixed + 8ull * n64;
-            }
-        }
+        if (q == (unsigned)P.ppf - 1 && warp == 0)
+            write_fixed_fields(rec, lane, P.first_index + f, P.wh, 2, (uint32_t)(excl + agg), P.frame_offsets, P.frame_sizes, f,
+                               P.slot_stride);
         __syncthreads();                                      // s_words / s_ticket are reused by the next partition
     }
 }
@@ -298,7 +289,7 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_crops_kernel(const Enc1
     __shared__ uint32_t s_wtot[2][kT16 / 32];                // each warp's word count, by chunk parity
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const size_t fpix = (size_t)P.W * (size_t)P.H;
-    const size_t fixed = 32 + 3 * (size_t)P.wh;
+    const size_t fixed = rec_fixed(P.wh, 2);
     const uint32_t wunit = (uint32_t)warp * kCropWarpUnits16;   // a multiple of 32: pad16(wunit + u) = pad16(wunit) + pad16(u)
     const uint32_t *su = reinterpret_cast<const uint32_t *>(s_words);
     unsigned cc = 0;                                         // chunks done by this CTA: selects the s_wtot half
@@ -320,23 +311,17 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_crops_kernel(const Enc1
 #pragma unroll
                 for (int i = 0; i < 32; i++) px[i] = 0;
             }
-            // dbde16_encode_kernel's tile: min / max (VIMNMX.U16x2), depth, the pair packer
-            uint32_t lo2 = px[0], hi2 = px[0];
-#pragma unroll
-            for (int i = 1; i < 32; i++) {
-                lo2 = __vminu2(lo2, px[i]);
-                hi2 = __vmaxu2(hi2, px[i]);
-            }
-            const uint32_t mn = min(lo2 & 0xffffu, lo2 >> 16), mx = max(hi2 & 0xffffu, hi2 >> 16);
-            const int k = 32 - __clz((int)(mx - mn));        // 0 for the zeros past the crop's last tile
+            // dbde16_encode_kernel's tile: min, depth (0 for the zeros past the crop's last tile), the pair packer
+            uint32_t mn;
+            const int k = tile_stats16(px, mn);
             const uint32_t incl = warp_inclusive_scan((uint32_t)k, lane);
             if (lane == 31) s_wtot[cc & 1][warp] = incl;
             if (k > 0) pack_tile16(smem_u32(s_words), wunit + 2u * (incl - (uint32_t)k), k, mn, px);
             // depth and minimum planes (dbde_util.cpp:156-157), the minimum little-endian U16
             if (valid) {
-                rec[24 + (size_t)t] = (uint8_t)k;
-                rec[28 + (size_t)P.wh + 2 * (size_t)t] = (uint8_t)mn;
-                rec[29 + (size_t)P.wh + 2 * (size_t)t] = (uint8_t)(mn >> 8);
+                rec[kRecDepth + (size_t)t] = (uint8_t)k;
+                rec[rec_min(P.wh) + 2 * (size_t)t] = (uint8_t)mn;
+                rec[rec_min(P.wh) + 1 + 2 * (size_t)t] = (uint8_t)(mn >> 8);
             }
             __syncthreads();                                 // every warp's count is in shared memory
             uint32_t wbase = 0, tot = 0;
@@ -358,24 +343,9 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_crops_kernel(const Enc1
             carry += tot;
             __syncwarp();                                    // the copy has read the staging before the next chunk packs into it
         }
-        if (warp == 0) {
-            // the fixed fields (dbde_util.cpp:141-146,182-188,191), as dbde16_encode_kernel writes them
-            const uint64_t index = P.first_index + (uint64_t)f;
-            const uint32_t wh = (uint32_t)P.wh;
-            uint32_t b;
-            uint8_t *d8;
-            if (lane < 4) { b = (2u >> (8 * lane)) & 0xff; d8 = rec + lane; }
-            else if (lane < 12) { b = (uint32_t)(index >> (8 * (lane - 4))) & 0xff; d8 = rec + lane; }
-            else if (lane < 20) { b = 0; d8 = rec + lane; }
-            else if (lane < 24) { b = (wh >> (8 * (lane - 20))) & 0xff; d8 = rec + lane; }
-            else if (lane < 28) { b = ((2u * wh) >> (8 * (lane - 24))) & 0xff; d8 = rec + 24 + (size_t)wh + (lane - 24); }
-            else { b = (carry >> (8 * (lane - 28))) & 0xff; d8 = rec + 28 + 3 * (size_t)wh + (lane - 28); }
-            *d8 = (uint8_t)b;
-            if (lane == 0) {
-                P.frame_offsets[j] = (uint64_t)j * P.slot_stride;
-                P.frame_sizes[j] = fixed + 8ull * carry;
-            }
-        }
+        if (warp == 0)   // wh widened from unsigned: from int, ptxas reschedules the chunk loop and the crops encode 2.5 % slower
+            write_fixed_fields(rec, lane, P.first_index + (uint64_t)f, (uint32_t)P.wh, 2, carry, P.frame_offsets, P.frame_sizes, j,
+                               P.slot_stride);
     }
 }
 
@@ -386,28 +356,13 @@ __global__ void __launch_bounds__(kT16, 4) dbde16_encode_crops_kernel(const Enc1
 __global__ void __launch_bounds__(256) dbde16_scan_kernel(const Dec16Params P) {
     __shared__ uint32_t s_warp[8], s_flag;
     const int f = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint64_t off = P.frame_offsets[f];
-    const uint64_t fixed = 32 + 3 * (uint64_t)P.wh;
     const int ng = (P.wh + 31) / 32;
     uint32_t *wp = P.wprefix + (size_t)f * (ng + 1);
-    if (off > P.stream_bytes || P.stream_bytes - off < fixed) {   // no wrap for any off
-        if (tid == 0) {
-            P.status[f] = kStTruncated;
-            if (P.indices) P.indices[f] = 0;
-        }
-        return;
-    }
-    const uint64_t room = P.stream_bytes - off - fixed;      // payload bytes the stream has after the fixed fields
-    const uint8_t *rec = P.stream + off;
-    auto le32 = [](const uint8_t *p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); };
-    uint32_t status = 0;
-    if (le32(rec) != 2u) status |= kStBadFrameHeader;
-    if (le32(rec + 20) != (uint32_t)P.wh) status |= kStBadDepthCount;
-    if (le32(rec + 24 + P.wh) != 2u * (uint32_t)P.wh) status |= kStBadMinCount;
-    const uint32_t n64 = le32(rec + 28 + 3 * (size_t)P.wh);
+    ScanHead h;
+    if (!scan_head(P.stream, P.stream_bytes, P.frame_offsets[f], P.wh, 2, f, P.status, P.indices, h)) return;
     if (tid == 0) s_flag = 0;
     __syncthreads();
-    const uint8_t *dp = rec + 24;
+    const uint8_t *dp = h.rec + kRecDepth;
     bool big = false;
     for (int g0 = warp * 4; g0 < ng; g0 += 32) {              // four groups in flight per warp
         uint32_t d[4];
@@ -425,42 +380,8 @@ __global__ void __launch_bounds__(256) dbde16_scan_kernel(const Dec16Params P) {
     }
     if (big) atomicOr(&s_flag, 1u);
     __syncthreads();
-    uint32_t carry = 0;
-    for (int base = 0; base < ng; base += 2048) {
-        uint32_t v[8], local = 0;
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            const int idx = base + tid * 8 + i;
-            v[i] = idx < ng ? wp[idx] : 0u;
-            local += v[i];
-        }
-        const uint32_t incl = warp_inclusive_scan(local, lane);
-        if (lane == 31) s_warp[warp] = incl;
-        __syncthreads();
-        uint32_t pre = carry + incl - local, tot = 0;
-#pragma unroll
-        for (int wv = 0; wv < 8; wv++) {
-            const uint32_t x = s_warp[wv];
-            if (wv < warp) pre += x;
-            tot += x;
-        }
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            const int idx = base + tid * 8 + i;
-            if (idx < ng) wp[idx] = pre;
-            pre += v[i];
-        }
-        carry += tot;
-        __syncthreads();
-    }
-    if (tid == 0) {
-        wp[ng] = carry;
-        if (carry != n64) status |= kStBadWordCount;
-        if (s_flag) status |= kStDepthTooBig;
-        if (room < 8ull * carry) status |= kStTruncated;
-        P.status[f] = status;
-        if (P.indices) P.indices[f] = (uint64_t)le32(rec + 4) | ((uint64_t)le32(rec + 8) << 32);
-    }
+    const uint32_t total = scan_items(wp, ng, s_warp, tid, warp, lane);
+    if (tid == 0) scan_finish(h, wp, ng, total, s_flag != 0, f, P.status, P.indices);
 }
 
 // ------------------------------------------------------------------ decoder: unpack
@@ -558,28 +479,41 @@ __device__ __forceinline__ void store_bins16(uint16_t *op, int Wb, int ncb, int 
     }
 }
 
-// A partition's agg words at src (any alignment), coalesced over the CTA's threads, into the padded layout of
-// unpack_tile16 at s_words.  Padded layout (pad16): after every 32 units comes one padding unit, and that padding
-// unit holds a COPY of the unit that follows it, so the reader's "this unit and the next" is always two adjacent loads.
-__device__ __forceinline__ void stage_words16(uint8_t *s_words, const uint8_t *src, uint32_t agg, int tid) {
-    uint32_t *su = reinterpret_cast<uint32_t *>(s_words);
+// agg words at src (any alignment), spread over nlanes threads (this one is `lane`), into the padded layout of
+// unpack_tile16 at su.  Padded layout (pad16): after every 32 units comes one padding unit, and that padding unit holds a
+// COPY of the unit that follows it, so the reader's "this unit and the next" is always two adjacent loads.
+// CROP = false, the full decoders: each partition is read once, streaming (__ldcs), and a run that is not 8-byte aligned
+// is copied a byte at a time, the code these decoders have always had.  CROP = true, the crop decoder: loads take the
+// read-only path, and an unaligned run is read four bytes per 32-bit unit -- with byte copies its 1001x1003 crops ran
+// 21 % slower.
+template <bool CROP>
+__device__ __forceinline__ void stage_words16(uint32_t *su, const uint8_t *src, uint32_t agg, uint32_t lane, uint32_t nlanes) {
     if (((uintptr_t)src & 7) == 0) {
-        for (uint32_t i = (uint32_t)tid; i < agg; i += kT16) {
-            const uint64_t v = __ldcs(reinterpret_cast<const uint64_t *>(src) + i);
+        for (uint32_t i = lane; i < agg; i += nlanes) {
+            const uint64_t *p = reinterpret_cast<const uint64_t *>(src) + i;
+            const uint64_t v = CROP ? __ldg(p) : __ldcs(p);
             const uint32_t at = pad16(2u * i);                                  // units 2i and 2i+1 share a block of 32
             su[at] = (uint32_t)v;
             su[at + 1u] = (uint32_t)(v >> 32);
             if (((2u * i) & 31u) == 0u && i > 0u) su[at - 1u] = (uint32_t)v;    // the copy in the padding slot before it
         }
+    } else if (CROP) {
+        for (uint32_t u = lane; u < 2u * agg; u += nlanes) {
+            const uint32_t v = ld_le32(src + 4u * u);
+            const uint32_t at = pad16(u);
+            su[at] = v;
+            if ((u & 31u) == 0u && u > 0u) su[at - 1u] = v;
+        }
     } else {
-        for (uint32_t i = (uint32_t)tid; i < 8u * agg; i += kT16) {
+        uint8_t *s8 = reinterpret_cast<uint8_t *>(su);
+        for (uint32_t i = lane; i < 8u * agg; i += nlanes) {
             const uint32_t u = i >> 2;
-            s_words[4u * pad16(u) + (i & 3u)] = src[i];
-            if ((u & 31u) == 0u && u > 0u) s_words[4u * (pad16(u) - 1u) + (i & 3u)] = src[i];
+            s8[4u * pad16(u) + (i & 3u)] = src[i];
+            if ((u & 31u) == 0u && u > 0u) s8[4u * (pad16(u) - 1u) + (i & 3u)] = src[i];
         }
     }
-    if (tid < 2) {                                                            // the reader looks one unit past the end
-        const uint32_t u = 2u * agg + (uint32_t)tid;
+    if (lane < 2) {                                                           // the reader looks one unit past the end
+        const uint32_t u = 2u * agg + lane;
         su[pad16(u)] = 0u;
         if ((u & 31u) == 0u && u > 0u) su[pad16(u) - 1u] = 0u;
     }
@@ -598,15 +532,15 @@ __global__ void __launch_bounds__(kT16) dbde16_decode_kernel(const Dec16Params P
         const int g0 = (int)q * (kT16 / 32), g1 = min(g0 + kT16 / 32, ng);
         const uint32_t w0 = wp[g0], agg = wp[g1] - w0;
         // the partition's words, coalesced, into shared memory
-        const uint8_t *src = rec + 32 + 3 * (size_t)P.wh + 8ull * w0;
-        stage_words16(s_words, src, agg, tid);
+        const uint8_t *src = rec + rec_fixed(P.wh, 2) + 8ull * w0;
+        stage_words16<false>(reinterpret_cast<uint32_t *>(s_words), src, agg, (uint32_t)tid, kT16);
         const int tile = (int)q * kT16 + tid;
         const bool valid = tile < P.wh;
         int k = 0;
         uint32_t mn = 0;
         if (valid) {
-            k = rec[24 + tile];
-            const uint8_t *mp = rec + 28 + (size_t)P.wh + 2 * (size_t)tile;
+            k = rec[kRecDepth + tile];
+            const uint8_t *mp = rec + rec_min(P.wh) + 2 * (size_t)tile;
             mn = (uint32_t)mp[0] | ((uint32_t)mp[1] << 8);
         }
         const uint32_t incl = warp_inclusive_scan((uint32_t)k, lane);
@@ -641,14 +575,14 @@ __global__ void __launch_bounds__(kT16) dbde16_decode_binned_kernel(const Dec16P
         const uint32_t *wp = P.wprefix + (size_t)f * (ng + 1);
         const int g0 = (int)q * (kT16 / 32), g1 = min(g0 + kT16 / 32, ng);
         const uint32_t w0 = wp[g0], agg = wp[g1] - w0;
-        stage_words16(s_words, rec + 32 + 3 * (size_t)P.wh + 8ull * w0, agg, tid);
+        stage_words16<false>(reinterpret_cast<uint32_t *>(s_words), rec + rec_fixed(P.wh, 2) + 8ull * w0, agg, (uint32_t)tid, kT16);
         const int tile = (int)q * kT16 + tid;
         const bool valid = tile < P.wh;
         int k = 0;
         uint32_t mn = 0;
         if (valid) {
-            k = rec[24 + tile];
-            const uint8_t *mp = rec + 28 + (size_t)P.wh + 2 * (size_t)tile;
+            k = rec[kRecDepth + tile];
+            const uint8_t *mp = rec + rec_min(P.wh) + 2 * (size_t)tile;
             mn = (uint32_t)mp[0] | ((uint32_t)mp[1] << 8);
         }
         const uint32_t incl = warp_inclusive_scan((uint32_t)k, lane);
@@ -666,26 +600,14 @@ __global__ void __launch_bounds__(kT16) dbde16_decode_binned_kernel(const Dec16P
 }
 
 // ------------------------------------------------------------------ decoder: crops
-// ncrops rectangles of crop_w x crop_h per frame at int32 corners, after dbde16_scan_kernel.  The scan's word prefix
-// item g covers tiles [32 g, 32 g + 32) in raster order, so a run of consecutive tiles of one tile row has ONE
-// contiguous payload run, starting at the item's prefix plus the depths of the item's tiles before the run.
-// One warp == up to 32 consecutive tile columns of one tile row of a crop of one frame, one lane == one tile; a crop
-// narrower than 32 tiles gives each tile row a SEGMENT of S lanes (the next power of two >= its width in tiles) and a
-// warp 32 / S tile rows.  A segment stages its run in the padded layout and unpacks with unpack_tile16.  Lanes whose
-// tile lies outside the frame load nothing and unpack depth 0 with the pad value as minimum; a crop entirely outside
-// the frame reads nothing of the record.  Rows are cropped on all four sides and leave as aligned 16-byte words
-// assembled across lanes.
+// ncrops rectangles of crop_w x crop_h per frame at int32 corners, after dbde16_scan_kernel, on the task grid of the
+// 8-bit crop decoder (crop_task): one warp == up to 32 consecutive tile columns of one tile row of a crop of one frame,
+// one lane == one tile, in segments of S lanes for crops narrower than 32 tiles.  A segment stages its payload run in
+// the padded layout and unpacks with unpack_tile16.  Lanes whose tile lies outside the frame unpack depth 0 with the
+// pad value as minimum.  Rows are cropped on all four sides and leave as aligned 16-byte words assembled across lanes.
 struct Crop16Params {
-    const uint8_t *stream;
-    const uint64_t *frame_offsets;
-    const uint32_t *status;     // from the scan: frames with status != 0 are skipped
-    const uint32_t *wprefix;    // nframes * (ng + 1)
-    const int32_t *corners;     // {x0, y0} of crop r of frame f at corners + 2 * (f * corner_stride + r)
+    CropGrid g;                 // the scan's outputs, the frame, the crops and their tasks
     uint16_t *out;              // nframes * ncrops * crop_w * crop_h, tightly packed, 2-byte aligned
-    int W, H, w, h, wh, ng;     // the frame in pixels and tiles, word-prefix items per frame
-    int crop_w, crop_h, ncrops, corner_stride;   // corner_stride: ncrops (per-frame corners) or 0 (shared)
-    int nchunks, seg_shift, nrg;                 // 32-tile chunks per tile row, log2 lanes per segment, warps per chunk
-    unsigned long long ntasks;                   // nframes * ncrops * nrg * nchunks warps
     uint32_t pad2;              // the pad value in both halves
 };
 
@@ -728,95 +650,27 @@ __device__ __forceinline__ void crop16_store_row(uint16_t *row, int pos, uint4 x
 
 __global__ void __launch_bounds__(kCrop16Warps * 32) dbde16_decode_crops_kernel(const Crop16Params P) {
     __shared__ __align__(16) uint32_t s_buf[kCrop16Warps][kCrop16BufUnits];
+    const CropGrid &G = P.g;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const unsigned long long task = (unsigned long long)blockIdx.x * kCrop16Warps + warp;
-    if (task >= P.ntasks) return;
-    // task = ((f * ncrops + r) * nrg + row group) * nchunks + chunk: neighbouring warps read neighbouring payloads
-    const int chunk = (int)(task % (unsigned)P.nchunks);
-    const unsigned long long fr = task / (unsigned)P.nchunks;
-    const unsigned long long fc = fr / (unsigned)P.nrg;
-    const int rg = (int)(fr - fc * (unsigned)P.nrg);
-    const int f = (int)(fc / (unsigned)P.ncrops);
-    const int r = (int)(fc - (unsigned long long)f * (unsigned)P.ncrops);
-    if (P.status[f] != 0) return;                            // rejected by the scan: its crops stay untouched
-    const int32_t *cp = P.corners + 2 * ((size_t)f * (size_t)P.corner_stride + (size_t)r);
-    const int x0 = __ldg(cp), y0 = __ldg(cp + 1);
-    // floor division (negative corners), the far edge in 64 bits (corners up to INT32_MAX)
-    const int tx0 = x0 >> 3, ty0 = y0 >> 3;
-    const int tx_end = (int)(((long long)x0 + P.crop_w + 7) >> 3);
-    const int nty = (int)(((long long)y0 + P.crop_h + 7) >> 3) - ty0;
-    uint16_t *rout = P.out + (size_t)fc * ((size_t)P.crop_w * (size_t)P.crop_h);
-    const int S = 1 << P.seg_shift;
-    const int seg = lane >> P.seg_shift, sl = lane & (S - 1);
-    const int rowi = (rg << (5 - P.seg_shift)) + seg;        // tile row of the crop
-    const bool rowok = rowi < nty;
-    const int ty = ty0 + rowi;
-    const int txc = tx0 + 32 * chunk;                        // my segment's first tile column
-    const int tx = txc + sl;
-    const bool live = rowok && tx < tx_end;
-    // the segment's tiles inside the frame: columns [txa, txb) of tile row ty, one contiguous payload run
-    const int txa = max(txc, 0), txb = min(min(txc + S, tx_end), P.w);
-    const bool segin = rowok && ty >= 0 && ty < P.h && txa < txb;
-    const bool inframe = live && segin && tx >= 0 && tx < P.w;
-    const uint8_t *rec = P.stream + P.frame_offsets[f];
-    const int t0 = segin ? ty * P.w + txa : 0;               // the run's first raster tile
-    const int item = t0 >> 5, rem = t0 & 31;
-    const int tl = inframe ? ty * P.w + tx : 0;              // my tile
-
-    // word offset of tile t0: the item's exclusive prefix plus the depths of the item's tiles before t0
-    uint32_t before = 0;
-    if (segin)
-        for (int j = sl; j < rem; j += S) before += rec[24 + 32 * item + j];
-    for (int o = 1; o < S; o <<= 1) before += __shfl_xor_sync(0xffffffffu, before, o);
-    int k = 0;
+    CropTask T;
+    if (!crop_task<true>(G, (unsigned long long)blockIdx.x * kCrop16Warps + warp, lane, T)) return;
+    const int S = T.S, sl = T.sl, tx = T.tx;
     uint32_t mn = P.pad2 & 0xffffu;                          // outside the frame: depth 0 with the pad value as minimum
-    if (inframe) {
-        k = rec[24 + tl];
-        const uint8_t *mp = rec + 28 + (size_t)P.wh + 2 * (size_t)tl;
+    if (T.inframe) {
+        const uint8_t *mp = T.rec + rec_min(G.wh) + 2 * (size_t)T.tl;
         mn = (uint32_t)mp[0] | ((uint32_t)mp[1] << 8);
     }
-    const uint32_t wbase = segin ? P.wprefix[(size_t)f * (P.ng + 1) + item] + before : 0u;
-    uint32_t incl = (uint32_t)k;                             // inclusive scan of the depths inside the segment
-    for (int d = 1; d < S; d <<= 1) {
-        const uint32_t t = __shfl_up_sync(0xffffffffu, incl, d, S);
-        if (sl >= d) incl += t;
-    }
-    const uint32_t nwords = __shfl_sync(0xffffffffu, incl, S - 1, S);
-
-    // stage the segment's run (nothing outside it is read): 8-byte loads when it is 8-byte aligned, else 4 byte loads
-    // per unit
-    uint32_t *su = s_buf[warp] + seg * (33 * S + 2);
-    const uint8_t *src = rec + 32 + 3 * (size_t)P.wh + 8 * (size_t)wbase;
-    if (((uintptr_t)src & 7) == 0) {
-        for (uint32_t i = (uint32_t)sl; i < nwords; i += (uint32_t)S) {
-            const uint64_t v = __ldg(reinterpret_cast<const unsigned long long *>(src) + i);
-            const uint32_t at = pad16(2u * i);
-            su[at] = (uint32_t)v;
-            su[at + 1u] = (uint32_t)(v >> 32);
-            if (((2u * i) & 31u) == 0u && i > 0u) su[at - 1u] = (uint32_t)v;
-        }
-    } else {
-        for (uint32_t u = (uint32_t)sl; u < 2u * nwords; u += (uint32_t)S) {
-            const uint8_t *b = src + 4u * u;
-            const uint32_t v = (uint32_t)b[0] | ((uint32_t)b[1] << 8) | ((uint32_t)b[2] << 16) | ((uint32_t)b[3] << 24);
-            const uint32_t at = pad16(u);
-            su[at] = v;
-            if ((u & 31u) == 0u && u > 0u) su[at - 1u] = v;
-        }
-    }
-    if (sl == 0) {                                           // the reader looks one unit past the end
-        const uint32_t u = 2u * nwords;
-        su[pad16(u)] = 0u;
-        if ((u & 31u) == 0u && u > 0u) su[pad16(u) - 1u] = 0u;
-    }
+    // stage the segment's run (nothing outside it is read)
+    uint32_t *su = s_buf[warp] + T.seg * (33 * S + 2);
+    stage_words16<true>(su, T.rec + rec_fixed(G.wh, 2) + 8 * (size_t)T.wbase, T.nwords, (uint32_t)sl, (uint32_t)S);
     __syncwarp();
 
     uint32_t px[32];
-    unpack_tile16(su, incl - (uint32_t)k, k, mn, px);
+    unpack_tile16(su, T.incl - T.k, (int)T.k, mn, px);
 
     // the frame's partial last tile column / row: pixels past column W and rows past H are pad
-    const int wc = inframe && tx == P.w - 1 ? (P.W & 7) : 0;              // kept pixels of each row, 0 = all
-    const int hr = inframe && ty == P.h - 1 ? P.H - 8 * ty : 8;           // kept rows
+    const int wc = T.inframe && tx == G.w - 1 ? (G.W & 7) : 0;          // kept pixels of each row, 0 = all
+    const int hr = T.inframe && T.ty == G.h - 1 ? G.H - 8 * T.ty : 8;     // kept rows
 #pragma unroll
     for (int j = 0; j < 4; j++) {
         const uint32_t m = wc == 0 || 2 * j + 2 <= wc ? ~0u : 2 * j + 1 == wc ? 0xffffu : 0u;
@@ -825,38 +679,25 @@ __global__ void __launch_bounds__(kCrop16Warps * 32) dbde16_decode_crops_kernel(
     }
     // crop and store: rows of the tile inside [y0, y0 + crop_h), columns inside [x0, x0 + crop_w).  Offsets are taken
     // from the crop's first tile, so corners near INT32_MAX do not overflow
-    const int pos = 8 * (tx - tx0) - (x0 & 7);
-    const bool last = sl == S - 1 || tx + 1 >= tx_end;
+    uint16_t *rout = P.out + (size_t)T.rect * ((size_t)G.crop_w * (size_t)G.crop_h);
+    const int pos = 8 * (tx - T.tx0) - (T.x0 & 7);
+    const bool last = sl == S - 1 || tx + 1 >= T.tx_end;
 #pragma unroll
     for (int rr = 0; rr < 8; rr++) {
-        const int yr = 8 * rowi + rr - (y0 & 7);                               // the same in every lane of a segment
-        const bool in = live && yr >= 0 && yr < P.crop_h;
-        crop16_store_row(rout + (in ? (size_t)yr * (size_t)P.crop_w : 0), pos,
-                         make_uint4(px[4 * rr], px[4 * rr + 1], px[4 * rr + 2], px[4 * rr + 3]), P.crop_w, in, sl == 0, last);
+        const int yr = 8 * T.rowi + rr - (T.y0 & 7);                           // the same in every lane of a segment
+        const bool in = T.live && yr >= 0 && yr < G.crop_h;
+        crop16_store_row(rout + (in ? (size_t)yr * (size_t)G.crop_w : 0), pos,
+                         make_uint4(px[4 * rr], px[4 * rr + 1], px[4 * rr + 2], px[4 * rr + 3]), G.crop_w, in, sl == 0, last);
     }
 }
 
 // ------------------------------------------------------------------ launches
-static size_t smem16() { return (size_t)kWordBytesPadded16; }
-
-template <typename Kern, typename Params>
-static cudaError_t launch16(Kern kern, const Params &P, unsigned nparts, int num_sms, cudaStream_t stream) {
-    int occ = 0;
-    cudaError_t e = cached_occupancy((const void *)kern, kT16, smem16(), &occ);
-    if (e != cudaSuccess) return e;
-    unsigned grid = (unsigned)(num_sms * occ);
-    if (grid > nparts) grid = nparts;
-    if (grid == 0) return cudaSuccess;
-    kern<<<grid, kT16, smem16(), stream>>>(P);
-    return cudaGetLastError();
-}
-
 cudaError_t launch_encode16(const Enc16Params &P, int num_sms, cudaStream_t stream) {
-    return launch16(dbde16_encode_kernel, P, P.nparts, num_sms, stream);
+    return launch_persistent(dbde16_encode_kernel, P, P.nparts, kT16, kWordBytesPadded16, num_sms, stream);
 }
 cudaError_t launch_encode16_crops(const Enc16CropParams &P, int num_sms, cudaStream_t stream) {
     if (P.nrec <= 0) return cudaSuccess;
-    return launch16(dbde16_encode_crops_kernel, P, (unsigned)P.nrec, num_sms, stream);
+    return launch_persistent(dbde16_encode_crops_kernel, P, (unsigned)P.nrec, kT16, kWordBytesPadded16, num_sms, stream);
 }
 cudaError_t launch_decode16_scan(const Dec16Params &P, cudaStream_t stream) {
     if (P.nframes <= 0) return cudaSuccess;
@@ -864,16 +705,16 @@ cudaError_t launch_decode16_scan(const Dec16Params &P, cudaStream_t stream) {
     return cudaGetLastError();
 }
 cudaError_t launch_decode16(const Dec16Params &P, int num_sms, cudaStream_t stream) {
-    return launch16(dbde16_decode_kernel, P, P.nparts, num_sms, stream);
+    return launch_persistent(dbde16_decode_kernel, P, P.nparts, kT16, kWordBytesPadded16, num_sms, stream);
 }
 
 cudaError_t launch_decode16_binned(const Dec16Params &scan, int factor, uint16_t *out, int num_sms, cudaStream_t stream) {
     Dec16Params P = scan;
     P.frames = out;
     switch (factor) {
-        case 2: return launch16(dbde16_decode_binned_kernel<2>, P, P.nparts, num_sms, stream);
-        case 4: return launch16(dbde16_decode_binned_kernel<4>, P, P.nparts, num_sms, stream);
-        case 8: return launch16(dbde16_decode_binned_kernel<8>, P, P.nparts, num_sms, stream);
+        case 2: return launch_persistent(dbde16_decode_binned_kernel<2>, P, P.nparts, kT16, kWordBytesPadded16, num_sms, stream);
+        case 4: return launch_persistent(dbde16_decode_binned_kernel<4>, P, P.nparts, kT16, kWordBytesPadded16, num_sms, stream);
+        case 8: return launch_persistent(dbde16_decode_binned_kernel<8>, P, P.nparts, kT16, kWordBytesPadded16, num_sms, stream);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -881,29 +722,17 @@ cudaError_t launch_decode16_binned(const Dec16Params &scan, int factor, uint16_t
 cudaError_t launch_decode16_crops(const Dec16Params &scan, const int32_t *corners, int ncrops, bool per_frame, int crop_w,
                                   int crop_h, int pad, uint16_t *out, cudaStream_t stream) {
     Crop16Params P = Crop16Params();
-    P.stream = scan.stream;
-    P.frame_offsets = scan.frame_offsets;
-    P.status = scan.status;
-    P.wprefix = scan.wprefix;
-    P.corners = corners;
-    P.out = out;
-    P.W = scan.W; P.H = scan.H; P.w = scan.w; P.h = scan.h; P.wh = scan.wh;
-    P.ng = (scan.wh + 31) / 32;
-    P.crop_w = crop_w; P.crop_h = crop_h; P.ncrops = ncrops;
-    P.corner_stride = per_frame ? ncrops : 0;
+    unsigned blocks = 0;
     // a crop starting 7 columns / rows into a tile spans one tile more than one starting on a tile boundary
-    const int span = (int)(((long long)crop_w + 14) / 8), nty = (int)(((long long)crop_h + 14) / 8);
-    P.nchunks = (span + 31) / 32;
-    P.seg_shift = 0;                                          // segments: the next power of two >= the span, <= 32 lanes
-    while ((1 << P.seg_shift) < span && P.seg_shift < 5) P.seg_shift++;
-    P.nrg = (nty + (32 >> P.seg_shift) - 1) / (32 >> P.seg_shift);
-    P.ntasks = (unsigned long long)scan.nframes * (unsigned long long)ncrops * (unsigned long long)P.nrg *
-               (unsigned long long)P.nchunks;
+    const cudaError_t e = crop_grid(P.g, scan, scan.W, scan.H, (scan.wh + 31) / 32, crop_w, crop_h, ncrops,
+                                    (int)(((long long)crop_w + 14) / 8), (int)(((long long)crop_h + 14) / 8), kCrop16Warps, &blocks);
+    if (e != cudaSuccess) return e;
+    if (blocks == 0) return cudaSuccess;
+    P.g.corners = corners;
+    P.g.corner_stride = per_frame ? ncrops : 0;
+    P.out = out;
     P.pad2 = (uint32_t)(pad & 0xFFFF) * 0x00010001u;
-    if (P.ntasks == 0) return cudaSuccess;
-    const unsigned long long blocks = (P.ntasks + kCrop16Warps - 1) / kCrop16Warps;
-    if (blocks > 0x7FFFFFFFull) return cudaErrorInvalidConfiguration;
-    dbde16_decode_crops_kernel<<<(unsigned)blocks, kCrop16Warps * 32, 0, stream>>>(P);
+    dbde16_decode_crops_kernel<<<blocks, kCrop16Warps * 32, 0, stream>>>(P);
     return cudaGetLastError();
 }
 

@@ -294,7 +294,7 @@ extern "C" int dbde_b200_set_chunk_frames(dbde_b200_ctx *c, int frames) {
 // ------------------------------------------------------------------ sizes
 extern "C" size_t dbde_b200_frame_record_bound(int W, int H) {
     const size_t wh = (size_t)((W + 7) / 8) * ((H + 7) / 8);
-    return 32 + 66 * wh;
+    return rec_bound(wh, 1);
 }
 extern "C" size_t dbde_b200_slot_stride(int W, int H) { return (dbde_b200_frame_record_bound(W, H) + 15) / 16 * 16; }
 extern "C" size_t dbde_b200_stream_bound(int W, int H, int nframes) {
@@ -418,7 +418,7 @@ struct Request {
         f.px = (size_t)fw * fh * (u16 ? 2 : 1);
         f.bound = u16 ? dbde_b200_frame_record_bound16(fw, fh) : dbde_b200_frame_record_bound(fw, fh);
         f.stride = (f.bound + 15) & ~(size_t)15;
-        f.delta = (16 - (32 + (u16 ? 3 : 2) * wh) % 16) % 16;
+        f.delta = (16 - rec_fixed(wh, u16 ? 2 : 1) % 16) % 16;
         return f;
     }
     int records() const { return form == Form::Crops ? ncrops : 1; }      // per frame
@@ -770,7 +770,7 @@ extern "C" int dbde_b200_decode_binned_device(dbde_b200_ctx *c, const uint8_t *s
 // ------------------------------------------------------------------ DBDE16 (SURVEY 8 f-4)
 extern "C" size_t dbde_b200_frame_record_bound16(int W, int H) {
     const size_t wh = (size_t)((W + 7) / 8) * ((H + 7) / 8);
-    return 32 + 3 * wh + 128 * wh;
+    return rec_bound(wh, 2);
 }
 extern "C" size_t dbde_b200_slot_stride16(int W, int H) { return (dbde_b200_frame_record_bound16(W, H) + 15) & ~(size_t)15; }
 
@@ -1521,12 +1521,12 @@ extern "C" int dbde_b200_decode_host_sharded(dbde_b200_ctx **ctxs, int nctx, con
 static long index_stream_impl(const uint8_t *p, size_t bytes, int W, int H, uint64_t *offs, long max_frames, size_t minbytes) {
     if (!p || !offs || !dims_ok(W, H, 0)) return fail(DBDE_B200_E_INVALID, "index_stream: bad argument");
     const size_t wh = (size_t)((W + 7) / 8) * ((H + 7) / 8);
-    const size_t fixed = 32 + (1 + minbytes) * wh;
+    const size_t fixed = rec_fixed(wh, minbytes);
     size_t cur = 0;
     long n = 0;
     while (cur + fixed <= bytes && n < max_frames) {
         uint32_t n64;
-        memcpy(&n64, p + cur + fixed - 4, 4);
+        memcpy(&n64, p + cur + rec_n64(wh, minbytes), 4);
         const size_t next = cur + fixed + 8 * (size_t)n64;
         if (next > bytes) break;
         offs[n++] = cur;

@@ -44,33 +44,15 @@ constexpr int kDecPlaneBytes = kTilesPerPart + 32;
 constexpr int kDecStageBytes = ((kDecPayloadBytes + 2 * kDecPlaneBytes + 127) / 128) * 128;
 
 // ------------------------------------------------------------------ scan / validate pre-pass
-__device__ __forceinline__ uint32_t ldg_u32_bytes(const uint8_t *p) {
-    return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
-}
-
 __global__ void __launch_bounds__(256) dbde_decode_scan_kernel(const DecParams P) {
     __shared__ uint32_t s_warp[8];
     __shared__ uint32_t s_flag;
     const PartGeom &g = P.g;
     const int f = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint64_t off = P.frame_offsets[f];
-    const uint64_t fixed = 32 + 2 * (uint64_t)g.wh;
     const int nitems = g.ppf * kConsumerWarps;
     uint32_t *wp = P.wprefix + (size_t)f * (nitems + 1);
-    if (off > P.stream_bytes || P.stream_bytes - off < fixed) {   // cannot even read the fixed fields (no wrap for any off)
-        if (tid == 0) {
-            P.status[f] = kStTruncated;
-            if (P.indices) P.indices[f] = 0;
-        }
-        return;
-    }
-    const uint64_t room = P.stream_bytes - off - fixed;      // payload bytes the stream has after the fixed fields
-    const uint8_t *rec = P.stream + off;
-    uint32_t status = 0;
-    if (ldg_u32_bytes(rec) != 2u) status |= kStBadFrameHeader;
-    if (ldg_u32_bytes(rec + 20) != (uint32_t)g.wh) status |= kStBadDepthCount;
-    if (ldg_u32_bytes(rec + 24 + g.wh) != (uint32_t)g.wh) status |= kStBadMinCount;
-    const uint32_t n64 = ldg_u32_bytes(rec + 28 + 2 * (size_t)g.wh);
+    ScanHead h;
+    if (!scan_head(P.stream, P.stream_bytes, P.frame_offsets[f], g.wh, 1, f, P.status, P.indices, h)) return;
     if (tid == 0) s_flag = 0;
     __syncthreads();
 
@@ -78,7 +60,7 @@ __global__ void __launch_bounds__(256) dbde_decode_scan_kernel(const DecParams P
     // takes a whole partition per step: lane l owns tiles 8l..8l+7 (8 depth bytes, summed with
     // two IDP.4A), four lanes make one 32-tile item.  Four partitions are loaded before any is
     // reduced so four global loads are in flight per lane.
-    const uint8_t *dp = rec + 24;
+    const uint8_t *dp = h.rec + kRecDepth;
     bool big = false;
     if (g.wh == kTilesPerPart * g.ppf && (((uintptr_t)dp) & 7) == 0) {
         // Every partition is a full run of 256 tiles starting at tile 256*q and the plane is 8-byte
@@ -157,46 +139,9 @@ __global__ void __launch_bounds__(256) dbde_decode_scan_kernel(const DecParams P
     if (big) atomicOr(&s_flag, 1u);
     __syncthreads();
 
-    // phase 2: exclusive scan of the nitems sums, in place, 2048 per round
-    uint32_t carry = 0;
-    for (int base = 0; base < nitems; base += 2048) {
-        uint32_t v[8], local = 0;
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            const int idx = base + tid * 8 + i;
-            v[i] = idx < nitems ? wp[idx] : 0u;
-            local += v[i];
-        }
-        const uint32_t incl = warp_inclusive_scan(local, lane);
-        if (lane == 31) s_warp[warp] = incl;
-        __syncthreads();
-        uint32_t pre = carry + incl - local, tot = 0;
-#pragma unroll
-        for (int wv = 0; wv < 8; wv++) {
-            const uint32_t t = s_warp[wv];
-            if (wv < warp) pre += t;
-            tot += t;
-        }
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            const int idx = base + tid * 8 + i;
-            if (idx < nitems) wp[idx] = pre;
-            pre += v[i];
-        }
-        carry += tot;
-        __syncthreads();
-    }
-    if (tid == 0) {
-        wp[nitems] = carry;
-        if (carry != n64) status |= kStBadWordCount;
-        if (s_flag) status |= kStDepthTooBig;
-        if (room < 8ull * carry) status |= kStTruncated;
-        P.status[f] = status;
-        if (P.indices) {
-            uint64_t idx = (uint64_t)ldg_u32_bytes(rec + 4) | ((uint64_t)ldg_u32_bytes(rec + 8) << 32);
-            P.indices[f] = idx;
-        }
-    }
+    // phase 2: exclusive scan of the nitems sums
+    const uint32_t total = scan_items(wp, nitems, s_warp, tid, warp, lane);
+    if (tid == 0) scan_finish(h, wp, nitems, total, s_flag != 0, f, P.status, P.indices);
 }
 
 // ------------------------------------------------------------------ main kernel
@@ -437,9 +382,9 @@ __device__ __forceinline__ void dec_producer(const DecParams &P, DecSmemT<NSTAGE
         const uint8_t *src = nullptr;
         uint32_t nbytes = 0;
         uint8_t *dst = stage;
-        if (lane == 0) { src = rec + 32 + 2 * (size_t)g.wh + 8ull * v0; nbytes = 8 * agg; }
-        if (lane == 1) { src = rec + 24 + pi.tfirst; nbytes = (uint32_t)pi.nt; dst = stage + kDecPayloadBytes; }
-        if (lane == 2) { src = rec + 28 + (size_t)g.wh + pi.tfirst; nbytes = (uint32_t)pi.nt; dst = stage + kDecPayloadBytes + kDecPlaneBytes; }
+        if (lane == 0) { src = rec + rec_fixed(g.wh, 1) + 8ull * v0; nbytes = 8 * agg; }
+        if (lane == 1) { src = rec + kRecDepth + pi.tfirst; nbytes = (uint32_t)pi.nt; dst = stage + kDecPayloadBytes; }
+        if (lane == 2) { src = rec + rec_min(g.wh) + pi.tfirst; nbytes = (uint32_t)pi.nt; dst = stage + kDecPayloadBytes + kDecPlaneBytes; }
         const uintptr_t a0 = (uintptr_t)src & ~(uintptr_t)15;
         const uintptr_t a1 = ((uintptr_t)src + nbytes + 15) & ~(uintptr_t)15;
         const uint32_t len = nbytes ? (uint32_t)(a1 - a0) : 0u;
@@ -968,22 +913,6 @@ static size_t stg_smem_bytes() {
     return ((sizeof(StgSmem) + 127) & ~(size_t)127) + (size_t)kStgStages * kDecStageBytes + kStgOut * (size_t)kStgOutBytes;
 }
 
-template <typename Kern>
-static cudaError_t launch_persistent(Kern kern, const DecParams &P, int threads, size_t smem, int num_sms, cudaStream_t stream) {
-    int occ = 0;
-    cudaError_t e = cached_occupancy((const void *)kern, threads, smem, &occ);
-    if (e != cudaSuccess) return e;
-    unsigned grid = (unsigned)(num_sms * occ);
-    if (grid > P.nparts) grid = P.nparts;
-    if (grid == 0) return cudaSuccess;
-    kern<<<grid, threads, smem, stream>>>(P);
-    return cudaGetLastError();
-}
-
-// Which kernel unpacks odd-size frames whose partitions span the full width (W <= 2048): "staged"
-// (image built in shared memory, one bulk store per partition: the default, 5-25 % faster on every
-// 1001x1003 workload) or "direct" (re-aligned row stores from registers, the kernel that serves wider odd
-// frames).  DBDE_B200_ODD_DECODE=staged|direct picks one for tests and A/B measurements.
 static bool odd_decode_staged() {
     const char *e = getenv("DBDE_B200_ODD_DECODE");       // read per launch: tests switch it inside one process
     return !(e && e[0] == 'd');
@@ -991,30 +920,30 @@ static bool odd_decode_staged() {
 
 cudaError_t launch_decode(const DecParams &P, bool fast, int num_sms, cudaStream_t stream) {
     const size_t smem = dec_smem_bytes(P.g);
-    if (fast && P.g.linear) return launch_persistent(dbde_decode_kernel<-2>, P, kDecThreads, smem, num_sms, stream);
-    if (fast) return launch_persistent(dbde_decode_kernel<-1>, P, kDecThreads, smem, num_sms, stream);
+    if (fast && P.g.linear) return launch_persistent(dbde_decode_kernel<-2>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+    if (fast) return launch_persistent(dbde_decode_kernel<-1>, P, P.nparts, kDecThreads, smem, num_sms, stream);
     if (P.g.nseg == 1 && odd_decode_staged()) {
         const size_t ss = stg_smem_bytes();
         switch (P.g.W & 7) {
-            case 0: return launch_persistent(dbde_decode_staged_kernel<0>, P, kStgThreads, ss, num_sms, stream);
-            case 1: return launch_persistent(dbde_decode_staged_kernel<1>, P, kStgThreads, ss, num_sms, stream);
-            case 2: return launch_persistent(dbde_decode_staged_kernel<2>, P, kStgThreads, ss, num_sms, stream);
-            case 3: return launch_persistent(dbde_decode_staged_kernel<3>, P, kStgThreads, ss, num_sms, stream);
-            case 4: return launch_persistent(dbde_decode_staged_kernel<4>, P, kStgThreads, ss, num_sms, stream);
-            case 5: return launch_persistent(dbde_decode_staged_kernel<5>, P, kStgThreads, ss, num_sms, stream);
-            case 6: return launch_persistent(dbde_decode_staged_kernel<6>, P, kStgThreads, ss, num_sms, stream);
-            default: return launch_persistent(dbde_decode_staged_kernel<7>, P, kStgThreads, ss, num_sms, stream);
+            case 0: return launch_persistent(dbde_decode_staged_kernel<0>, P, P.nparts, kStgThreads, ss, num_sms, stream);
+            case 1: return launch_persistent(dbde_decode_staged_kernel<1>, P, P.nparts, kStgThreads, ss, num_sms, stream);
+            case 2: return launch_persistent(dbde_decode_staged_kernel<2>, P, P.nparts, kStgThreads, ss, num_sms, stream);
+            case 3: return launch_persistent(dbde_decode_staged_kernel<3>, P, P.nparts, kStgThreads, ss, num_sms, stream);
+            case 4: return launch_persistent(dbde_decode_staged_kernel<4>, P, P.nparts, kStgThreads, ss, num_sms, stream);
+            case 5: return launch_persistent(dbde_decode_staged_kernel<5>, P, P.nparts, kStgThreads, ss, num_sms, stream);
+            case 6: return launch_persistent(dbde_decode_staged_kernel<6>, P, P.nparts, kStgThreads, ss, num_sms, stream);
+            default: return launch_persistent(dbde_decode_staged_kernel<7>, P, P.nparts, kStgThreads, ss, num_sms, stream);
         }
     }
     switch (P.g.W & 7) {
-        case 0: return launch_persistent(dbde_decode_kernel<0>, P, kDecThreads, smem, num_sms, stream);
-        case 1: return launch_persistent(dbde_decode_kernel<1>, P, kDecThreads, smem, num_sms, stream);
-        case 2: return launch_persistent(dbde_decode_kernel<2>, P, kDecThreads, smem, num_sms, stream);
-        case 3: return launch_persistent(dbde_decode_kernel<3>, P, kDecThreads, smem, num_sms, stream);
-        case 4: return launch_persistent(dbde_decode_kernel<4>, P, kDecThreads, smem, num_sms, stream);
-        case 5: return launch_persistent(dbde_decode_kernel<5>, P, kDecThreads, smem, num_sms, stream);
-        case 6: return launch_persistent(dbde_decode_kernel<6>, P, kDecThreads, smem, num_sms, stream);
-        default: return launch_persistent(dbde_decode_kernel<7>, P, kDecThreads, smem, num_sms, stream);
+        case 0: return launch_persistent(dbde_decode_kernel<0>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        case 1: return launch_persistent(dbde_decode_kernel<1>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        case 2: return launch_persistent(dbde_decode_kernel<2>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        case 3: return launch_persistent(dbde_decode_kernel<3>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        case 4: return launch_persistent(dbde_decode_kernel<4>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        case 5: return launch_persistent(dbde_decode_kernel<5>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        case 6: return launch_persistent(dbde_decode_kernel<6>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        default: return launch_persistent(dbde_decode_kernel<7>, P, P.nparts, kDecThreads, smem, num_sms, stream);
     }
 }
 
@@ -1023,9 +952,9 @@ cudaError_t launch_decode_binned(const DecParams &scan, int factor, uint8_t *out
     P.frames = out;
     const size_t smem = dec_smem_bytes(P.g);
     switch (factor) {
-        case 2: return launch_persistent(dbde_decode_binned_kernel<2>, P, kDecThreads, smem, num_sms, stream);
-        case 4: return launch_persistent(dbde_decode_binned_kernel<4>, P, kDecThreads, smem, num_sms, stream);
-        case 8: return launch_persistent(dbde_decode_binned_kernel<8>, P, kDecThreads, smem, num_sms, stream);
+        case 2: return launch_persistent(dbde_decode_binned_kernel<2>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        case 4: return launch_persistent(dbde_decode_binned_kernel<4>, P, P.nparts, kDecThreads, smem, num_sms, stream);
+        case 8: return launch_persistent(dbde_decode_binned_kernel<8>, P, P.nparts, kDecThreads, smem, num_sms, stream);
         default: return cudaErrorInvalidValue;
     }
 }

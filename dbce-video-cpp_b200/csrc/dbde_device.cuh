@@ -7,6 +7,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "dbde_record.h"
 
 #if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ < 1000)
 #error "dbde_b200 kernels are written for sm_100a (B200) only"
@@ -570,6 +571,32 @@ __device__ __forceinline__ void pack_low_depths(const uint32_t (&px)[16], int k,
     } else if (k == 1) {
         asm volatile("st.shared.v2.u32 [%0], {%1, %2};" ::"r"(addr), "r"(r[0] + (r[1] << 16)), "r"(r[2] + (r[3] << 16)) : "memory");
     }
+}
+
+// ------------------------------------------------------------------ record fixed fields
+// Warp-wide, after the record's last word count is known: lane i writes byte i of {I32 2 | U64 index | F64 0.0 | I32 wh}
+// and the lanes above write the two counts behind the planes, {I32 mb*wh} and {I32 n64} (dbde_util.cpp:141-146,
+// 182-188,191); lane 0 stores record j's offset (j slots of slot_stride bytes) and size.
+__device__ __forceinline__ void write_fixed_fields(uint8_t *rec, int lane, uint64_t index, size_t wh, uint32_t mb, uint32_t n64,
+                                                   uint64_t *offsets, uint64_t *sizes, uint64_t j, uint64_t slot_stride) {
+    uint32_t b;
+    size_t at = lane;
+    if (lane < 4) b = 2u >> (8 * lane);
+    else if (lane < 12) b = (uint32_t)(index >> (8 * (lane - 4)));
+    else if (lane < 20) b = 0;
+    else if (lane < 24) b = (uint32_t)wh >> (8 * (lane - 20));
+    else if (lane < 28) { b = (uint32_t)(mb * wh) >> (8 * (lane - 24)); at = rec_min_count(wh) + (lane - 24); }
+    else { b = n64 >> (8 * (lane - 28)); at = rec_n64(wh, mb) + (lane - 28); }
+    rec[at] = (uint8_t)b;
+    if (lane == 0) {
+        offsets[j] = j * slot_stride;
+        sizes[j] = rec_fixed(wh, mb) + 8ull * n64;
+    }
+}
+
+// a little-endian U32 at any byte address
+__device__ __forceinline__ uint32_t ld_le32(const uint8_t *p) {
+    return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
 }
 #endif  // __CUDACC__
 

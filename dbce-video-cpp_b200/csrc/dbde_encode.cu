@@ -333,7 +333,7 @@ __global__ void __launch_bounds__(kEncThreads, 3) dbde_encode_kernel(const EncPa
                 excl = lookback_exclusive<true>(P.desc, p, p - (unsigned)q, lane);
             }
             if (lane == 0) st_relaxed_u64(P.desc + p, desc_make(kDescPrefix, excl + agg));
-            const size_t fixed = 32 + 2 * (size_t)g.wh;     // frame header + lengths + planes
+            const size_t fixed = rec_fixed(g.wh, 1);        // frame header + lengths + planes
             uint8_t *frame = P.out + (size_t)f * P.slot_stride;
             __syncwarp();
             if (lane == 0) {
@@ -342,7 +342,9 @@ __global__ void __launch_bounds__(kEncThreads, 3) dbde_encode_kernel(const EncPa
                 mbar_arrive(&S.basebar[ss]);
             }
             if (q == g.ppf - 1) {
-                // last partition of the frame: the fixed fields (dbde_util.cpp:141-146,182-188,191)
+                // last partition of the frame: the fixed fields, byte for byte write_fixed_fields(frame, lane, index,
+                // g.wh, 1, n64, ...).  Kept as its own copy: with the shared writer ptxas schedules this kernel
+                // differently, and the micro-2048 encode measured 0.5 % slower (B200, 1000 W power limit)
                 const uint32_t n64 = (uint32_t)(excl + agg);
                 const uint64_t index = P.first_index + (uint64_t)f;
                 uint32_t b;      // lane i writes one byte of {I32 2 | U64 index | F64 0.0 | I32 wh} {I32 wh} {I32 n64}
@@ -351,8 +353,8 @@ __global__ void __launch_bounds__(kEncThreads, 3) dbde_encode_kernel(const EncPa
                 else if (lane < 12) { b = (uint32_t)(index >> (8 * (lane - 4))) & 0xff; dst = frame + lane; }
                 else if (lane < 20) { b = 0; dst = frame + lane; }
                 else if (lane < 24) { b = ((uint32_t)g.wh >> (8 * (lane - 20))) & 0xff; dst = frame + lane; }
-                else if (lane < 28) { b = ((uint32_t)g.wh >> (8 * (lane - 24))) & 0xff; dst = frame + 24 + g.wh + (lane - 24); }
-                else { b = (n64 >> (8 * (lane - 28))) & 0xff; dst = frame + 28 + 2 * (size_t)g.wh + (lane - 28); }
+                else if (lane < 28) { b = ((uint32_t)g.wh >> (8 * (lane - 24))) & 0xff; dst = frame + rec_min_count(g.wh) + (lane - 24); }
+                else { b = (n64 >> (8 * (lane - 28))) & 0xff; dst = frame + rec_n64(g.wh, 1) + (lane - 28); }
                 *dst = (uint8_t)b;
                 if (lane == 0) {
                     P.frame_offsets[f] = (uint64_t)f * P.slot_stride;
@@ -370,7 +372,7 @@ __global__ void __launch_bounds__(kEncThreads, 3) dbde_encode_kernel(const EncPa
             stx = tid - sb * g.w;
         }
         const uint32_t toff = (uint32_t)(sb * 8) * (uint32_t)g.pitch + (uint32_t)stx * 8u;   // my tile inside a stage
-        const size_t fixed = 32 + 2 * (size_t)g.wh;
+        const size_t fixed = rec_fixed(g.wh, 1);
         // deferred partition (iteration it-1): its depth/min/word count stay in registers until its
         // addresses are known.  d_km = depth | min << 8 | valid << 16.
         uint32_t d_km = 0, d_wtot = 0;
@@ -385,8 +387,8 @@ __global__ void __launch_bounds__(kEncThreads, 3) dbde_encode_kernel(const EncPa
             // ---- depth and minimum planes (dbde_util.cpp:156-157)
             if (WIDE || (d_km >> 16)) {
                 uint8_t *pl = frame + d_tfirst + tid;
-                pl[24] = (uint8_t)d_km;
-                pl[28 + (size_t)g.wh] = (uint8_t)(d_km >> 8);
+                pl[kRecDepth] = (uint8_t)d_km;
+                pl[rec_min(g.wh)] = (uint8_t)(d_km >> 8);
             }
             // ---- this warp's words, by this warp: one coalesced run per warp
             uint8_t *dst = frame + fixed + 8 * ((size_t)b.z + S.wbase[ds][warp]);
@@ -619,7 +621,7 @@ __global__ void __launch_bounds__(kTilesPerPart) dbde_encode_crops_kernel(const 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint8_t *stage_out = s_words[warp];
     const size_t fbytes = (size_t)P.W * (size_t)P.H;
-    const size_t fixed = 32 + 2 * (size_t)P.wh;
+    const size_t fixed = rec_fixed(P.wh, 1);
     unsigned cc = 0;                                   // chunks done by this CTA: selects the s_wtot half
     for (int j = blockIdx.x; j < P.nrec; j += gridDim.x) {
         const int f = j / P.ncrops, r = j - f * P.ncrops;
@@ -680,8 +682,8 @@ __global__ void __launch_bounds__(kTilesPerPart) dbde_encode_crops_kernel(const 
             }
             // depth and minimum planes (dbde_util.cpp:156-157)
             if (valid) {
-                rec[24 + (size_t)t] = (uint8_t)k;
-                rec[28 + (size_t)P.wh + (size_t)t] = (uint8_t)mn;
+                rec[kRecDepth + t] = (uint8_t)k;
+                rec[rec_min(P.wh) + t] = (uint8_t)mn;
             }
             // this warp's words: one coalesced run
             const uint32_t n = s_wtot[cc & 1][warp];
@@ -695,36 +697,15 @@ __global__ void __launch_bounds__(kTilesPerPart) dbde_encode_crops_kernel(const 
             carry += tot;
             __syncwarp();                              // the copy has read the staging before the next chunk packs into it
         }
-        if (warp == 0) {
-            // the fixed fields (dbde_util.cpp:141-146,182-188,191), as the frame encoder's scan warp writes them
-            const uint64_t index = P.first_index + (uint64_t)f;
-            const uint32_t wh = (uint32_t)P.wh;
-            uint32_t b;
-            uint8_t *dst;
-            if (lane < 4) { b = (2u >> (8 * lane)) & 0xff; dst = rec + lane; }
-            else if (lane < 12) { b = (uint32_t)(index >> (8 * (lane - 4))) & 0xff; dst = rec + lane; }
-            else if (lane < 20) { b = 0; dst = rec + lane; }
-            else if (lane < 24) { b = (wh >> (8 * (lane - 20))) & 0xff; dst = rec + lane; }
-            else if (lane < 28) { b = (wh >> (8 * (lane - 24))) & 0xff; dst = rec + 24 + (size_t)wh + (lane - 24); }
-            else { b = (carry >> (8 * (lane - 28))) & 0xff; dst = rec + 28 + 2 * (size_t)wh + (lane - 28); }
-            *dst = (uint8_t)b;
-            if (lane == 0) {
-                P.frame_offsets[j] = (uint64_t)j * P.slot_stride;
-                P.frame_sizes[j] = fixed + 8ull * carry;
-            }
-        }
+        if (warp == 0)
+            write_fixed_fields(rec, lane, P.first_index + (uint64_t)f, P.wh, 1, carry, P.frame_offsets, P.frame_sizes,
+                               j, P.slot_stride);
     }
 }
 
 cudaError_t launch_encode_crops(const EncCropParams &P, int num_sms, cudaStream_t stream) {
     if (P.nrec <= 0) return cudaSuccess;
-    int occ = 0;
-    cudaError_t e = cached_occupancy((const void *)dbde_encode_crops_kernel, kTilesPerPart, 0, &occ);
-    if (e != cudaSuccess) return e;
-    unsigned grid = (unsigned)(num_sms * occ);
-    if (grid > (unsigned)P.nrec) grid = (unsigned)P.nrec;
-    dbde_encode_crops_kernel<<<grid, kTilesPerPart, 0, stream>>>(P);
-    return cudaGetLastError();
+    return launch_persistent(dbde_encode_crops_kernel, P, (unsigned)P.nrec, kTilesPerPart, 0, num_sms, stream);
 }
 
 // ------------------------------------------------------------------ record compaction
@@ -887,14 +868,7 @@ cudaError_t launch_encode(const EncParams &Pin, bool fast, int num_sms, cudaStre
         case 6: kern = dbde_encode_kernel<false, false, true, 6>; break;
         default: kern = dbde_encode_kernel<false, false, true, 7>; break;
     }
-    int occ = 0;
-    cudaError_t e = cached_occupancy((const void *)kern, kEncThreads, smem, &occ);
-    if (e != cudaSuccess) return e;
-    unsigned grid = (unsigned)(num_sms * occ);
-    if (grid > P.nparts) grid = P.nparts;
-    if (grid == 0) return cudaSuccess;
-    kern<<<grid, kEncThreads, smem, stream>>>(P);
-    return cudaGetLastError();
+    return launch_persistent(kern, P, P.nparts, kEncThreads, smem, num_sms, stream);
 }
 
 }  // namespace dbde

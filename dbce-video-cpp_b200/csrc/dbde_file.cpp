@@ -7,6 +7,7 @@
 //   * the reader decodes a batch on the GPU while a background thread reads the next bytes ahead,
 // so disk I/O overlaps the PCIe copies.  Host code only: no codec arithmetic lives here.
 #include "../../include/dbde_b200.h"
+#include "dbde_record.h"
 
 #include <stdio.h>
 #include <string.h>
@@ -224,7 +225,7 @@ extern "C" int dbde_b200_reader_open(dbde_b200_ctx *ctx, const char *path, int b
     r->batch = batch_frames > 0 ? batch_frames : 16;
     r->rec_bound = dbde_b200_frame_record_bound(r->W, r->H);
     const size_t wh = (size_t)((r->W + 7) / 8) * ((r->H + 7) / 8);
-    r->fixed = 32 + 2 * wh;
+    r->fixed = dbde::rec_fixed(wh, 1);
     // each buffer: [carry-over half | read-ahead half], each half holds a full batch of worst-case records
     r->cap = 2 * (r->rec_bound * (size_t)r->batch + 64);
     for (int i = 0; i < 2; i++) {

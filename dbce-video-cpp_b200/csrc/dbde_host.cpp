@@ -9,6 +9,7 @@
 bool dbde_advance_file_buffer(dbde_file_walker &w);      // exported by the reference object, not in its header
 #pragma GCC visibility pop
 #include "../../include/dbde_b200.h"
+#include "dbde_record.h"
 
 #include <stdlib.h>
 #include <string.h>
@@ -203,10 +204,11 @@ video_header dbde_unpack_video_header(uint8_t **packed) {
 // rejects (documented deviation) -- so a malformed or foreign buffer never reaches the GPU path.
 namespace {
 bool image_block_ok(const uint8_t *blk, size_t wh, size_t *n64_out) {
+    using namespace dbde;
     if (get32(blk) != (uint32_t)wh) return false;                   // nb != w*h  (:296)
-    const uint8_t *depth = blk + 4;
-    if (get32(blk + 4 + wh) != (uint32_t)wh) return false;          // nm != w*h  (:299)
-    const uint32_t n64 = get32(blk + 8 + 2 * wh);
+    const uint8_t *depth = blk + (kRecDepth - kRecDepthCount);
+    if (get32(blk + (rec_min_count(wh) - kRecDepthCount)) != (uint32_t)wh) return false;   // nm != w*h  (:299)
+    const uint32_t n64 = get32(blk + (rec_n64(wh, 1) - kRecDepthCount));
     uint64_t sum = 0;
     uint32_t big = 0;
     for (size_t i = 0; i < wh; i++) {
@@ -246,13 +248,13 @@ frame_header dbde_unpack_frame(uint8_t **packed, int W, int H, uint8_t *image) {
         fh.u64s = (uint32_t)-1;
         return fh;
     }
-    const size_t bytes = 32 + 2 * wh + 8 * n64;
+    const size_t fixed = dbde::rec_fixed(wh, 1), bytes = fixed + 8 * n64;
     uint8_t hdr_ok[4];
     put32(hdr_ok, 2);                                          // image validity is independent of the tag (:341)
     std::vector<uint8_t> tmp;
     const uint8_t *src = rec;
     if (get32(rec) != 2) {
-        tmp.assign(rec, rec + (bytes < 32 + 2 * wh ? 32 + 2 * wh : bytes));
+        tmp.assign(rec, rec + (bytes < fixed ? fixed : bytes));
         memcpy(tmp.data(), hdr_ok, 4);
         src = tmp.data();
     }
@@ -269,7 +271,7 @@ size_t dbde_unpack_image(uint8_t *packed, int W, int H, uint8_t *image) {
     const size_t wh = (size_t)((W + 7) / 8) * ((H + 7) / 8);
     size_t n64 = 0;
     if (!image_block_ok(packed, wh, &n64)) return 0;           // :296,299,303 before anything else is read
-    const size_t body = 12 + 2 * wh + 8 * n64;
+    const size_t body = dbde::rec_fixed(wh, 1) - dbde::kRecDepthCount + 8 * n64;
     uint8_t *rec = scratch_record(20 + body);
     frame_header fh = {2, 0, 0};
     dbde_pack_frame_header(fh, rec);
@@ -283,11 +285,12 @@ size_t dbde_unpack_image(uint8_t *packed, int W, int H, uint8_t *image) {
 // reference dbde_util.cpp:105-135: an (downmargin x rightmargin) corner IS a W=rightmargin,
 // H=downmargin frame; the device clamp-pads it exactly as dbde_pack_8x8_partial does
 uint32_t dbde_pack_8x8_partial(uint8_t *image, int stride, int rightmargin, int downmargin, uint8_t *target) {
-    uint8_t px[64], rec[32 + 66];
+    using namespace dbde;
+    uint8_t px[64], rec[rec_bound(1, 1)];
     for (int y = 0; y < downmargin; y++) memcpy(px + y * rightmargin, image + (size_t)y * stride, rightmargin);
     const size_t n = dbde_pack_frame(0, px, rightmargin, downmargin, rec);
-    const uint32_t depth = rec[24], mn = rec[29];
-    memcpy(target, rec + 34, n - 34);                          // exactly 8*depth bytes
+    const uint32_t depth = rec[kRecDepth], mn = rec[rec_min(1)];
+    memcpy(target, rec + rec_fixed(1, 1), n - rec_fixed(1, 1));          // exactly 8*depth bytes
     return (depth << 8) | mn;
 }
 // reference dbde_util.cpp:22-103
@@ -297,15 +300,16 @@ uint32_t dbde_pack_8x8(uint8_t *image, int stride, uint8_t *target) {
 // reference dbde_util.cpp:216-279 (depth >= 8 reads 64 raw bytes, :229)
 void dbde_unpack_8x8(uint8_t depth, uint8_t minval, uint8_t *packed, size_t stride, uint8_t *image) {
     const uint32_t k = depth > 8 ? 8 : depth;
-    uint8_t rec[34 + 64], px[64];
+    using namespace dbde;
+    uint8_t rec[rec_bound(1, 1)], px[64];
     frame_header fh = {2, 0, 0};
     dbde_pack_frame_header(fh, rec);
-    put32(rec + 20, 1);
-    rec[24] = (uint8_t)k;
-    put32(rec + 25, 1);
-    rec[29] = minval;
-    put32(rec + 30, k);
-    memcpy(rec + 34, packed, 8 * k);
+    put32(rec + kRecDepthCount, 1);
+    rec[kRecDepth] = (uint8_t)k;
+    put32(rec + rec_min_count(1), 1);
+    rec[rec_min(1)] = minval;
+    put32(rec + rec_n64(1, 1), k);
+    memcpy(rec + rec_fixed(1, 1), packed, 8 * k);
     uint8_t *p = rec;
     dbde_unpack_frame(&p, 8, 8, px);
     for (int y = 0; y < 8; y++) memcpy(image + y * stride, px + 8 * y, 8);
@@ -320,7 +324,7 @@ void dbde_unpack_8x8_partial(uint8_t depth, uint8_t minval, uint8_t *packed, siz
 
 // ---------------------------------------------------------------- file walker
 // Same interface and field meanings as the reference (dbde_util.cpp:362-426) but: the buffer is
-// sized for the true worst-case record (32 + 66*wh, not npix + npix/8 + 32, which under-sizes
+// sized for the true worst-case record (rec_bound(wh, 1), not npix + npix/8 + 32, which under-sizes
 // small odd frames), it is freed in dbde_end_file_walk, and frames are decoded on the GPU in
 // batches of `frames_buffered`.  A helper thread reads, indexes and decodes batch k+1 (fread -> page-locked
 // file buffer -> H2D -> kernels -> D2H into a pinned batch buffer) while the caller is still being handed
