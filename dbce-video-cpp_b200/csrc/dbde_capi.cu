@@ -180,7 +180,7 @@ static PartGeom make_geom(int W, int H, bool fast) {
 
 static bool dims_ok(int W, int H, int nframes) {
     if (W <= 0 || H <= 0 || nframes < 0) return false;
-    const long long wh = (long long)((W + 7) / 8) * ((H + 7) / 8);
+    const long long wh = (((long long)W + 7) / 8) * (((long long)H + 7) / 8);   // W + 7 overflows int near INT32_MAX
     return wh <= 0x0FFFFFFF && (long long)W * H <= 0x7FFFFFFFLL;
 }
 
